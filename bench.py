@@ -10,10 +10,12 @@ replicas, no data-path collective: weak scaling).
   python bench.py --gpus 1 --steps 3 --warmup 3
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
   python bench.py --impl reference ...     # the reference's own CPU path on the host cores
+  python bench.py --gpus 1 --steps 3 --warmup 3 --dump-outputs DIR
 
 Prints ONE JSON line (rank 0).  `value` = images/s with inputs resident in HBM; `e2e` = the same
 through the C ABI with host buffers (pinned H2D of every input ciphertext and D2H of the 10 output
-ciphertexts per image inside the timed region).
+ciphertexts per image inside the timed region).  The inputs are seeded: the same arguments give the
+same inputs, so --dump-outputs of two builds can be compared array for array (see dump_outputs).
 """
 import argparse
 import json
@@ -61,7 +63,7 @@ W = 8  # bytes per residue
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--batch", type=int, default=8, help="images per step per GPU")
@@ -80,7 +82,41 @@ def parse():
                          "network's conv / fc layers split by output neuron across the GPUs with NCCL all-gathers of the "
                          "activation ciphertexts (BASELINE config 3, strong scaling); crt: the plaintext modulus ~2^30 split into "
                          "one CRT modulus per GPU, independent instances of the WoPad network on the same images (BASELINE config 4)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the score ciphertexts rank 0's last timed step computed (replicas and crt "
+                         "modes): DIR/scores.npy holds every residue as four exact 16-bit words in float32, least significant first "
+                         "(words, not values: compare exactly), DIR/scores_coeff_index.npy the coefficient positions kept")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.mode == "shard"):
+        ap.error("--dump-outputs needs --impl b200 and --mode replicas or crt")
+    return args
+
+
+DUMP_BYTES = 60 * 10**6   # scores.npy stays below this; with the index file and headers the dump is under 64 MB
+DUMP_SEED = 20240
+
+
+def dump_outputs(directory, scores, budget=DUMP_BYTES, seed=DUMP_SEED):
+    """Writes score ciphertexts ([batch][outputs][2][K][n+1] uint64 residues, pad word last) as exact float32 arrays:
+
+      scores.npy              [batch][outputs][2][K][m][4]: each residue as four 16-bit words, least significant first
+      scores_coeff_index.npy  [m]: the coefficient positions kept, all n of them when they fit in `budget` bytes, else a
+                              fixed sample drawn with `seed`, so two runs with the same arguments keep the same positions
+
+    A float32 holds every integer below 2^24, so the words are exact and two builds' dumps compare with np.array_equal; a
+    residue that is off by one changes a word by one, which no tolerance meant for float data lets through."""
+    scores = np.asarray(scores, dtype=np.uint64)
+    n = scores.shape[-1] - 1
+    per_coeff = scores[..., 0].size * 4 * 4
+    m = min(n, budget // per_coeff)
+    index = np.arange(n) if m == n else np.sort(np.random.default_rng(seed).choice(n, size=m, replace=False))
+    kept = scores[..., index]
+    words = np.stack([(kept >> np.uint64(16 * i)) & np.uint64(0xFFFF) for i in range(4)], axis=-1).astype(np.float32)
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "scores.npy"), words)
+    np.save(os.path.join(directory, "scores_coeff_index.npy"), index.astype(np.float32))
 
 
 # ------------------------------------------------------------------------------------------
@@ -479,8 +515,9 @@ def main_b200(args, rank, world, local_rank):
     net.resident_run(max(3, args.warmup))
     _barrier(dist)
     eng.prof_reset(); eng.prof_enable(True)
+    last_scores = np.empty(B * n_scores * ct_words, dtype=np.uint64) if args.dump_outputs else None
     sampler = ClockSampler(local_rank); sampler.start()
-    ms_total, per_layer_list = net.resident_run(args.steps)
+    ms_total, per_layer_list = net.resident_run(args.steps, out=last_scores)
     _barrier(dist)
     clocks = sampler.stop()
     net.resident_end()
@@ -494,6 +531,8 @@ def main_b200(args, rank, world, local_rank):
     alloc0 = eng.alloc_stats()
     ms_e2e = net.serve(own_in.ptr, own_out.ptr, B, args.steps)
     _barrier(dist)
+    if last_scores is not None and not np.array_equal(last_scores, np.asarray(pin_out)):
+        raise RuntimeError("scores of the last timed resident step differ from the serving loop's scores of the same input")
     alloc1 = eng.alloc_stats()
     alloc_e2e = {k: alloc1[k] - alloc0[k] for k in ("pool_mallocs", "cache_hits", "cache_bypass", "flushes", "small_mallocs")}
     serve_done = net.serve_times()
@@ -712,6 +751,8 @@ def main_b200(args, rank, world, local_rank):
         except Exception as e:
             if rank == 0:
                 line["shard"] = {"failed": repr(e)}
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_scores.reshape(B, n_scores, 2, K, n + 1))
     if rank == 0:
         emit(line)
     if dist is not None:

@@ -86,7 +86,8 @@ int crcnn_host_forward_range(const uint64_t *in_words, int batch, int zd, int xd
 // every one from a fresh coefficient-form copy of the resident input (so the input transform is inside the timed region), timed with
 // CUDA events on the context's stream (ms_total) and per layer (per_layer_ms, mean over the steps; may be null); end: release.
 // Warm-up and timed steps are separate run() calls on the SAME resident tensor, so the caller can put its barrier between them and the
-// stream-ordered allocator sees one steady allocation pattern.
+// stream-ordered allocator sees one steady allocation pattern.  last_out (may be null): host words [batch][outputs] ciphertexts that
+// receive the output of the last step, downloaded after the timing has ended.
 int crcnn_host_resident_begin(const uint64_t *pinned_in, int batch) {
     return guarded([&] {
         if (!g_net) throw std::invalid_argument("no network built");
@@ -96,7 +97,7 @@ int crcnn_host_resident_begin(const uint64_t *pinned_in, int batch) {
         g_x0.reset(new DeviceTensor(x0, g_zd, g_xd, g_yd, batch));
     });
 }
-int crcnn_host_resident_run(int steps, double *ms_total, double *per_layer_ms) {
+int crcnn_host_resident_run(int steps, double *ms_total, double *per_layer_ms, uint64_t *last_out) {
     return guarded([&] {
         if (!g_net || !g_x0) throw std::invalid_argument("crcnn_host_resident_begin has not been called");
         Runtime &rt = Runtime::get();
@@ -105,6 +106,7 @@ int crcnn_host_resident_run(int steps, double *ms_total, double *per_layer_ms) {
         const int L = g_net->getNumLayers();
         std::vector<void *> ev((size_t)steps * (L + 1), nullptr);
         for (auto &e : ev) rt.check(crcnn_event_create(ctx, &e));
+        DeviceTensor last;
         for (int s = 0; s < steps; s++) {
             crcnn_tensor *c = nullptr;
             rt.check(crcnn_tensor_slice(ctx, g_x0->t, 0, count, &c));
@@ -116,6 +118,7 @@ int crcnn_host_resident_run(int steps, double *ms_total, double *per_layer_ms) {
             x = g_net->forward_dev(std::move(x), 0, L);
             g_net->after_layer = nullptr;
             rt.check(crcnn_event_record(ctx, ev[(size_t)s * (L + 1) + L], nullptr));
+            if (last_out && s == steps - 1) last = std::move(x);
         }
         if (steps > 0 && ms_total) rt.check(crcnn_event_elapsed_ms(ctx, ev[0], ev[(size_t)(steps - 1) * (L + 1) + L], ms_total));
         if (per_layer_ms)
@@ -126,6 +129,10 @@ int crcnn_host_resident_run(int steps, double *ms_total, double *per_layer_ms) {
             }
         rt.check(crcnn_ctx_sync(ctx));
         for (auto &e : ev) crcnn_event_destroy(ctx, e);
+        if (last.t) {
+            if (last.count() != (long)g_x0->batch * g_outputs) throw std::logic_error("network output is not [batch][outputs] ciphertexts");
+            rt.check(crcnn_tensor_download(ctx, last.t, last_out));
+        }
     });
 }
 int crcnn_host_resident_end() { return guarded([&] { g_x0.reset(); }); }

@@ -36,7 +36,7 @@ def load():
     h.crcnn_host_layer_name.argtypes = [_I, C.c_char_p, _I]
     h.crcnn_host_forward_range.argtypes = [_vp, _I, _I, _I, _I, _I, _I, _vp, C.c_long, C.POINTER(_I)]
     h.crcnn_host_resident_begin.argtypes = [_vp, _I]
-    h.crcnn_host_resident_run.argtypes = [_I, _dp, _dp]
+    h.crcnn_host_resident_run.argtypes = [_I, _dp, _dp, _vp]
     h.crcnn_host_serve.argtypes = [_vp, _vp, _I, C.c_long, _dp]
     h.crcnn_host_set_fusion.argtypes = [_I]
     h.crcnn_host_serve_times.argtypes = [_dp, _I]
@@ -117,12 +117,17 @@ class HostNetwork:
     def resident_begin(self, pinned_ptr, batch):
         """Upload the batch once; resident_run() then times forwards that start from a fresh device copy of it."""
         self._chk(self.h.crcnn_host_resident_begin(pinned_ptr, batch))
+        self.resident_batch = batch
 
-    def resident_run(self, steps):
-        """(total ms by CUDA events, [ms per layer]) of `steps` forwards of the resident batch."""
+    def resident_run(self, steps, out=None):
+        """(total ms by CUDA events, [ms per layer]) of `steps` forwards of the resident batch.  out: a uint64 array of
+        [batch * outputs][2][K][n+1] words that receives the scores of the last of those forwards."""
         ms = C.c_double()
         per = (C.c_double * self.num_layers)()
-        self._chk(self.h.crcnn_host_resident_run(steps, C.byref(ms), per))
+        if out is not None and not (out.dtype == np.uint64 and out.flags.c_contiguous and out.flags.writeable
+                                    and out.size == self.resident_batch * self.outputs * self.ct_words()):
+            raise ValueError("out must be a writable contiguous uint64 array of batch * outputs ciphertexts")
+        self._chk(self.h.crcnn_host_resident_run(steps, C.byref(ms), per, None if out is None else out.ctypes.data))
         return ms.value, list(per)
 
     def resident_end(self):

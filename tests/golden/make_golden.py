@@ -75,6 +75,21 @@ def case_chain_hashes():
     json.dump(out, open(os.path.join(HERE, "chain_hashes.json"), "w"), indent=1)
 
 
+def case_reference_ops():
+    """SHA-256 digests of the reference's output of every evaluator / layer case of tests/test_oracle_vs_reference.py
+    (util.ref_ops: inputs regenerated from splitmix64 seeds by the test)."""
+    import json
+    sys.path.insert(0, os.path.dirname(HERE))
+    import util
+    out = {}
+    for n, (t, seed) in util.REF_OPS.items():
+        r = Ref(n, t, seed=seed)
+        outs = util.ref_ops("ref", r, n, r.primes, t, seed)
+        out[str(n)] = dict(t=t, seed=seed, primes=[int(q) for q in r.primes], digests={k: util.sha(v) for k, v in outs.items()})
+    json.dump(out, open(os.path.join(HERE, "reference_ops.json"), "w"), indent=1)
+
+
 if __name__ == "__main__":
     case_layers(2048, 1 << 10, 7, "layers_n2048.npz")
     case_chain_hashes()
+    case_reference_ops()

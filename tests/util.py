@@ -109,3 +109,57 @@ def run_chain(backend, kind, x, p, evk, sizes, dbc):
         t = g.square_layer(t, g.evk_upload(evk, sizes, dbc)); outs.append(g.download(t))
         t = g.fc(t, e(p["fc_w"]), e(p["fc_b"]), 1, 12, 4); outs.append(g.download(t))
     return outs
+
+
+# the evaluator and layer cases pinned on the reference (tests/test_oracle_vs_reference.py, tests/golden/reference_ops.json)
+ENC_VALUES = [0.0867, -3.25, 0.0, 1.0, -1.0, 7.0, 0.25, 2.8215, -0.4242, 1 / 9.0, -17.5, 1e-9, 123456.789]
+REF_OPS = {2048: (1 << 16, 2048), 4096: (1 << 18, 4096), 8192: (1 << 30, 8192)}   # n: (t, seed)
+
+
+def ref_ops(kind, r, n, primes, t, seed):
+    """Runs the cases on `r` (kind: 'ref' = oracle.ref.Ref, 'oracle' = oracle.port.Oracle) and returns {name: output array}.
+    Inputs are splitmix64 residues, floats and evaluation keys, the same for both; the pool case `avgpool9` encodes the
+    DOUBLE 1/9 as the reference does (avgPoolingLayer.cpp:10-13)."""
+    out = {}
+    for i, v in enumerate(ENC_VALUES + [float(v) for v in det_floats(seed, 40) * 3]):
+        a, cc = r.encode(float(v))
+        out["encode_%02d" % i] = np.append(a, np.uint64(cc))
+    evk, sizes, dbc = det_evk(seed, n, primes)
+    if kind == "ref":
+        r.set_evk(evk, sizes, dbc)
+    x = det_cts(seed + 1, n, primes, 5)
+    xn = r.ct_transform(x)
+    out["ct_ntt"], out["ct_intt"] = xn, r.ct_transform(xn, inverse=True)
+    w, _ = r.encode(0.0867)
+    wn = r.plain_to_ntt(w)
+    out["plain_ntt"], out["multiply_plain_ntt"] = wn, r.multiply_plain_ntt(xn, wn)
+    dense = np.zeros(n + 1, dtype=np.uint64)
+    dense[:n] = splitmix64(seed * 31 + 5, n) % np.uint64(t)
+    for j, plain in enumerate((w, dense, np.array([t - 2], dtype=np.uint64), np.array([3], dtype=np.uint64))):
+        for op in ("mul", "add", "sub"):
+            out["plain_%s_%d" % (op, j)] = r.plain_op(x, plain, op)
+    out["add_many"] = r.add_many(x)
+    s3 = r.square(det_cts(seed + 2, n, primes, 3))
+    out["square"] = s3
+    out["relinearize"] = r.relinearize(s3) if kind == "ref" else r.relinearize(s3, evk, sizes, dbc)
+    xi = det_cts(seed + 3, n, primes, 2 * 3 * 3)
+    wv, bv, wf, bf = det_floats(seed + 4, 16), det_floats(seed + 5, 2), det_floats(seed + 6, 3 * 18), det_floats(seed + 7, 3)
+    mean, invstd = [0.3, -0.2], [1.7, 0.9]
+    if kind == "ref":
+        out["conv"] = r.conv(xi, 3, 3, 2, 1, 1, 2, 2, 2, wv, bv)
+        out["fc"] = r.fc3d(xi, 2, 3, 3, 3, wf, bf)
+        out["pool"] = r.pool(xi, 3, 3, 2, 1, 1, 2, 2)
+        out["avgpool"] = r.pool(xi, 3, 3, 2, 1, 1, 2, 2, avg=True)
+        out["avgpool9"] = r.pool(xi, 3, 3, 2, 1, 1, 3, 3, avg=True)
+        out["bn"] = r.bn(xi, 2, 3, 3, mean, invstd)
+        out["square_layer"] = r.square_layer(xi[:4], 1, 2, 2)
+    else:
+        e = r.encode_many
+        out["conv"] = r.conv(xi, 3, 3, 2, 1, 1, 2, 2, 2, e(wv), e(bv))
+        out["fc"] = r.fc(xi, 18, 3, e(wf), e(bf))
+        out["pool"] = r.pool(xi, 3, 3, 2, 1, 1, 2, 2)
+        out["avgpool"] = r.pool(xi, 3, 3, 2, 1, 1, 2, 2, *r.encode(0.25))
+        out["avgpool9"] = r.pool(xi, 3, 3, 2, 1, 1, 3, 3, *r.encode(1.0 / 9.0))
+        out["bn"] = r.bn(xi, 2, 3, 3, e(mean), e(invstd))
+        out["square_layer"] = r.square_layer(xi[:4], evk, sizes, dbc)
+    return out
