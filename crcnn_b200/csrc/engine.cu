@@ -110,6 +110,7 @@ struct crcnn_ctx {
     int tap_mode = 1;                // 1: avg-pool / batch-norm on coefficient-form inputs multiply in the coefficient domain (tapmul_kernel); env CRCNN_TAP
     int relin_mode = 1;              // 1: relinearize through 30-bit auxiliary primes when exact for the parameters (relin32.cuh); 0: 64-bit transforms
     int tcn_mode = 1;                // 1: weighted sums whose staged weights fit the weight cache run as the NTT-domain limb-split GEMM (tcn_mac.cuh)
+    int sq_lean = 1;                 // 1 (default): square's tensor products reduce through the 2^k - delta fold when every modulus allows, and the inverse transforms feeding the BEHZ lift / floor leave n^-1 to their constants (params.h: *_n); 0: Barrett products, n^-1 in the transforms; same bytes; env CRCNN_SQ_LEAN
     int tcn_fold = 1;                // 1 (default): the limb-split GEMM reduces its class sums through the 2^k - delta shape of the primes when every prime has it (modarith.cuh: tcn_fold_reduce), 0: 128-bit recombination + Barrett; same bytes; env CRCNN_TCN_FOLD
     size_t tc_scratch_bytes = 12ull << 30;
     std::string err;
@@ -621,6 +622,7 @@ int crcnn_ctx_create(int n, int K, const uint64_t *q, uint64_t t, int device, cr
     if (const char *e = getenv("CRCNN_TCN")) c->tcn_mode = atoi(e);
     if (const char *e = getenv("CRCNN_TAP")) c->tap_mode = atoi(e);
     if (const char *e = getenv("CRCNN_TCN_FOLD")) c->tcn_fold = atoi(e);
+    if (const char *e = getenv("CRCNN_SQ_LEAN")) c->sq_lean = atoi(e);
     // stream-ordered allocator: keep freed blocks cached
     cudaMemPool_t pool;
     if (cudaDeviceGetDefaultMemPool(&pool, device) == cudaSuccess) {
@@ -1579,6 +1581,9 @@ int crcnn_square(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_tensor **out3) {
     // An NTT-form input (the usual case: the convolution before the activation leaves NTT form) keeps its transformed q
     // limbs: the base conversion works on an inverse-transformed COPY, and only the Bsk limbs are transformed again.
     const bool have_ntt = in->ntt != 0;
+    // lean: the tensor stage leaves n^-1 to the floor's constants (and reduces on the fold where it applies); so does the INTT copy
+    // to the lift's -- not a coefficient-form input, whose q limbs the lift copies into ext unscaled
+    const bool lean = ctx->sq_lean != 0, fold = lean && behz_fold_ok(ctx->hp.d), copy_ninv = !(lean && have_ntt);
     crcnn_tensor *o = nullptr;
     int rc = new_tensor(ctx, in->count, 3, 0, &o);
     if (rc) return rc;
@@ -1597,9 +1602,10 @@ int crcnn_square(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_tensor **out3) {
         cudaError_t e = cudaSuccess;
         if (have_ntt) {
             ProfScope ps(ctx, KC_NTT_INV, 2 * lp_bytes(ctx, (double)cur * 2 * ctx->K), lp_bfly(ctx, (double)cur * 2 * ctx->K));
-            e = launch_ntt_grouped(ctx->dP, ctx->logn, coef, cur * 2 * ctx->K, 0, ctx->K, true, ctx->K, 0, ctx->stream, src);  // out of place
+            e = launch_ntt_grouped(ctx->dP, ctx->logn, coef, cur * 2 * ctx->K, 0, ctx->K, true, ctx->K, 0, ctx->stream, src,  // out of place
+                                   nullptr, 1, 1, copy_ninv);
         }
-        if (e == cudaSuccess) { ProfScope ps(ctx, KC_BEHZ_LIFT, lp_bytes(ctx, (double)cur * 2 * (ctx->K + (have_ntt ? ctx->S : KS))), (double)cur * 2 * n * ctx->S * (ctx->K + 1)); e = launch_behz_lift(ctx->hp.d, ctx->n, have_ntt ? coef : src, have_ntt ? src : nullptr, cur, ext, ctx->stream); }
+        if (e == cudaSuccess) { ProfScope ps(ctx, KC_BEHZ_LIFT, lp_bytes(ctx, (double)cur * 2 * (ctx->K + (have_ntt ? ctx->S : KS))), (double)cur * 2 * n * ctx->S * (ctx->K + 1)); e = launch_behz_lift(ctx->hp.d, ctx->n, have_ntt ? coef : src, have_ntt ? src : nullptr, cur, ext, ctx->stream, copy_ninv); }
         if (e == cudaSuccess) {
             if (have_ntt) {   // Bsk limbs only
                 ProfScope ps(ctx, KC_NTT_FWD, 2 * lp_bytes(ctx, (double)cur * 2 * ctx->S), lp_bfly(ctx, (double)cur * 2 * ctx->S));
@@ -1612,10 +1618,10 @@ int crcnn_square(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_tensor **out3) {
         if (e == cudaSuccess) {
             // tensor products formed while the inverse transform loads its polynomial (bytes: 2 inputs + 3 outputs per limb)
             ProfScope ps(ctx, KC_SQ_TENSOR, lp_bytes(ctx, (double)cur * 5 * KS), lp_bfly(ctx, (double)cur * 3 * KS));
-            e = launch_ntt_inv_tensor(ctx->dP, ctx->logn, ext, have_ntt ? src : nullptr, cur, KS, prod, ctx->stream);
+            e = launch_ntt_inv_tensor(ctx->dP, ctx->logn, ext, have_ntt ? src : nullptr, cur, KS, prod, fold, !lean, ctx->stream);
         }
         if (e == cudaSuccess) { ProfScope ps(ctx, KC_BEHZ_FLOOR, lp_bytes(ctx, (double)cur * 3 * (KS + ctx->K)),
-                                                     (double)cur * 3 * n * (ctx->S * (ctx->K + 1) + ctx->S + ctx->K * ctx->S)); e = launch_behz_floor(ctx->hp.d, ctx->n, prod, cur, o->d + c0 * 3 * pw, ctx->stream); }
+                                                     (double)cur * 3 * n * (ctx->S * (ctx->K + 1) + ctx->S + ctx->K * ctx->S)); e = launch_behz_floor(ctx->hp.d, ctx->n, prod, cur, o->d + c0 * 3 * pw, ctx->stream, !lean); }
         if (e != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
     }
     dev_free(ctx, coef);

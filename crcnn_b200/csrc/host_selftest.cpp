@@ -86,6 +86,58 @@ int main(int argc, char **argv) {
                 if (reduce128_fold(z, f) != want || barrett128(z, m) != want) { printf("FOLD128 MISMATCH\n"); return 1; }
             }
         }
+        // square without n^-1 in its inverse transforms: the lift / floor constants that absorb it (params.h: *_n)
+        typedef unsigned __int128 u128;
+        for (int s = 0; s < d.K + d.S; s++) {
+            const uint64_t q = d.tab[s].mod.q;
+            const bool ok_ninv = (u128)d.tab[s].ninv * (uint64_t)n % q == 1;
+            bool ok = ok_ninv;
+            if (s < d.K) {
+                ok = ok && d.mt_inv_qhat_n[s] < q && (u128)d.mt_inv_qhat_n[s] * (uint64_t)n % q == d.mt_inv_qhat[s];
+                ok = ok && d.fl_c_n[s] < q && (u128)d.fl_c_n[s] * (uint64_t)n % q == d.fl_c[s];
+            } else {
+                ok = ok && d.fl_T_n[s - d.K] < q && (u128)d.fl_T_n[s - d.K] * (uint64_t)n % q == d.fl_T[s - d.K];
+            }
+            printf("ninv %d ok %d\n", s, ok ? 1 : 0);
+            if (!ok) { printf("NINV CONSTANT MISMATCH\n"); return 1; }
+        }
+        // the transforms' approximate Shoup product (modarith.cuh: mulshoup_lazy4, host form of the same quotient estimate) on edge
+        // operands: result in [0,4q) and = w*y mod q; and the three-partial-product square of the tensor stage
+        for (int s = 0; s < d.K + d.S; s++) {
+            const uint64_t q = d.tab[s].mod.q, nq = 0 - q;
+            const uint64_t ws[] = {0, 1, q - 1, q / 2, 0x5555555555555555ULL % q, 0};
+            long checked = 0;
+            for (int wi = 0; wi < 6; wi++) {
+                uint64_t w = ws[wi];
+                for (int it = 0; it < 20000; it++) {
+                    x = x * 6364136223846793005ULL + 1442695040888963407ULL;
+                    y = y * 2862933555777941757ULL + 3037000493ULL;
+                    if (wi == 5) w = y % q;
+                    const uint64_t wp = (uint64_t)(((u128)w << 64) / q);
+                    const int mode = it % 8;
+                    const uint64_t yv = mode == 0 ? 0 : mode == 1 ? ~0ull : mode == 2 ? (x % (~0ull / q + 1)) * q
+                                      : mode == 3 ? (~0ull / q) * q : mode == 4 ? q - 1 : mode == 5 ? 8 * q - 1 - (x & 7) : x;
+                    const uint64_t r = mulshoup_lazy4(yv, w, wp, nq);
+                    if (r >= 4 * q || r % q != (uint64_t)((u128)w * yv % q)) { printf("SHOUP4 MISMATCH\n"); return 1; }
+                    const uint64_t a = x % q;
+                    const U128 z = sqr128(a);
+                    if (((u128)z.hi << 64 | z.lo) != (u128)a * a) { printf("SQR128 MISMATCH\n"); return 1; }
+                    checked++;
+                }
+            }
+            printf("shoup4 %d checked %ld\n", s, checked);
+            // one-fold reduction of the forward transforms' final store (modarith.cuh: reduce64_shape), any 64-bit input
+            const int k = reduce64_shape_k(q);
+            if (k) {
+                for (int it = 0; it < 200000; it++) {
+                    x = x * 6364136223846793005ULL + 1442695040888963407ULL;
+                    const int mode = it % 6;
+                    const uint64_t v = mode == 0 ? ~0ull : mode == 1 ? 0 : mode == 2 ? q : mode == 3 ? q - 1 : mode == 4 ? (x % 16) * q + (x >> 60) : x;
+                    if (reduce64_shape(v, q, k) != v % q || reduce64(v, d.tab[s].mod) != v % q) { printf("REDUCE64 MISMATCH\n"); return 1; }
+                }
+            }
+            printf("reduce64_shape %d k %d\n", s, k);
+        }
         // fractional encoder
         for (int i = 4; i >= 0; i--) {
             double vals[] = {0.0867, -3.25, 0.0, 1.0, 2.8215};

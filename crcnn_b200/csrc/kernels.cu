@@ -3,6 +3,7 @@
 #include "devcfg.cuh"
 #include "ntt.cuh"
 #include <cstdlib>
+#include <cstring>
 
 namespace crcnn {
 
@@ -22,7 +23,7 @@ ntt_fwd_kernel(uint64_t *__restrict__ data, const DeviceParams *__restrict__ P, 
     smem_store_poly_canonical<LOGN>(sm, poly, tb.mod);
 }
 
-template <int LOGN>
+template <int LOGN, bool NINV>
 __global__ void __launch_bounds__(NttPlan<LOGN>::THREADS, NttPlan<LOGN>::MIN_CTAS)
 ntt_inv_kernel(uint64_t *__restrict__ data, const DeviceParams *__restrict__ P, int slot_base, int slot_count, int group_polys,
                int group_off, const uint64_t *__restrict__ src, const uint64_t *__restrict__ addend, int add_group, int add_stride) {
@@ -34,13 +35,36 @@ ntt_inv_kernel(uint64_t *__restrict__ data, const DeviceParams *__restrict__ P, 
     smem_load_poly<LOGN>(sm, src ? src + off : poly);   // src: out-of-place transform (same indexing), data is only written
     __syncthreads();
     // addend (relinearize): polynomial p adds polynomial (p / add_group) * add_stride + p % add_group of `addend`
-    ntt_inverse_from_smem<LOGN>(sm, poly, tb, addend ? addend + ((p / add_group) * add_stride + p % add_group) * (1L << LOGN) : nullptr);
+    ntt_inverse_from_smem<LOGN, NINV>(sm, poly, tb, addend ? addend + ((p / add_group) * add_stride + p % add_group) * (1L << LOGN) : nullptr);
 }
+
+// Reductions of the BEHZ kernels.  FOLD: the three-fold reduction through the 2^k - delta shape every SEAL modulus on this path has
+// (coefficient primes, the 61-bit Bsk primes and m_sk; modarith.cuh: reduce128_fold, host-checked against unsigned __int128 in
+// host_selftest.cpp); its constants are derived from q on the spot (5 instructions).  The launcher takes it only when
+// fold128_make(q).ok holds for EVERY modulus of the context (caller-supplied primes of another shape get the generic 128-bit
+// Barrett step); env CRCNN_BEHZ_FOLD=0 forces Barrett.  Measured on B200 (profiles/r02a_first.txt): behz_lift 9.0 -> 7.8 ms,
+// behz_floor 21.2 -> 18.0 ms per step of the bench network; both give the canonical residue, i.e. the same bytes.
+template <bool FOLD>
+__device__ __forceinline__ uint64_t behz_reduce(U128 z, const Mod &m) {
+    if constexpr (FOLD) {
+        Fold128 f;
+        const int k = 64 - __clzll((long long)m.q);
+        f.q = m.q; f.delta = (uint32_t)((1ull << k) - m.q); f.sh = (uint32_t)(k - 32); f.mask = (1u << (k - 32)) - 1; f.ok = 1;
+        return reduce128_fold(z, f);
+    } else {
+        return barrett128(z, m);
+    }
+}
+template <bool FOLD>
+__device__ __forceinline__ uint64_t behz_mulmod(uint64_t a, uint64_t b, const Mod &m) { return behz_reduce<FOLD>(mul128(a, b), m); }
 
 // Tensor square fused into the inverse transform (evaluator.cpp:783-848): the CTA of output limb-polynomial (ct, k, j)
 // forms c0*c0 (k = 0), 2*c0*c1 (k = 1) or c1*c1 (k = 2) mod the j-th prime of q U Bsk while loading, then inverse-transforms it.
 // Saves the write and re-read of the 3(K+S) product polynomials of every ciphertext.
-template <int LOGN>
+// FOLD: products reduced by behz_reduce<true> (three folds through 2^k - delta, 6 IMAD.WIDE) instead of barrett128 (~18 multiplier
+// instructions); a square takes 3 32x32 partial products instead of 4.  NINV = false: the output is left multiplied by n (the
+// floor kernel's constants carry n^-1, params.h: fl_c_n / fl_T_n).  Every variant stores the same canonical residues up to that factor.
+template <int LOGN, bool FOLD, bool NINV>
 __global__ void __launch_bounds__(NttPlan<LOGN>::THREADS, NttPlan<LOGN>::MIN_CTAS)
 ntt_inv_tensor_kernel(const DeviceParams *__restrict__ P, const uint64_t *__restrict__ ext, const uint64_t *__restrict__ qntt, int KS,
                       uint64_t *__restrict__ prod) {
@@ -59,27 +83,34 @@ ntt_inv_tensor_kernel(const DeviceParams *__restrict__ P, const uint64_t *__rest
     if (k == 1) {
 #pragma unroll 8
         for (int i = threadIdx.x; i < N; i += NttPlan<LOGN>::THREADS) {
-            const uint64_t ab = mulmod(__ldg(c0 + i), __ldg(c1 + i), tb.mod);
-            sm[ntt_pad(i)] = addmod(ab, ab, tb.mod.q);
+            if (FOLD) {
+                U128 z = mul128(__ldg(c0 + i), __ldg(c1 + i));   // < 2^122: doubling cannot wrap
+                z.hi = (z.hi << 1) | (z.lo >> 63);
+                z.lo <<= 1;
+                sm[ntt_pad(i)] = behz_reduce<true>(z, tb.mod);
+            } else {
+                const uint64_t ab = mulmod(__ldg(c0 + i), __ldg(c1 + i), tb.mod);
+                sm[ntt_pad(i)] = addmod(ab, ab, tb.mod.q);
+            }
         }
     } else {
         const uint64_t *c = k == 0 ? c0 : c1;
 #pragma unroll 8
         for (int i = threadIdx.x; i < N; i += NttPlan<LOGN>::THREADS) {
             const uint64_t a = __ldg(c + i);
-            sm[ntt_pad(i)] = mulmod(a, a, tb.mod);
+            sm[ntt_pad(i)] = FOLD ? behz_reduce<true>(sqr128(a), tb.mod) : mulmod(a, a, tb.mod);
         }
     }
     __syncthreads();
-    ntt_inverse_from_smem<LOGN>(sm, prod + b * N, tb);
+    ntt_inverse_from_smem<LOGN, NINV>(sm, prod + b * N, tb);
 }
 
-template <int LOGN>
+template <int LOGN, bool FOLD, bool NINV>
 static cudaError_t launch_ntt_inv_tensor_t(const DeviceParams *P, const uint64_t *ext, const uint64_t *qntt, long count, int KS, uint64_t *prod,
                                            cudaStream_t stream) {
     using Pl = NttPlan<LOGN>;
     const size_t smem = Pl::SMEM_WORDS * sizeof(uint64_t);
-    auto kf = ntt_inv_tensor_kernel<LOGN>;
+    auto kf = ntt_inv_tensor_kernel<LOGN, FOLD, NINV>;
     static DeviceOnce once;
     if (once.first()) {
         cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -89,15 +120,24 @@ static cudaError_t launch_ntt_inv_tensor_t(const DeviceParams *P, const uint64_t
     return cudaGetLastError();
 }
 
+template <int LOGN>
+static cudaError_t launch_ntt_inv_tensor_l(const DeviceParams *P, const uint64_t *ext, const uint64_t *qntt, long count, int KS, uint64_t *prod,
+                                           bool fold, bool ninv, cudaStream_t stream) {
+    if (!ninv) return fold ? launch_ntt_inv_tensor_t<LOGN, true, false>(P, ext, qntt, count, KS, prod, stream)
+                           : launch_ntt_inv_tensor_t<LOGN, false, false>(P, ext, qntt, count, KS, prod, stream);
+    if (fold) return cudaErrorInvalidValue;   // not instantiated: the folded products come only with the n^-1-free output
+    return launch_ntt_inv_tensor_t<LOGN, false, true>(P, ext, qntt, count, KS, prod, stream);
+}
+
 cudaError_t launch_ntt_inv_tensor(const DeviceParams *P, int logn, const uint64_t *ext, const uint64_t *qntt, long count, int KS, uint64_t *prod,
-                                  cudaStream_t stream) {
+                                  bool fold, bool ninv, cudaStream_t stream) {
     if (count <= 0) return cudaSuccess;
     switch (logn) {
-        case 10: return launch_ntt_inv_tensor_t<10>(P, ext, qntt, count, KS, prod, stream);
-        case 11: return launch_ntt_inv_tensor_t<11>(P, ext, qntt, count, KS, prod, stream);
-        case 12: return launch_ntt_inv_tensor_t<12>(P, ext, qntt, count, KS, prod, stream);
-        case 13: return launch_ntt_inv_tensor_t<13>(P, ext, qntt, count, KS, prod, stream);
-        case 14: return launch_ntt_inv_tensor_t<14>(P, ext, qntt, count, KS, prod, stream);
+        case 10: return launch_ntt_inv_tensor_l<10>(P, ext, qntt, count, KS, prod, fold, ninv, stream);
+        case 11: return launch_ntt_inv_tensor_l<11>(P, ext, qntt, count, KS, prod, fold, ninv, stream);
+        case 12: return launch_ntt_inv_tensor_l<12>(P, ext, qntt, count, KS, prod, fold, ninv, stream);
+        case 13: return launch_ntt_inv_tensor_l<13>(P, ext, qntt, count, KS, prod, fold, ninv, stream);
+        case 14: return launch_ntt_inv_tensor_l<14>(P, ext, qntt, count, KS, prod, fold, ninv, stream);
         default: return cudaErrorInvalidValue;
     }
 }
@@ -105,35 +145,38 @@ cudaError_t launch_ntt_inv_tensor(const DeviceParams *P, int logn, const uint64_
 template <int LOGN>
 static cudaError_t launch_ntt_t(const DeviceParams *P, uint64_t *data, long npolys, int slot_base, int slot_count,
                                 bool inverse, int group_polys, int group_off, const uint64_t *src, const uint64_t *addend,
-                                int add_group, int add_stride, cudaStream_t stream) {
+                                int add_group, int add_stride, bool ninv, cudaStream_t stream) {
     using Pl = NttPlan<LOGN>;
     size_t smem = Pl::SMEM_WORDS * sizeof(uint64_t);
     auto kf = ntt_fwd_kernel<LOGN>;
-    auto ki = ntt_inv_kernel<LOGN>;
+    auto ki = ntt_inv_kernel<LOGN, true>;
+    auto kn = ntt_inv_kernel<LOGN, false>;
     static DeviceOnce once;
     if (once.first()) {
         cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         cudaFuncSetAttribute(ki, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaFuncSetAttribute(kn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         // without this the driver sizes the carve-out for ONE resident CTA (seen in ncu: occupancy limit 1)
         cudaFuncSetAttribute(kf, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
         cudaFuncSetAttribute(ki, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        cudaFuncSetAttribute(kn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     }
     if (npolys <= 0) return cudaSuccess;
-    if ((src || addend) && !inverse) return cudaErrorInvalidValue;
-    if (inverse) ki<<<(unsigned)npolys, Pl::THREADS, smem, stream>>>(data, P, slot_base, slot_count, group_polys, group_off, src, addend, add_group, add_stride);
+    if ((src || addend || !ninv) && !inverse) return cudaErrorInvalidValue;
+    if (inverse) (ninv ? ki : kn)<<<(unsigned)npolys, Pl::THREADS, smem, stream>>>(data, P, slot_base, slot_count, group_polys, group_off, src, addend, add_group, add_stride);
     else kf<<<(unsigned)npolys, Pl::THREADS, smem, stream>>>(data, P, slot_base, slot_count, group_polys, group_off);
     return cudaGetLastError();
 }
 
 cudaError_t launch_ntt_grouped(const DeviceParams *P, int logn, uint64_t *data, long npolys, int slot_base, int slot_count,
                                bool inverse, int group_polys, int group_off, cudaStream_t stream, const uint64_t *src,
-                               const uint64_t *addend, int add_group, int add_stride) {
+                               const uint64_t *addend, int add_group, int add_stride, bool ninv) {
     switch (logn) {
-        case 10: return launch_ntt_t<10>(P, data, npolys, slot_base, slot_count, inverse, group_polys, group_off, src, addend, add_group, add_stride, stream);
-        case 11: return launch_ntt_t<11>(P, data, npolys, slot_base, slot_count, inverse, group_polys, group_off, src, addend, add_group, add_stride, stream);
-        case 12: return launch_ntt_t<12>(P, data, npolys, slot_base, slot_count, inverse, group_polys, group_off, src, addend, add_group, add_stride, stream);
-        case 13: return launch_ntt_t<13>(P, data, npolys, slot_base, slot_count, inverse, group_polys, group_off, src, addend, add_group, add_stride, stream);
-        case 14: return launch_ntt_t<14>(P, data, npolys, slot_base, slot_count, inverse, group_polys, group_off, src, addend, add_group, add_stride, stream);
+        case 10: return launch_ntt_t<10>(P, data, npolys, slot_base, slot_count, inverse, group_polys, group_off, src, addend, add_group, add_stride, ninv, stream);
+        case 11: return launch_ntt_t<11>(P, data, npolys, slot_base, slot_count, inverse, group_polys, group_off, src, addend, add_group, add_stride, ninv, stream);
+        case 12: return launch_ntt_t<12>(P, data, npolys, slot_base, slot_count, inverse, group_polys, group_off, src, addend, add_group, add_stride, ninv, stream);
+        case 13: return launch_ntt_t<13>(P, data, npolys, slot_base, slot_count, inverse, group_polys, group_off, src, addend, add_group, add_stride, ninv, stream);
+        case 14: return launch_ntt_t<14>(P, data, npolys, slot_base, slot_count, inverse, group_polys, group_off, src, addend, add_group, add_stride, ninv, stream);
         default: return cudaErrorInvalidValue;
     }
 }
@@ -769,26 +812,6 @@ plain_op_kernel(const DeviceParams *__restrict__ P, uint64_t *__restrict__ data,
     x[0] = a; x[1] = b;
 }
 
-// Reductions of the BEHZ kernels.  FOLD: the three-fold reduction through the 2^k - delta shape every SEAL modulus on this path has
-// (coefficient primes, the 61-bit Bsk primes and m_sk; modarith.cuh: reduce128_fold, host-checked against unsigned __int128 in
-// host_selftest.cpp); its constants are derived from q on the spot (5 instructions).  The launcher takes it only when
-// fold128_make(q).ok holds for EVERY modulus of the context (caller-supplied primes of another shape get the generic 128-bit
-// Barrett step); env CRCNN_BEHZ_FOLD=0 forces Barrett.  Measured on B200 (profiles/r02a_first.txt): behz_lift 9.0 -> 7.8 ms,
-// behz_floor 21.2 -> 18.0 ms per step of the bench network; both give the canonical residue, i.e. the same bytes.
-template <bool FOLD>
-__device__ __forceinline__ uint64_t behz_reduce(U128 z, const Mod &m) {
-    if constexpr (FOLD) {
-        Fold128 f;
-        const int k = 64 - __clzll((long long)m.q);
-        f.q = m.q; f.delta = (uint32_t)((1ull << k) - m.q); f.sh = (uint32_t)(k - 32); f.mask = (1u << (k - 32)) - 1; f.ok = 1;
-        return reduce128_fold(z, f);
-    } else {
-        return barrett128(z, m);
-    }
-}
-template <bool FOLD>
-__device__ __forceinline__ uint64_t behz_mulmod(uint64_t a, uint64_t b, const Mod &m) { return behz_reduce<FOLD>(mul128(a, b), m); }
-
 // =====================================================================================
 // BEHZ square pieces
 // =====================================================================================
@@ -1095,7 +1118,7 @@ cudaError_t launch_plain_op(const DeviceParams *P, int n, int K, uint64_t *data,
     } while (0)
 
 // every modulus the BEHZ kernels reduce by (coefficient primes, Bsk primes incl. m_sk) has the 2^k - delta shape reduce128_fold needs
-static bool behz_fold_ok(const DeviceParams &hp) {
+bool behz_fold_ok(const DeviceParams &hp) {
     static const int env = [] { const char *e = getenv("CRCNN_BEHZ_FOLD"); return e ? atoi(e) : 1; }();
     if (!env) return false;
     for (int i = 0; i < hp.K + hp.S; i++)
@@ -1103,17 +1126,33 @@ static bool behz_fold_ok(const DeviceParams &hp) {
     return true;
 }
 
-cudaError_t launch_behz_lift(const DeviceParams &hp, int n, const uint64_t *in, const uint64_t *in_ntt, long count, uint64_t *ext,
-                                cudaStream_t stream) {
+// The kernels take the parameter block by value, so an input left multiplied by n (ninv_in = false) is served by a copy of
+// the block whose first-step constants carry n^-1 -- the kernels themselves do not change.
+cudaError_t launch_behz_lift(const DeviceParams &P, int n, const uint64_t *in, const uint64_t *in_ntt, long count, uint64_t *ext,
+                                cudaStream_t stream, bool ninv_in) {
     if (count <= 0) return cudaSuccess;
+    if (!ninv_in && !in_ntt) return cudaErrorInvalidValue;   // the copied q limbs would carry the factor n
+    DeviceParams scaled;
+    if (!ninv_in) {
+        scaled = P;
+        std::memcpy(scaled.mt_inv_qhat, P.mt_inv_qhat_n, sizeof scaled.mt_inv_qhat);
+    }
+    const DeviceParams &hp = ninv_in ? P : scaled;
     const unsigned grid = (unsigned)(count * 2 * (n / 128));
     CRCNN_BEHZ_DISPATCH(behz_lift_kernel, grid, in, in_ntt, ext);
     return cudaGetLastError();
 }
 
-cudaError_t launch_behz_floor(const DeviceParams &hp, int n, const uint64_t *prod, long count, uint64_t *out,
-                                 cudaStream_t stream) {
+cudaError_t launch_behz_floor(const DeviceParams &P, int n, const uint64_t *prod, long count, uint64_t *out,
+                                 cudaStream_t stream, bool ninv_in) {
     if (count <= 0) return cudaSuccess;
+    DeviceParams scaled;
+    if (!ninv_in) {
+        scaled = P;
+        std::memcpy(scaled.fl_c, P.fl_c_n, sizeof scaled.fl_c);
+        std::memcpy(scaled.fl_T, P.fl_T_n, sizeof scaled.fl_T);
+    }
+    const DeviceParams &hp = ninv_in ? P : scaled;
     const unsigned grid = (unsigned)(count * 3 * (n / 128));
     CRCNN_BEHZ_DISPATCH(behz_floor_kernel, grid, prod, out);
     return cudaGetLastError();

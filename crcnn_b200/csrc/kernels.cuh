@@ -16,9 +16,11 @@ cudaError_t launch_ntt(const DeviceParams *P, int logn, uint64_t *data, long npo
 // (e.g. only the Bsk limbs of [count][2][K+S][n]).
 // src (inverse transform only): read the polynomials from src instead of data (out of place, same indexing).
 // addend (inverse only): output polynomial p = transform + polynomial (p / add_group) * add_stride + p % add_group of addend.
+// ninv = false (inverse only): the output is n times the inverse transform, canonical -- for a consumer that multiplies
+// every residue by a constant carrying n^-1 next (launch_behz_lift with ninv_in = false).
 cudaError_t launch_ntt_grouped(const DeviceParams *P, int logn, uint64_t *data, long npolys, int slot_base, int slot_count,
                                bool inverse, int group_polys, int group_off, cudaStream_t stream, const uint64_t *src = nullptr,
-                               const uint64_t *addend = nullptr, int add_group = 1, int add_stride = 1);
+                               const uint64_t *addend = nullptr, int add_group = 1, int add_stride = 1, bool ninv = true);
 
 // ---- plaintext packs: sparse coefficient form -> dense NTT form, one CTA per (plaintext, limb).
 // mode 0: lifted residues (multiplicative use: weights, scale factors)  [evaluator.cpp:1465-1486]
@@ -91,10 +93,16 @@ cudaError_t launch_plain_op(const DeviceParams *P, int n, int K, uint64_t *data,
 // base-conversion constant is a constant-bank operand)
 // in_ntt (optional): the same ciphertexts in NTT form; the q limbs of ext are then left unwritten (launch_ntt_inv_tensor reads them from in_ntt) and only the Bsk
 // limbs still need the forward transform
+// ninv_in = false: `in` holds n times the coefficients (an inverse transform without its n^-1, launch_ntt_grouped ninv = false);
+// the lift then multiplies by mt_inv_qhat_n.  Only together with in_ntt: the q limbs of `in` are not copied to ext then.
 cudaError_t launch_behz_lift(const DeviceParams &hp, int n, const uint64_t *in, const uint64_t *in_ntt, long count, uint64_t *ext,
-                             cudaStream_t stream);
+                             cudaStream_t stream, bool ninv_in = true);
 // floor:  prod (coefficient form) -> out [count][3][K][n]: multiply by t, fast_floor, fastbconv_sk
-cudaError_t launch_behz_floor(const DeviceParams &hp, int n, const uint64_t *prod, long count, uint64_t *out, cudaStream_t stream);
+// ninv_in = false: prod holds n times the products (launch_ntt_inv_tensor with ninv = false); fl_c_n / fl_T_n absorb the factor.
+cudaError_t launch_behz_floor(const DeviceParams &hp, int n, const uint64_t *prod, long count, uint64_t *out, cudaStream_t stream,
+                              bool ninv_in = true);
+// true when every modulus of the context (q and Bsk) has the 2^k - delta shape of reduce128_fold (modarith.cuh)
+bool behz_fold_ok(const DeviceParams &hp);
 
 // ---- relinearize 3 -> 2 with 16-bit digits (evaluator.cpp:934-1069)
 // in3 [count][3][K][n] (coefficient), keys: for prime i, digit k: polys (2k, 2k+1) at
@@ -113,8 +121,10 @@ struct RelinArgs {
 // ---- tensor square (c0*c0, 2*c0*c1, c1*c1 in q U Bsk) fused into the inverse transform of each product polynomial:
 // ext = [count][2][KS][n] NTT form (qntt != null: its q limbs are taken from qntt = [count][2][K][n] instead),
 // prod = [count][3][KS][n] coefficient form
+// fold: reduce the products with reduce128_fold (requires behz_fold_ok; only with ninv = false).  ninv = false: prod holds n times
+// the products, for launch_behz_floor with ninv_in = false.
 cudaError_t launch_ntt_inv_tensor(const DeviceParams *P, int logn, const uint64_t *ext, const uint64_t *qntt, long count, int KS, uint64_t *prod,
-                                  cudaStream_t stream);
+                                  bool fold, bool ninv, cudaStream_t stream);
 
 // stages 1-3 (scale, digit NTTs, key MAC); then the caller inverse-NTTs `acc` and calls launch_relin_finish
 cudaError_t launch_relin(const DeviceParams *P, int logn, int K, const RelinArgs &a, cudaStream_t stream);

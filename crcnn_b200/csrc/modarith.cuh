@@ -39,6 +39,16 @@ CRCNN_HD U128 mul128(uint64_t a, uint64_t b) {
     return r;
 }
 
+// a*a for a < 2^63 from three 32x32 partial products: a1^2 2^64 + 2 a0 a1 2^32 + a0^2 (2 a0 a1 < 2^64).
+CRCNN_HD U128 sqr128(uint64_t a) {
+    const uint64_t a0 = (uint32_t)a, a1 = a >> 32;
+    const uint64_t lo = a0 * a0, mid = (a0 * a1) << 1, hi = a1 * a1;
+    U128 r;
+    r.lo = lo + (mid << 32);
+    r.hi = hi + (mid >> 32) + (r.lo < lo);
+    return r;
+}
+
 // acc += a*b (mod 2^128).  Callers bound the number of accumulated terms so this never wraps.
 CRCNN_HD void mac128(U128 &acc, uint64_t a, uint64_t b) {
     uint64_t lo = a * b;
@@ -129,6 +139,20 @@ CRCNN_HD uint64_t reduce64(uint64_t x, const Mod &m) {
     return r >= m.q ? r - m.q : r;
 }
 
+// x mod q for any 64-bit x when q = 2^k - delta with k >= 48 and delta < 2^27 (every SEAL coefficient prime and Bsk prime): one fold
+// x = lo + hi 2^k = lo + hi delta (mod q), hi < 2^16 so hi delta < 2^43 is ONE 32x32 IMAD.WIDE, and lo + hi delta < 2^k + 2^43 < 2q,
+// so one conditional subtraction gives the canonical residue -- the same value as reduce64.  shape_k = k, or 0 when q lacks the shape.
+CRCNN_HD int reduce64_shape_k(uint64_t q) {
+    int k = 0;
+    for (uint64_t v = q; v; v >>= 1) k++;
+    return (k >= 48 && k <= 63 && ((1ull << k) - q) < (1ull << 27)) ? k : 0;
+}
+CRCNN_HD uint64_t reduce64_shape(uint64_t x, uint64_t q, int k) {
+    const uint32_t delta = (uint32_t)((1ull << k) - q), hi = (uint32_t)(x >> k);
+    const uint64_t r = (x & ((1ull << k) - 1)) + (uint64_t)hi * delta;
+    return r >= q ? r - q : r;
+}
+
 CRCNN_HD uint64_t mulmod(uint64_t a, uint64_t b, const Mod &m) { return barrett128(mul128(a, b), m); }
 
 CRCNN_HD uint64_t addmod(uint64_t a, uint64_t b, uint64_t q) {
@@ -148,16 +172,21 @@ CRCNN_HD uint64_t mulshoup_lazy(uint64_t y, uint64_t w, uint64_t wp, uint64_t q)
 // Cheaper Shoup product for the transforms: the quotient estimate drops the low partial products,
 //   h' = wp1*y1 + hi32(wp1*y0) + hi32(wp0*y1)  in  {h-2, h-1, h},   h = floor(wp*y / 2^64),
 // so the result  y*w - h'*q  (mod 2^64)  is w*y mod q as a representative in [0, 4q) for any 64-bit y
-// (q < 2^62).  nq = 2^64 - q turns the subtraction into a multiply-add: 3 IMAD.WIDE + 2 IMAD.HI + 4 IMAD and
-// two carry adds, against 6 IMAD.WIDE + 5 IMAD and ~9 adds for the exact form.
+// (q < 2^62).  nq = 2^64 - q turns the subtraction into a multiply-add.  The two hi32 terms are taken as the high
+// word of a mul.wide.u32 (IMAD.WIDE.U32, 2.17 clk per warp instruction on the multiplier pipe) rather than
+// mul.hi.u32 (IMAD.HI, 4 clk; profiles/r01_pipe_probe.txt) -- the same value: 5 IMAD.WIDE + 4 IMAD and two carry
+// adds, against 6 IMAD.WIDE + 5 IMAD and ~9 adds for the exact form.
 CRCNN_HD uint64_t mulshoup_lazy4(uint64_t y, uint64_t w, uint64_t wp, uint64_t nq) {
 #if defined(__CUDA_ARCH__)
     uint32_t y0 = (uint32_t)y, y1 = (uint32_t)(y >> 32), p0 = (uint32_t)wp, p1 = (uint32_t)(wp >> 32);
     uint32_t w0 = (uint32_t)w, w1 = (uint32_t)(w >> 32), n0 = (uint32_t)nq, n1 = (uint32_t)(nq >> 32);
     uint32_t a, b, h0, h1, r0, r1;
-    asm("mul.hi.u32 %0, %2, %3;\n\t"
-        "mul.hi.u32 %1, %4, %5;\n\t"
-        : "=r"(a), "=r"(b) : "r"(p1), "r"(y0), "r"(p0), "r"(y1));
+    uint64_t wa, wb;
+    asm("mul.wide.u32 %0, %2, %3;\n\t"
+        "mul.wide.u32 %1, %4, %5;\n\t"
+        : "=l"(wa), "=l"(wb) : "r"(p1), "r"(y0), "r"(p0), "r"(y1));
+    a = (uint32_t)(wa >> 32);
+    b = (uint32_t)(wb >> 32);
     asm("mad.lo.cc.u32 %0, %2, %3, %4;\n\t"
         "madc.hi.u32 %1, %2, %3, 0;\n\t"
         "add.cc.u32 %0, %0, %5;\n\t"
@@ -270,8 +299,8 @@ CRCNN_HD uint64_t tcn_fold_reduce(const uint32_t (&s)[13], uint64_t bias, const 
 // The same idea for ANY 128-bit value (the lazy sums of the BEHZ and relinearize kernels): z mod q for q = 2^k - delta, 54 <= k <= 61,
 // delta < 2^27 -- every coefficient prime and every Bsk prime of SEAL 2.3.1 (SEAL/seal/util/globals.cpp:50-74, 321-340).  Three folds of
 // the bits above k through delta (6 IMAD.WIDE in all, against 18 multiply-pipe instructions of barrett128) and one conditional
-// subtraction; canonical result, so it equals barrett128(z, mod) bit for bit.  NOT wired into any kernel yet (DESIGN.md section 9 item 5);
-// host_selftest.cpp checks it against unsigned __int128 for every modulus of the context.
+// subtraction; canonical result, so it equals barrett128(z, mod) bit for bit.  Used by the BEHZ kernels and the tensor products of
+// `square` (kernels.cu: behz_reduce); host_selftest.cpp checks it against unsigned __int128 for every modulus of the context.
 struct Fold128 {
     uint64_t q;
     uint32_t delta, sh, mask, ok;   // 2^k - q, k - 32, 2^(k-32) - 1

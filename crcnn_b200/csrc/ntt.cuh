@@ -12,7 +12,8 @@
 //     primes of `square`) keep the exact product and the correction.
 //   * inverse: the n^-1 factor is applied once at the end (one Shoup product per residue) instead of a
 //     halving in every butterfly, so the tables hold the plain inverse powers; for q < 2^57 the butterflies
-//     keep values in [0,4q) with the same approximate product.
+//     keep values in [0,4q) with the same approximate product.  Callers that multiply every output residue by a
+//     constant next can leave n^-1 out altogether (NINV = false) and fold it into their constant.
 // Both remove ALU-pipe work, which ncu showed to be the binding pipe (profiles/r01b_*).
 //
 // Schedule: log2(n) stages are grouped into passes of 3 or 4 stages done in registers
@@ -223,8 +224,10 @@ __device__ __forceinline__ void inv_first_pass(uint64_t *sm, const NttTable &tb)
     }
 }
 
-// DST_GLOBAL marks the last pass: the n^-1 scaling and the canonical store happen there.
-template <int LOGN, int B, bool DST_GLOBAL, bool CORR>
+// DST_GLOBAL marks the last pass: the n^-1 scaling and the canonical store happen there.  NINV = false stores
+// n * (the inverse transform) instead, still canonical, for a consumer whose first operation on every residue is a
+// product by a constant that has absorbed n^-1 (the BEHZ lift and floor of `square`, params.h: *_n).
+template <int LOGN, int B, bool DST_GLOBAL, bool CORR, bool NINV = true>
 __device__ __forceinline__ void inv_pass(uint64_t *sm, uint64_t *__restrict__ gdst, const NttTable &tb, int g,
                                          const uint64_t *__restrict__ gadd = nullptr) {
     constexpr int N = 1 << LOGN;
@@ -241,7 +244,12 @@ __device__ __forceinline__ void inv_pass(uint64_t *sm, uint64_t *__restrict__ gd
 #pragma unroll
         for (int k = 0; k < (1 << B); k++) {
             if (DST_GLOBAL) {
-                uint64_t v = mulshoup_lazy(x[k], tb.ninv, tb.ninvp, q);  // exact product: [0,2q) for any 64-bit input
+                uint64_t v;
+                if (NINV) {
+                    v = mulshoup_lazy(x[k], tb.ninv, tb.ninvp, q);  // exact product: [0,2q) for any 64-bit input
+                } else {
+                    v = x[k] >= 2 * q ? x[k] - 2 * q : x[k];          // [0,4q) (lazy) or [0,2q) (exact) -> [0,2q)
+                }
                 v = v >= q ? v - q : v;
                 if (gadd) v = addmod(v, __ldg(gadd + base + k * g), q);   // fused "+ c_p" of relinearize
                 gdst[base + k * g] = v;
@@ -295,7 +303,7 @@ __device__ __forceinline__ void ntt_forward_in_smem(uint64_t *sm, const NttTable
 // Inverse transform of the polynomial in padded shared memory (values < 2q, < 4q on the lazy path) -> dst
 // (global, canonical).  Pass order mirrors the forward plan (narrow passes first so the last, HBM-writing pass
 // is strided).
-template <int LOGN, bool CORR>
+template <int LOGN, bool CORR, bool NINV>
 __device__ __forceinline__ void ntt_inverse_passes(uint64_t *sm, uint64_t *__restrict__ dst, const NttTable &tb,
                                                    const uint64_t *__restrict__ add) {
     using P = NttPlan<LOGN>;
@@ -307,14 +315,15 @@ __device__ __forceinline__ void ntt_inverse_passes(uint64_t *sm, uint64_t *__res
         g <<= P::bits(p);
         __syncthreads();
     }
-    if (P::bits(0) == 4) inv_pass<LOGN, 4, true, CORR>(sm, dst, tb, g, add); else inv_pass<LOGN, 3, true, CORR>(sm, dst, tb, g, add);
+    if (P::bits(0) == 4) inv_pass<LOGN, 4, true, CORR, NINV>(sm, dst, tb, g, add); else inv_pass<LOGN, 3, true, CORR, NINV>(sm, dst, tb, g, add);
 }
 
-template <int LOGN>
+// NINV = false: the output is n times the inverse transform (see inv_pass)
+template <int LOGN, bool NINV = true>
 __device__ __forceinline__ void ntt_inverse_from_smem(uint64_t *sm, uint64_t *__restrict__ dst, const NttTable &tb,
                                                       const uint64_t *__restrict__ add = nullptr) {
-    if (ntt_inv_exact(tb.mod.q)) ntt_inverse_passes<LOGN, true>(sm, dst, tb, add);
-    else ntt_inverse_passes<LOGN, false>(sm, dst, tb, add);
+    if (ntt_inv_exact(tb.mod.q)) ntt_inverse_passes<LOGN, true, NINV>(sm, dst, tb, add);
+    else ntt_inverse_passes<LOGN, false, NINV>(sm, dst, tb, add);
 }
 
 // Coalesced copies between global (unpadded) and shared (padded).
@@ -323,11 +332,18 @@ __device__ __forceinline__ void smem_load_poly(uint64_t *sm, const uint64_t *__r
 #pragma unroll 8
     for (int i = threadIdx.x; i < (1 << LOGN); i += NttPlan<LOGN>::THREADS) sm[ntt_pad(i)] = src[i];
 }
-// Lazy forward output (any value below 2^63) -> canonical residues in global memory.
+// Lazy forward output (any 64-bit value) -> canonical residues in global memory.  Primes of the 2^k - delta shape take the one-fold
+// reduction (1 IMAD.WIDE per residue instead of the ~9 multiplier instructions of reduce64); same residues.
 template <int LOGN>
 __device__ __forceinline__ void smem_store_poly_canonical(const uint64_t *sm, uint64_t *__restrict__ dst, const Mod &mod) {
+    const int k = reduce64_shape_k(mod.q);
+    if (k) {
 #pragma unroll 8
-    for (int i = threadIdx.x; i < (1 << LOGN); i += NttPlan<LOGN>::THREADS) dst[i] = reduce64(sm[ntt_pad(i)], mod);
+        for (int i = threadIdx.x; i < (1 << LOGN); i += NttPlan<LOGN>::THREADS) dst[i] = reduce64_shape(sm[ntt_pad(i)], mod.q, k);
+    } else {
+#pragma unroll 8
+        for (int i = threadIdx.x; i < (1 << LOGN); i += NttPlan<LOGN>::THREADS) dst[i] = reduce64(sm[ntt_pad(i)], mod);
+    }
 }
 
 }  // namespace crcnn

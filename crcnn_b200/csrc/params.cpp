@@ -212,6 +212,11 @@ HostParams derive_params(int n, int K, const uint64_t *q, uint64_t t) {
         }
     }
     for (int i = 0; i < d.L; i++) d.fl_P[i] = mulmod(d.Mhat_mod_msk[i], d.inv_M_mod_msk, msk);
+    for (int j = 0; j < K; j++) {
+        d.mt_inv_qhat_n[j] = mulmod(d.mt_inv_qhat[j], d.tab[j].ninv, d.tab[j].mod);
+        d.fl_c_n[j] = mulmod(d.fl_c[j], d.tab[j].ninv, d.tab[j].mod);
+    }
+    for (int k = 0; k < d.S; k++) d.fl_T_n[k] = mulmod(d.fl_T[k], d.tab[K + k].ninv, d.tab[K + k].mod);
     return hp;
 }
 

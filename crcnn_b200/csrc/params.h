@@ -73,6 +73,11 @@ struct DeviceParams {
     uint64_t fl_T[MAXS];                // t * q^-1 [* (M/m_k)^-1 for k < L] mod p_k
     uint64_t fl_N[MAXS][MAXK];          // -(q/q_i mod p_k) * q^-1 [* (M/m_k)^-1 for k < L] mod p_k
     uint64_t fl_P[MAXS];                // (M/m_i mod m_sk) * M^-1 mod m_sk
+    // The same first-step constants times n^-1 (mod q_i resp. p_k): for lift / floor inputs that an inverse transform left
+    // multiplied by n (kernels.cuh: ninv_in = false), so the transform saves its n^-1 product per residue.
+    uint64_t mt_inv_qhat_n[MAXK];       // mt_inv_qhat * n^-1 mod q_i
+    uint64_t fl_c_n[MAXK];              // fl_c * n^-1 mod q_i
+    uint64_t fl_T_n[MAXS];              // fl_T * n^-1 mod p_k
 };
 
 // Host copy: the scalar part of DeviceParams plus the tables as vectors.
