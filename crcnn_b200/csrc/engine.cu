@@ -62,9 +62,11 @@ struct crcnn_plain {
     int tc_state = 0;              // 0 not examined, 1 eligible, -1 not (support outside x^(n-32..n-1) or digits other than +-1)
     int8_t *tc_A = nullptr;
     int tc_R = 0, tc_Kpad = 0;
-    // limb-split tensor-core form (tcn_mac.cuh): byte planes of the NTT-form weights [K*n][7][count/R][Kpad]
+    // limb-split tensor-core form (tcn_mac.cuh): byte planes of the NTT-form weights [K*n][7][count/R][Kpad]; pre-shifted
+    // (tcn_pre): seven such blocks, block b holding the planes of W 2^(8b) mod q_j (block 0 is the plain staging)
     uint8_t *tcn_W = nullptr;
     int tcn_R = 0;
+    bool tcn_pre = false;
     // fused average pooling + batch-norm (this pack = the batch-norm factors): C[z] = scale (.) invstd[z] with Shoup companions and
     // D[z] = mean[z] (.) invstd[z] in NTT form, valid for the (scale, mean) packs they were made from
     uint64_t *fused_C = nullptr, *fused_Csh = nullptr, *fused_D = nullptr;
@@ -111,6 +113,7 @@ struct crcnn_ctx {
     int relin_mode = 1;              // 1: relinearize through 30-bit auxiliary primes when exact for the parameters (relin32.cuh); 0: 64-bit transforms
     int tcn_mode = 1;                // 1: weighted sums whose staged weights fit the weight cache run as the NTT-domain limb-split GEMM (tcn_mac.cuh)
     int sq_lean = 1;                 // 1 (default): square's tensor products reduce through the 2^k - delta fold when every modulus allows, and the inverse transforms feeding the BEHZ lift / floor leave n^-1 to their constants (params.h: *_n); 0: Barrett products, n^-1 in the transforms; same bytes; env CRCNN_SQ_LEAN
+    int tcn_preshift = 1;            // 1 (default): convolution weights of fan-in <= 32 are staged pre-shifted and run on the seven-class kernel (tcn_mac.cu: tcn2p_mac_kernel) when 7x the planes fit the weight cache; 0: 13-class kernel; same bytes; env CRCNN_TCN2_PRESHIFT
     int tcn_fold = 1;                // 1 (default): the limb-split GEMM reduces its class sums through the 2^k - delta shape of the primes when every prime has it (modarith.cuh: tcn_fold_reduce), 0: 128-bit recombination + Barrett; same bytes; env CRCNN_TCN_FOLD
     size_t tc_scratch_bytes = 12ull << 30;
     std::string err;
@@ -452,36 +455,56 @@ int run_weighted_sum_tc(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_
 }
 
 // Byte planes of the whole pack's NTT-form weights, staged once (tcn_mac.cuh); the dense NTT form is released afterwards.
-int ensure_tcn_weights(crcnn_ctx *ctx, crcnn_plain *w, int R) {
+// preshift: also the planes of W 2^(8b) mod q_j for b = 1..6 (the seven-class kernel).  A pack keeps its first staging: a
+// pre-shifted one serves the 13-class kernels through its first block.
+int ensure_tcn_weights(crcnn_ctx *ctx, crcnn_plain *w, int R, bool preshift) {
     if (w->tcn_W && w->tcn_R == R) return CRCNN_OK;
     int rc = ensure_form(ctx, w, PF_NTT_MUL);
     if (rc) return rc;
     if (w->tcn_W) { dev_free(ctx, w->tcn_W); w->tcn_W = nullptr; }
     const int Mall = (int)(w->count / R), Kpad = tcn_kpad(R);
-    rc = dev_alloc(ctx, tcn_w_bytes(7, Mall, Kpad, ctx->K, ctx->n), (void **)&w->tcn_W);
+    const size_t block = tcn_w_bytes(7, Mall, Kpad, ctx->K, ctx->n);
+    const int blocks = preshift ? 7 : 1;
+    rc = dev_alloc(ctx, block * blocks, (void **)&w->tcn_W);
     if (rc) return rc;
+    const long words = (long)w->count * (long)poly_words(ctx);
+    uint64_t *shifted = nullptr;
+    if (preshift) {
+        rc = dev_alloc(ctx, (size_t)words * 8, (void **)&shifted);
+        if (rc) { dev_free(ctx, w->tcn_W); w->tcn_W = nullptr; return rc; }
+    }
+    uint64_t q[MAXK];
+    for (int j = 0; j < ctx->K; j++) q[j] = ctx->hp.d.tab[j].mod.q;
     TcnSplitArgs s{};
-    s.src = w->ntt_mul; s.index = nullptr; s.dst = w->tcn_W; s.item_polys = 1;
+    s.index = nullptr; s.item_polys = 1;
     s.R = R; s.Kpad = Kpad; s.planes = 7; s.ncols = Mall; s.slot0 = 0; s.nslots = ctx->K * ctx->n; s.n = ctx->n; s.K = ctx->K;
-    {
-        ProfScope ps(ctx, KC_TCN_SPLIT, lp_bytes(ctx, (double)w->count * ctx->K) + (double)tcn_w_bytes(7, Mall, Kpad, ctx->K, ctx->n), 0);
+    for (int b = 0; b < blocks; b++) {
+        if (b) CU(launch_tcn_preshift(q, w->ntt_mul, shifted, words, b, ctx->n, ctx->K, ctx->stream));
+        s.src = b ? shifted : w->ntt_mul;
+        s.dst = w->tcn_W + block * b;
+        ProfScope ps(ctx, KC_TCN_SPLIT, lp_bytes(ctx, (double)w->count * ctx->K) + (double)block, 0);
         CU(launch_tcn_split(s, ctx->stream));
     }
+    if (shifted) dev_free(ctx, shifted);
     dev_free(ctx, w->ntt_mul); w->ntt_mul = nullptr;
     if (w->ntt_mul_sh) { dev_free(ctx, w->ntt_mul_sh); w->ntt_mul_sh = nullptr; }
     w->tcn_R = R;
+    w->tcn_pre = preshift;
     return CRCNN_OK;
 }
 
 // Weighted sum as the NTT-domain limb-split GEMM on the tensor cores: NTT-form inputs and outputs.
 int run_weighted_sum_tcn(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_plain *b, const int *d_index, int R,
                          int Npos, int Pimg, int m_first, int M, crcnn_tensor *out) {
+    const int Kpad = tcn_kpad(R), ncols = 2 * Npos, total = ctx->K * ctx->n;
+    const int variant = ctx->tcn_mode >= 2 ? ctx->tcn_mode - 1 : 0;
+    const bool want_pre = ctx->tcn_preshift && tcn_preshift_shape(R, ncols, M, variant) &&
+                          7 * tcn_w_bytes(7, (int)(w->count / R), Kpad, ctx->K, ctx->n) <= ctx->weight_cache_bytes;
     int rc = ensure_domain(ctx, in, 1);
     if (!rc) rc = ensure_form(ctx, b, PF_NTT_ADD);
-    if (!rc) rc = ensure_tcn_weights(ctx, w, R);
+    if (!rc) rc = ensure_tcn_weights(ctx, w, R, want_pre);
     if (rc) return rc;
     const size_t pw = poly_words(ctx);
-    const int Kpad = tcn_kpad(R), ncols = 2 * Npos, total = ctx->K * ctx->n;
     const size_t per_slot = tcn_x_bytes_per_slot(7, ncols, Kpad);
     long chunk = (long)(ctx->tc_scratch_bytes / per_slot) / 32 * 32;
     chunk = std::max<long>(32, std::min<long>(chunk, total));
@@ -496,7 +519,8 @@ int run_weighted_sum_tcn(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn
     a.Mall = (int)(w->count / R); a.m_first = m_first; a.M = M;
     a.R = R; a.Kpad = Kpad; a.planes = 7; a.ncols = ncols;
     a.Pimg = Pimg; a.Mtotal = M; a.m0 = 0; a.n = ctx->n; a.K = ctx->K;
-    a.variant = ctx->tcn_mode >= 2 ? ctx->tcn_mode - 1 : 0;
+    a.variant = variant;
+    a.preshift = want_pre && w->tcn_pre;
     a.use_fold = ctx->tcn_fold;
     for (int j = 0; j < ctx->K; j++) a.fold[j] = tcn_fold_make(ctx->hp.d.tab[j].mod.q);
     for (long s0 = 0; s0 < total && !rc; s0 += chunk) {
@@ -507,7 +531,7 @@ int run_weighted_sum_tcn(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn
         { ProfScope ps(ctx, KC_TCN_SPLIT, (double)ncols * R * ns * 8.0 + xbytes, 0); e = launch_tcn_split(s, ctx->stream); }
         if (e == cudaSuccess) {
             // ops: int8 multiply-accumulates of the unpadded problem (49 plane pairs per residue product)
-            ProfScope ps(ctx, KC_TCN_MAC, xbytes + (double)ns * 7 * M * Kpad + (double)ncols * M * ns * 8.0, (double)ns * ncols * M * R * 49.0);
+            ProfScope ps(ctx, KC_TCN_MAC, xbytes + (double)ns * 7 * M * Kpad * (a.preshift ? 7 : 1) + (double)ncols * M * ns * 8.0, (double)ns * ncols * M * R * 49.0);
             e = launch_tcn_mac(ctx->dP, a, ctx->sm_count, ctx->stream);
         }
         if (e != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, std::string("limb-split tensor-core weighted sum: ") + cudaGetErrorString(e));
@@ -622,6 +646,7 @@ int crcnn_ctx_create(int n, int K, const uint64_t *q, uint64_t t, int device, cr
     if (const char *e = getenv("CRCNN_TCN")) c->tcn_mode = atoi(e);
     if (const char *e = getenv("CRCNN_TAP")) c->tap_mode = atoi(e);
     if (const char *e = getenv("CRCNN_TCN_FOLD")) c->tcn_fold = atoi(e);
+    if (const char *e = getenv("CRCNN_TCN2_PRESHIFT")) c->tcn_preshift = atoi(e);
     if (const char *e = getenv("CRCNN_SQ_LEAN")) c->sq_lean = atoi(e);
     // stream-ordered allocator: keep freed blocks cached
     cudaMemPool_t pool;
@@ -1215,7 +1240,7 @@ static int compose_fc(crcnn_ctx *ctx, crcnn_plain *w1, crcnn_plain *b1, crcnn_pl
     if (rc) return done(rc);
     CU(cudaMemcpy2DAsync(B->ntt_add, pw * 8, O->d, 2 * pw * 8, pw * 8, out_dim, cudaMemcpyDeviceToDevice, ctx->stream));
     if (C) CU(launch_fold_fc_input_affine(ctx->dP, W->ntt_mul, out_dim, in_dim, (long)pw, per_channel, C, D, B->ntt_add, ctx->stream));
-    rc = ensure_tcn_weights(ctx, W, in_dim);      // byte planes of the composed weights; releases the dense form
+    rc = ensure_tcn_weights(ctx, W, in_dim, false);   // byte planes of the composed weights; releases the dense form
     if (rc) return done(rc);
     w1->folded_w = W; w1->folded_b = B;
     return done(CRCNN_OK);
@@ -1479,8 +1504,7 @@ int crcnn_conv_pool_bn_forward_shard(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_pla
         rc = ensure_form(ctx, w->folded_w, PF_NTT_MUL);
         if (rc) return rc;
         CU(launch_fold_affine(ctx->dP, w->folded_w->ntt_mul, (long)nf * R, (long)pw, R, invstd->fused_C, nullptr, ctx->stream));
-        rc = ensure_tcn_weights(ctx, w->folded_w, R);
-        if (rc) return rc;
+        // staged as byte planes by the first weighted sum below, which knows the shape (pre-shifted or not); it releases the dense form
         // B' : |window| * (Delta-scaled bias) in NTT form, times C[m], minus D[m]
         rc = make_plain(ctx, std::vector<uint32_t>(b->off), std::vector<uint32_t>(b->idx), std::vector<uint64_t>(b->val), &w->folded_b);
         if (rc) return rc;

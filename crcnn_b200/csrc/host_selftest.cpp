@@ -69,6 +69,50 @@ int main(int argc, char **argv) {
                 if (tcn_fold_reduce(s, bias, f, m.q) != want) { printf("FOLD MISMATCH\n"); return 1; }
             }
         }
+        // pre-shifted limb-split GEMM (tcn_mac.cu: tcn2p_mac_kernel): the byte planes of W' = W 2^(8b) mod q recombine to W' and give
+        // W X mod q through the seven classes; tcn7_fold_reduce and tcn7_combine against unsigned __int128, all-(q-1) operands at R = 4096
+        for (int j = 0; j < d.K; j++) {
+            const Mod &m = d.tab[j].mod;
+            const TcnFold f = tcn_fold_make(m.q);
+            long checked = 0;
+            for (int it = 0; it < 20000; it++) {
+                x = x * 6364136223846793005ULL + 1442695040888963407ULL;
+                y = y * 2862933555777941757ULL + 3037000493ULL;
+                const uint64_t W = it < 2 ? m.q - 1 : x % m.q, X = it < 2 ? m.q - 1 : y % m.q;
+                uint32_t C[7] = {0, 0, 0, 0, 0, 0, 0};
+                for (int b = 0; b < 7; b++) {
+                    const uint64_t wb = (uint64_t)(((unsigned __int128)1 << (8 * b)) % m.q);
+                    const uint64_t wbp = (uint64_t)(((unsigned __int128)wb << 64) / m.q);
+                    uint64_t Wb = mulshoup_lazy(W, wb, wbp, m.q);
+                    Wb = Wb >= m.q ? Wb - m.q : Wb;
+                    if (Wb != (uint64_t)(((unsigned __int128)W << (8 * b)) % m.q)) { printf("PRESHIFT MISMATCH\n"); return 1; }
+                    uint64_t back = 0;
+                    for (int a = 6; a >= 0; a--) back = (back << 8) | ((Wb >> (8 * a)) & 0xff);
+                    if (back != Wb) { printf("PLANE MISMATCH\n"); return 1; }
+                    for (int a = 0; a < 7; a++) C[a] += (uint32_t)(((X >> (8 * b)) & 0xff) * ((Wb >> (8 * a)) & 0xff));
+                }
+                const uint64_t bias = (it & 1) ? y % m.q : 0;
+                const uint64_t want = (uint64_t)(((unsigned __int128)W * X + bias) % m.q);
+                const U128 z = tcn7_combine(C);
+                if (addmod(barrett128(z, m), bias, m.q) != want) { printf("SEVEN-CLASS MISMATCH\n"); return 1; }
+                if (f.ok7 && tcn7_fold_reduce(C, bias, f, m.q) != want) { printf("FOLD7 MISMATCH\n"); return 1; }
+                checked++;
+            }
+            // largest class sums the kernel admits: every byte 0xff in all 7 x 4096 plane pairs of a class
+            const uint32_t cmax = 7u * 4096u * 255u * 255u;
+            for (int it = 0; it < 2000 && f.ok7; it++) {
+                uint32_t C[7];
+                x = x * 6364136223846793005ULL + 1442695040888963407ULL;
+                for (int a = 0; a < 7; a++) C[a] = it == 0 ? cmax : cmax - (uint32_t)((x >> (4 * a)) % 4096);
+                const uint64_t bias = it == 0 ? m.q - 1 : x % m.q;
+                unsigned __int128 z = 0;
+                for (int a = 6; a >= 0; a--) z = (z << 8) + C[a];
+                if (z >> 80) { printf("FOLD7 BOUND\n"); return 1; }
+                if (tcn7_fold_reduce(C, bias, f, m.q) != (uint64_t)((z + bias) % m.q)) { printf("FOLD7 MISMATCH\n"); return 1; }
+                checked++;
+            }
+            printf("fold7 %d ok7 %u checked %ld\n", j, f.ok7, checked);
+        }
         // three-fold reduction of arbitrary 128-bit values (modarith.cuh: reduce128_fold) for every modulus, against barrett128 and __int128
         for (int sidx = 0; sidx < d.K + d.S; sidx++) {
             const Mod &m = d.tab[sidx].mod;

@@ -226,7 +226,20 @@ struct TcnFold {
     uint32_t sh, mask;    // k - 32, 2^(k-32) - 1
     uint32_t c8, c16, c24;
     uint32_t ok;          // 0: this prime does not have the shape (the kernels then take the generic path)
+    uint32_t ok7;         // tcn7_fold_reduce is exact for this prime (seven-class sums of the pre-shifted GEMM)
 };
+
+// worst case of tcn7_fold_reduce (below) for q = 2^k - delta: every class sum 2^31 - 1, bias q - 1
+inline bool tcn7_fold_bound(uint64_t q, int k, uint64_t delta) {
+    typedef unsigned __int128 u128;
+    const u128 one = 1, cmax = 0x7fffffffu;
+    u128 z = 0;
+    for (int a = 6; a >= 0; a--) z = (z << 8) + cmax;
+    const u128 h = z >> k;
+    const u128 v = h * delta + ((one << k) - 1) + (q - 1);
+    if (h >> 32 || v >> 64) return false;
+    return (v >> k) * delta + ((one << k) - 1) < 2 * (u128)q;
+}
 
 // Worst-case magnitudes of every intermediate for S_w <= 2^31 - 1 and bias <= q - 1, checked numerically.
 inline TcnFold tcn_fold_make(uint64_t q) {
@@ -254,6 +267,7 @@ inline TcnFold tcn_fold_make(uint64_t q) {
     if (g * delta + ((one << k) - 1) >= 2 * (u128)q) return f;
     f.T = (uint32_t)T; f.delta = (uint32_t)delta; f.sh = (uint32_t)(k - 32); f.mask = (1u << (k - 32)) - 1;
     f.c8 = 1u << 8; f.c16 = 1u << 16; f.c24 = 1u << 24; f.ok = 1;
+    f.ok7 = tcn7_fold_bound(q, k, delta) ? 1 : 0;
     return f;
 }
 
@@ -293,6 +307,36 @@ CRCNN_HD uint64_t tcn_fold_reduce(const uint32_t (&s)[13], uint64_t bias, const 
     const uint64_t lo = ((uint64_t)(V1 & f.mask) << 32) | (uint32_t)v;
     const uint64_t r = (uint64_t)g * f.delta + lo;
     return r >= q ? r - q : r;
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// Reduction of the SEVEN accumulator classes of the pre-shifted limb-split GEMM (tcn_mac.cuh: the weights are staged as
+// W'_b = W 2^(8b) mod q, so every product lands in class a = weight byte and z = sum_a C_a 2^(8a)).  C_a < 2^31 gives
+// z < 2^80 = 2^(48+32): for 48 <= k <= 56 the bits above k are ONE word h, and two folds through delta (the bias joins the
+// first) leave r < 2q.  tcn_fold_make checks the worst case per prime (TcnFold::ok7); the result is canonical, so it equals
+// (z + bias) mod q bit for bit (host_selftest.cpp checks it against unsigned __int128).
+// C[a] = class sum of weight byte a (< 2^31), bias < q (0 when there is none)
+CRCNN_HD uint64_t tcn7_fold_reduce(const uint32_t (&C)[7], uint64_t bias, const TcnFold &f, uint64_t q) {
+    const uint64_t La = (uint64_t)C[3] * f.c24 + ((uint64_t)C[2] * f.c16 + ((uint64_t)C[1] * f.c8 + C[0]));   // weight 2^0, < 2^56
+    const uint64_t Lb = (uint64_t)C[6] * f.c16 + ((uint64_t)C[5] * f.c8 + C[4]);                             // weight 2^32, < 2^48
+    const uint64_t m1 = (La >> 32) + (uint32_t)Lb;
+    const uint32_t y0 = (uint32_t)La, y1 = (uint32_t)m1, y2 = (uint32_t)(Lb >> 32) + (uint32_t)(m1 >> 32);
+    const uint32_t h = tcn_shr64(y1, y2, f.sh);                                   // z >> k: one word since z < 2^(k+32)
+    const uint64_t v = (uint64_t)h * f.delta + ((((uint64_t)(y1 & f.mask)) << 32) | y0) + bias;
+    const uint32_t vh = (uint32_t)(v >> 32);
+    const uint64_t r = (uint64_t)(vh >> f.sh) * f.delta + ((((uint64_t)(vh & f.mask)) << 32) | (uint32_t)v);
+    return r >= q ? r - q : r;
+}
+
+// The same 80-bit value as a U128, for the generic (Barrett) reduction
+CRCNN_HD U128 tcn7_combine(const uint32_t (&C)[7]) {
+    const uint64_t La = ((uint64_t)C[3] << 24) + (((uint64_t)C[2] << 16) + (((uint64_t)C[1] << 8) + C[0]));
+    const uint64_t Lb = ((uint64_t)C[6] << 16) + (((uint64_t)C[5] << 8) + C[4]);
+    const uint64_t m1 = (La >> 32) + (uint32_t)Lb;
+    U128 z;
+    z.lo = (m1 << 32) | (uint32_t)La;
+    z.hi = (Lb >> 32) + (m1 >> 32);
+    return z;
 }
 
 // ------------------------------------------------------------------------------------------------------------

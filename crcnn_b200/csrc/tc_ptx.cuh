@@ -57,6 +57,12 @@ __device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap *map
         "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
         : "memory");
 }
+__device__ __forceinline__ void tma_load_5d(uint32_t dst, const CUtensorMap *map, uint32_t bar, int c0, int c1, int c2, int c3, int c4) {
+    asm volatile(
+        "cp.async.bulk.tensor.5d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], [%2];" ::"r"(dst),
+        "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
+        : "memory");
+}
 __device__ __forceinline__ void prefetch_tmap(const CUtensorMap *map) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory");
 }

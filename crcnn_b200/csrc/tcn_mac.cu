@@ -1,6 +1,7 @@
 // NTT-domain limb-split weighted sum on tcgen05 kind::i8 (see tcn_mac.cuh for the algorithm and the exactness argument).
 #include <cuda.h>
 #include <cuda_runtime.h>
+#include <algorithm>
 #include <cstdio>
 #include <cstdlib>
 #include "devcfg.cuh"
@@ -489,6 +490,221 @@ tcn2_mac_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__
     if (warp == 0) tmem_dealloc(tmem_base, TCN_TMEM_COLS);
 }
 
+// ------------------------------------------------------------------------------------ the column-major GEMM on pre-shifted weights
+// The weights are staged as W'_b = W 2^(8b) mod q_j for b = 0..6, each split into its 7 byte planes W'_(b,a).  Then
+//       W X = sum_b X_b W'_b = sum_a 2^(8a) C_a  (mod q_j),      C_a = sum_b sum_r Xb[col][r] W'_(b,a)[m][r],
+// SEVEN classes instead of 13 (C_a <= 7 R 255^2 < 2^31 as before; the recombined value is < 2^80).  Input plane b is
+// multiplied against the 7 stacked planes of W'_b (N = 224) into the SAME 224 accumulator columns for every b: no
+// column shift, no special first step, and two accumulators fit TMEM (2 x 224 of 512 columns), so the epilogue of one
+// (chunk, slot) runs while the MMAs of the next one are issued.  Fan-in <= 32 (one 32-byte K block: conv1) and four
+// consecutive slots per item, as tcn2_mac_kernel<32, ., 1, 4, .>: the pre-shifted planes of the four slots stay resident
+// (4 x 49 KB), which leaves no shared memory for output staging -- instead each epilogue thread keeps the results of
+// slots 0-2 in registers and slot 3 writes all four as one 32-byte sector (STAGED, layers of at most 24 outputs).
+constexpr int TCN2P_NS = 4;
+constexpr int TCN2P_WB = TCN_PLANES * TCN2_MT * 32;           // one b block [a][32 outputs][32 bytes]
+constexpr int TCN2P_WSLOT = TCN_PLANES * TCN2P_WB;            // [b][a][32][32] of one slot
+constexpr int TCN2P_X = TCN2_CB * 32;                         // one input plane tile [128][32]
+constexpr int TCN2P_STAGES = 7;
+constexpr int TCN2P_ACC = TCN_PLANES * TCN2_MT;               // 224 columns per accumulator
+// groups of 4 outputs per epilogue warp: 3 cover a 32-output tile; the STAGED kernel keeps 2 x 4 x 3 results in registers and
+// takes tiles of at most 24 outputs (3 groups would need more registers than 448 threads can have)
+template <bool STAGED> __host__ __device__ constexpr int tcn2p_gpw() { return STAGED ? 2 : (TCN2_MT / 4 + TCN2_EPI_WARPS / 4 - 1) / (TCN2_EPI_WARPS / 4); }
+constexpr int TCN2P_STAGED_MAX_M = 4 * 2 * (TCN2_EPI_WARPS / 4);
+constexpr size_t TCN2P_SMEM = 1024 + (size_t)TCN2P_NS * TCN2P_WSLOT + (size_t)TCN2P_STAGES * TCN2P_X + 8 * (2 * TCN2P_STAGES + 6) + 16;
+
+template <bool FOLD, bool STAGED>
+__global__ void __launch_bounds__(TCN2_THREADS, 1)
+tcn2p_mac_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmX,
+                 const DeviceParams *__restrict__ P, TcnMacArgs a) {
+    constexpr int NS = TCN2P_NS, STAGES = TCN2P_STAGES, GPW = tcn2p_gpw<STAGED>();
+    constexpr uint32_t ID = (2u << 4) | ((uint32_t)(TCN2_CB >> 4) << 24) | ((uint32_t)(TCN2P_ACC >> 3) << 17);   // S32, u8 x u8, M 128, N 224
+
+    extern __shared__ uint8_t smem_raw[];
+    const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
+    uint8_t *base_ptr = smem_raw + (base - smem_u32(smem_raw));
+    const uint32_t sW = base, sX = base + NS * TCN2P_WSLOT;
+    const uint32_t off_bar = NS * TCN2P_WSLOT + STAGES * TCN2P_X;
+    const uint32_t bar_full = base + off_bar, bar_empty = bar_full + 8 * STAGES;
+    const uint32_t bar_wfull = bar_empty + 8 * STAGES, bar_wempty = bar_wfull + 8;
+    const uint32_t bar_tfull = bar_wempty + 8, bar_tempty = bar_tfull + 16;   // one pair per accumulator
+    const uint32_t tmem_slot = bar_tempty + 16;
+    volatile uint32_t *tmem_slot_ptr = reinterpret_cast<volatile uint32_t *>(base_ptr + off_bar + 8 * (2 * STAGES + 6));
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int n = a.n;
+    const int m_tiles = (a.M + TCN2_MT - 1) / TCN2_MT;
+    const long groups = a.nslots / NS;
+    const long items = (groups > blockIdx.x ? (groups - blockIdx.x + gridDim.x - 1) / gridDim.x : 0) * m_tiles;   // items of THIS CTA
+    auto item_group = [&](long it) { return (long)blockIdx.x + (it / m_tiles) * gridDim.x; };
+    const int chunks = (a.ncols + TCN2_CB - 1) / TCN2_CB;
+
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < STAGES; s++) { mbar_init(bar_full + 8 * s, 1); mbar_init(bar_empty + 8 * s, 1); }
+        mbar_init(bar_wfull, 1);
+        mbar_init(bar_wempty, 1);
+        for (int b = 0; b < 2; b++) { mbar_init(bar_tfull + 8 * b, 1); mbar_init(bar_tempty + 8 * b, TCN2_EPI_WARPS); }
+        fence_barrier_init();
+        prefetch_tmap(&tmW);
+        prefetch_tmap(&tmX);
+    }
+    if (warp == 0) tmem_alloc(tmem_slot, TCN_TMEM_COLS);
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem_base = *tmem_slot_ptr;
+
+    if (warp == 0) {
+        // ===================================================================== TMA producer
+        if (lane == 0) {
+            int stage = 0;
+            uint32_t phase = 0, wphase = 0;
+            for (long item = 0; item < items; item++) {
+                const int sl = (int)item_group(item) * NS, mt = (int)(item % m_tiles);
+                mbar_wait(bar_wempty, wphase ^ 1);
+                mbar_expect_tx(bar_wfull, NS * TCN2P_WSLOT);
+                for (int s = 0; s < NS; s++) tma_load_5d(sW + s * TCN2P_WSLOT, &tmW, bar_wfull, 0, mt * TCN2_MT, 0, a.slot0 + sl + s, 0);
+                wphase ^= 1;
+                for (int ch = 0; ch < chunks; ch++)
+                    for (int s = 0; s < NS; s++)
+                        for (int b = 0; b < TCN_PLANES; b++) {
+                            mbar_wait(bar_empty + 8 * stage, phase ^ 1);
+                            TCN2_TR(0, b);                          // stage free: load of plane b issued now
+                            mbar_expect_tx(bar_full + 8 * stage, TCN2P_X);
+                            tma_load_4d(sX + stage * TCN2P_X, &tmX, bar_full + 8 * stage, 0, ch * TCN2_CB, b, sl + s);
+                            if (++stage == STAGES) { stage = 0; phase ^= 1; }
+                        }
+            }
+        }
+        __syncwarp();
+    } else if (warp == 1) {
+        // ===================================================================== MMA issuer
+        if (lane == 0) {
+            int stage = 0;
+            uint32_t phase = 0, wphase = 0, use = 0;   // use: accumulator fills so far; buffer use & 1, its phase (use >> 1) & 1
+            for (long item = 0; item < items; item++) {
+                mbar_wait(bar_wfull, wphase);
+                wphase ^= 1;
+                tc_fence_after();
+                for (int chs = 0; chs < chunks * NS; chs++, use++) {   // (chunk, slot of the item), slot fastest
+                    const int s = chs % NS;
+                    const uint32_t buf = use & 1;
+                    TCN2_TR(1, 100);                                // waiting for the accumulator
+                    mbar_wait(bar_tempty + 8 * buf, ((use >> 1) & 1) ^ 1);
+                    TCN2_TR(1, 101);                                // accumulator free
+                    tc_fence_after();
+                    const uint32_t acc = tmem_base + buf * TCN2P_ACC;
+                    for (int b = 0; b < TCN_PLANES; b++) {
+                        mbar_wait(bar_full + 8 * stage, phase);
+                        TCN2_TR(1, b);                              // plane tile arrived
+                        tc_fence_after();
+                        // D[column, (a, output)] += X_b[column] . W'_(b,a)[output]
+                        umma_i8(acc, umma_desc_sw32(sX + stage * TCN2P_X), umma_desc_sw32(sW + s * TCN2P_WSLOT + b * TCN2P_WB), ID, b ? 1u : 0u);
+                        umma_commit(bar_empty + 8 * stage);
+                        if (++stage == STAGES) { stage = 0; phase ^= 1; }
+                    }
+                    umma_commit(bar_tfull + 8 * buf);
+                    TCN2_TR(1, 102);                                // all MMAs of the chunk issued
+                }
+                umma_commit(bar_wempty);   // every MMA that reads this item's weights has been issued before this commit
+            }
+        }
+        __syncwarp();
+    } else {
+        // ===================================================================== epilogue
+        // TMEM lane = column of the chunk; a warp owns lane quadrant warp % 4, the three warps of a quadrant take the tile's
+        // groups of 4 outputs round robin (at most GPW each)
+        const int qd = warp & 3, sub = (warp - 2) >> 2;
+        const long pw = (long)a.K * n;
+        const long m_stride = 2L * a.Pimg * pw;      // words between consecutive outputs of one column
+        uint32_t use = 0;
+        for (long item = 0; item < items; item++) {
+            const int sl = (int)item_group(item) * NS, mt = (int)(item % m_tiles);
+            const int slot = a.slot0 + sl, j = slot / n, c = slot - j * n;   // first slot of the item; its NS slots share the limb j
+            const Mod mod = P->tab[j].mod;
+            const TcnFold fold = a.fold[FOLD ? j : 0];
+            const long slot_off = (long)j * n + c;
+            const int m_valid = min(TCN2_MT, a.M - mt * TCN2_MT);
+            const int groups = (m_valid + 3) >> 2;
+            // lane m holds the bias residues of output m of this item; the loop broadcasts them by shuffle
+            uint64_t bias_lane[NS];
+#pragma unroll
+            for (int s = 0; s < NS; s++)
+                bias_lane[s] = (a.bias && lane < m_valid) ? __ldg(a.bias + (long)(mt * TCN2_MT + lane) * pw + slot_off + s) : 0;
+            for (int ch = 0; ch < chunks; ch++) {
+                const int col = ch * TCN2_CB + qd * 32 + lane;
+                const bool valid = col < a.ncols;
+                const int p = col >> 1, poly = col & 1;
+                const long colbase = (long)(p / a.Pimg) * ((long)a.Mtotal * a.Pimg) + p % a.Pimg;
+                uint64_t *out_col = a.out + (colbase * 2 + poly) * pw + slot_off + (long)(a.m0 + mt * TCN2_MT) * m_stride;
+                const bool add_bias = poly == 0 && a.bias != nullptr;
+                uint64_t keep[GPW][4][NS - 1];    // STAGED: results of slots 0 .. NS-2 until slot NS-1 completes the sector
+#pragma unroll
+                for (int s = 0; s < NS; s++, use++) {   // slot sl + s of the item: residue position c + s
+                    const uint32_t buf = use & 1;
+                    if (warp == 2 && lane == 0) TCN2_TR(2, 200);    // waiting for the accumulator
+                    mbar_wait(bar_tfull + 8 * buf, (use >> 1) & 1);
+                    if (warp == 2 && lane == 0) TCN2_TR(2, 201);    // accumulator complete
+                    tc_fence_after();
+#pragma unroll
+                    for (int gi = 0; gi < GPW; gi++) {
+                        const int g = sub + gi * (TCN2_EPI_WARPS / 4);
+                        if (g >= groups) break;                   // warp uniform
+                        const int mloc = g * 4;
+                        uint32_t C[TCN_PLANES][4];
+#pragma unroll
+                        for (int w = 0; w < TCN_PLANES; w++)
+                            tmem_ld4(tmem_base + ((uint32_t)(qd * 32) << 16) + buf * TCN2P_ACC + w * TCN2_MT + mloc, C[w]);
+                        tmem_ld_wait();
+                        uint64_t *op = out_col + (long)mloc * m_stride + s;
+#pragma unroll
+                        for (int i = 0; i < 4; i++) {
+                            if (mloc + i < m_valid) {                // warp uniform
+                                const uint64_t bias_m = __shfl_sync(0xffffffffu, bias_lane[s], mloc + i);
+                                uint32_t Ci[TCN_PLANES];
+#pragma unroll
+                                for (int w = 0; w < TCN_PLANES; w++) Ci[w] = C[w][i];
+                                uint64_t r;
+                                if constexpr (FOLD) {
+                                    r = tcn7_fold_reduce(Ci, add_bias ? bias_m : 0, fold, mod.q);
+                                } else {
+                                    r = barrett128(tcn7_combine(Ci), mod);
+                                    if (add_bias) r = addmod(r, bias_m, mod.q);
+                                }
+                                if constexpr (STAGED) {
+                                    if (s < NS - 1) keep[gi][i][s < NS - 1 ? s : 0] = r;
+                                    else if (valid) tcn_store_sector(op - (NS - 1), keep[gi][i][0], keep[gi][i][1], keep[gi][i][2], r);
+                                } else if (valid) {
+                                    *op = r;
+                                }
+                            }
+                            op += m_stride;
+                        }
+                    }
+                    tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive(bar_tempty + 8 * buf);
+                    if (warp == 2 && lane == 0) TCN2_TR(2, 202);    // this warp's share of the chunk recombined and stored
+                }
+            }
+        }
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 0) tmem_dealloc(tmem_base, TCN_TMEM_COLS);
+}
+
+// W'_b = W 2^(8b) mod q_j (Shoup product by a per-limb constant), b = 1..6, for the pre-shifted staging
+struct TcnShift { uint64_t q[MAXK], w[MAXK], wp[MAXK]; };   // per limb: q_j, 2^(8b) mod q_j, floor(w 2^64 / q_j)
+__global__ void tcn_preshift_kernel(const uint64_t *__restrict__ src, uint64_t *__restrict__ dst, long words, int n, int K, TcnShift c) {
+    const long pw = (long)K * n;
+    for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < words; i += (long)gridDim.x * blockDim.x) {
+        const int j = (int)((i % pw) / n);
+        const uint64_t q = c.q[j];
+        const uint64_t r = mulshoup_lazy(__ldg(src + i), c.w[j], c.wp[j], q);
+        dst[i] = r >= q ? r - q : r;
+    }
+}
+
 // ------------------------------------------------------------------------------------ operand staging
 // dst[slot - slot0][l][col][r] = byte l of src item (col group, r), polynomial col % item_polys, residue of `slot`.
 // One CTA: 32 consecutive slots x 128 consecutive (column, term) bytes of a plane row -- one column x 128 terms, or
@@ -622,7 +838,61 @@ cudaError_t launch_tcn2_mac_t(const DeviceParams *P, const TcnMacArgs &a, int sm
     return cudaGetLastError();
 }
 
+template <bool FOLD, bool STAGED>
+cudaError_t launch_tcn2p_mac_t(const DeviceParams *P, const TcnMacArgs &a, int sm_count, cudaStream_t stream) {
+    EncodeTiledFn enc = encode_tiled();
+    if (!enc) return cudaErrorNotSupported;
+    CUtensorMap tmW, tmX;
+    {
+        // pre-shifted planes [b][K*n][a][Mall][Kpad]; one box = the 49 planes of 32 outputs of one slot, landing as [b][a][m][32]
+        const cuuint64_t rowsW = (cuuint64_t)a.Mall * a.Kpad, slotW = rowsW * TCN_PLANES;
+        cuuint64_t dims[5] = {(cuuint64_t)a.Kpad, (cuuint64_t)a.M, (cuuint64_t)TCN_PLANES, (cuuint64_t)a.K * a.n, (cuuint64_t)TCN_PLANES};
+        cuuint64_t strides[4] = {(cuuint64_t)a.Kpad, rowsW, slotW, slotW * a.K * a.n};
+        cuuint32_t box[5] = {32, TCN2_MT, TCN_PLANES, 1, TCN_PLANES}, es[5] = {1, 1, 1, 1, 1};
+        if (enc(&tmW, CU_TENSOR_MAP_DATA_TYPE_UINT8, 5, (void *)(a.W + (size_t)a.m_first * a.Kpad), dims, strides, box, es,
+                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+            return cudaErrorInvalidValue;
+    }
+    {
+        const cuuint64_t rowsX = (cuuint64_t)a.ncols * a.Kpad;
+        cuuint64_t dims[4] = {(cuuint64_t)a.Kpad, (cuuint64_t)a.ncols, (cuuint64_t)TCN_PLANES, (cuuint64_t)a.nslots};
+        cuuint64_t strides[3] = {(cuuint64_t)a.Kpad, rowsX, rowsX * TCN_PLANES};
+        cuuint32_t box[4] = {32, TCN2_CB, 1, 1}, es[4] = {1, 1, 1, 1};
+        if (enc(&tmX, CU_TENSOR_MAP_DATA_TYPE_UINT8, 4, (void *)a.X, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_32B,
+                CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+            return cudaErrorInvalidValue;
+    }
+    auto k = tcn2p_mac_kernel<FOLD, STAGED>;
+    static DeviceOnce once;
+    if (once.first()) {
+        cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TCN2P_SMEM);
+        if (e != cudaSuccess) return e;
+    }
+    const long groups = a.nslots / TCN2P_NS;
+    const unsigned grid = (unsigned)(groups < sm_count ? groups : sm_count);
+    k<<<grid, TCN2_THREADS, TCN2P_SMEM, stream>>>(tmW, tmX, P, a);
+    return cudaGetLastError();
+}
+
 }  // namespace
+
+bool tcn_preshift_shape(int R, int ncols, int M, int variant) {
+    return R >= 1 && R <= 32 && variant != 1 && (variant == 2 || ncols >= 4 * M);
+}
+
+cudaError_t launch_tcn_preshift(const uint64_t *q, const uint64_t *src, uint64_t *dst, long words, int b, int n, int K, cudaStream_t stream) {
+    if (words <= 0) return cudaSuccess;
+    if (b < 1 || b >= TCN_PLANES || K > MAXK) return cudaErrorInvalidValue;
+    TcnShift c{};
+    for (int j = 0; j < K; j++) {
+        c.q[j] = q[j];
+        c.w[j] = (uint64_t)(((unsigned __int128)1 << (8 * b)) % q[j]);
+        c.wp[j] = (uint64_t)(((unsigned __int128)c.w[j] << 64) / q[j]);
+    }
+    const long blocks = std::min<long>((words + 255) / 256, 148L * 16);
+    tcn_preshift_kernel<<<(unsigned)blocks, 256, 0, stream>>>(src, dst, words, n, K, c);
+    return cudaGetLastError();
+}
 
 size_t tcn_x_bytes_per_slot(int planes, int ncols, int Kpad) { return (size_t)planes * ncols * Kpad; }
 size_t tcn_w_bytes(int planes, int Mall, int Kpad, int K, int n) { return (size_t)K * n * planes * Mall * Kpad; }
@@ -655,8 +925,18 @@ cudaError_t launch_tcn_mac(const DeviceParams *P, const TcnMacArgs &a, int sm_co
     // the four-slot kernel with 8-byte stores (A/B runs; same bytes).
     static const int ns_env = [] { const char *e = getenv("CRCNN_TCN2_NS"); return e ? atoi(e) : 4; }();
     static const int stage_env = [] { const char *e = getenv("CRCNN_TCN2_STAGE"); return e ? atoi(e) : 1; }();
+    // Pre-shifted weights (a.preshift, staged by the caller for tcn_preshift_shape): seven accumulator classes, double-buffered
+    // accumulator, four slots per item; CRCNN_TCN2_STAGE=0 gives 8-byte stores here too
+    if (a.preshift) {
+        if (!tcn_preshift_shape(a.R, a.ncols, a.M, forced) || a.nslots % TCN2P_NS || a.slot0 % TCN2P_NS || a.n % TCN2P_NS) return cudaErrorInvalidValue;
+        bool fold7 = a.use_fold != 0;
+        for (int j = 0; j < a.K && fold7; j++) fold7 = a.fold[j].ok7 != 0;
+        if (stage_env && a.M <= TCN2P_STAGED_MAX_M && (reinterpret_cast<uintptr_t>(a.out) & 31) == 0)
+            return fold7 ? launch_tcn2p_mac_t<true, true>(P, a, sm_count, stream) : launch_tcn2p_mac_t<false, true>(P, a, sm_count, stream);
+        return fold7 ? launch_tcn2p_mac_t<true, false>(P, a, sm_count, stream) : launch_tcn2p_mac_t<false, false>(P, a, sm_count, stream);
+    }
     if (use2 && ns_env == 4 && bk == 32 && a.nslots % 4 == 0 && a.slot0 % 4 == 0 && a.n % 4 == 0) {
-        if (stage_env && (reinterpret_cast<uintptr_t>(a.out) & 31) == 0)
+        if (stage_env && a.M <= TCN2P_STAGED_MAX_M && (reinterpret_cast<uintptr_t>(a.out) & 31) == 0)
             return fold ? launch_tcn2_mac_t<32, true, 1, 4, true>(P, a, sm_count, stream) : launch_tcn2_mac_t<32, false, 1, 4, true>(P, a, sm_count, stream);
         return fold ? launch_tcn2_mac_t<32, true, 1, 4>(P, a, sm_count, stream) : launch_tcn2_mac_t<32, false, 1, 4>(P, a, sm_count, stream);
     }

@@ -72,11 +72,17 @@ struct TcnMacArgs {
     int use_fold;          // 1: reduce the class sums with tcn_fold_reduce when fold[j].ok for every prime (0: 128-bit recombination + Barrett)
     TcnFold fold[MAXK];    // per coefficient prime (modarith.cuh: tcn_fold_make)
     int variant;           // 0: pick by shape; 1: outputs on the UMMA rows (64 x 32 tiles); 2: columns on the UMMA rows (128 x 32 tiles, fan-in <= 256)
+    int preshift;          // 1: W holds the pre-shifted planes [7 (b)][K*n][planes][Mall][Kpad] (W 2^(8b) mod q_j; block b = 0 is the
+                           //    plain staging) and the shape is tcn_preshift_shape: seven-class kernel.  0: 13-class kernels on block 0
 };
 
 size_t tcn_x_bytes_per_slot(int planes, int ncols, int Kpad);
 size_t tcn_w_bytes(int planes, int Mall, int Kpad, int K, int n);
 cudaError_t launch_tcn_split(const TcnSplitArgs &a, cudaStream_t stream);
+// shapes that run on pre-shifted weights: fan-in <= 32 on the column-major kernel (variant as in TcnMacArgs)
+bool tcn_preshift_shape(int R, int ncols, int M, int variant);
+// dst = src 2^(8b) mod q_j for every residue of `words` limb-major words ([..][K][n]); q = the K primes (host array), 1 <= b <= 6
+cudaError_t launch_tcn_preshift(const uint64_t *q, const uint64_t *src, uint64_t *dst, long words, int b, int n, int K, cudaStream_t stream);
 cudaError_t launch_tcn_mac(const DeviceParams *P, const TcnMacArgs &a, int sm_count, cudaStream_t stream);
 
 }  // namespace crcnn
