@@ -21,8 +21,11 @@ std::unique_ptr<BatchServer> g_srv;
 std::unique_ptr<DeviceTensor> g_x0;   // resident input of crcnn_host_resident_*
 int g_zd = 0, g_xd = 0, g_yd = 0, g_outputs = 0, g_batch = 0;
 
+int g_oob_layer = -1;                 // layer of the last OutOfBudgetException
+
 template <class F> int guarded(F &&f) {
     try { f(); return 0; }
+    catch (const OutOfBudgetException &e) { g_err = e.what(); g_oob_layer = e.last_layer_computed; return CRCNN_ERR_OUT_OF_BUDGET; }
     catch (const std::invalid_argument &e) { g_err = e.what(); return CRCNN_ERR_INVALID_ARGUMENT; }
     catch (const std::exception &e) { g_err = e.what(); return CRCNN_ERR_CUDA; }
 }
@@ -164,6 +167,53 @@ int crcnn_host_set_fusion(int on) {
         if (!g_net) throw std::invalid_argument("no network built");
         g_net->fuse_fc_fc = g_net->fuse_conv_pool_bn = g_net->fuse_pool_bn = on != 0;
     });
+}
+
+// The key holder's keys for the built network (Network::use_device_keys; with device_reencryption, use_device_reencryption with
+// `seed`): secret_key_ntt [K][n+1], public_key_ntt [2][K][n+1] words, NTT form, as SEAL keeps them.
+int crcnn_host_use_keys(const uint64_t *secret_key_ntt, const uint64_t *public_key_ntt, int device_reencryption, uint64_t seed) {
+    return guarded([&] {
+        if (!g_net) throw std::invalid_argument("no network built");
+        if (!secret_key_ntt || !public_key_ntt) throw std::invalid_argument("null key");
+        g_net->reencrypt_dev = nullptr;
+        if (device_reencryption) g_net->use_device_reencryption(secret_key_ntt, public_key_ntt, seed);
+        else g_net->use_device_keys(secret_key_ntt, public_key_ntt);
+    });
+}
+// Network::reencrypt_below_budget (-1: the fixed re-encryption point; >= 0: budget-driven re-encryption)
+int crcnn_host_set_budget_threshold(int threshold) {
+    return guarded([&] {
+        if (!g_net) throw std::invalid_argument("no network built");
+        g_net->reencrypt_below_budget = threshold;
+    });
+}
+// Network::forward_dev_adaptive on `batch` images given as host words [batch][zd][xd][yd] ciphertexts; output as in
+// crcnn_host_forward_range.  An OutOfBudgetException returns CRCNN_ERR_OUT_OF_BUDGET with its layer in *failed_layer (may be null).
+int crcnn_host_forward_adaptive(const uint64_t *in_words, int batch, uint64_t *out_words, long out_cap, int *out_shape, int *failed_layer) {
+    g_oob_layer = -1;
+    const int rc = guarded([&] {
+        if (!g_net) throw std::invalid_argument("no network built");
+        Runtime &rt = Runtime::get();
+        crcnn_tensor *t = nullptr;
+        rt.check(crcnn_tensor_upload(rt.ctx(), in_words, (long)batch * g_zd * g_xd * g_yd, 2, &t));
+        DeviceTensor y = g_net->forward_dev_adaptive(DeviceTensor(t, g_zd, g_xd, g_yd, batch));
+        if ((long)y.count() * (long)rt.ct_words(2) > out_cap) throw std::invalid_argument("output buffer too small");
+        rt.check(crcnn_tensor_download(rt.ctx(), y.t, out_words));
+        out_shape[0] = y.zd; out_shape[1] = y.xd; out_shape[2] = y.yd;
+    });
+    if (failed_layer) *failed_layer = g_oob_layer;
+    return rc;
+}
+// Network::budget_log of the last adaptive forward: (layer, minimum budget, re-encrypted) per check; returns how many there are.
+int crcnn_host_budget_log(int *layer, int *min_budget, int *reencrypted, int cap) {
+    if (!g_net) return 0;
+    const int n = (int)g_net->budget_log.size();
+    for (int i = 0; i < n && i < cap; i++) {
+        layer[i] = g_net->budget_log[i].layer;
+        min_budget[i] = g_net->budget_log[i].min_budget;
+        reencrypted[i] = g_net->budget_log[i].reencrypted ? 1 : 0;
+    }
+    return n;
 }
 
 // Host-clock completion time (ms since the start of the last crcnn_host_serve) of each of its requests; returns how many there are.

@@ -94,6 +94,7 @@ struct crcnn_keys {
     uint64_t *sk = nullptr;   // [K][n]    secret key, NTT form
     uint64_t *pk = nullptr;   // [2][K][n] public key, NTT form
     ReencConsts c;
+    BudgetConsts b;
 };
 
 struct crcnn_ctx {
@@ -2098,6 +2099,7 @@ int crcnn_keys_upload(crcnn_ctx *ctx, const uint64_t *secret_key_ntt, const uint
     CU(cudaSetDevice(ctx->device));
     auto *k = new crcnn_keys;
     k->c = make_reenc_consts(ctx->hp.d);
+    k->b = make_budget_consts(ctx->hp.d);
     const size_t pw = poly_words(ctx);
     int rc = dev_alloc(ctx, pw * 8, (void **)&k->sk);
     if (!rc) rc = dev_alloc(ctx, 2 * pw * 8, (void **)&k->pk);
@@ -2119,11 +2121,11 @@ int crcnn_keys_free(crcnn_ctx *ctx, crcnn_keys *k) {
 }
 
 namespace {
-// plaintext polynomials [count][n] of ciphertexts [first, first+count) of t (Decryptor::decrypt); scratch = count*K*n words
-int decrypt_range(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, long first, long count, uint64_t *scratch, uint64_t *plain) {
-    const size_t n = ctx->n, pw = poly_words(ctx);
+// c0 + c1 s of ciphertexts [first, first+count) of t into scratch (count*K*n words), coefficient form -- except that for a
+// coefficient-form t the "+ c0" is left to the consumer, which gets *c0 = the ciphertexts (null when c0 is already in scratch)
+int dec_dot_range(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, long first, long count, uint64_t *scratch, const uint64_t **c0) {
+    const size_t pw = poly_words(ctx);
     const uint64_t *ct = t->d + first * 2 * pw;
-    ProfScope ps(ctx, KC_REENC, lp_bytes(ctx, (double)count * 2 * ctx->K) + (double)count * n * 8, lp_bfly(ctx, (double)count * 2 * ctx->K));
     if (!t->ntt) {
         // copy the c1 polynomials and transform them (decryptor.cpp:153-158)
         CU(cudaMemcpy2DAsync(scratch, pw * 8, ct + pw, 2 * pw * 8, pw * 8, count, cudaMemcpyDeviceToDevice, ctx->stream));
@@ -2131,7 +2133,27 @@ int decrypt_range(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, long first, lo
     }
     CU(launch_dec_dot(k->c, ct, t->ntt, k->sk, scratch, count, ctx->stream));
     CU(launch_ntt(ctx->dP, ctx->logn, scratch, count * ctx->K, 0, ctx->K, true, ctx->stream));
-    CU(launch_dec_scale(k->c, t->ntt ? nullptr : ct, scratch, plain, count, ctx->stream));
+    *c0 = t->ntt ? nullptr : ct;
+    return CRCNN_OK;
+}
+
+// plaintext polynomials [count][n] of ciphertexts [first, first+count) of t (Decryptor::decrypt); scratch = count*K*n words
+int decrypt_range(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, long first, long count, uint64_t *scratch, uint64_t *plain) {
+    ProfScope ps(ctx, KC_REENC, lp_bytes(ctx, (double)count * 2 * ctx->K) + (double)count * ctx->n * 8, lp_bfly(ctx, (double)count * 2 * ctx->K));
+    const uint64_t *c0 = nullptr;
+    int rc = dec_dot_range(ctx, k, t, first, count, scratch, &c0);
+    if (rc) return rc;
+    CU(launch_dec_scale(k->c, c0, scratch, plain, count, ctx->stream));
+    return CRCNN_OK;
+}
+
+// noise bit lengths of ciphertexts [first, first+count) of t, atomically maximised into bits[count] (Decryptor::invariant_noise_budget)
+int noise_bits_range(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, long first, long count, uint64_t *scratch, int *bits) {
+    ProfScope ps(ctx, KC_REENC, lp_bytes(ctx, (double)count * 2 * ctx->K) + (double)count * 4, lp_bfly(ctx, (double)count * 2 * ctx->K));
+    const uint64_t *c0 = nullptr;
+    int rc = dec_dot_range(ctx, k, t, first, count, scratch, &c0);
+    if (rc) return rc;
+    CU(launch_noise_bits(k->b, c0, scratch, bits, count, ctx->stream));
     return CRCNN_OK;
 }
 }  // namespace
@@ -2158,6 +2180,40 @@ int crcnn_decrypt(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, uint64_t *host
     }
     dev_free(ctx, scratch); dev_free(ctx, plain);
     return rc;
+}
+
+int crcnn_noise_budget(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, int *host_budgets, int *min_budget) {
+    if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
+    REQUIRE(k && t, "null argument");
+    REQUIRE(t->size == 2, "the noise budget is implemented for size-2 ciphertexts");
+    REQUIRE(t->count > 0, "empty tensor");
+    CU(cudaSetDevice(ctx->device));
+    const size_t n = ctx->n;
+    const long step = std::max<long>(1, std::min<long>(t->count, (long)((1ull << 30) / ((size_t)(ctx->K + 1) * n * 8))));   // crcnn_decrypt's chunks
+    uint64_t *scratch = nullptr;
+    int *bits = nullptr;
+    int rc = dev_alloc(ctx, (size_t)step * ctx->K * n * 8, (void **)&scratch);
+    if (!rc) rc = dev_alloc(ctx, (size_t)t->count * sizeof(int), (void **)&bits);
+    if (!rc) { cudaError_t e = cudaMemsetAsync(bits, 0, (size_t)t->count * sizeof(int), ctx->stream); if (e != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e)); }
+    for (long c0 = 0; c0 < t->count && !rc; c0 += step)
+        rc = noise_bits_range(ctx, k, t, c0, std::min<long>(step, t->count - c0), scratch, bits + c0);
+    std::vector<int> hb;
+    if (!rc) {
+        hb.resize((size_t)t->count);
+        cudaError_t e = cudaMemcpyAsync(hb.data(), bits, hb.size() * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+        if (e != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
+    }
+    dev_free(ctx, scratch); dev_free(ctx, bits);
+    if (rc) return rc;
+    int mn = k->b.q_bits;
+    for (long i = 0; i < t->count; i++) {
+        const int b = std::max(0, k->b.q_bits - hb[(size_t)i] - 1);     // the -1 accounts for scaling the invariant noise by 2
+        if (host_budgets) host_budgets[i] = b;
+        mn = std::min(mn, b);
+    }
+    if (min_budget) *min_budget = mn;
+    return CRCNN_OK;
 }
 
 int crcnn_reencrypt(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *in, uint64_t seed, double noise_standard_deviation,

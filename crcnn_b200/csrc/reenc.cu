@@ -33,6 +33,37 @@ ReencConsts make_reenc_consts(const DeviceParams &d) {
     return c;
 }
 
+// w[NB_WORDS] *= v
+static void words_mul(uint64_t *w, uint64_t v) {
+    u128h carry = 0;
+    for (int j = 0; j < NB_WORDS; j++) {
+        const u128h p = (u128h)w[j] * v + carry;
+        w[j] = (uint64_t)p;
+        carry = p >> 64;
+    }
+}
+
+BudgetConsts make_budget_consts(const DeviceParams &d) {
+    BudgetConsts c{};
+    c.n = d.n; c.K = d.K;
+    c.qw[0] = 1;
+    for (int i = 0; i < d.K; i++) {
+        const Mod &m = d.tab[i].mod;
+        c.q[i] = m;
+        c.c[i] = mulmod(d.t % m.q, d.inv_qhat[i], m);
+        c.qhat[i][0] = 1;
+        for (int j = 0; j < d.K; j++)
+            if (j != i) words_mul(c.qhat[i], d.tab[j].mod.q);
+        words_mul(c.qw, m.q);
+    }
+    // (q + 1) / 2: q is odd, so this is q / 2 rounded up = (q >> 1) + 1
+    for (int j = 0; j < NB_WORDS; j++) c.half[j] = (c.qw[j] >> 1) | (j + 1 < NB_WORDS ? c.qw[j + 1] << 63 : 0);
+    for (int j = 0; j < NB_WORDS && ++c.half[j] == 0; j++) {}
+    for (int j = 0; j < NB_WORDS; j++)
+        if (c.qw[j]) c.q_bits = 64 * j + 64 - __builtin_clzll(c.qw[j]);
+    return c;
+}
+
 // ---------------------------------------------------------------------------------------------- decrypt
 __global__ void __launch_bounds__(256)
 dec_dot_kernel(const __grid_constant__ ReencConsts c, const uint64_t *__restrict__ ct, int ct_is_ntt, const uint64_t *__restrict__ sk,
@@ -75,6 +106,88 @@ dec_scale_kernel(const __grid_constant__ ReencConsts c, const uint64_t *__restri
     if (a_g > (c.gamma >> 1)) r = addmod(a_t, reduce64(c.gamma - a_g, c.tm), c.t);          // :207-217
     else r = submod(a_t, reduce64(a_g, c.tm), c.t);                                         // :219-224
     plain[w] = mulmod(r, c.inv_gamma_t, c.tm);                                              // :233-234
+}
+
+// x -= y when x >= y (NB_WORDS words each); returns whether it subtracted
+__device__ __forceinline__ bool words_sub_if_ge(uint64_t (&x)[NB_WORDS], const uint64_t (&y)[NB_WORDS]) {
+    uint64_t d[NB_WORDS], borrow = 0;
+#pragma unroll
+    for (int j = 0; j < NB_WORDS; j++) {
+        const uint64_t yj = y[j] + borrow;
+        const uint64_t nb = (uint64_t)(yj < borrow) | (uint64_t)(x[j] < yj);
+        d[j] = x[j] - yj;
+        borrow = nb;
+    }
+    if (borrow) return false;
+#pragma unroll
+    for (int j = 0; j < NB_WORDS; j++) x[j] = d[j];
+    return true;
+}
+
+// One thread per coefficient: the K residues of c0 + c1 s -> bit length of the centred t (c0 + c1 s) mod q (decryptor.cpp:
+// invariant_noise_budget), maximised over the ciphertext's n coefficients into bits[cti].  Every thread reaches the warp reduction
+// (no early return); n is a multiple of 32 and blocks are 128 threads, so a warp never straddles two ciphertexts or the end.
+__global__ void __launch_bounds__(128)
+noise_bits_kernel(const __grid_constant__ BudgetConsts c, const uint64_t *__restrict__ ct, const uint64_t *__restrict__ tmp,
+                  int *__restrict__ bits, long total) {
+    const long w = (long)blockIdx.x * 128 + threadIdx.x;
+    const int n = c.n, K = c.K;
+    const long cti = w / n;
+    int b = 0;
+    if (w < total) {
+        const int k = (int)(w % n);
+        uint64_t x[NB_WORDS];
+#pragma unroll
+        for (int j = 0; j < NB_WORDS; j++) x[j] = 0;
+#pragma unroll
+        for (int i = 0; i < MAXK; i++) {
+            if (i >= K) break;
+            uint64_t d = __ldg(tmp + (cti * K + i) * (long)n + k);
+            if (ct) d += __ldg(ct + (cti * 2 * K + i) * (long)n + k);   // lazy "+ c0": < 2 q_i, the product below reduces it
+            const uint64_t a = mulmod(d, c.c[i], c.q[i]);              // [t y_i (q/q_i)^-1]_{q_i}  (baseconverter.cpp: compose)
+            // x += a (q/q_i): q/q_i has at most K-1 nonzero words; the partial sum stays below K q < 2^(64 K + 3), so the carry out of
+            // word K-1 lands in word K without overflowing it
+            uint64_t carry = 0;
+#pragma unroll
+            for (int j = 0; j < MAXK; j++) {
+                if (j >= K) break;
+                const uint64_t lo = a * c.qhat[i][j], hi = __umul64hi(a, c.qhat[i][j]);
+                uint64_t s = x[j] + lo;
+                uint64_t cy = s < lo;
+                s += carry;
+                cy += s < carry;
+                x[j] = s;
+                carry = hi + cy;              // a * qhat + x + carry < 2^128: no overflow
+            }
+#pragma unroll
+            for (int j = 1; j < NB_WORDS; j++)
+                if (j == K) x[j] += carry;
+        }
+        // x < K q: at most K - 1 subtractions of q bring it into [0, q)  (compose's final modulo_uint_inplace)
+#pragma unroll 1
+        for (int r = 1; r < K; r++)
+            if (!words_sub_if_ge(x, c.qw)) break;
+        // |x| = q - x for x >= (q + 1) / 2 (poly_infty_norm_coeffmod)
+        uint64_t h[NB_WORDS];
+#pragma unroll
+        for (int j = 0; j < NB_WORDS; j++) h[j] = x[j];
+        if (words_sub_if_ge(h, c.half)) {
+            uint64_t borrow = 0;
+#pragma unroll
+            for (int j = 0; j < NB_WORDS; j++) {
+                const uint64_t xj = x[j] + borrow;
+                const uint64_t nb = (uint64_t)(xj < borrow) | (uint64_t)(c.qw[j] < xj);
+                x[j] = c.qw[j] - xj;
+                borrow = nb;
+            }
+        }
+#pragma unroll
+        for (int j = 0; j < NB_WORDS; j++)
+            if (x[j]) b = 64 * j + 64 - __clzll((long long)x[j]);     // get_significant_bit_count_uint
+    }
+    // the bit length of the maximum is the maximum of the bit lengths: no multi-word maximum is needed
+    b = __reduce_max_sync(0xffffffffu, b);
+    if ((threadIdx.x & 31) == 0 && w < total) atomicMax(bits + cti, b);
 }
 
 // ---------------------------------------------------------------------------------------------- decode -> float -> encode
@@ -232,6 +345,13 @@ cudaError_t launch_dec_scale(const ReencConsts &c, const uint64_t *ct, const uin
     const long total = count * (long)c.n;
     if (total <= 0) return cudaSuccess;
     dec_scale_kernel<<<blocks(total, 128), 128, 0, s>>>(c, ct, tmp, plain, total);
+    return cudaGetLastError();
+}
+cudaError_t launch_noise_bits(const BudgetConsts &c, const uint64_t *ct, const uint64_t *tmp, int *bits, long count, cudaStream_t s) {
+    const long total = count * (long)c.n;
+    if (total <= 0) return cudaSuccess;
+    if (c.n % 32) return cudaErrorInvalidValue;      // the warp reduction needs whole warps per ciphertext
+    noise_bits_kernel<<<blocks(total, 128), 128, 0, s>>>(c, ct, tmp, bits, total);
     return cudaGetLastError();
 }
 cudaError_t launch_reencode(const ReencConsts &c, const uint64_t *plain, uint64_t *slots, float *values, long count, cudaStream_t s) {

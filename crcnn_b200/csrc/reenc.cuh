@@ -32,11 +32,28 @@ struct ReencConsts {
 
 ReencConsts make_reenc_consts(const DeviceParams &d);
 
+// Decryptor::invariant_noise_budget (SEAL/seal/decryptor.cpp): t (c0 + c1 s) mod q composed by CRT (BaseConverter::compose) as
+// sum_i [y_i (q/q_i)^-1]_{q_i} (q/q_i), reduced below q, centred (poly_infty_norm_coeffmod).  Multi-word integers are MAXK + 1
+// little-endian 64-bit words: primes are <= 60 bits, so q < 2^480 and a sum of K terms below q stays below 2^(64 K + 3).
+constexpr int NB_WORDS = MAXK + 1;
+struct BudgetConsts {
+    int n, K, q_bits;                     // q_bits: total_coeff_modulus_bit_count
+    Mod q[MAXK];
+    uint64_t c[MAXK];                     // t (q/q_i)^-1 mod q_i: multiply_poly_scalar_coeffmod by t and compose's first step folded
+    uint64_t qhat[MAXK][NB_WORDS];        // q/q_i
+    uint64_t qw[NB_WORDS], half[NB_WORDS];   // q and (q + 1) / 2 (modulus_neg_threshold)
+};
+
+BudgetConsts make_budget_consts(const DeviceParams &d);
+
 // tmp[count][K][n] = NTT(c1) on entry (coefficient-form input) -> tmp (.) sk;  NTT-form input: tmp = c1 (.) sk + c0
 cudaError_t launch_dec_dot(const ReencConsts &c, const uint64_t *ct, int ct_is_ntt, const uint64_t *sk, uint64_t *tmp, long count, cudaStream_t s);
 // tmp = INTT(...) on entry; plain[count][n] = Decryptor::decrypt's result
 cudaError_t launch_dec_scale(const ReencConsts &c, const uint64_t *ct /* null when c0 is already in tmp */, const uint64_t *tmp,
                              uint64_t *plain, long count, cudaStream_t s);
+// tmp as for launch_dec_scale; bits[count] (zeroed by the caller) = max over coefficients of the bit length of |t (c0 + c1 s) mod q|
+cudaError_t launch_noise_bits(const BudgetConsts &c, const uint64_t *ct /* null when c0 is already in tmp */, const uint64_t *tmp,
+                              int *bits, long count, cudaStream_t s);
 // decode -> (float) -> encode: slots[count][96] = coefficients 0..63 and n-32..n-1 of the re-encoded plaintext; values[count] (may be null)
 cudaError_t launch_reencode(const ReencConsts &c, const uint64_t *plain, uint64_t *slots, float *values, long count, cudaStream_t s);
 // u (as residues, U[count][K][n]) and e[count][2][n] (int8): sampled from (seed, ciphertext index, coefficient) or copied from `given`

@@ -41,12 +41,28 @@ def load():
     h.crcnn_host_set_fusion.argtypes = [_I]
     h.crcnn_host_serve_times.argtypes = [_dp, _I]
     h.crcnn_host_serve_times.restype = _I
+    h.crcnn_host_use_keys.argtypes = [_vp, _vp, _I, C.c_uint64]
+    h.crcnn_host_set_budget_threshold.argtypes = [_I]
+    h.crcnn_host_forward_adaptive.argtypes = [_vp, _I, _vp, C.c_long, C.POINTER(_I), C.POINTER(_I)]
+    h.crcnn_host_budget_log.argtypes = [C.POINTER(_I)] * 3 + [_I]
+    h.crcnn_host_budget_log.restype = _I
     _h = h
     return h
 
 
 class HostError(RuntimeError):
     pass
+
+
+CRCNN_ERR_OUT_OF_BUDGET = -6
+
+
+class OutOfBudget(HostError):
+    """OutOfBudgetException of the host library: the activation after `layer` has no noise budget left to go on with."""
+
+    def __init__(self, msg, layer):
+        super().__init__(msg)
+        self.layer = layer
 
 
 def weights_h5(model, directory=None):
@@ -145,6 +161,38 @@ class HostNetwork:
         ms = C.c_double()
         self._chk(self.h.crcnn_host_serve(pinned_in_ptr, pinned_out_ptr, batch, requests, C.byref(ms)))
         return ms.value
+
+    def use_keys(self, secret_key_ntt, public_key_ntt, device_reencryption=False, seed=0):
+        """Network::use_device_keys (or use_device_reencryption with `seed`): the key holder's keys on the device."""
+        sk = np.ascontiguousarray(secret_key_ntt, dtype=np.uint64)
+        pk = np.ascontiguousarray(public_key_ntt, dtype=np.uint64)
+        assert sk.size == self.K * self.stride and pk.size == 2 * self.K * self.stride
+        self._chk(self.h.crcnn_host_use_keys(sk.ctypes.data, pk.ctypes.data, int(bool(device_reencryption)), C.c_uint64(seed)))
+
+    def set_budget_threshold(self, threshold):
+        """Network::reencrypt_below_budget: -1 keeps the fixed re-encryption point, >= 0 re-encrypts when the budget falls to it."""
+        self._chk(self.h.crcnn_host_set_budget_threshold(int(threshold)))
+
+    def forward_adaptive(self, x, batch=1):
+        """Network::forward_dev_adaptive on host ciphertexts x ([batch * z*x*y][2][K][n+1]) -> (output array, (z, x, y)).
+        Raises OutOfBudget (with .layer) where the network throws OutOfBudgetException."""
+        x = np.ascontiguousarray(x, dtype=np.uint64)
+        cap = max(x.size, batch * 64 * 64 * 64 * 2 * self.K * self.stride // 64)
+        out = np.empty(cap, dtype=np.uint64)
+        oshape, failed = (_I * 3)(), _I(-1)
+        rc = self.h.crcnn_host_forward_adaptive(x.ctypes.data, batch, out.ctypes.data, cap, oshape, C.byref(failed))
+        if rc == CRCNN_ERR_OUT_OF_BUDGET:
+            raise OutOfBudget(self.h.crcnn_host_last_error().decode(), failed.value)
+        self._chk(rc)
+        cnt = batch * oshape[0] * oshape[1] * oshape[2]
+        return out[:cnt * self.ct_words()].reshape(cnt, 2, self.K, self.stride).copy(), (oshape[0], oshape[1], oshape[2])
+
+    def budget_log(self):
+        """Network::budget_log of the last adaptive forward: [(layer, min budget, re-encrypted)]."""
+        cap = 256
+        a, b, c = (_I * cap)(), (_I * cap)(), (_I * cap)()
+        k = min(self.h.crcnn_host_budget_log(a, b, c, cap), cap)
+        return [(a[i], b[i], bool(c[i])) for i in range(k)]
 
     def set_fusion(self, on):
         """Layer fusion (conv+pool+bn on the pooled grid, pool+bn, fc+fc composed) on / off; off = one call per reference layer."""

@@ -99,6 +99,7 @@ SYMBOLS = [
     ("crcnn_keys_upload", _I, [_vp, _vp, _vp, _vpp]),
     ("crcnn_keys_free", _I, [_vp, _vp]),
     ("crcnn_decrypt", _I, [_vp, _vp, _vp, _vp]),
+    ("crcnn_noise_budget", _I, [_vp, _vp, _vp, _i32p, _i32p]),
     ("crcnn_reencrypt", _I, [_vp, _vp, _vp, C.c_uint64, C.c_double, _vp, _vpp, _vp, _vp]),
     ("crcnn_probe_pipe", _I, [_vp, _I, _I, _I, _I, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
 ]
@@ -326,6 +327,19 @@ class Engine:
         out = np.zeros((self.count(t), self.stride), dtype=np.uint64)
         self._chk(self.lib.crcnn_decrypt(self.h, keys.ptr, t.ptr, out.ctypes.data))
         return out
+
+    def noise_budget(self, keys, t):
+        """Decryptor::invariant_noise_budget of every ciphertext of t -> int32[count]."""
+        out = np.zeros(self.count(t), dtype=np.int32)
+        self._chk(self.lib.crcnn_noise_budget(self.h, keys.ptr if keys is not None else None, t.ptr if t is not None else None,
+                                              out.ctypes.data_as(_i32p), None))
+        return out
+
+    def min_noise_budget(self, keys, t):
+        """The minimum invariant noise budget over t (crcnn_noise_budget's min_budget)."""
+        m = C.c_int()
+        self._chk(self.lib.crcnn_noise_budget(self.h, keys.ptr if keys is not None else None, t.ptr, None, C.byref(m)))
+        return m.value
 
     def reencrypt(self, keys, t, seed=0, sigma=0.0, noise=None, want_plain=False):
         """decrypt -> decode -> float -> encode -> encrypt on the device; noise: optional int8 [count][3][n] (u, e0, e1).

@@ -43,7 +43,8 @@ typedef enum {
     CRCNN_ERR_CUDA = -2,
     CRCNN_ERR_NO_DEVICE = -3,
     CRCNN_ERR_OUT_OF_MEMORY = -4,
-    CRCNN_ERR_UNSUPPORTED = -5
+    CRCNN_ERR_UNSUPPORTED = -5,
+    CRCNN_ERR_OUT_OF_BUDGET = -6     /* the host library's OutOfBudgetException (crcnn_b200.hpp): a ciphertext ran out of noise budget */
 } crcnn_status;
 
 /* Message for the most recent failing call on `ctx` (or, with ctx == NULL, for the most recent
@@ -304,6 +305,9 @@ int crcnn_keys_free(crcnn_ctx *ctx, crcnn_keys *keys);   /* the device copy of t
 /* Decryptor::decrypt of every (size-2) ciphertext of t: host_plain gets count plaintexts of n+1 words (values < t, pad word 0),
  * bit-identical to SEAL's. */
 int crcnn_decrypt(crcnn_ctx *ctx, crcnn_keys *keys, crcnn_tensor *t, uint64_t *host_plain);
+/* Decryptor::invariant_noise_budget (SEAL/seal/decryptor.cpp) of every size-2 ciphertext of t, either domain.
+ * host_budgets: count ints (may be NULL); min_budget: the minimum over t (may be NULL). Needs the secret key. */
+int crcnn_noise_budget(crcnn_ctx *ctx, crcnn_keys *keys, crcnn_tensor *t, int *host_budgets, int *min_budget);
 /* decrypt -> decode -> (float) -> encode -> encrypt of every ciphertext of `in`, activations never leaving the device.  The three
  * sampled polynomials of an encryption (u uniform in {-1,0,1}; e0, e1 clipped normal, standard deviation
  * noise_standard_deviation (<= 0: SEAL's default 3.19), redrawn beyond 6 sigma, truncated toward zero) come from a counter-based
