@@ -891,6 +891,51 @@ public:
         Runtime::get().check(crcnn_noise_budget(Runtime::get().ctx(), require_keys(), x.t, nullptr, &m));
         return m;
     }
+    // encryptImage / decryptImage (CrCNN/src/globals.cpp:127-142, 207-233) on the device with the installed keys; need use_device_keys.
+    // encrypt_images_dev: images[b][z][x][y] -> one tensor [batch][z][x][y], the layout upload_batch produces (crcnn_encrypt_values).
+    // Every call draws fresh randomness from (seed, call number), as reencrypt_dev does; do not hand the same seed to both.
+    DeviceTensor encrypt_images_dev(const std::vector<floatCube> &images, std::uint64_t seed) {
+        crcnn_keys *keys = require_keys();
+        if (images.empty() || images[0].empty() || images[0][0].empty() || images[0][0][0].empty()) throw std::invalid_argument("empty batch");
+        const int B = (int)images.size(), zd = (int)images[0].size(), xd = (int)images[0][0].size(), yd = (int)images[0][0][0].size();
+        std::vector<float> v;
+        v.reserve((size_t)B * zd * xd * yd);
+        for (auto &img : images) {
+            if ((int)img.size() != zd) throw std::invalid_argument("images of a batch must have one shape");
+            for (auto &plane : img) {
+                if ((int)plane.size() != xd) throw std::invalid_argument("images of a batch must have one shape");
+                for (auto &row : plane) {
+                    if ((int)row.size() != yd) throw std::invalid_argument("images of a batch must have one shape");
+                    v.insert(v.end(), row.begin(), row.end());
+                }
+            }
+        }
+        Runtime &rt = Runtime::get();
+        crcnn_tensor *t = nullptr;
+        rt.check(crcnn_encrypt_values(rt.ctx(), keys, v.data(), (long)v.size(), seed + 0x9E3779B97F4A7C15ull * encrypt_calls_++, 0.0, nullptr, &t));
+        return DeviceTensor(t, zd, xd, yd, B);
+    }
+    // x as x.count() / (zd*xd*yd) images of [zd][xd][yd] floats (crcnn_decrypt_values: only the floats leave the device).
+    std::vector<floatCube> decrypt_images_dev(const DeviceTensor &x, int zd, int xd, int yd) {
+        crcnn_keys *keys = require_keys();
+        const long per = (long)zd * xd * yd;
+        if (per <= 0 || x.count() % per) throw std::invalid_argument("tensor is not a whole number of images of that shape");
+        std::vector<float> v((size_t)x.count());
+        Runtime::get().check(crcnn_decrypt_values(Runtime::get().ctx(), keys, x.t, v.data()));
+        std::vector<floatCube> out((size_t)(x.count() / per), floatCube(zd, std::vector<std::vector<float>>(xd, std::vector<float>(yd))));
+        size_t i = 0;
+        for (auto &img : out)
+            for (auto &plane : img)
+                for (auto &row : plane)
+                    for (auto &f : row) f = v[i++];
+        return out;
+    }
+    // The reference program's encrypt -> forward -> decrypt (CrCNN/src/mainparams.cpp:84-111) for a batch, activations never leaving
+    // the device: encrypt_images_dev, forward_batch's path (fusion, fixed or budget-driven re-encryption), decrypt_images_dev.
+    std::vector<floatCube> predict(const std::vector<floatCube> &images, std::uint64_t seed) {
+        DeviceTensor y = forward_batch_dev(encrypt_images_dev(images, seed));
+        return decrypt_images_dev(y, y.zd, y.xd, y.yd);
+    }
 
     // Budget-driven re-encryption, the reference's commented-out alternative to the fixed point (network.cpp:52-96): at a value
     // >= 0, forward / forward_batch run forward_dev_adaptive instead of re-encrypting before layer_before_reenc.  -1: off.
@@ -1027,7 +1072,7 @@ public:
     std::function<void(int)> after_layer;
     bool needs_reencryption() const { return layer_before_reenc > 0 && layer_before_reenc < (int)layers.size(); }
     crcnn_keys *require_keys() {
-        if (!device_keys) throw std::logic_error("crcnn_b200::Network: noise budgets need the key holder's keys (use_device_keys)");
+        if (!device_keys) throw std::logic_error("crcnn_b200::Network: noise budgets, encryption and decryption need the key holder's keys (use_device_keys)");
         return device_keys.get();
     }
     ciphertext3D forward(ciphertext3D input) {
@@ -1045,19 +1090,22 @@ public:
         return download(forward_dev(upload(input), 0, L));
     }
     // Same for a batch of independent images in one pass (what the reference's per-image loop, mainparams.cpp:84-111, does one by one).
-    std::vector<ciphertext3D> forward_batch(const std::vector<ciphertext3D> &inputs) {
+    std::vector<ciphertext3D> forward_batch(const std::vector<ciphertext3D> &inputs) { return download_batch(forward_batch_dev(upload_batch(inputs))); }
+    // forward_batch's path on a device tensor [batch][z][x][y]
+    DeviceTensor forward_batch_dev(DeviceTensor x) {
         const int L = (int)layers.size();
-        if (reencrypt_below_budget >= 0) return download_batch(forward_dev_adaptive(upload_batch(inputs)));
+        if (reencrypt_below_budget >= 0) return forward_dev_adaptive(std::move(x));
         if (needs_reencryption() && !skip_reencryption) {
-            if (reencrypt_dev)
-                return download_batch(forward_dev(reencrypt_dev(forward_dev(upload_batch(inputs), 0, layer_before_reenc)), layer_before_reenc, L));
+            if (reencrypt_dev) return forward_dev(reencrypt_dev(forward_dev(std::move(x), 0, layer_before_reenc)), layer_before_reenc, L);
             if (!reencrypt) throw std::logic_error("crcnn_b200::Network::forward_batch: re-encryption before layer " + std::to_string(layer_before_reenc) + " is not installed (see Network::forward)");
-            std::vector<ciphertext3D> mid = download_batch(forward_dev(upload_batch(inputs), 0, layer_before_reenc));
+            std::vector<ciphertext3D> mid = download_batch(forward_dev(std::move(x), 0, layer_before_reenc));
             for (auto &m : mid) m = reencrypt(m);
-            return download_batch(forward_dev(upload_batch(mid), layer_before_reenc, L));
+            return forward_dev(upload_batch(mid), layer_before_reenc, L);
         }
-        return download_batch(forward_dev(upload_batch(inputs), 0, L));
+        return forward_dev(std::move(x), 0, L);
     }
+private:
+    std::uint64_t encrypt_calls_ = 0;   // encrypt_images_dev's call number
 };
 
 // ------------------------------------------------------------------------------------------------

@@ -204,6 +204,35 @@ int crcnn_host_forward_adaptive(const uint64_t *in_words, int batch, uint64_t *o
     if (failed_layer) *failed_layer = g_oob_layer;
     return rc;
 }
+// Network::predict on `batch` images given as floats [batch][zd][xd][yd] (the built network's input shape): encrypted on the device
+// with the installed keys (use_keys) from `seed` and the call number, forward_batch's path, decrypted on the device into
+// scores[batch][outputs].  An OutOfBudgetException returns CRCNN_ERR_OUT_OF_BUDGET with its layer in *failed_layer (may be null).
+int crcnn_host_predict_values(const float *images, int batch, uint64_t seed, float *scores, int *failed_layer) {
+    g_oob_layer = -1;
+    const int rc = guarded([&] {
+        if (!g_net) throw std::invalid_argument("no network built");
+        if (!images || !scores || batch <= 0) throw std::invalid_argument("bad predict arguments");
+        std::vector<floatCube> in((size_t)batch, floatCube(g_zd, std::vector<std::vector<float>>(g_xd, std::vector<float>(g_yd))));
+        const float *p = images;
+        for (auto &img : in)
+            for (auto &plane : img)
+                for (auto &row : plane)
+                    for (auto &f : row) f = *p++;
+        const std::vector<floatCube> out = g_net->predict(in, seed);
+        size_t i = 0;
+        for (auto &img : out) {
+            long per = 0;
+            for (auto &plane : img)
+                for (auto &row : plane) per += (long)row.size();
+            if (per != g_outputs) throw std::logic_error("network output is not [batch][outputs] values");
+            for (auto &plane : img)
+                for (auto &row : plane)
+                    for (float f : row) scores[i++] = f;
+        }
+    });
+    if (failed_layer) *failed_layer = g_oob_layer;
+    return rc;
+}
 // Network::budget_log of the last adaptive forward: (layer, minimum budget, re-encrypted) per check; returns how many there are.
 int crcnn_host_budget_log(int *layer, int *min_budget, int *reencrypted, int cap) {
     if (!g_net) return 0;

@@ -2156,6 +2156,36 @@ int noise_bits_range(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, long first,
     CU(launch_noise_bits(k->b, c0, scratch, bits, count, ctx->stream));
     return CRCNN_OK;
 }
+
+// ciphertexts per chunk of the decrypting calls: a dot-product scratch (K*n words) and a plaintext (n words) each, 1 GiB in all
+long decrypt_step(const crcnn_ctx *ctx, long count) {
+    return std::max<long>(1, std::min<long>(count, (long)((1ull << 30) / ((size_t)(ctx->K + 1) * ctx->n * 8))));
+}
+
+// ciphertexts per chunk of the encrypting calls, 1 GiB in all: K*n words (dot product / u), n words (plaintext), 96 slots,
+// 2n + 3n noise bytes, a float
+long encrypt_step(const crcnn_ctx *ctx, long count) {
+    const size_t n = ctx->n, per_ct = (size_t)(ctx->K + 1) * n * 8 + REENC_SLOTS * 8 + 5 * n + 8;
+    return std::max<long>(1, std::min<long>(count, (long)((1ull << 30) / per_ct)));
+}
+
+// Encryptor::encrypt (SEAL/seal/encryptor.cpp:95-200) of the plaintexts slots[count][96] into dst[count][2][K][n], coefficient form.
+// u, e0, e1 of ciphertext r come from (seed, first + r, coefficient) or, with host_noise (this range's int8 rows [count][3][n]),
+// are copied through `given`.  U: count*K*n words, e: count*2*n bytes of scratch.
+cudaError_t encrypt_range(crcnn_ctx *ctx, crcnn_keys *k, const uint64_t *slots, uint64_t seed, long first, double noise_standard_deviation,
+                          const int8_t *host_noise, int8_t *given, uint64_t *U, int8_t *e, uint64_t *dst, long count) {
+    const int K = ctx->K;
+    const double sigma = noise_standard_deviation > 0 ? noise_standard_deviation : 3.19;   // SEAL/seal/util/globals.cpp: default_noise_standard_deviation
+    const double max_dev = 6.0 * sigma;                                                   // noise_distribution_width_multiplier = 6 (encryptionparams.h:204-211)
+    cudaError_t er = cudaSuccess;
+    if (host_noise) er = cudaMemcpyAsync(given, host_noise, (size_t)count * 3 * ctx->n, cudaMemcpyHostToDevice, ctx->stream);
+    if (er == cudaSuccess) er = launch_enc_sample(k->c, seed, first, sigma, max_dev, host_noise ? given : nullptr, U, e, count, ctx->stream);
+    if (er == cudaSuccess) er = launch_ntt(ctx->dP, ctx->logn, U, count * K, 0, K, false, ctx->stream);
+    if (er == cudaSuccess) er = launch_enc_mul(k->c, U, k->pk, dst, count, ctx->stream);
+    if (er == cudaSuccess) er = launch_ntt(ctx->dP, ctx->logn, dst, count * 2 * K, 0, K, true, ctx->stream);
+    if (er == cudaSuccess) er = launch_enc_finish(k->c, slots, e, dst, count, ctx->stream);
+    return er;
+}
 }  // namespace
 
 int crcnn_decrypt(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, uint64_t *host_plain) {
@@ -2164,7 +2194,7 @@ int crcnn_decrypt(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, uint64_t *host
     REQUIRE(t->size == 2, "decrypt is implemented for size-2 ciphertexts");
     CU(cudaSetDevice(ctx->device));
     const size_t n = ctx->n;
-    const long step = std::max<long>(1, std::min<long>(t->count, (long)((1ull << 30) / ((size_t)(ctx->K + 1) * n * 8))));
+    const long step = decrypt_step(ctx, t->count);
     uint64_t *scratch = nullptr, *plain = nullptr;
     int rc = dev_alloc(ctx, (size_t)step * ctx->K * n * 8, (void **)&scratch);
     if (!rc) rc = dev_alloc(ctx, (size_t)step * n * 8, (void **)&plain);
@@ -2189,7 +2219,7 @@ int crcnn_noise_budget(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, int *host
     REQUIRE(t->count > 0, "empty tensor");
     CU(cudaSetDevice(ctx->device));
     const size_t n = ctx->n;
-    const long step = std::max<long>(1, std::min<long>(t->count, (long)((1ull << 30) / ((size_t)(ctx->K + 1) * n * 8))));   // crcnn_decrypt's chunks
+    const long step = decrypt_step(ctx, t->count);
     uint64_t *scratch = nullptr;
     int *bits = nullptr;
     int rc = dev_alloc(ctx, (size_t)step * ctx->K * n * 8, (void **)&scratch);
@@ -2224,14 +2254,10 @@ int crcnn_reencrypt(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *in, uint64_t se
     CU(cudaSetDevice(ctx->device));
     const size_t n = ctx->n, pw = poly_words(ctx);
     const int K = ctx->K;
-    const double sigma = noise_standard_deviation > 0 ? noise_standard_deviation : 3.19;   // SEAL/seal/util/globals.cpp: default_noise_standard_deviation
-    const double max_dev = 6.0 * sigma;                                                   // noise_distribution_width_multiplier = 6 (encryptionparams.h:204-211)
     crcnn_tensor *o = nullptr;
     int rc = new_tensor(ctx, in->count, 2, 0, &o);
     if (rc) return rc;
-    // per ciphertext of a chunk: K*n words (dot product / u), n words (plaintext), 96 slots, 2n + 3n noise bytes
-    const size_t per_ct = (size_t)(K + 1) * n * 8 + REENC_SLOTS * 8 + 5 * n + 8;
-    const long step = std::max<long>(1, std::min<long>(in->count, (long)((1ull << 30) / per_ct)));
+    const long step = encrypt_step(ctx, in->count);
     uint64_t *scratch = nullptr, *plain = nullptr, *slots = nullptr;
     int8_t *e = nullptr, *given = nullptr;
     float *vals = nullptr;
@@ -2250,12 +2276,9 @@ int crcnn_reencrypt(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *in, uint64_t se
         {
             ProfScope ps(ctx, KC_REENC, lp_bytes(ctx, (double)cnt * 2 * K), lp_bfly(ctx, (double)cnt * 3 * K));
             er = launch_reencode(k->c, plain, slots, vals, cnt, ctx->stream);
-            if (er == cudaSuccess && host_noise) er = cudaMemcpyAsync(given, host_noise + c0 * 3 * n, (size_t)cnt * 3 * n, cudaMemcpyHostToDevice, ctx->stream);
-            if (er == cudaSuccess) er = launch_enc_sample(k->c, seed, c0, sigma, max_dev, given, scratch, e, cnt, ctx->stream);
-            if (er == cudaSuccess) er = launch_ntt(ctx->dP, ctx->logn, scratch, cnt * K, 0, K, false, ctx->stream);
-            if (er == cudaSuccess) er = launch_enc_mul(k->c, scratch, k->pk, dst, cnt, ctx->stream);
-            if (er == cudaSuccess) er = launch_ntt(ctx->dP, ctx->logn, dst, cnt * 2 * K, 0, K, true, ctx->stream);
-            if (er == cudaSuccess) er = launch_enc_finish(k->c, slots, e, dst, cnt, ctx->stream);
+            if (er == cudaSuccess)
+                er = encrypt_range(ctx, k, slots, seed, c0, noise_standard_deviation, host_noise ? host_noise + c0 * 3 * n : nullptr, given, scratch, e,
+                                   dst, cnt);
         }
         if (er == cudaSuccess && host_reencoded) {     // the re-encoded plaintexts, n+1 words each (parity checks)
             std::vector<uint64_t> hs((size_t)cnt * REENC_SLOTS);
@@ -2279,6 +2302,78 @@ int crcnn_reencrypt(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *in, uint64_t se
     if (rc) { crcnn_tensor_free(ctx, o); return rc; }
     *out = o;
     return CRCNN_OK;
+}
+
+int crcnn_encrypt_values(crcnn_ctx *ctx, crcnn_keys *k, const float *host_values, long count, uint64_t seed, double noise_standard_deviation,
+                         const int8_t *host_noise, crcnn_tensor **out) {
+    if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
+    REQUIRE(k && host_values && out, "null argument");
+    REQUIRE(count > 0, "no values to encrypt");
+    CU(cudaSetDevice(ctx->device));
+    const size_t n = ctx->n, pw = poly_words(ctx);
+    const int K = ctx->K;
+    crcnn_tensor *o = nullptr;
+    int rc = new_tensor(ctx, count, 2, 0, &o);
+    if (rc) return rc;
+    const long step = encrypt_step(ctx, count);
+    uint64_t *U = nullptr, *slots = nullptr;
+    int8_t *e = nullptr, *given = nullptr;
+    float *vals = nullptr;
+    rc = dev_alloc(ctx, (size_t)step * K * n * 8, (void **)&U);
+    if (!rc) rc = dev_alloc(ctx, (size_t)step * REENC_SLOTS * 8, (void **)&slots);
+    if (!rc) rc = dev_alloc(ctx, (size_t)step * 2 * n, (void **)&e);
+    if (!rc && host_noise) rc = dev_alloc(ctx, (size_t)step * 3 * n, (void **)&given);
+    if (!rc) rc = dev_alloc(ctx, (size_t)count * 4, (void **)&vals);
+    if (!rc) { cudaError_t er = cudaMemcpyAsync(vals, host_values, (size_t)count * 4, cudaMemcpyHostToDevice, ctx->stream); if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(er)); }
+    for (long c0 = 0; c0 < count && !rc; c0 += step) {
+        const long cnt = std::min<long>(step, count - c0);
+        cudaError_t er;
+        {
+            ProfScope ps(ctx, KC_REENC, lp_bytes(ctx, (double)cnt * 2 * K), lp_bfly(ctx, (double)cnt * 3 * K));
+            er = launch_encode_values(k->c, vals + c0, slots, cnt, ctx->stream);
+            if (er == cudaSuccess)
+                er = encrypt_range(ctx, k, slots, seed, c0, noise_standard_deviation, host_noise ? host_noise + c0 * 3 * n : nullptr, given, U, e,
+                                   o->d + c0 * 2 * pw, cnt);
+        }
+        if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, std::string("encryption: ") + cudaGetErrorString(er));
+    }
+    // the host buffers must stay untouched until their copies have run
+    if (!rc) { cudaError_t er = cudaStreamSynchronize(ctx->stream); if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(er)); }
+    dev_free(ctx, U); dev_free(ctx, slots); dev_free(ctx, e); dev_free(ctx, given); dev_free(ctx, vals);
+    if (rc) { crcnn_tensor_free(ctx, o); return rc; }
+    *out = o;
+    return CRCNN_OK;
+}
+
+int crcnn_decrypt_values(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, float *host_values) {
+    if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
+    REQUIRE(k && t && host_values, "null argument");
+    REQUIRE(t->size == 2, "decrypt is implemented for size-2 ciphertexts");
+    REQUIRE(t->count > 0, "empty tensor");
+    CU(cudaSetDevice(ctx->device));
+    const size_t n = ctx->n;
+    const long step = decrypt_step(ctx, t->count);
+    uint64_t *scratch = nullptr, *plain = nullptr;
+    float *vals = nullptr;
+    int rc = dev_alloc(ctx, (size_t)step * ctx->K * n * 8, (void **)&scratch);
+    if (!rc) rc = dev_alloc(ctx, (size_t)step * n * 8, (void **)&plain);
+    if (!rc) rc = dev_alloc(ctx, (size_t)t->count * 4, (void **)&vals);
+    for (long c0 = 0; c0 < t->count && !rc; c0 += step) {
+        const long cnt = std::min<long>(step, t->count - c0);
+        rc = decrypt_range(ctx, k, t, c0, cnt, scratch, plain);
+        if (!rc) {
+            ProfScope ps(ctx, KC_REENC, (double)cnt * n * 8 + (double)cnt * 4, 0);
+            cudaError_t er = launch_decode_values(k->c, plain, vals + c0, cnt, ctx->stream);
+            if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(er));
+        }
+    }
+    if (!rc) {
+        cudaError_t er = cudaMemcpyAsync(host_values, vals, (size_t)t->count * 4, cudaMemcpyDeviceToHost, ctx->stream);
+        if (er == cudaSuccess) er = cudaStreamSynchronize(ctx->stream);
+        if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(er));
+    }
+    dev_free(ctx, scratch); dev_free(ctx, plain); dev_free(ctx, vals);
+    return rc;
 }
 
 }  // extern "C"

@@ -56,6 +56,10 @@ cudaError_t launch_noise_bits(const BudgetConsts &c, const uint64_t *ct /* null 
                               int *bits, long count, cudaStream_t s);
 // decode -> (float) -> encode: slots[count][96] = coefficients 0..63 and n-32..n-1 of the re-encoded plaintext; values[count] (may be null)
 cudaError_t launch_reencode(const ReencConsts &c, const uint64_t *plain, uint64_t *slots, float *values, long count, cudaStream_t s);
+// slots[count][96] = FractionalEncoder::encode((double) values[i]), laid out as launch_reencode's
+cudaError_t launch_encode_values(const ReencConsts &c, const float *values, uint64_t *slots, long count, cudaStream_t s);
+// values[count] = (float) FractionalEncoder::decode(plain[i]), plain[count][n] as launch_dec_scale leaves it
+cudaError_t launch_decode_values(const ReencConsts &c, const uint64_t *plain, float *values, long count, cudaStream_t s);
 // u (as residues, U[count][K][n]) and e[count][2][n] (int8): sampled from (seed, ciphertext index, coefficient) or copied from `given`
 // ([count][3][n] int8: u, e0, e1)
 cudaError_t launch_enc_sample(const ReencConsts &c, uint64_t seed, long first_ct, double sigma, double max_dev, const int8_t *given,

@@ -46,6 +46,7 @@ def load():
     h.crcnn_host_forward_adaptive.argtypes = [_vp, _I, _vp, C.c_long, C.POINTER(_I), C.POINTER(_I)]
     h.crcnn_host_budget_log.argtypes = [C.POINTER(_I)] * 3 + [_I]
     h.crcnn_host_budget_log.restype = _I
+    h.crcnn_host_predict_values.argtypes = [C.POINTER(C.c_float), _I, C.c_uint64, C.POINTER(C.c_float), C.POINTER(_I)]
     _h = h
     return h
 
@@ -186,6 +187,22 @@ class HostNetwork:
         self._chk(rc)
         cnt = batch * oshape[0] * oshape[1] * oshape[2]
         return out[:cnt * self.ct_words()].reshape(cnt, 2, self.K, self.stride).copy(), (oshape[0], oshape[1], oshape[2])
+
+    def predict_values(self, images, batch=1, seed=0):
+        """Network::predict: float32 images ([batch][z][x][y] values) encrypted on the device with the keys of use_keys, the network's
+        forward (as forward_batch runs it), the scores decrypted on the device -> float32 [batch][outputs].  Each call draws its
+        randomness from (seed, call number).  Raises OutOfBudget (with .layer) where the network throws OutOfBudgetException."""
+        x = np.ascontiguousarray(images, dtype=np.float32).ravel()
+        if x.size != batch * self.zd * self.xd * self.yd:
+            raise ValueError("images must hold batch * %d values" % (self.zd * self.xd * self.yd))
+        out = np.zeros((batch, self.outputs), dtype=np.float32)
+        fp = C.POINTER(C.c_float)
+        failed = _I(-1)
+        rc = self.h.crcnn_host_predict_values(x.ctypes.data_as(fp), batch, C.c_uint64(seed), out.ctypes.data_as(fp), C.byref(failed))
+        if rc == CRCNN_ERR_OUT_OF_BUDGET:
+            raise OutOfBudget(self.h.crcnn_host_last_error().decode(), failed.value)
+        self._chk(rc)
+        return out
 
     def budget_log(self):
         """Network::budget_log of the last adaptive forward: [(layer, min budget, re-encrypted)]."""

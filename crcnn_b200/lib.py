@@ -101,6 +101,8 @@ SYMBOLS = [
     ("crcnn_decrypt", _I, [_vp, _vp, _vp, _vp]),
     ("crcnn_noise_budget", _I, [_vp, _vp, _vp, _i32p, _i32p]),
     ("crcnn_reencrypt", _I, [_vp, _vp, _vp, C.c_uint64, C.c_double, _vp, _vpp, _vp, _vp]),
+    ("crcnn_encrypt_values", _I, [_vp, _vp, _f32p, C.c_long, C.c_uint64, C.c_double, _vp, _vpp]),
+    ("crcnn_decrypt_values", _I, [_vp, _vp, _vp, _f32p]),
     ("crcnn_probe_pipe", _I, [_vp, _I, _I, _I, _I, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
 ]
 
@@ -357,6 +359,23 @@ class Engine:
                                            plain.ctypes.data if want_plain else None, vals.ctypes.data if want_plain else None))
         h = Handle(self, out, "tensor")
         return (h, plain, vals) if want_plain else h
+
+    def encrypt_values(self, keys, values, seed=0, sigma=0.0, noise=None):
+        """FractionalEncoder::encode + Encryptor::encrypt of every value (float32) on the device -> coefficient-form tensor of
+        len(values) ciphertexts.  noise: optional int8 [count][3][n] (u, e0, e1) instead of the generator keyed by `seed`."""
+        v = np.ascontiguousarray(values, dtype=np.float32).ravel()
+        nz = None
+        if noise is not None:
+            nz = np.ascontiguousarray(noise, dtype=np.int8)
+            assert nz.size == len(v) * 3 * self.n
+        return self._new(self.lib.crcnn_encrypt_values, "tensor", keys.ptr if keys is not None else None, v.ctypes.data_as(_f32p), len(v),
+                         C.c_uint64(seed), C.c_double(sigma), nz.ctypes.data if nz is not None else None)
+
+    def decrypt_values(self, keys, t):
+        """(float) FractionalEncoder::decode(Decryptor::decrypt(ct)) of every ciphertext of t -> float32[count]."""
+        out = np.zeros(self.count(t), dtype=np.float32)
+        self._chk(self.lib.crcnn_decrypt_values(self.h, keys.ptr if keys is not None else None, t.ptr, out.ctypes.data_as(_f32p)))
+        return out
 
     # ---- layers
     def conv(self, x, w, b, batch, xd, yd, zd, xs, ys, xf, yf, nf, shard=None):

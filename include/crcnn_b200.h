@@ -316,6 +316,21 @@ int crcnn_noise_budget(crcnn_ctx *ctx, crcnn_keys *keys, crcnn_tensor *t, int *h
 int crcnn_reencrypt(crcnn_ctx *ctx, crcnn_keys *keys, crcnn_tensor *in, uint64_t seed, double noise_standard_deviation,
                     const int8_t *host_noise, crcnn_tensor **out, uint64_t *host_reencoded, float *host_values);
 
+/* ---- the client's two ends on the device (opt-in, the same keys) ----------------------------------------
+ * Replaces: encryptImage / decryptImage (CrCNN/src/globals.cpp:127-142, 207-233) for a key holder who runs the evaluator.
+ * encryptImage's inner loop: FractionalEncoder(64, 32, base 3).encode((double) v) + Encryptor::encrypt for every value; *out is a
+ * new coefficient-form tensor of `count` size-2 ciphertexts, ciphertext i encrypting host_values[i].  Noise as crcnn_reencrypt:
+ * (seed, ciphertext index, coefficient) -> Philox, or host_noise int8[count][3][n] = u, e0, e1.  The values are encoded exactly as
+ * crcnn_plain_encode encodes them, which accepts every float; SEAL leaves the integer part of a value outside the int64 range (and
+ * NaN) undefined, and so does this call.
+ * Seeds: the same (seed, ciphertext index) always draws the same u, e0, e1 -- in this call and in crcnn_reencrypt alike -- so a seed
+ * must never serve two calls: two encryptions under one u reveal the difference of their plaintexts. */
+int crcnn_encrypt_values(crcnn_ctx *ctx, crcnn_keys *keys, const float *host_values, long count, uint64_t seed,
+                         double noise_standard_deviation, const int8_t *host_noise, crcnn_tensor **out);
+/* decryptImage's inner loop: host_values[i] = (float) FractionalEncoder::decode(Decryptor::decrypt(ciphertext i of t)), size-2
+ * ciphertexts in either domain; only the count floats leave the device. */
+int crcnn_decrypt_values(crcnn_ctx *ctx, crcnn_keys *keys, crcnn_tensor *t, float *host_values);
+
 /* ---- measurement ------------------------------------------------------------------------------
  * Kernel classes are timed with CUDA events on the context's stream while profiling is on. */
 int crcnn_prof_enable(crcnn_ctx *ctx, int on);
