@@ -357,10 +357,12 @@ int get_index_table(crcnn_ctx *ctx, const std::vector<int> &key, const std::vect
 }
 
 // The coefficient-domain multiply (tapmul_kernel) applies to this pack: FractionalEncoder digits only, primes below 2^56.
+// tapmul_kernel reads value 1 as +1 and value t-1 as -1; multiply_plain lifts 1 to +1 only when 1 < (t+1)/2, that is t >= 3
+// (at t = 2 both digits are the value 1 and it lifts to q-1), so t = 2 takes the NTT-domain multiply.
 bool tap_eligible(crcnn_ctx *ctx, crcnn_plain *p) {
     if (p->tap_state == 0) {
-        p->tap_state = (p->sparse_shape && tcn_planes_for(ctx->hp.d) == 7 && ctx->n % 1024 == 0) ? 1 : -1;
         const uint64_t t = ctx->hp.d.t;
+        p->tap_state = (p->sparse_shape && tcn_planes_for(ctx->hp.d) == 7 && ctx->n % 1024 == 0 && t >= 3) ? 1 : -1;
         for (size_t e = 0; e < p->val.size() && p->tap_state == 1; e++)
             if (p->val[e] != 1 && p->val[e] != t - 1) p->tap_state = -1;
         for (long i = 0; i < p->count && p->tap_state == 1; i++)
@@ -389,6 +391,8 @@ int ensure_tc_form(crcnn_ctx *ctx, crcnn_plain *w, int R) {
     if (w->tc_state == 1 && w->tc_R == R) return CRCNN_OK;
     const uint32_t n = (uint32_t)ctx->n;
     const uint64_t t = ctx->hp.d.t;
+    // the digits are read as +1 (value 1) and -1 (value t-1), which is multiply_plain's lift only for t >= 3 (tap_eligible)
+    if (t < 3) { w->tc_state = -1; return CRCNN_OK; }
     for (size_t e = 0; e < w->idx.size(); e++)
         if (w->idx[e] < n - TC_TAPS || (w->val[e] != 1 && w->val[e] != t - 1)) { w->tc_state = -1; return CRCNN_OK; }
     if (w->count % R) { w->tc_state = -1; return CRCNN_OK; }

@@ -70,8 +70,11 @@ int main(int argc, char **argv) {
             }
         }
         // pre-shifted limb-split GEMM (tcn_mac.cu: tcn2p_mac_kernel): the byte planes of W' = W 2^(8b) mod q recombine to W' and give
-        // W X mod q through the seven classes; tcn7_fold_reduce and tcn7_combine against unsigned __int128, all-(q-1) operands at R = 4096
-        for (int j = 0; j < d.K; j++) {
+        // W X mod q through the seven classes; tcn7_fold_reduce and tcn7_combine against unsigned __int128, all-(q-1) operands at R = 4096.
+        // Seven byte planes hold residues of primes up to 56 bits only; above that the engine does not take the limb-split GEMM.
+        bool seven_planes = true;
+        for (int j = 0; j < d.K; j++) seven_planes = seven_planes && (d.tab[j].mod.q >> 56) == 0;
+        for (int j = 0; j < d.K && seven_planes; j++) {
             const Mod &m = d.tab[j].mod;
             const TcnFold f = tcn_fold_make(m.q);
             long checked = 0;

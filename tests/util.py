@@ -14,6 +14,29 @@ from oracle import ref as oref  # noqa: E402
 PRIMES = oport.DEFAULT_PRIMES_128
 T_FOR_N = {2048: 1 << 16, 4096: 1 << 18, 8192: 1 << 30, 16384: 1 << 30}
 
+# Parameter sets beyond SEAL's defaults: {name: (n, primes, t)}.  Every prime is = 1 (mod 2n).  They take the kernels' other
+# branches: 56-bit primes (the full top byte plane of the limb-split GEMM), 57-60-bit primes (8 byte planes in the ternary GEMM,
+# no limb-split GEMM, mode 2 of the forward transform on q, partial sums in the CUDA-core MAC, R * q >= 2^64), primes without
+# the 2^k - delta shape (Barrett instead of the folds), small primes (other relinearization digit counts), K not a power of two
+# (the generic BEHZ and the 64-bit relinearize), an extra auxiliary prime (L = K + 1) and odd or tiny plain moduli.
+PARAM_SETS = {
+    "P56": (4096, [0xfffffffff78001, 0xfffffffff70001], 1 << 18),
+    "P57": (4096, [0x1fffffffffc0001], 1 << 18),
+    "P57n16384": (16384, [0x1fffffffffc0001], 1 << 18),
+    "P60a": (4096, [0xffffffffffe8001], 1 << 30),
+    "P60b": (4096, [0xffffffffffe8001, 0xffffffffffd8001], (1 << 31) - 1),
+    "U50": (4096, [0x2fffffff50001, 0x2ffffffee0001], 1 << 18),
+    "U40": (2048, [0xbffffe8001], 1 << 8),
+    "U30": (2048, [0x2ffd0001], 1 << 4),
+    "K3": (8192, PRIMES[16384][:3], 1 << 30),
+    "K5": (8192, PRIMES[16384][:5], 1 << 30),
+    "K7": (8192, PRIMES[16384][:7], 1 << 30),
+    "T2": (4096, PRIMES[4096], 2),
+    "T3": (4096, PRIMES[4096], 3),
+    "T5": (4096, PRIMES[4096], 5),
+    "T32771": (4096, PRIMES[4096], 32771),
+}
+
 
 def have_ref():
     return oref.available()
