@@ -934,10 +934,13 @@ relin_scale_kernel(const DeviceParams *__restrict__ P, const uint64_t *__restric
     dsc[ct * pw + lw] = mulmod(__ldg(in3 + (ct * 3 + 2) * pw + lw), P->inv_qhat[i], P->tab[i].mod);
 }
 
+// crcnn_relinearize admits up to 63 digits (the 128-bit lazy sum of relin_mac_kernel, evaluator.cpp:972-976): keys of 1-bit
+// digits over a 54-bit prime, or 4-bit digits over four 55-bit primes, have more than 32
+constexpr int RELIN_MAXD = 64;
 struct DigitMap {
-    int D;                    // total digits = sum_i digits_i
-    unsigned char prime[32];  // digit d belongs to prime i
-    unsigned char shift[32];  // and is (d_i >> shift) & mask
+    int D;                             // total digits = sum_i digits_i
+    unsigned char prime[RELIN_MAXD];   // digit d belongs to prime i
+    unsigned char shift[RELIN_MAXD];   // and is (d_i >> shift) & mask
 };
 
 template <int LOGN>
@@ -1016,7 +1019,7 @@ cudaError_t launch_relin(const DeviceParams *P, int logn, int K, const RelinArgs
     DigitMap map{};
     for (int i = 0; i < K; i++)
         for (int k = 0; k < a.digits[i]; k++) {
-            if (map.D >= 32) return cudaErrorInvalidValue;
+            if (map.D >= RELIN_MAXD) return cudaErrorInvalidValue;
             map.prime[map.D] = (unsigned char)i;
             map.shift[map.D] = (unsigned char)(k * a.dbc);
             map.D++;

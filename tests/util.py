@@ -186,3 +186,93 @@ def ref_ops(kind, r, n, primes, t, seed):
         out["bn"] = r.bn(xi, 2, 3, 3, e(mean), e(invstd))
         out["square_layer"] = r.square_layer(xi[:4], evk, sizes, dbc)
     return out
+
+
+# ---- worst-case operands at the weighted sums' accumulator limits (tests/test_limits_oracle.py proves these on the oracle,
+# tests/test_gpu_limits.py runs them on the device)
+def class_sums(w, x, planes=7):
+    """One term w * x of the limb-split GEMM (tcn_mac.cuh): both split into `planes` unsigned bytes, class c = a + b collects
+    byte_a(w) * byte_b(x).  Returns the 2 * planes - 1 class values; a layer of fan-in R with uniform operands sums R of them."""
+    wb = [(int(w) >> (8 * a)) & 0xff for a in range(planes)]
+    xb = [(int(x) >> (8 * b)) & 0xff for b in range(planes)]
+    return [sum(wb[a] * xb[c - a] for a in range(max(0, c - planes + 1), min(c, planes - 1) + 1)) for c in range(2 * planes - 1)]
+
+
+def ones_below(q, width=8):
+    """Values below q whose low digits of `width` bits are all ones (one per digit count), and q - 1."""
+    out = {int(q) - 1}
+    for s in range(width, int(q).bit_length(), width):
+        top = ((int(q) - 1) >> s) - 1
+        if top >= 0:
+            out.add((top << s) | ((1 << s) - 1))
+    return sorted(out)
+
+
+def worst_operands(primes, t):
+    """(k, [x_j]) maximising the largest class sum: weights are the constant plaintext t - k, which lifts to q_j - k in every NTT slot
+    of every prime (k <= (t - 1) / 2), slot values x_j < q_j.  k is shared by the primes (one plaintext), x_j is per prime."""
+    kmax = (int(t) - 1) // 2
+    ks = set(range(1, min(kmax, 255) + 1))
+    for q in primes:
+        ks.update(int(q) - v for v in ones_below(q) if 1 <= int(q) - v <= kmax)
+    best = None
+    for k in sorted(ks):
+        xs, score = [], 0
+        for q in primes:
+            m, x = max((max(class_sums(int(q) - k, v)), v) for v in ones_below(q))
+            xs.append(x)
+            score += m
+        if best is None or score > best[0]:
+            best = (score, k, xs)
+    return best[1], best[2]
+
+
+def acc7_even(w, x, terms, carry=0):
+    """The 128-bit `even` half of the CUDA-core MAC's split accumulator (modarith.cuh: Acc7) after `terms` products w * x on top of a
+    reduced residue `carry`: sum of lo32(x) lo32(w) + hi32(x) hi32(w) 2^64.  Must stay below 2^128 for chunk_terms terms."""
+    x0, x1, w0, w1 = int(x) & 0xffffffff, int(x) >> 32, int(w) & 0xffffffff, int(w) >> 32
+    return int(carry) + terms * (x0 * w0 + ((x1 * w1) << 64))
+
+
+def const_weight_fc_slots(k, xb, d, primes, bias=None):
+    """Closed form of a fully connected layer in the NTT domain with constant-plaintext weights: weight (m, r) is q_j - k[m][r] in every
+    slot, input slot (b, r, poly, j, s) is xb[j] - d[b][r][poly][j][s].  Then
+        Y[b][m][poly][j][s] = sum_r (q_j - k[m][r]) (xb[j] - d[...]) = sum_r k[m][r] d[...] - xb[j] sum_r k[m][r]   (mod q_j)
+    (+ bias[m][j][s] on polynomial 0).  k: [M][R] ints, d: [B][R][2][K][n] small ints.  Returns [B][M][2][K][n] uint64.
+    The products k d are exact in float64 while R * max(k) * max(d) < 2^53."""
+    k = np.asarray(k, dtype=np.int64)
+    M, R = k.shape
+    B, _, _, K, n = d.shape
+    assert R * int(k.max()) * max(1, int(d.max())) < (1 << 53)
+    ks = [int(v) for v in k.sum(axis=1)]
+    out = np.zeros((B, M, 2, K, n), dtype=np.uint64)
+    kf = k.astype(np.float64)
+    for b in range(B):
+        kd = (kf @ d[b].reshape(R, -1).astype(np.float64)).astype(np.int64).reshape(M, 2, K, n)
+        for j, q in enumerate(primes):
+            q = int(q)
+            for m in range(M):
+                a = int(xb[j]) * ks[m] % q
+                y = (kd[m, :, j, :] % q - a) % q
+                if bias is not None:
+                    y[0] = (y[0] + bias[m][j].astype(np.int64)) % q
+                out[b, m, :, j, :] = y.astype(np.uint64)
+    return out
+
+
+def slots_to_words(slots):
+    """[..][K][n] slot values -> [..][K][n + 1] SEAL-layout words (the unused last word 0)."""
+    out = np.zeros(slots.shape[:-1] + (slots.shape[-1] + 1,), dtype=np.uint64)
+    out[..., :-1] = slots
+    return out
+
+
+def bias_slots(orc, bias_plain):
+    """NTT slots [M][K][n] the bias of a layer adds to polynomial 0: the transform of Delta * b (add_plain on a zero ciphertext)."""
+    M = len(bias_plain)
+    z = np.zeros((M, 2, orc.K, orc.n + 1), dtype=np.uint64)
+    out = np.zeros((M, orc.K, orc.n), dtype=np.uint64)
+    for m in range(M):
+        y = orc.ct_transform(orc.plain_op(z[m:m + 1], bias_plain[m], "add"))
+        out[m] = y[0, 0, :, :orc.n]
+    return out
