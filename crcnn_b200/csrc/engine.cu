@@ -113,8 +113,6 @@ struct crcnn_ctx {
     int tap_mode = 1;                // 1: avg-pool / batch-norm on coefficient-form inputs multiply in the coefficient domain (tapmul_kernel); env CRCNN_TAP
     int relin_mode = 1;              // 1: relinearize through 30-bit auxiliary primes when exact for the parameters (relin32.cuh); 0: 64-bit transforms
     int tcn_mode = 1;                // 1: weighted sums whose staged weights fit the weight cache run as the NTT-domain limb-split GEMM (tcn_mac.cuh)
-    int sq_lean = 1;                 // 1 (default): square's tensor products reduce through the 2^k - delta fold when every modulus allows, and the inverse transforms feeding the BEHZ lift / floor leave n^-1 to their constants (params.h: *_n); 0: Barrett products, n^-1 in the transforms; same bytes; env CRCNN_SQ_LEAN
-    int tcn_preshift = 1;            // 1 (default): convolution weights of fan-in <= 32 are staged pre-shifted and run on the seven-class kernel (tcn_mac.cu: tcn2p_mac_kernel) when 7x the planes fit the weight cache; 0: 13-class kernel; same bytes; env CRCNN_TCN2_PRESHIFT
     int tcn_fold = 1;                // 1 (default): the limb-split GEMM reduces its class sums through the 2^k - delta shape of the primes when every prime has it (modarith.cuh: tcn_fold_reduce), 0: 128-bit recombination + Barrett; same bytes; env CRCNN_TCN_FOLD
     size_t tc_scratch_bytes = 12ull << 30;
     std::string err;
@@ -503,7 +501,8 @@ int run_weighted_sum_tcn(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn
                          int Npos, int Pimg, int m_first, int M, crcnn_tensor *out) {
     const int Kpad = tcn_kpad(R), ncols = 2 * Npos, total = ctx->K * ctx->n;
     const int variant = ctx->tcn_mode >= 2 ? ctx->tcn_mode - 1 : 0;
-    const bool want_pre = ctx->tcn_preshift && tcn_preshift_shape(R, ncols, M, variant) &&
+    // fan-in <= 32: pre-shifted weights (7x the planes) and the seven-class kernel, when they fit the weight cache
+    const bool want_pre = tcn_preshift_shape(R, ncols, M, variant) &&
                           7 * tcn_w_bytes(7, (int)(w->count / R), Kpad, ctx->K, ctx->n) <= ctx->weight_cache_bytes;
     int rc = ensure_domain(ctx, in, 1);
     if (!rc) rc = ensure_form(ctx, b, PF_NTT_ADD);
@@ -651,8 +650,6 @@ int crcnn_ctx_create(int n, int K, const uint64_t *q, uint64_t t, int device, cr
     if (const char *e = getenv("CRCNN_TCN")) c->tcn_mode = atoi(e);
     if (const char *e = getenv("CRCNN_TAP")) c->tap_mode = atoi(e);
     if (const char *e = getenv("CRCNN_TCN_FOLD")) c->tcn_fold = atoi(e);
-    if (const char *e = getenv("CRCNN_TCN2_PRESHIFT")) c->tcn_preshift = atoi(e);
-    if (const char *e = getenv("CRCNN_SQ_LEAN")) c->sq_lean = atoi(e);
     // stream-ordered allocator: keep freed blocks cached
     cudaMemPool_t pool;
     if (cudaDeviceGetDefaultMemPool(&pool, device) == cudaSuccess) {
@@ -1610,9 +1607,9 @@ int crcnn_square(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_tensor **out3) {
     // An NTT-form input (the usual case: the convolution before the activation leaves NTT form) keeps its transformed q
     // limbs: the base conversion works on an inverse-transformed COPY, and only the Bsk limbs are transformed again.
     const bool have_ntt = in->ntt != 0;
-    // lean: the tensor stage leaves n^-1 to the floor's constants (and reduces on the fold where it applies); so does the INTT copy
+    // The tensor stage leaves n^-1 to the floor's constants (and reduces on the fold where it applies); so does the INTT copy
     // to the lift's -- not a coefficient-form input, whose q limbs the lift copies into ext unscaled
-    const bool lean = ctx->sq_lean != 0, fold = lean && behz_fold_ok(ctx->hp.d), copy_ninv = !(lean && have_ntt);
+    const bool fold = behz_fold_ok(ctx->hp.d);
     crcnn_tensor *o = nullptr;
     int rc = new_tensor(ctx, in->count, 3, 0, &o);
     if (rc) return rc;
@@ -1632,9 +1629,9 @@ int crcnn_square(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_tensor **out3) {
         if (have_ntt) {
             ProfScope ps(ctx, KC_NTT_INV, 2 * lp_bytes(ctx, (double)cur * 2 * ctx->K), lp_bfly(ctx, (double)cur * 2 * ctx->K));
             e = launch_ntt_grouped(ctx->dP, ctx->logn, coef, cur * 2 * ctx->K, 0, ctx->K, true, ctx->K, 0, ctx->stream, src,  // out of place
-                                   nullptr, 1, 1, copy_ninv);
+                                   nullptr, 1, 1, false);
         }
-        if (e == cudaSuccess) { ProfScope ps(ctx, KC_BEHZ_LIFT, lp_bytes(ctx, (double)cur * 2 * (ctx->K + (have_ntt ? ctx->S : KS))), (double)cur * 2 * n * ctx->S * (ctx->K + 1)); e = launch_behz_lift(ctx->hp.d, ctx->n, have_ntt ? coef : src, have_ntt ? src : nullptr, cur, ext, ctx->stream, copy_ninv); }
+        if (e == cudaSuccess) { ProfScope ps(ctx, KC_BEHZ_LIFT, lp_bytes(ctx, (double)cur * 2 * (ctx->K + (have_ntt ? ctx->S : KS))), (double)cur * 2 * n * ctx->S * (ctx->K + 1)); e = launch_behz_lift(ctx->hp.d, ctx->n, have_ntt ? coef : src, have_ntt ? src : nullptr, cur, ext, ctx->stream, !have_ntt); }
         if (e == cudaSuccess) {
             if (have_ntt) {   // Bsk limbs only
                 ProfScope ps(ctx, KC_NTT_FWD, 2 * lp_bytes(ctx, (double)cur * 2 * ctx->S), lp_bfly(ctx, (double)cur * 2 * ctx->S));
@@ -1647,10 +1644,10 @@ int crcnn_square(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_tensor **out3) {
         if (e == cudaSuccess) {
             // tensor products formed while the inverse transform loads its polynomial (bytes: 2 inputs + 3 outputs per limb)
             ProfScope ps(ctx, KC_SQ_TENSOR, lp_bytes(ctx, (double)cur * 5 * KS), lp_bfly(ctx, (double)cur * 3 * KS));
-            e = launch_ntt_inv_tensor(ctx->dP, ctx->logn, ext, have_ntt ? src : nullptr, cur, KS, prod, fold, !lean, ctx->stream);
+            e = launch_ntt_inv_tensor(ctx->dP, ctx->logn, ext, have_ntt ? src : nullptr, cur, KS, prod, fold, ctx->stream);
         }
         if (e == cudaSuccess) { ProfScope ps(ctx, KC_BEHZ_FLOOR, lp_bytes(ctx, (double)cur * 3 * (KS + ctx->K)),
-                                                     (double)cur * 3 * n * (ctx->S * (ctx->K + 1) + ctx->S + ctx->K * ctx->S)); e = launch_behz_floor(ctx->hp.d, ctx->n, prod, cur, o->d + c0 * 3 * pw, ctx->stream, !lean); }
+                                                     (double)cur * 3 * n * (ctx->S * (ctx->K + 1) + ctx->S + ctx->K * ctx->S)); e = launch_behz_floor(ctx->hp.d, ctx->n, prod, cur, o->d + c0 * 3 * pw, ctx->stream); }
         if (e != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
     }
     dev_free(ctx, coef);

@@ -133,7 +133,8 @@ int main(int argc, char **argv) {
                 if (reduce128_fold(z, f) != want || barrett128(z, m) != want) { printf("FOLD128 MISMATCH\n"); return 1; }
             }
         }
-        // square without n^-1 in its inverse transforms: the lift / floor constants that absorb it (params.h: *_n)
+        // square without n^-1 in its inverse transforms: the lift / floor constants that absorb it (params.h: mt_inv_qhat_n, fl_c,
+        // fl_T), times n against their definitions
         typedef unsigned __int128 u128;
         for (int s = 0; s < d.K + d.S; s++) {
             const uint64_t q = d.tab[s].mod.q;
@@ -141,9 +142,11 @@ int main(int argc, char **argv) {
             bool ok = ok_ninv;
             if (s < d.K) {
                 ok = ok && d.mt_inv_qhat_n[s] < q && (u128)d.mt_inv_qhat_n[s] * (uint64_t)n % q == d.mt_inv_qhat[s];
-                ok = ok && d.fl_c_n[s] < q && (u128)d.fl_c_n[s] * (uint64_t)n % q == d.fl_c[s];
+                ok = ok && d.fl_c[s] < q && (u128)d.fl_c[s] * (uint64_t)n % q == (u128)(d.t % q) * d.inv_qhat[s] % q;
             } else {
-                ok = ok && d.fl_T_n[s - d.K] < q && (u128)d.fl_T_n[s - d.K] * (uint64_t)n % q == d.fl_T[s - d.K];
+                const int k = s - d.K;
+                const uint64_t fold = k < d.L ? (uint64_t)((u128)d.inv_q_mod_bsk[k] * d.inv_Mhat[k] % q) : d.inv_q_mod_bsk[k];
+                ok = ok && d.fl_T[k] < q && (u128)d.fl_T[k] * (uint64_t)n % q == (u128)(d.t % q) * fold % q;
             }
             printf("ninv %d ok %d\n", s, ok ? 1 : 0);
             if (!ok) { printf("NINV CONSTANT MISMATCH\n"); return 1; }

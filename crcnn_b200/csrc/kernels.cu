@@ -2,7 +2,6 @@
 #include "kernels.cuh"
 #include "devcfg.cuh"
 #include "ntt.cuh"
-#include <cstdlib>
 #include <cstring>
 
 namespace crcnn {
@@ -42,7 +41,7 @@ ntt_inv_kernel(uint64_t *__restrict__ data, const DeviceParams *__restrict__ P, 
 // (coefficient primes, the 61-bit Bsk primes and m_sk; modarith.cuh: reduce128_fold, host-checked against unsigned __int128 in
 // host_selftest.cpp); its constants are derived from q on the spot (5 instructions).  The launcher takes it only when
 // fold128_make(q).ok holds for EVERY modulus of the context (caller-supplied primes of another shape get the generic 128-bit
-// Barrett step); env CRCNN_BEHZ_FOLD=0 forces Barrett.  Measured on B200 (profiles/r02a_first.txt): behz_lift 9.0 -> 7.8 ms,
+// Barrett step).  Measured on B200 (profiles/r02a_first.txt): behz_lift 9.0 -> 7.8 ms,
 // behz_floor 21.2 -> 18.0 ms per step of the bench network; both give the canonical residue, i.e. the same bytes.
 template <bool FOLD>
 __device__ __forceinline__ uint64_t behz_reduce(U128 z, const Mod &m) {
@@ -62,9 +61,9 @@ __device__ __forceinline__ uint64_t behz_mulmod(uint64_t a, uint64_t b, const Mo
 // forms c0*c0 (k = 0), 2*c0*c1 (k = 1) or c1*c1 (k = 2) mod the j-th prime of q U Bsk while loading, then inverse-transforms it.
 // Saves the write and re-read of the 3(K+S) product polynomials of every ciphertext.
 // FOLD: products reduced by behz_reduce<true> (three folds through 2^k - delta, 6 IMAD.WIDE) instead of barrett128 (~18 multiplier
-// instructions); a square takes 3 32x32 partial products instead of 4.  NINV = false: the output is left multiplied by n (the
-// floor kernel's constants carry n^-1, params.h: fl_c_n / fl_T_n).  Every variant stores the same canonical residues up to that factor.
-template <int LOGN, bool FOLD, bool NINV>
+// instructions); a square takes 3 32x32 partial products instead of 4.  The output is left multiplied by n (the floor kernel's
+// constants carry n^-1, params.h: fl_c / fl_T).
+template <int LOGN, bool FOLD>
 __global__ void __launch_bounds__(NttPlan<LOGN>::THREADS, NttPlan<LOGN>::MIN_CTAS)
 ntt_inv_tensor_kernel(const DeviceParams *__restrict__ P, const uint64_t *__restrict__ ext, const uint64_t *__restrict__ qntt, int KS,
                       uint64_t *__restrict__ prod) {
@@ -102,15 +101,15 @@ ntt_inv_tensor_kernel(const DeviceParams *__restrict__ P, const uint64_t *__rest
         }
     }
     __syncthreads();
-    ntt_inverse_from_smem<LOGN, NINV>(sm, prod + b * N, tb);
+    ntt_inverse_from_smem<LOGN, false>(sm, prod + b * N, tb);
 }
 
-template <int LOGN, bool FOLD, bool NINV>
+template <int LOGN, bool FOLD>
 static cudaError_t launch_ntt_inv_tensor_t(const DeviceParams *P, const uint64_t *ext, const uint64_t *qntt, long count, int KS, uint64_t *prod,
                                            cudaStream_t stream) {
     using Pl = NttPlan<LOGN>;
     const size_t smem = Pl::SMEM_WORDS * sizeof(uint64_t);
-    auto kf = ntt_inv_tensor_kernel<LOGN, FOLD, NINV>;
+    auto kf = ntt_inv_tensor_kernel<LOGN, FOLD>;
     static DeviceOnce once;
     if (once.first()) {
         cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -122,22 +121,20 @@ static cudaError_t launch_ntt_inv_tensor_t(const DeviceParams *P, const uint64_t
 
 template <int LOGN>
 static cudaError_t launch_ntt_inv_tensor_l(const DeviceParams *P, const uint64_t *ext, const uint64_t *qntt, long count, int KS, uint64_t *prod,
-                                           bool fold, bool ninv, cudaStream_t stream) {
-    if (!ninv) return fold ? launch_ntt_inv_tensor_t<LOGN, true, false>(P, ext, qntt, count, KS, prod, stream)
-                           : launch_ntt_inv_tensor_t<LOGN, false, false>(P, ext, qntt, count, KS, prod, stream);
-    if (fold) return cudaErrorInvalidValue;   // not instantiated: the folded products come only with the n^-1-free output
-    return launch_ntt_inv_tensor_t<LOGN, false, true>(P, ext, qntt, count, KS, prod, stream);
+                                           bool fold, cudaStream_t stream) {
+    return fold ? launch_ntt_inv_tensor_t<LOGN, true>(P, ext, qntt, count, KS, prod, stream)
+                : launch_ntt_inv_tensor_t<LOGN, false>(P, ext, qntt, count, KS, prod, stream);
 }
 
 cudaError_t launch_ntt_inv_tensor(const DeviceParams *P, int logn, const uint64_t *ext, const uint64_t *qntt, long count, int KS, uint64_t *prod,
-                                  bool fold, bool ninv, cudaStream_t stream) {
+                                  bool fold, cudaStream_t stream) {
     if (count <= 0) return cudaSuccess;
     switch (logn) {
-        case 10: return launch_ntt_inv_tensor_l<10>(P, ext, qntt, count, KS, prod, fold, ninv, stream);
-        case 11: return launch_ntt_inv_tensor_l<11>(P, ext, qntt, count, KS, prod, fold, ninv, stream);
-        case 12: return launch_ntt_inv_tensor_l<12>(P, ext, qntt, count, KS, prod, fold, ninv, stream);
-        case 13: return launch_ntt_inv_tensor_l<13>(P, ext, qntt, count, KS, prod, fold, ninv, stream);
-        case 14: return launch_ntt_inv_tensor_l<14>(P, ext, qntt, count, KS, prod, fold, ninv, stream);
+        case 10: return launch_ntt_inv_tensor_l<10>(P, ext, qntt, count, KS, prod, fold, stream);
+        case 11: return launch_ntt_inv_tensor_l<11>(P, ext, qntt, count, KS, prod, fold, stream);
+        case 12: return launch_ntt_inv_tensor_l<12>(P, ext, qntt, count, KS, prod, fold, stream);
+        case 13: return launch_ntt_inv_tensor_l<13>(P, ext, qntt, count, KS, prod, fold, stream);
+        case 14: return launch_ntt_inv_tensor_l<14>(P, ext, qntt, count, KS, prod, fold, stream);
         default: return cudaErrorInvalidValue;
     }
 }
@@ -389,19 +386,6 @@ static cudaError_t launch_mac_t(const DeviceParams *P, const MacArgs &a, cudaStr
 
 cudaError_t launch_mac(const DeviceParams *P, const MacArgs &a, cudaStream_t stream) {
     if (a.M <= 0 || a.Npos <= 0) return cudaSuccess;
-    // tile override for tuning sweeps: CRCNN_MAC_TILE=<TM><TN>, e.g. 22
-    static const int forced = [] { const char *e = getenv("CRCNN_MAC_TILE"); return e ? atoi(e) : 0; }();
-    switch (forced) {
-        case 42: return launch_mac_t<4, 2>(P, a, stream);
-        case 22: return launch_mac_t<2, 2>(P, a, stream);
-        case 24: return launch_mac_t<2, 4>(P, a, stream);
-        case 41: return launch_mac_t<4, 1>(P, a, stream);
-        case 21: return launch_mac_t<2, 1>(P, a, stream);
-        case 81: return launch_mac_t<8, 1>(P, a, stream);
-        case 12: return launch_mac_t<1, 2>(P, a, stream);
-        case 14: return launch_mac_t<1, 4>(P, a, stream);
-        default: break;
-    }
     if (a.Npos == 1) return launch_mac_t<4, 1>(P, a, stream);
     return launch_mac_t<2, 2>(P, a, stream);
 }
@@ -1122,8 +1106,6 @@ cudaError_t launch_plain_op(const DeviceParams *P, int n, int K, uint64_t *data,
 
 // every modulus the BEHZ kernels reduce by (coefficient primes, Bsk primes incl. m_sk) has the 2^k - delta shape reduce128_fold needs
 bool behz_fold_ok(const DeviceParams &hp) {
-    static const int env = [] { const char *e = getenv("CRCNN_BEHZ_FOLD"); return e ? atoi(e) : 1; }();
-    if (!env) return false;
     for (int i = 0; i < hp.K + hp.S; i++)
         if (!fold128_make(hp.tab[i].mod.q).ok) return false;
     return true;
@@ -1146,16 +1128,8 @@ cudaError_t launch_behz_lift(const DeviceParams &P, int n, const uint64_t *in, c
     return cudaGetLastError();
 }
 
-cudaError_t launch_behz_floor(const DeviceParams &P, int n, const uint64_t *prod, long count, uint64_t *out,
-                                 cudaStream_t stream, bool ninv_in) {
+cudaError_t launch_behz_floor(const DeviceParams &hp, int n, const uint64_t *prod, long count, uint64_t *out, cudaStream_t stream) {
     if (count <= 0) return cudaSuccess;
-    DeviceParams scaled;
-    if (!ninv_in) {
-        scaled = P;
-        std::memcpy(scaled.fl_c, P.fl_c_n, sizeof scaled.fl_c);
-        std::memcpy(scaled.fl_T, P.fl_T_n, sizeof scaled.fl_T);
-    }
-    const DeviceParams &hp = ninv_in ? P : scaled;
     const unsigned grid = (unsigned)(count * 3 * (n / 128));
     CRCNN_BEHZ_DISPATCH(behz_floor_kernel, grid, prod, out);
     return cudaGetLastError();

@@ -98,9 +98,8 @@ cudaError_t launch_plain_op(const DeviceParams *P, int n, int K, uint64_t *data,
 cudaError_t launch_behz_lift(const DeviceParams &hp, int n, const uint64_t *in, const uint64_t *in_ntt, long count, uint64_t *ext,
                              cudaStream_t stream, bool ninv_in = true);
 // floor:  prod (coefficient form) -> out [count][3][K][n]: multiply by t, fast_floor, fastbconv_sk
-// ninv_in = false: prod holds n times the products (launch_ntt_inv_tensor with ninv = false); fl_c_n / fl_T_n absorb the factor.
-cudaError_t launch_behz_floor(const DeviceParams &hp, int n, const uint64_t *prod, long count, uint64_t *out, cudaStream_t stream,
-                              bool ninv_in = true);
+// prod holds n times the products (launch_ntt_inv_tensor); fl_c / fl_T absorb the factor.
+cudaError_t launch_behz_floor(const DeviceParams &hp, int n, const uint64_t *prod, long count, uint64_t *out, cudaStream_t stream);
 // true when every modulus of the context (q and Bsk) has the 2^k - delta shape of reduce128_fold (modarith.cuh)
 bool behz_fold_ok(const DeviceParams &hp);
 
@@ -121,10 +120,10 @@ struct RelinArgs {
 // ---- tensor square (c0*c0, 2*c0*c1, c1*c1 in q U Bsk) fused into the inverse transform of each product polynomial:
 // ext = [count][2][KS][n] NTT form (qntt != null: its q limbs are taken from qntt = [count][2][K][n] instead),
 // prod = [count][3][KS][n] coefficient form
-// fold: reduce the products with reduce128_fold (requires behz_fold_ok; only with ninv = false).  ninv = false: prod holds n times
-// the products, for launch_behz_floor with ninv_in = false.
+// fold: reduce the products with reduce128_fold (requires behz_fold_ok).  prod holds n times the products (the inverse
+// transforms leave n^-1 to launch_behz_floor).
 cudaError_t launch_ntt_inv_tensor(const DeviceParams *P, int logn, const uint64_t *ext, const uint64_t *qntt, long count, int KS, uint64_t *prod,
-                                  bool fold, bool ninv, cudaStream_t stream);
+                                  bool fold, cudaStream_t stream);
 
 // stages 1-3 (scale, digit NTTs, key MAC); then the caller inverse-NTTs `acc` and calls launch_relin_finish
 cudaError_t launch_relin(const DeviceParams *P, int logn, int K, const RelinArgs &a, cudaStream_t stream);

@@ -200,23 +200,22 @@ HostParams derive_params(int n, int K, const uint64_t *q, uint64_t t) {
     }
     d.inv_M_mod_msk = inv_mod(product_mod(bsk.data(), d.L, -1, msk), kMsk);
     // folded constants (see params.h)
-    for (int j = 0; j < K; j++) d.fl_c[j] = mulmod(t % d.tab[j].mod.q, d.inv_qhat[j], d.tab[j].mod);
+    for (int j = 0; j < K; j++) {
+        const Mod &m = d.tab[j].mod;
+        d.fl_c[j] = mulmod(mulmod(t % m.q, d.inv_qhat[j], m), d.tab[j].ninv, m);
+        d.mt_inv_qhat_n[j] = mulmod(d.mt_inv_qhat[j], d.tab[j].ninv, m);
+    }
     for (int k = 0; k < d.S; k++) {
         const Mod &m = d.tab[K + k].mod;
         const uint64_t fold = k < d.L ? mulmod(d.inv_q_mod_bsk[k], d.inv_Mhat[k], m) : d.inv_q_mod_bsk[k];
         d.lift_b[k] = mulmod(d.q_mod_bsk[k], d.inv_mt_mod_bsk[k], m);
-        d.fl_T[k] = mulmod(t % m.q, fold, m);
+        d.fl_T[k] = mulmod(mulmod(t % m.q, fold, m), d.tab[K + k].ninv, m);
         for (int i = 0; i < K; i++) {
             d.lift_a[k][i] = mulmod(d.qhat_mod_bsk[k][i], d.inv_mt_mod_bsk[k], m);
             d.fl_N[k][i] = negmod(mulmod(d.qhat_mod_bsk[k][i], fold, m), m.q);
         }
     }
     for (int i = 0; i < d.L; i++) d.fl_P[i] = mulmod(d.Mhat_mod_msk[i], d.inv_M_mod_msk, msk);
-    for (int j = 0; j < K; j++) {
-        d.mt_inv_qhat_n[j] = mulmod(d.mt_inv_qhat[j], d.tab[j].ninv, d.tab[j].mod);
-        d.fl_c_n[j] = mulmod(d.fl_c[j], d.tab[j].ninv, d.tab[j].mod);
-    }
-    for (int k = 0; k < d.S; k++) d.fl_T_n[k] = mulmod(d.fl_T[k], d.tab[K + k].ninv, d.tab[K + k].mod);
     return hp;
 }
 

@@ -69,15 +69,14 @@ struct DeviceParams {
     // 128-bit sum followed by ONE Barrett reduction (same residues, fewer reductions).
     uint64_t lift_a[MAXS][MAXK];        // (q/q_i mod p_k) * m_tilde^-1 mod p_k
     uint64_t lift_b[MAXS];              // (q mod p_k) * m_tilde^-1 mod p_k
-    uint64_t fl_c[MAXK];                // t * (q/q_i)^-1 mod q_i
-    uint64_t fl_T[MAXS];                // t * q^-1 [* (M/m_k)^-1 for k < L] mod p_k
+    uint64_t fl_c[MAXK];                // t * (q/q_i)^-1 * n^-1 mod q_i
+    uint64_t fl_T[MAXS];                // t * q^-1 [* (M/m_k)^-1 for k < L] * n^-1 mod p_k
     uint64_t fl_N[MAXS][MAXK];          // -(q/q_i mod p_k) * q^-1 [* (M/m_k)^-1 for k < L] mod p_k
     uint64_t fl_P[MAXS];                // (M/m_i mod m_sk) * M^-1 mod m_sk
-    // The same first-step constants times n^-1 (mod q_i resp. p_k): for lift / floor inputs that an inverse transform left
-    // multiplied by n (kernels.cuh: ninv_in = false), so the transform saves its n^-1 product per residue.
+    // The floor's first-step constants fl_c / fl_T carry n^-1 (mod q_i resp. p_k): its input comes from inverse transforms that
+    // leave the products multiplied by n (kernels.cuh: launch_ntt_inv_tensor), so they save their n^-1 product per residue.  The
+    // lift takes the same saving through this copy of mt_inv_qhat when its input is such a transform (kernels.cuh: ninv_in = false).
     uint64_t mt_inv_qhat_n[MAXK];       // mt_inv_qhat * n^-1 mod q_i
-    uint64_t fl_c_n[MAXK];              // fl_c * n^-1 mod q_i
-    uint64_t fl_T_n[MAXS];              // fl_T * n^-1 mod p_k
 };
 
 // Host copy: the scalar part of DeviceParams plus the tables as vectors.

@@ -4,7 +4,6 @@
 #include "devcfg.cuh"
 #include "modarith.cuh"
 #include <cmath>
-#include <cstdlib>
 #include <vector>
 
 namespace crcnn {
@@ -48,9 +47,7 @@ struct Plan32 {
     static constexpr int N = 1 << LOGN;
     static constexpr int THREADS = N / 32 < 32 ? 32 : N / 32;
     static constexpr int SMEM_WORDS = N + N / 8;
-#ifndef R32_TPS
-#define R32_TPS 1024  // resident threads per SM the register budget is sized for (64 registers per thread; measured 6 % faster than 768 -> 85)
-#endif
+    static constexpr int R32_TPS = 1024;  // resident threads per SM the register budget is sized for (64 registers per thread; measured 6 % faster than 768 -> 85)
     static constexpr int MIN_CTAS = R32_TPS / THREADS > 16 ? 16 : (R32_TPS / THREADS < 1 ? 1 : R32_TPS / THREADS);
     static constexpr int LAST = 5;
     static constexpr int REST = LOGN - LAST;
@@ -721,11 +718,10 @@ cudaError_t run_t(const DeviceParams *dP, int K, const Relin32 &r, const uint64_
         const unsigned gz = (unsigned)((count + cpb - 1) / cpb);
         const size_t ksmem = (size_t)c.D * 2 * K * 4;  // bytes per staged coefficient
         cudaError_t e = cudaSuccess;
-        const bool generic = std::getenv("CRCNN_R32_GENERIC_MAC") != nullptr;  // A/B switch for tools/ntt_ab.py
-        if (!generic && c.D == 4 * K && K == 1) e = launch_mac_reg<4, 2>(dig, r, N, count, cpb, gz, acc, stream);
-        else if (!generic && c.D == 4 * K && K == 2) e = launch_mac_reg<8, 4>(dig, r, N, count, cpb, gz, acc, stream);
-        else if (!generic && c.D == 4 * K && K == 4) e = launch_mac_reg<16, 8>(dig, r, N, count, cpb, gz, acc, stream);
-        else if (!generic && c.D == 4 * K && K == 8) e = launch_mac_reg<32, 16>(dig, r, N, count, cpb, gz, acc, stream);
+        if (c.D == 4 * K && K == 1) e = launch_mac_reg<4, 2>(dig, r, N, count, cpb, gz, acc, stream);
+        else if (c.D == 4 * K && K == 2) e = launch_mac_reg<8, 4>(dig, r, N, count, cpb, gz, acc, stream);
+        else if (c.D == 4 * K && K == 4) e = launch_mac_reg<16, 8>(dig, r, N, count, cpb, gz, acc, stream);
+        else if (c.D == 4 * K && K == 8) e = launch_mac_reg<32, 16>(dig, r, N, count, cpb, gz, acc, stream);
         else
         switch (2 * K) {
             case 2: e = launch_mac<4, 2, 64>(dig, r, N, count, cpb, gz, ksmem, acc, stream); break;
@@ -737,10 +733,8 @@ cudaError_t run_t(const DeviceParams *dP, int K, const Relin32 &r, const uint64_
         if (e != cudaSuccess) return e;
     }
     if constexpr (LOGN <= 13) {
-        // fused inverse transform + reconstruction: 43.1 -> 41.4 ms per step of the headline network (two CTAs of 8 warps per SM hold it back);
-        // CRCNN_R32_FUSED=0 selects the two-kernel form (same bytes)
-        static const bool fused = !(std::getenv("CRCNN_R32_FUSED") && std::atoi(std::getenv("CRCNN_R32_FUSED")) == 0);
-        if (fused && c.S3 == 3) {
+        // fused inverse transform + reconstruction: 43.1 -> 41.4 ms per step of the headline network (two CTAs of 8 warps per SM hold it back)
+        if (c.S3 == 3) {
             static DeviceOnce once3;
             const int smem3 = 3 * Pl::SMEM_WORDS * 4;
             if (once3.first()) {

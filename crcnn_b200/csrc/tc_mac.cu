@@ -2,7 +2,6 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <cstdio>
-#include <cstdlib>
 #include "devcfg.cuh"
 #include "modarith.cuh"
 #include "tc_mac.cuh"
@@ -20,13 +19,15 @@ constexpr int TC_SCRATCH_WARP = 64 * 32 * 4;
 using namespace tcptx;
 
 // ------------------------------------------------------------------------------------ the GEMM kernel
-// SUB = K blocks of 128 bytes per ring stage (one barrier flip and one tcgen05.commit per stage): 1 -> 4 stages of 44 KB, 2 -> 2 stages of 88 KB
-template <int PLANES, int SUB = 1>
+template <int PLANES>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 tc_mac_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
               const DeviceParams *__restrict__ P, TcMacArgs a) {
     constexpr int N = PLANES * TC_CB;               // UMMA N: 224 or 256
     constexpr int B_BLK = N * TC_BK;                // 28 / 32 KB
+    // two 128-byte K blocks per ring stage (2 stages of 88 KB, half as many barrier flips and tcgen05.commits as four stages of
+    // 44 KB): fc3 of the bench 64.8 -> 62.1 ms on B200
+    constexpr int SUB = 2;
     constexpr int TC_STAGES = 4 / SUB;
     constexpr int NACC = 2;                                 // accumulators in tensor memory
     constexpr uint32_t TMEM_COLS = 512;
@@ -202,204 +203,6 @@ tc_mac_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
     if (warp == 0) tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
-// ------------------------------------------------------------------------------------ the GEMM kernel, CTA pairs
-// Same GEMM on pairs of SMs (clusters of two CTAs, tcgen05.mma.cta_group::2, M = 256): the pair works on TWO neighbouring row
-// tiles (8 outputs) of one limb-polynomial.  Each CTA stages its own 128 rows of A and only HALF of every B tile (16 of the 32
-// coefficients of each plane), so a K block costs a CTA 16 + 14 KB of shared-memory fill instead of 16 + 28 KB for the same
-// number of multiply-accumulates -- the one-CTA kernel is bound by exactly that traffic (ncu: tensor pipe 58 % active, epilogue
-// and MMA warps waiting for the TMA ring; 44 KB per 476 tensor-clocks = 92 B/clk/SM at full rate).  The smaller stages also allow
-// a 6-deep ring.  N index of the pair's tile: (coefficient half, plane, coefficient mod 16), i.e. the 7 x 16 rows CTA 0 loaded
-// followed by CTA 1's; each CTA's TMEM holds its own 128 rows (= its 4 outputs x 32 taps) of all N columns, so the epilogue is
-// the one-CTA epilogue with another column map.  Barriers: the leader's `full` collects the transaction bytes of both CTAs'
-// loads, tcgen05.commit multicasts `empty` / `tfull` to both CTAs, the epilogue warps of both CTAs arrive on the leader's `tempty`.
-constexpr int TC2_THREADS = 192;
-
-template <int PLANES>
-struct Tc2Cfg {
-    static constexpr int NH = PLANES * (TC_CB / 2);        // N rows per CTA: 112 / 128
-    static constexpr int N = 2 * NH;                       // UMMA N: 224 / 256
-    static constexpr int B_STAGE = NH * TC_BK;             // 14 / 16 KB
-    static constexpr int STAGE = TC_A_STAGE + B_STAGE;     // 30 / 32 KB
-    static constexpr int STAGES = PLANES == 7 ? 6 : 5;
-    static constexpr size_t SMEM = 1024 + (size_t)STAGES * STAGE + 4 * TC_SCRATCH_WARP + 16 * STAGES + 32 + 16;
-};
-
-// DBG (timing builds only, results wrong by construction): 1 = epilogue does nothing but the barrier hand-shake, 2 = no MMAs are issued
-template <int PLANES, int DBG = 0>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC2_THREADS, 1)
-tc_mac2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-               const DeviceParams *__restrict__ P, TcMacArgs a) {
-    using C = Tc2Cfg<PLANES>;
-    constexpr int STAGES = C::STAGES;
-    constexpr uint32_t IDESC = (2u << 4)            // accumulator format S32
-                               | (1u << 7)          // A = signed 8 bit
-                               | (0u << 10)         // B = unsigned 8 bit
-                               | ((uint32_t)(C::N >> 3) << 17) | ((uint32_t)((2 * TC_BM) >> 4) << 24);  // K-major A and B, M = 256
-
-    extern __shared__ uint8_t smem_raw[];
-    const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    uint8_t *base_ptr = smem_raw + (base - smem_u32(smem_raw));
-    const uint32_t sA = base, sB = base + STAGES * TC_A_STAGE;
-    const uint32_t off_scratch = STAGES * C::STAGE;
-    const uint32_t off_bar = off_scratch + 4 * TC_SCRATCH_WARP;
-    const uint32_t bar_full = base + off_bar, bar_empty = bar_full + 8 * STAGES;
-    const uint32_t bar_tfull = bar_empty + 8 * STAGES, bar_tempty = bar_tfull + 16;
-    const uint32_t tmem_slot = bar_tempty + 16;
-    volatile uint32_t *tmem_slot_ptr = reinterpret_cast<volatile uint32_t *>(base_ptr + off_bar + 16 * STAGES + 32);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t rank = cluster_ctarank();
-    const int n = a.n, K = a.K;
-    const int m_tiles = a.Mpad / TC_BM, pair_tiles = (m_tiles + 1) / 2;
-    const long items = (long)a.npos * 2 * K * pair_tiles;
-    const long cluster = blockIdx.x >> 1, nclusters = gridDim.x >> 1;
-    const int NU = n / TC_CB + 1;
-    const int ksteps = (a.R + 31) / 32;
-    const int KB = (ksteps + 3) / 4;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < STAGES; s++) { mbar_init(bar_full + 8 * s, 1); mbar_init(bar_empty + 8 * s, 1); }
-        for (int s = 0; s < 2; s++) { mbar_init(bar_tfull + 8 * s, 1); mbar_init(bar_tempty + 8 * s, 8); }
-        fence_barrier_init();
-        prefetch_tmap(&tmA);
-        prefetch_tmap(&tmB);
-    }
-    __syncthreads();
-    cluster_sync_all();                  // both CTAs' barriers exist before anything remote touches them
-    if (warp == 0) tmem_alloc_pair(tmem_slot, 512);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot_ptr;
-
-    if (warp == 0) {
-        // ===================================================================== TMA producer (both CTAs)
-        if (lane == 0) {
-            int stage = 0;
-            uint32_t phase = 0;
-            for (long item = cluster; item < items; item += nclusters) {
-                const int g = (int)(item / pair_tiles), pt = (int)(item % pair_tiles);
-                const int mt = min(2 * pt + (int)rank, m_tiles - 1);   // an odd tile count: the last pair's second half recomputes the last tile (never stored)
-                for (int u = 0; u < NU; u++)
-                    for (int kb = 0; kb < KB; kb++) {
-                        if (DBG == 3) continue;
-                        mbar_wait(bar_empty + 8 * stage, phase ^ 1);
-                        if (rank == 0) mbar_expect_tx(bar_full + 8 * stage, 2 * C::STAGE);
-                        tma_load_2d_pair(sA + stage * TC_A_STAGE, &tmA, bar_full + 8 * stage, kb * TC_BK, mt * TC_BM);
-                        tma_load_4d_pair(sB + stage * C::B_STAGE, &tmB, bar_full + 8 * stage, kb * TC_BK, u * TC_CB + (int)rank * (TC_CB / 2), 0, g);
-                        if (++stage == STAGES) { stage = 0; phase ^= 1; }
-                    }
-            }
-        }
-        __syncwarp();
-    } else if (warp == 1) {
-        // ===================================================================== MMA issuer (leader CTA only)
-        if (lane == 0 && rank == 0) {
-            int stage = 0, acc = 0;
-            uint32_t phase = 0, acc_phase = 0;
-            for (long item = cluster; item < items; item += nclusters)
-                for (int u = 0; u < NU; u++) {
-                    mbar_wait(bar_tempty + 8 * acc, acc_phase ^ 1);
-                    tc_fence_after();
-                    const uint32_t d_tmem = tmem_base + acc * TC_ACC_STRIDE;
-                    for (int kb = 0; kb < KB; kb++) {
-                        if (DBG != 3) mbar_wait(bar_full + 8 * stage, phase);
-                        tc_fence_after();
-                        const uint64_t da = umma_desc_sw128(sA + stage * TC_A_STAGE), db = umma_desc_sw128(sB + stage * C::B_STAGE);
-                        const int nks = min(4, ksteps - kb * 4);
-                        if (DBG != 2)
-                            for (int ks = 0; ks < nks; ks++)
-                                umma_i8_pair(d_tmem, da + 2 * ks, db + 2 * ks, IDESC, (kb | ks) != 0);
-                        umma_commit_pair(bar_empty + 8 * stage);
-                        if (++stage == STAGES) { stage = 0; phase ^= 1; }
-                    }
-                    umma_commit_pair(bar_tfull + 8 * acc);
-                    if ((acc ^= 1) == 0) acc_phase ^= 1;
-                }
-        }
-        __syncwarp();
-    } else {
-        // ===================================================================== epilogue (both CTAs, own row tile)
-        const int lg = warp & 3;
-        int acc = 0;
-        uint32_t acc_phase = 0;
-        for (long item = cluster; item < items; item += nclusters) {
-            const int g = (int)(item / pair_tiles), pt = (int)(item % pair_tiles);
-            const int mt = 2 * pt + (int)rank;
-            const int j = g % K, poly = (g / K) & 1, p = g / (2 * K);
-            const int m = mt * 4 + lg;
-            const bool valid = mt < m_tiles && m < a.M;
-            const Mod mod = P->tab[j].mod;
-            const int s = 85 - (64 - __clzll(mod.q));
-            const uint64_t off_lo = mod.q << s, off_hi = mod.q >> (64 - s);
-            const int pg = a.p0 + p;
-            const long oct = (long)(pg / a.Pimg) * ((long)a.Mtotal * a.Pimg) + (long)(a.m0 + m) * a.Pimg + pg % a.Pimg;
-            uint64_t *optr = a.out + ((oct * 2 + poly) * K + j) * (long)n;
-            const uint64_t *bptr = (a.bias && poly == 0 && valid) ? a.bias + ((long)m * K + j) * n : nullptr;
-            int carry[PLANES];
-#pragma unroll
-            for (int l = 0; l < PLANES; l++) carry[l] = 0;
-            for (int u = 0; u < NU; u++) {
-                mbar_wait(bar_tfull + 8 * acc, acc_phase);
-                tc_fence_after();
-                int lo[PLANES], hi[PLANES];
-#pragma unroll
-                for (int l = 0; l < PLANES; l++) {
-                    if (DBG == 1 || DBG == 3) { lo[l] = hi[l] = u; continue; }
-                    int v[32];
-                    const uint32_t t0 = tmem_base + ((uint32_t)(lg * 32) << 16) + acc * TC_ACC_STRIDE + l * (TC_CB / 2);
-                    tmem_ld16_nowait(t0, v);                 // coefficients 0..15 of plane l: CTA 0's rows of B
-                    tmem_ld16_nowait(t0 + C::NH, v + 16);    // coefficients 16..31: CTA 1's
-                    tmem_ld_wait();
-                    // diagonal sum by warp shuffles (no shared memory: the skew scratch of the one-CTA kernel competes with the TMA
-                    // writes and the UMMA operand reads for the SM's shared-memory bandwidth).  Entry (tap lane L, column cc) belongs to
-                    // row cc - L + 31 of the skewed array; lane l collects rows l (previous block, cc <= l) and l + 32 (this block,
-                    // cc > l), and for a given cc exactly one source lane qualifies: L = (cc + 31 - l) mod 32.
-                    int slo = 0, shi = 0;
-#pragma unroll
-                    for (int cc = 0; cc < 32; cc++) {
-                        const int x = __shfl_sync(0xffffffffu, v[cc], (cc + 31 - lane) & 31);
-                        if (cc > lane) shi += x; else slo += x;
-                    }
-                    lo[l] = slo;
-                    hi[l] = shi;
-                }
-                tc_fence_before();
-                __syncwarp();
-                if (lane == 0) {
-                    if (rank == 0) mbar_arrive(bar_tempty + 8 * acc); else mbar_arrive_remote(bar_tempty + 8 * acc, 0);
-                }
-                if ((acc ^= 1) == 0) acc_phase ^= 1;
-                if (u >= 1 && valid && DBG != 1 && DBG != 3) {
-                    long long v0 = 0, v1 = 0;
-#pragma unroll
-                    for (int l = 0; l < PLANES; l++) {
-                        const long long pl = (long long)(carry[l] + lo[l]);
-                        if (l < 4) v0 += pl << (8 * l); else v1 += pl << (8 * (l - 4));
-                    }
-                    U128 z;
-                    const uint64_t t_lo = (uint64_t)v1 << 32;
-                    z.lo = (uint64_t)v0 + t_lo;
-                    z.hi = (uint64_t)(v0 >> 63) + (uint64_t)(v1 >> 32) + (z.lo < t_lo);
-                    const uint64_t l2 = z.lo + off_lo;
-                    z.hi += off_hi + (l2 < off_lo);
-                    z.lo = l2;
-                    uint64_t r = barrett128(z, mod);
-                    const int c = (u - 1) * TC_CB + lane;
-                    if (bptr) r = addmod(r, __ldg(bptr + c), mod.q);
-                    optr[c] = r;
-                }
-#pragma unroll
-                for (int l = 0; l < PLANES; l++) carry[l] = hi[l];
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync_all();                  // no CTA leaves (or frees TMEM) while its peer may still signal it
-    if (warp == 0) tmem_dealloc_pair(tmem_base, 512);
-}
-
 // ------------------------------------------------------------------------------------ tensor-pipe roofline probe
 // kind::i8 UMMA peak of this GPU: one CTA per SM issues M = 128, N = 256, K = 32 tcgen05.mma instructions back to back on operand
 // tiles that stay in shared memory (no TMA, no epilogue), alternating between two TMEM accumulators.  What it measures is the
@@ -513,19 +316,15 @@ cudaError_t launch_tc_mac_t(const DeviceParams *P, const TcMacArgs &a, int sm_co
                 CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
             return cudaErrorInvalidValue;
     }
-    // two 128-byte K blocks per ring stage (2 stages of 88 KB, half as many barrier flips and commits): fc3 of the bench 64.8 -> 62.1 ms on B200; CRCNN_TC_SUB=1 = four 44 KB stages
-    static const int sub_env = [] { const char *e = getenv("CRCNN_TC_SUB"); return e ? atoi(e) : 2; }();
-    auto k = sub_env == 2 ? tc_mac_kernel<PLANES, 2> : tc_mac_kernel<PLANES, 1>;
     const size_t smem = tc_smem_bytes<PLANES>();
     static DeviceOnce once;
     if (once.first()) {
-        cudaError_t e = cudaFuncSetAttribute(tc_mac_kernel<PLANES, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(tc_mac_kernel<PLANES, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(tc_mac_kernel<PLANES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
     const long items = (long)a.npos * 2 * a.K * (a.Mpad / TC_BM);
     const unsigned grid = (unsigned)(items < sm_count ? items : sm_count);
-    k<<<grid, TC_THREADS, smem, stream>>>(tmA, tmB, P, a);
+    tc_mac_kernel<PLANES><<<grid, TC_THREADS, smem, stream>>>(tmA, tmB, P, a);
     return cudaGetLastError();
 }
 
@@ -562,65 +361,9 @@ cudaError_t launch_tc_split(const DeviceParams *P, const TcMacArgs &a, cudaStrea
     return cudaGetLastError();
 }
 
-template <int PLANES>
-cudaError_t launch_tc_mac2_t(const DeviceParams *P, const TcMacArgs &a, int sm_count, cudaStream_t stream) {
-    using C = Tc2Cfg<PLANES>;
-    EncodeTiledFn enc = encode_tiled();
-    if (!enc) return cudaErrorNotSupported;
-    CUtensorMap tmA, tmB;
-    {
-        cuuint64_t dims[2] = {(cuuint64_t)a.Kpad, (cuuint64_t)a.Mpad};
-        cuuint64_t strides[1] = {(cuuint64_t)a.Kpad};
-        cuuint32_t box[2] = {TC_BK, TC_BM}, es[2] = {1, 1};
-        if (enc(&tmA, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, (void *)a.A, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-            return cudaErrorInvalidValue;
-    }
-    {
-        const cuuint64_t rows = (cuuint64_t)a.n + 32, groups = (cuuint64_t)a.npos * 2 * a.K;
-        cuuint64_t dims[4] = {(cuuint64_t)a.Kpad, rows, (cuuint64_t)PLANES, groups};
-        cuuint64_t strides[3] = {(cuuint64_t)a.Kpad, rows * a.Kpad, rows * a.Kpad * PLANES};
-        cuuint32_t box[4] = {TC_BK, TC_CB / 2, PLANES, 1}, es[4] = {1, 1, 1, 1};
-        if (enc(&tmB, CU_TENSOR_MAP_DATA_TYPE_UINT8, 4, (void *)a.B, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-            return cudaErrorInvalidValue;
-    }
-    static const int dbg_env = [] { const char *e = getenv("CRCNN_TC_DEBUG"); return e ? atoi(e) : 0; }();
-    auto k = dbg_env == 1 ? tc_mac2_kernel<PLANES, 1> : dbg_env == 2 ? tc_mac2_kernel<PLANES, 2> : dbg_env == 3 ? tc_mac2_kernel<PLANES, 3> : tc_mac2_kernel<PLANES, 0>;
-    static DeviceOnce once;
-    static int max_clusters[64];
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaLaunchConfig_t cfg{};
-    cfg.blockDim = dim3(TC2_THREADS);
-    cfg.dynamicSmemBytes = C::SMEM;
-    cfg.stream = stream;
-    if (once.first()) {
-        cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM);
-        if (e != cudaSuccess) return e;
-        cfg.gridDim = dim3((unsigned)(sm_count & ~1));
-        int nc = 0;
-        e = cudaOccupancyMaxActiveClusters(&nc, k, &cfg);      // pairs that can be co-resident (a GPC with an odd SM count strands one SM)
-        max_clusters[dev & 63] = (e == cudaSuccess && nc > 0) ? nc : sm_count / 2;
-    }
-    const int m_tiles = a.Mpad / TC_BM;
-    const long items = (long)a.npos * 2 * a.K * ((m_tiles + 1) / 2);
-    const long clusters = items < max_clusters[dev & 63] ? items : max_clusters[dev & 63];
-    cfg.gridDim = dim3((unsigned)(2 * clusters));
-    return cudaLaunchKernelEx(&cfg, k, tmA, tmB, P, a);
-}
-
 cudaError_t launch_tc_mac(const DeviceParams *P, const TcMacArgs &a, int sm_count, cudaStream_t stream) {
     if (a.npos <= 0 || a.M <= 0) return cudaSuccess;
     if (a.Kpad % TC_BK || a.Mpad % TC_BM || a.n % TC_CB || (long)a.npos * 2 * a.K > 65535) return cudaErrorInvalidValue;
-    // CRCNN_TC_PAIR=1: CTA pairs (tcgen05 cta_group::2, tc_mac2_kernel) for layers with at least two row tiles.  Bit-exact (tests/
-    // test_gpu_tc.py runs it), but NOT faster on B200 (fc3 of the bench: 67.0 vs 66.1 ms), so the one-CTA kernel stays the default;
-    // DESIGN.md section 6 has the measurements that rule out operand traffic as this GEMM's limiter.
-    static const int pair_env = [] { const char *e = getenv("CRCNN_TC_PAIR"); return e ? atoi(e) : 0; }();
-    if (pair_env && a.Mpad / TC_BM >= 2) {
-        if (a.planes == 7) return launch_tc_mac2_t<7>(P, a, sm_count, stream);
-        if (a.planes == 8) return launch_tc_mac2_t<8>(P, a, sm_count, stream);
-    }
     if (a.planes == 7) return launch_tc_mac_t<7>(P, a, sm_count, stream);
     if (a.planes == 8) return launch_tc_mac_t<8>(P, a, sm_count, stream);
     return cudaErrorInvalidValue;

@@ -102,74 +102,6 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, int (&v)[32]) {
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-
-// 16 consecutive 32-bit columns of this warp's 32 TMEM lanes (no wait: pair with tmem_ld_wait)
-__device__ __forceinline__ void tmem_ld16_nowait(uint32_t taddr, int *v) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-          "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr)
-        : "memory");
-}
-
-// ---- CTA pairs (cta_group::2): two CTAs of a cluster of 2 run one M = 256 UMMA; the leader (cluster rank 0) issues it,
-// each CTA stages its own 128 rows of A and its half of B's N rows in its own shared memory, at identical offsets.
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// shared::cta addresses of the two CTAs of a pair differ in bit 24 of the shared::cluster window; clearing it names the leader's copy
-constexpr uint32_t PAIR_LEADER_MASK = 0xFEFFFFFFu;
-__device__ __forceinline__ void tma_load_2d_pair(uint32_t dst, const CUtensorMap *map, uint32_t bar, int c0, int c1) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(dst),
-        "l"(map), "r"(bar & PAIR_LEADER_MASK), "r"(c0), "r"(c1)
-        : "memory");
-}
-__device__ __forceinline__ void tma_load_4d_pair(uint32_t dst, const CUtensorMap *map, uint32_t bar, int c0, int c1, int c2, int c3) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];" ::"r"(dst),
-        "l"(map), "r"(bar & PAIR_LEADER_MASK), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_pair(uint32_t dst_smem, uint32_t cols) {   // one warp of EACH CTA of the pair
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t cols) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-__device__ __forceinline__ void umma_i8_pair(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-        "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// arrives (once the MMAs issued so far have completed) on the barrier at this offset in BOTH CTAs of the pair
-__device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-                 "h"((uint16_t)3)
-                 : "memory");
-}
-// arrive on the barrier at the same offset in CTA `rank` of the cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t bar, uint32_t rank) {
-    asm volatile(
-        "{\n\t.reg .b32 ra;\n\t"
-        "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-        "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}" ::"r"(bar),
-        "r"(rank)
-        : "memory");
-}
-
 // 4 consecutive 32-bit columns of this warp's 32 TMEM lanes
 __device__ __forceinline__ void tmem_ld4(uint32_t taddr, uint32_t (&v)[4]) {
     asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];"

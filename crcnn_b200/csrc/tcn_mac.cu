@@ -3,7 +3,6 @@
 #include <cuda_runtime.h>
 #include <algorithm>
 #include <cstdio>
-#include <cstdlib>
 #include "devcfg.cuh"
 #include "modarith.cuh"
 #include "tc_ptx.cuh"
@@ -246,18 +245,15 @@ __device__ int g_tcn2_trace_n[3];
 template <int BK> struct Tcn2Cfg {
     static constexpr int W_BLOCK = TCN_PLANES * TCN2_MT * BK;   // weight planes of one K block: [7][32][BK]
     static constexpr int X_STAGE = TCN2_CB * BK;                // one input plane of one K block: [128][BK]
-#ifndef TCN2_STAGES_SMALL
-#define TCN2_STAGES_SMALL 8
-#define TCN2_STAGES_BIG 6
-#endif
+    static constexpr int NS = BK == 32 ? 4 : 1;                 // consecutive slots per work item (see tcn2_mac_kernel)
     // ring depth: measured on B200, 40 / 9 stages instead of 8 / 6 made conv1 slower (42.6 -> 62.8 ms) and left conv2 unchanged,
     // although 39 % of the samples of the 8-stage kernel wait on the accumulator-full barrier (profiles/r01f_ncu_source_top.txt)
-    static constexpr int STAGES = BK == 128 ? TCN2_STAGES_BIG : TCN2_STAGES_SMALL;
+    static constexpr int STAGES = BK == 128 ? 6 : 8;
     static constexpr size_t BARS = (8 * (2 * STAGES + 4) + 16 + 127) / 128 * 128;   // barriers + TMEM slot, padded so that the output staging is 128-byte aligned
-    // staged: results of the first ns - 1 slots of an item wait in shared memory, [slot][output][column] words, for the whole-sector store
-    static constexpr size_t smem(int ns, bool staged) {
-        const size_t ops = 1024 + (size_t)ns * TCN2_KBMAX * W_BLOCK + (size_t)STAGES * X_STAGE;
-        return staged ? ops + BARS + (size_t)(ns - 1) * TCN2_MT * TCN2_CB * 8 : ops + 8 * (2 * STAGES + 4) + 16;
+    // staged: results of the first NS - 1 slots of an item wait in shared memory, [slot][output][column] words, for the whole-sector store
+    static constexpr size_t smem(bool staged) {
+        const size_t ops = 1024 + (size_t)NS * TCN2_KBMAX * W_BLOCK + (size_t)STAGES * X_STAGE;
+        return staged ? ops + BARS + (size_t)(NS - 1) * TCN2_MT * TCN2_CB * 8 : ops + 8 * (2 * STAGES + 4) + 16;
     }
 };
 
@@ -266,22 +262,19 @@ __device__ __forceinline__ void tcn_store_sector(uint64_t *p, uint64_t a, uint64
     asm volatile("st.global.v4.u64 [%0], {%1, %2, %3, %4};" ::"l"(p), "l"(a), "l"(b), "l"(c), "l"(d) : "memory");
 }
 
-// BIAS: 0 = the bias residue of an output is loaded where it is added; 1 = lane m fetches the bias of output m once per item and
-// the loop broadcasts it by shuffle; 2 = as 1 with the output stores dropped (timing experiments only, results are not written).
-// Measured on B200 (PlainModel.h5, batch 8): BIAS 1 takes conv2 (BK 128) from 35.3 to 33.4 ms and conv1 (BK 32) from 42.5 to 70 ms,
-// so the launcher uses 1 for BK 128 and 0 for BK 32 (DESIGN.md section 6 on why conv1 dislikes a quicker epilogue).
-// NS: consecutive slots per work item.  1 = one slot per item (what every measured number of round 1 is).  4 (EXPERIMENTAL: six parity tests
-// at n = 2048 and one timing run on B200 so far, conv1 36 ms against 24 ms for the shipped kernel; CRCNN_TCN2_NS=4, BK 32 only) = the four slots of one 32-byte output sector belong to ONE item, loop order chunk-outer /
-// slot-inner with the four slots' weight planes resident, so a sector's four 8-byte writes come from the same thread a few microseconds apart
-// instead of from four CTAs that have to stay in step (DESIGN.md section 6, "Correction").
-// STAGED (NS = 4 only; NOT YET RUN ON HARDWARE, CRCNN_TCN2_STAGE=1): the results of slots 0-2 wait in shared memory (each thread reads back
-// only what it wrote, no synchronisation) and slot 3 writes all four as ONE 32-byte sector per (column, output): a quarter of the sector writes.
-template <int BK, bool FOLD, int BIAS, int NS, bool STAGED = false>
+// NS = Tcn2Cfg<BK>::NS consecutive slots per work item.  BK 128 (fan-in > 32): one slot per item.  BK 32 (fan-in <= 32: conv1):
+// the four slots of one 32-byte output sector belong to ONE item, loop order chunk-outer / slot-inner with the four slots' weight
+// planes resident, so a sector's four 8-byte writes come from the same thread a few microseconds apart instead of from four CTAs
+// that have to stay in step (DESIGN.md section 6, "Correction").
+// STAGED (BK 32 only): the results of slots 0-2 wait in shared memory (each thread reads back only what it wrote, no
+// synchronisation) and slot 3 writes all four as ONE 32-byte sector per (column, output): a quarter of the sector writes.
+template <int BK, bool FOLD, bool STAGED = false>
 __global__ void __launch_bounds__(TCN2_THREADS, 1)
 tcn2_mac_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmX,
                 const DeviceParams *__restrict__ P, TcnMacArgs a) {
     using Cfg = Tcn2Cfg<BK>;
-    constexpr int STAGES = Cfg::STAGES, W_BLOCK = Cfg::W_BLOCK, X_STAGE = Cfg::X_STAGE;
+    constexpr int NS = Cfg::NS, STAGES = Cfg::STAGES, W_BLOCK = Cfg::W_BLOCK, X_STAGE = Cfg::X_STAGE;
+    static_assert(!STAGED || NS == 4, "the staged whole-sector store needs four slots per item");
     constexpr uint32_t IDESC_BASE = (2u << 4) | ((uint32_t)(TCN2_CB >> 4) << 24);  // S32 accumulators, u8 x u8, K-major, M = 128
     constexpr uint32_t ID_ALL = IDESC_BASE | ((uint32_t)((TCN_PLANES * TCN2_MT) >> 3) << 17);
     constexpr uint32_t ID_HI = IDESC_BASE | ((uint32_t)(((TCN_PLANES - 1) * TCN2_MT) >> 3) << 17);
@@ -427,15 +420,14 @@ tcn2_mac_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__
             uint64_t bias_lane[NS];
 #pragma unroll
             for (int s = 0; s < NS; s++)
-                bias_lane[s] = (BIAS != 0 && a.bias && lane < m_valid) ? __ldg(a.bias + (long)(mt * TCN2_MT + lane) * pw + slot_off + s) : 0;
-            const uint64_t *bias_p = a.bias ? a.bias + (long)(mt * TCN2_MT) * pw + slot_off : nullptr;
+                bias_lane[s] = (a.bias && lane < m_valid) ? __ldg(a.bias + (long)(mt * TCN2_MT + lane) * pw + slot_off + s) : 0;
             for (int ch = 0; ch < chunks; ch++) {
                 const int col = ch * TCN2_CB + qd * 32 + lane;
                 const bool valid = col < a.ncols;
                 const int p = col >> 1, poly = col & 1;
                 const long colbase = (long)(p / a.Pimg) * ((long)a.Mtotal * a.Pimg) + p % a.Pimg;
                 uint64_t *out_col = a.out + (colbase * 2 + poly) * pw + slot_off + (long)(a.m0 + mt * TCN2_MT) * m_stride;
-                const bool add_bias = poly == 0 && (BIAS != 0 || bias_p != nullptr);
+                const bool add_bias = poly == 0;
 #pragma unroll
               for (int s = 0; s < NS; s++) {                    // slot sl + s of the item: residue position c + s
                 if (warp == 2 && lane == 0) TCN2_TR(2, 200);    // waiting for the accumulator
@@ -451,13 +443,10 @@ tcn2_mac_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__
                         tmem_ld4(tmem_base + ((uint32_t)(qd * 32) << 16) + w * TCN2_MT + mloc, S[w]);
                     tmem_ld_wait();
                     uint64_t *op = out_col + (long)mloc * m_stride + s;
-                    const uint64_t *bp = bias_p + (long)mloc * pw + s;
 #pragma unroll
                     for (int i = 0; i < 4; i++) {
                         if (mloc + i < m_valid) {                // warp uniform
-                            uint64_t bias_m = 0;
-                            if constexpr (BIAS != 0) bias_m = __shfl_sync(0xffffffffu, bias_lane[s], mloc + i);
-                            else if (add_bias) bias_m = __ldg(bp);
+                            const uint64_t bias_m = __shfl_sync(0xffffffffu, bias_lane[s], mloc + i);
                             uint64_t r;
                             if constexpr (FOLD) {
                                 r = tcn_fold_out(S, i, add_bias ? bias_m : 0, fold, mod.q);
@@ -465,15 +454,13 @@ tcn2_mac_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__
                                 r = barrett128(tcn_combine(S, i), mod);
                                 if (add_bias) r = addmod(r, bias_m, mod.q);
                             }
-                            if constexpr (BIAS == 2) { if (valid && r == ~0ull) *op = r; }   // never true: r < q
-                            else if constexpr (STAGED && NS == 4) {
+                            if constexpr (STAGED) {
                                 uint64_t *st = out_stage + (mloc + i) * TCN2_CB + qd * 32 + lane;
                                 if (s < NS - 1) st[s * (TCN2_MT * TCN2_CB)] = r;
                                 else if (valid) tcn_store_sector(op - (NS - 1), st[0], st[TCN2_MT * TCN2_CB], st[2 * TCN2_MT * TCN2_CB], r);
                             } else if (valid) *op = r;
                         }
                         op += m_stride;
-                        bp += pw;
                     }
                 }
                 tc_fence_before();
@@ -497,7 +484,7 @@ tcn2_mac_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__
 // multiplied against the 7 stacked planes of W'_b (N = 224) into the SAME 224 accumulator columns for every b: no
 // column shift, no special first step, and two accumulators fit TMEM (2 x 224 of 512 columns), so the epilogue of one
 // (chunk, slot) runs while the MMAs of the next one are issued.  Fan-in <= 32 (one 32-byte K block: conv1) and four
-// consecutive slots per item, as tcn2_mac_kernel<32, ., 1, 4, .>: the pre-shifted planes of the four slots stay resident
+// consecutive slots per item, as tcn2_mac_kernel<32, .>: the pre-shifted planes of the four slots stay resident
 // (4 x 49 KB), which leaves no shared memory for output staging -- instead each epilogue thread keeps the results of
 // slots 0-2 in registers and slot 3 writes all four as one 32-byte sector (STAGED, layers of at most 24 outputs).
 constexpr int TCN2P_NS = 4;
@@ -801,7 +788,7 @@ cudaError_t launch_tcn_mac_t(const DeviceParams *P, const TcnMacArgs &a, int sm_
     return cudaGetLastError();
 }
 
-template <int BK, bool FOLD, int BIAS, int NS = 1, bool STAGED = false>
+template <int BK, bool FOLD, bool STAGED = false>
 cudaError_t launch_tcn2_mac_t(const DeviceParams *P, const TcnMacArgs &a, int sm_count, cudaStream_t stream) {
     EncodeTiledFn enc = encode_tiled();
     if (!enc) return cudaErrorNotSupported;
@@ -825,14 +812,14 @@ cudaError_t launch_tcn2_mac_t(const DeviceParams *P, const TcnMacArgs &a, int sm
                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
             return cudaErrorInvalidValue;
     }
-    auto k = tcn2_mac_kernel<BK, FOLD, BIAS, NS, STAGED>;
-    const size_t smem = Tcn2Cfg<BK>::smem(NS, STAGED);
+    auto k = tcn2_mac_kernel<BK, FOLD, STAGED>;
+    const size_t smem = Tcn2Cfg<BK>::smem(STAGED);
     static DeviceOnce once;
     if (once.first()) {
         cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
-    const long groups = a.nslots / NS;      // a CTA runs every output tile of its slot groups
+    const long groups = a.nslots / Tcn2Cfg<BK>::NS;      // a CTA runs every output tile of its slot groups
     const unsigned grid = (unsigned)(groups < sm_count ? groups : sm_count);
     k<<<grid, TCN2_THREADS, smem, stream>>>(tmW, tmX, P, a);
     return cudaGetLastError();
@@ -916,42 +903,28 @@ cudaError_t launch_tcn_mac(const DeviceParams *P, const TcnMacArgs &a, int sm_co
     // folded reduction of the class sums (modarith.cuh: tcn_fold_reduce) when every prime of the context has SEAL's shape
     bool fold = a.use_fold != 0;
     for (int j = 0; j < a.K && fold; j++) fold = a.fold[j].ok != 0;
-    // CRCNN_TCN2_BIAS=0|1 overrides where the column-major kernel takes its bias from (A/B runs; same bytes either way)
-    static const int bias_env = [] { const char *e = getenv("CRCNN_TCN2_BIAS"); return e ? atoi(e) : -1; }();
-    // The 32-byte-row kernel (fan-in <= 32: conv1) takes items of FOUR consecutive slots with the per-item bias, stages slots 0-2 of an
-    // item in shared memory and writes whole 32-byte sectors (one STG.E.256 per (column, output)): a sector is then completed by ONE
-    // thread instead of four CTAs that have to stay in step (DESIGN.md section 6).  Measured on B200 (profiles/r02a_first.txt): conv1's
-    // GEMM 23.6 -> 21.3 ms per step (20.1 with the folded reduction).  CRCNN_TCN2_NS=1 selects the one-slot kernel, CRCNN_TCN2_STAGE=0
-    // the four-slot kernel with 8-byte stores (A/B runs; same bytes).
-    static const int ns_env = [] { const char *e = getenv("CRCNN_TCN2_NS"); return e ? atoi(e) : 4; }();
-    static const int stage_env = [] { const char *e = getenv("CRCNN_TCN2_STAGE"); return e ? atoi(e) : 1; }();
+    // staged whole-sector stores (STG.E.256) need a 32-byte aligned output, and the pre-shift kernel's register budget at most
+    // TCN2P_STAGED_MAX_M outputs
+    const bool staged = a.M <= TCN2P_STAGED_MAX_M && (reinterpret_cast<uintptr_t>(a.out) & 31) == 0;
     // Pre-shifted weights (a.preshift, staged by the caller for tcn_preshift_shape): seven accumulator classes, double-buffered
-    // accumulator, four slots per item; CRCNN_TCN2_STAGE=0 gives 8-byte stores here too
+    // accumulator, four slots per item
     if (a.preshift) {
         if (!tcn_preshift_shape(a.R, a.ncols, a.M, forced) || a.nslots % TCN2P_NS || a.slot0 % TCN2P_NS || a.n % TCN2P_NS) return cudaErrorInvalidValue;
         bool fold7 = a.use_fold != 0;
         for (int j = 0; j < a.K && fold7; j++) fold7 = a.fold[j].ok7 != 0;
-        if (stage_env && a.M <= TCN2P_STAGED_MAX_M && (reinterpret_cast<uintptr_t>(a.out) & 31) == 0)
-            return fold7 ? launch_tcn2p_mac_t<true, true>(P, a, sm_count, stream) : launch_tcn2p_mac_t<false, true>(P, a, sm_count, stream);
+        if (staged) return fold7 ? launch_tcn2p_mac_t<true, true>(P, a, sm_count, stream) : launch_tcn2p_mac_t<false, true>(P, a, sm_count, stream);
         return fold7 ? launch_tcn2p_mac_t<true, false>(P, a, sm_count, stream) : launch_tcn2p_mac_t<false, false>(P, a, sm_count, stream);
     }
-    if (use2 && ns_env == 4 && bk == 32 && a.nslots % 4 == 0 && a.slot0 % 4 == 0 && a.n % 4 == 0) {
-        if (stage_env && a.M <= TCN2P_STAGED_MAX_M && (reinterpret_cast<uintptr_t>(a.out) & 31) == 0)
-            return fold ? launch_tcn2_mac_t<32, true, 1, 4, true>(P, a, sm_count, stream) : launch_tcn2_mac_t<32, false, 1, 4, true>(P, a, sm_count, stream);
-        return fold ? launch_tcn2_mac_t<32, true, 1, 4>(P, a, sm_count, stream) : launch_tcn2_mac_t<32, false, 1, 4>(P, a, sm_count, stream);
+    // The 32-byte-row kernel (fan-in <= 32: conv1) takes items of FOUR consecutive slots, stages slots 0-2 of an item in shared
+    // memory and writes whole 32-byte sectors (one STG.E.256 per (column, output)): a sector is then completed by ONE thread
+    // instead of four CTAs that have to stay in step (DESIGN.md section 6).  Measured on B200 (profiles/r02a_first.txt): conv1's
+    // GEMM 23.6 -> 21.3 ms per step (20.1 with the folded reduction).
+    if (use2 && bk == 32) {
+        if (a.nslots % 4 || a.slot0 % 4 || a.n % 4) return cudaErrorInvalidValue;
+        if (staged) return fold ? launch_tcn2_mac_t<32, true, true>(P, a, sm_count, stream) : launch_tcn2_mac_t<32, false, true>(P, a, sm_count, stream);
+        return fold ? launch_tcn2_mac_t<32, true>(P, a, sm_count, stream) : launch_tcn2_mac_t<32, false>(P, a, sm_count, stream);
     }
-    if (use2) {
-        const int bias_var = bias_env >= 0 ? bias_env : (bk == 128 ? 1 : 0);
-#ifdef CRCNN_TCN2_TIMING   // timing builds only (make EXTRA=-DCRCNN_TCN2_TIMING OUT=../../ab/libS.so OBJDIR=../../build/objS): 2 drops the stores, results are NOT written
-        if (bias_var == 2) return bk == 128 ? launch_tcn2_mac_t<128, false, 2>(P, a, sm_count, stream) : launch_tcn2_mac_t<32, false, 2>(P, a, sm_count, stream);
-#endif
-        if (fold) {
-            if (bias_var) return bk == 128 ? launch_tcn2_mac_t<128, true, 1>(P, a, sm_count, stream) : launch_tcn2_mac_t<32, true, 1>(P, a, sm_count, stream);
-            return bk == 128 ? launch_tcn2_mac_t<128, true, 0>(P, a, sm_count, stream) : launch_tcn2_mac_t<32, true, 0>(P, a, sm_count, stream);
-        }
-        if (bias_var) return bk == 128 ? launch_tcn2_mac_t<128, false, 1>(P, a, sm_count, stream) : launch_tcn2_mac_t<32, false, 1>(P, a, sm_count, stream);
-        return bk == 128 ? launch_tcn2_mac_t<128, false, 0>(P, a, sm_count, stream) : launch_tcn2_mac_t<32, false, 0>(P, a, sm_count, stream);
-    }
+    if (use2) return fold ? launch_tcn2_mac_t<128, true>(P, a, sm_count, stream) : launch_tcn2_mac_t<128, false>(P, a, sm_count, stream);
     if (fold) return bk == 128 ? launch_tcn_mac_t<128, true>(P, a, sm_count, stream) : launch_tcn_mac_t<32, true>(P, a, sm_count, stream);
     return bk == 128 ? launch_tcn_mac_t<128, false>(P, a, sm_count, stream) : launch_tcn_mac_t<32, false>(P, a, sm_count, stream);
 }

@@ -13,11 +13,8 @@ launch counters which kernel ran, so that a silent fallback cannot pass.
     MAC reduces between chunks of 16 digits), the 64-bit path beyond, an error beyond 63 digits.
 Weights are constant plaintexts t - k (q - k in every NTT slot), inputs NTT-form slots of chosen residues: uniform ones for the largest
 accumulator values, and near-maximal ones that vary per (output, term, column, slot) so that a permuted row or column shows.
-Environment switches read once per process run the same cases in child processes.
 """
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -28,9 +25,7 @@ from oracle.port import Oracle
 
 pytestmark = pytest.mark.gpu
 
-HERE = os.path.abspath(__file__)
 TCN_MAX_R = 4096
-CHILD_FLAG = "CRCNN_LIMITS_CHILD"
 
 
 def _engine(n, primes, t):
@@ -78,41 +73,6 @@ def _explain(got, want):
         return "equal"
     first = tuple(int(v) for v in bad[0])
     return "%d of %d words differ; first at %s: got %d want %d" % (len(bad), got.size, first, int(got[first]), int(want[first]))
-
-
-def _child(switch, kfilter, path=HERE):
-    """Starts `path` -k kfilter in a child process with the environment switch set; returns the Popen."""
-    env = dict(os.environ, **{CHILD_FLAG: "1"})
-    for s in switch.split(","):
-        key, val = s.split("=")
-        env[key] = val
-    return subprocess.Popen([sys.executable, "-m", "pytest", path, "-q", "-x", "-m", "gpu", "-k", kfilter, "-p", "no:cacheprovider"],
-                            env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True,
-                            cwd=os.path.dirname(os.path.dirname(path)))
-
-
-def _run_children(jobs, parallel=3, timeout=1500):
-    """jobs: {label: (switch, kfilter, path)}.  Runs them, at most `parallel` at a time (every process keeps its own cache of device
-    memory), and asserts that every one passed and ran at least one test."""
-    failed, pending, running = [], list(jobs.items()), []
-    while pending or running:
-        while pending and len(running) < parallel:
-            label, args = pending.pop(0)
-            running.append((label, _child(*args)))
-        label, p = running.pop(0)
-        try:
-            out, _ = p.communicate(timeout=timeout)
-        except subprocess.TimeoutExpired:
-            p.kill()
-            out, _ = p.communicate()
-            failed.append("%s: timed out\n%s" % (label, out[-1500:]))
-            continue
-        if p.returncode != 0 or " passed" not in out:
-            failed.append("%s: exit %d\n%s" % (label, p.returncode, out[-1500:]))
-    assert not failed, "\n\n".join(failed)
-
-
-not_in_child = pytest.mark.skipif(os.environ.get(CHILD_FLAG) == "1", reason="spawns the child processes itself")
 
 
 # ============================================================================ limb-split GEMM
@@ -292,12 +252,6 @@ def test_ternary_gemm_at_large_fan_in(tc_env, R):
     assert np.array_equal(got, want), _explain(got, want)
 
 
-@not_in_child
-def test_ternary_gemm_variants_in_child():
-    """The cta_group::2 pair kernel (CRCNN_TC_PAIR=1) and the four-stage ring (CRCNN_TC_SUB=1) at the same limits."""
-    _run_children({s: (s, "ternary_gemm_at_large") for s in ("CRCNN_TC_PAIR=1", "CRCNN_TC_SUB=1")})
-
-
 # ============================================================================ CUDA-core MAC at chunk_terms
 @pytest.fixture(scope="module", params=["P60a", "P60b"])
 def p60_env(request):
@@ -311,14 +265,15 @@ def p60_env(request):
 def test_cuda_core_mac_at_chunk_terms(p60_env, R):
     """60-bit primes: 8 byte planes, so every weighted sum takes the CUDA-core MAC, which reduces its 128-bit accumulators every
     chunk_terms = 256 terms.  W = X = q - 1 gives R mod q in every slot (plus the bias); near-maximal operands (k in [1, 8], slot values
-    q - 1 - [0, 8)) follow the closed form; fan-in 257 is also compared with the oracle."""
+    q - 1 - [0, 8)) follow the closed form; fan-in 257 is also compared with the oracle.  Batch 2 runs the 2 x 2 output tile, batch 1
+    (one position) the 4 x 1 tile (kernels.cu: launch_mac)."""
     n, primes, t, eng, orc, rng = p60_env
-    K, M, B = len(primes), 3, 2
+    K, M = len(primes), 3
     bv = rng.uniform(-3, 3, size=M).astype(np.float32)
     b_ = eng.plain_encode(bv)
     bias = bias_slots(orc, orc.encode_many(bv))
     xb = [q - 1 for q in primes]
-    for kind in ("uniform", "varied"):
+    for B, kind in ((2, "uniform"), (2, "varied"), (1, "uniform"), (1, "varied")):
         k = np.ones((M, R), np.int64) if kind == "uniform" else rng.integers(1, 9, size=(M, R))
         d = np.zeros((B, R, 2, K, n), np.int64) if kind == "uniform" else rng.integers(0, 8, size=(B, R, 2, K, n))
         want = const_weight_fc_slots(k, xb, d, primes, bias)
@@ -331,19 +286,13 @@ def test_cuda_core_mac_at_chunk_terms(p60_env, R):
         cnt = _delta(eng, before)
         assert cnt["weighted_sum_mac"] == 1 and cnt["weighted_sum_tcn_i8"] == 0, cnt
         got = got.reshape(B, M, 2, K, n + 1)[..., :n]
-        assert np.array_equal(got, want), "%s: %s" % (kind, _explain(got, want))
+        assert np.array_equal(got, want), "B=%d %s: %s" % (B, kind, _explain(got, want))
         if kind == "varied" and R == 257:
             xc = orc.ct_transform(xw[:R], inverse=True)
             wp = np.zeros((M * R, n + 1), np.uint64)
             wp[:, 0] = t - k.ravel()
             ref = orc.ct_transform(orc.fc(xc, R, M, wp, orc.encode_many(bv)).reshape(M, 2, K, n + 1))[..., :n]
             assert np.array_equal(got[0], ref), _explain(got[0], ref)
-
-
-@not_in_child
-def test_every_mac_tile_in_child():
-    """Every CRCNN_MAC_TILE instantiation of the CUDA-core MAC (the switch is read once per process) at chunk_terms."""
-    _run_children({v: ("CRCNN_MAC_TILE=%s" % v, "cuda_core_mac_at_chunk_terms") for v in ("42", "22", "24", "41", "21", "81", "12", "14")}, parallel=4)
 
 
 # ============================================================================ 64-bit window sums at sum_fits_64
@@ -554,24 +503,3 @@ def test_relinearize_every_digit_width(relin_env):
     if n == 8192:
         assert {"register", "generic, 2 chunks", "64-bit, over 32 digits", "error"} <= seen, seen
 
-
-@not_in_child
-def test_relinearize_switches_in_child():
-    """The generic auxiliary-prime MAC also at D = 4K (CRCNN_R32_GENERIC_MAC=1), and the two-kernel inverse transform + reconstruction
-    (CRCNN_R32_FUSED=0), at every digit width."""
-    _run_children({s: (s, "relinearize_every_digit_width") for s in ("CRCNN_R32_GENERIC_MAC=1", "CRCNN_R32_FUSED=0")})
-
-
-# ============================================================================ limb-split kernel switches
-@not_in_child
-def test_limb_split_switches_in_child():
-    """Instantiations of the limb-split GEMM that the README says give the same bytes: the one-slot column-major kernel
-    (CRCNN_TCN2_NS=1), 8-byte stores (CRCNN_TCN2_STAGE=0), the bias read from either source (CRCNN_TCN2_BIAS=0 / 1).  The suites of the
-    limb-split and pre-shifted kernels and this file's limb-split limits run with each switch set."""
-    tests = os.path.dirname(HERE)
-    jobs = {}
-    for s in ("CRCNN_TCN2_NS=1", "CRCNN_TCN2_STAGE=0", "CRCNN_TCN2_BIAS=0", "CRCNN_TCN2_BIAS=1"):
-        jobs[s + " tcn"] = (s, "not opt_in", os.path.join(tests, "test_gpu_tcn.py"))
-        jobs[s + " preshift"] = (s, "not opt_in", os.path.join(tests, "test_gpu_tcn_preshift.py"))
-        jobs[s + " limits"] = (s, "limb_split_at_fan_in_limits", HERE)
-    _run_children(jobs)

@@ -153,18 +153,3 @@ def test_extreme_inputs_on_tensor_cores(env):
     assert _tc_launches(eng) == before + 1
     assert np.array_equal(got, want), _explain(got, want)
 
-
-@pytest.mark.parametrize("switch", ["CRCNN_TC_PAIR=1", "CRCNN_TC_SUB=1"])
-def test_opt_in_kernel_variants_stay_bit_exact(switch):
-    """The ternary GEMM ships two more instantiations behind environment switches (read once per process): the cta_group::2 pair
-    kernel and the four-stage ring.  Neither is faster on B200 (profiles/r02_tc_mac_ablation.txt), both must stay exact: the tests
-    above are re-run in a child process with the switch set."""
-    import os
-    import subprocess
-    import sys
-    key, val = switch.split("=")
-    env = dict(os.environ, **{key: val})
-    here = os.path.abspath(__file__)
-    res = subprocess.run([sys.executable, "-m", "pytest", here, "-q", "-x", "-k", "not opt_in", "-p", "no:cacheprovider"],
-                         env=env, capture_output=True, text=True, timeout=900, cwd=os.path.dirname(os.path.dirname(here)))
-    assert res.returncode == 0, res.stdout[-2000:] + res.stderr[-500:]

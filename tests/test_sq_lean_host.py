@@ -1,6 +1,6 @@
-"""CPU checks behind the lean square: the n^-1-scaled lift / floor constants (params.h: mt_inv_qhat_n, fl_c_n, fl_T_n) and the
-transforms' approximate Shoup product on edge operands, for every modulus of the n = 2048 ... 16384 contexts.  host_selftest
-compares both with unsigned __int128 and prints one line per modulus."""
+"""CPU checks behind the lean square: the n^-1-scaled lift / floor constants (params.h: mt_inv_qhat_n, fl_c, fl_T) against their
+definitions and the transforms' approximate Shoup product on edge operands, for every modulus of the n = 2048 ... 16384 contexts.
+host_selftest compares both with unsigned __int128 and prints one line per modulus."""
 import os
 import subprocess
 

@@ -2,7 +2,7 @@
 """Times a few layers of the bench network in seconds of box time (no torch import): per-kernel-class ms of `reps` forwards of layers
 [first, last) at the bench batch, from the engine's own CUDA-event counters.  For A/B runs of kernel switches set through the environment.
 
-  CRCNN_TCN2_NS=4 python tools/quick_layers.py --first 0 --last 1      # conv1 only
+  CRCNN_TCN_FOLD=0 python tools/quick_layers.py --first 0 --last 1      # conv1 only
 """
 import argparse
 import os

@@ -1,18 +1,14 @@
 #!/bin/bash
-# Round-end validation on the GPU box (under gpurun): full GPU suite, smoke, the bench line, one timing experiment, launch list.
+# Round-end validation on a B200: full GPU suite, smoke, the bench line, launch list.
 # usage: bash tools/round_end_check.sh <tag>
 tag=${1:-r01k}
 mkdir -p gpurun_out
 python -m pytest tests -m gpu -q > gpurun_out/${tag}_gputests.log 2>&1; echo "tests rc=$?"; tail -4 gpurun_out/${tag}_gputests.log
 python -c "import __graft_entry__ as g; g.smoke()" > gpurun_out/${tag}_smoke.log 2>&1; echo "smoke rc=$?"; tail -1 gpurun_out/${tag}_smoke.log
 python bench.py > gpurun_out/${tag}_bench_line.json 2> gpurun_out/${tag}_bench.err; echo "bench rc=$?"
-# timing build: column-major limb-split kernel with the per-item bias broadcast and NO output stores (results not written)
-if [ -f ab/libS.so ]; then
-  CRCNN_B200_LIB=$PWD/ab/libS.so CRCNN_TCN2_BIAS=2 python bench.py --no-cpu-baseline > gpurun_out/${tag}_bench_nostore.json 2> gpurun_out/${tag}_bench_nostore.err; echo "nostore rc=$?"
-fi
 python - <<P
 import json
-for f in ("${tag}_bench_line","${tag}_bench_nostore"):
+for f in ("${tag}_bench_line",):
     try:
         d=json.load(open("gpurun_out/%s.json"%f))
         print(f, round(d["value"],2), round(d["ms_per_step"],1), round(d["e2e"]["value"],2), {k:round(v,1) for k,v in d["per_layer_ms"].items()}, {k:round(v["ms_per_step"],1) for k,v in d["kernel_ms"].items() if "tcn" in k})
