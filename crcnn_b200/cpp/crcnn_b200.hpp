@@ -989,7 +989,9 @@ public:
         FcFc,          // FullyConnectedLayer directly followed by FullyConnectedLayer: one composed layer (crcnn_fc_fc_forward)
         PoolBn         // AvgPoolingLayer directly followed by BatchNormLayer: one pass instead of two (crcnn_pool_bn_forward)
     };
-    // The group forward_dev runs from layer i of the range [i, last), and its number of layers
+    // The group forward_dev runs from layer i of the range [i, last), and its number of layers.  ConvPoolBn tests no geometry here:
+    // BatchNormLayer::forward_after_conv_avgpool throws where the three shapes do not chain, so a mismatch is an error, never other
+    // bytes.  ConvPool tests it because the layer-by-layer path is what a conv + pool pair that does not chain must get.
     std::pair<Group, int> group_at(int i, int last) {
         auto at = [&](int k) { return layers[i + k].get(); };
         if (fuse_conv_pool_bn && i + 2 < last && dynamic_cast<ConvolutionalLayer *>(at(0)) && dynamic_cast<PoolingLayer *>(at(1)) &&

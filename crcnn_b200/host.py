@@ -14,6 +14,7 @@ from .h5write import write_h5
 _HERE = os.path.dirname(os.path.abspath(__file__))
 HOST_LIB_PATH = os.path.join(_HERE, "libcrcnn_b200_host.so")
 TOPOLOGY_OF = {"PlainModel": "PlainModel", "ApproxPlainModel": "Approx", "PlainModelWoPad": "WoPad", "PlainModelTiny": "Tiny"}
+MODEL_OF = {v: k for k, v in TOPOLOGY_OF.items()}
 _vp, _I, _dp = C.c_void_p, C.c_int, C.POINTER(C.c_double)
 
 _h = None
@@ -101,6 +102,9 @@ class HostNetwork:
         v = [_I() for _ in range(5)]
         self._chk(self.h.crcnn_host_shape(*[C.byref(x) for x in v]))
         self.zd, self.xd, self.yd, self.outputs, self.num_layers = [x.value for x in v]
+        # the largest activation per image (input or any layer's output): what forward() on any layer range may hand back
+        topo = nets.TOPOLOGIES[MODEL_OF.get(model, model)]
+        self.max_cts = max([self.zd * self.xd * self.yd] + [nets.layer_io_counts(layer)[1] for layer in topo["layers"]])
         name = C.create_string_buffer(128)
         self.layer_names = []
         for i in range(self.num_layers):
@@ -123,7 +127,7 @@ class HostNetwork:
         x = np.ascontiguousarray(x, dtype=np.uint64)
         zd, xd, yd = shape or (self.zd, self.xd, self.yd)
         last = self.num_layers if last is None else last
-        cap = max(x.size, batch * 64 * 64 * 64 * 2 * self.K * self.stride // 64)
+        cap = max(x.size, batch * self.max_cts * self.ct_words())
         out = np.empty(cap, dtype=np.uint64)
         oshape = (_I * 3)()
         self._chk(self.h.crcnn_host_forward_range(x.ctypes.data, batch, zd, xd, yd, first, last, out.ctypes.data, cap, oshape))
