@@ -922,7 +922,12 @@ public:
         if (per <= 0 || x.count() % per) throw std::invalid_argument("tensor is not a whole number of images of that shape");
         std::vector<float> v((size_t)x.count());
         Runtime::get().check(crcnn_decrypt_values(Runtime::get().ctx(), keys, x.t, v.data()));
-        std::vector<floatCube> out((size_t)(x.count() / per), floatCube(zd, std::vector<std::vector<float>>(xd, std::vector<float>(yd))));
+        return images_of(v, zd, xd, yd);
+    }
+    // v (a whole number of zd*xd*yd images, in order) as images [b][z][x][y]
+    static std::vector<floatCube> images_of(const std::vector<float> &v, int zd, int xd, int yd) {
+        const size_t per = (size_t)zd * xd * yd;
+        std::vector<floatCube> out(v.size() / per, floatCube(zd, std::vector<std::vector<float>>(xd, std::vector<float>(yd))));
         size_t i = 0;
         for (auto &img : out)
             for (auto &plane : img)
@@ -1292,6 +1297,78 @@ public:
 private:
     int world_, rank_;
     crcnn_comm *comm_ = nullptr;
+};
+
+// ------------------------------------------------------------------------------------------------
+// CrtEnsemble: a large plain modulus T split into pairwise coprime t_1 .. t_M (BASELINE config 4), one independent instance of the
+// network per GPU and process.  Each rank builds the whole network with CnnBuilder under Runtime::init(n, q, t_rank) and installs the
+// key holder's keys (use_device_keys; the instances may share one key set: FV keys depend on n and q only).  The ensemble recombines
+// the instances' plaintexts modulo T on the device (crcnn_crt_*), so the fixed re-encryption before layer_before_reenc and the final
+// decryption see what one network under T sees, and predict returns on every rank the floats of a single Network::predict under T.
+// The re-encryption and the decryption are collective: every rank must make the same calls in the same order.  That is why the
+// budget-driven policy (reencrypt_below_budget >= 0) is refused -- each rank would decide from its own budget whether to re-encrypt.
+// ------------------------------------------------------------------------------------------------
+class CrtEnsemble {
+public:
+    // Collective (crcnn_crt_create).  Installs the collective re-encryption as net.reencrypt_dev; every call draws fresh randomness
+    // from (reencrypt_seed, call number, rank).
+    CrtEnsemble(Network &net, const std::vector<std::uint64_t> &moduli, int world, int rank, const void *nccl_id128, std::uint64_t reencrypt_seed)
+        : net_(net) {
+        net.require_keys();
+        refuse_budget_policy();
+        Runtime &rt = Runtime::get();
+        rt.check(crcnn_comm_create(rt.ctx(), nccl_id128, world, rank, &comm_));
+        try {
+            rt.check(crcnn_crt_create(rt.ctx(), comm_, moduli.data(), (int)moduli.size(), &crt_));
+        } catch (...) {
+            crcnn_comm_destroy(rt.ctx(), comm_);
+            throw;
+        }
+        Network *np = &net;
+        crcnn_crt *crt = crt_;
+        auto calls = std::make_shared<std::uint64_t>(0);
+        net.reencrypt_dev = [np, crt, reencrypt_seed, calls](DeviceTensor x) {
+            if (np->reencrypt_below_budget >= 0) throw std::logic_error(budget_policy_refused);
+            Runtime &r = Runtime::get();
+            crcnn_tensor *o = nullptr;
+            r.check(crcnn_crt_reencrypt(r.ctx(), crt, np->require_keys(), x.t, reencrypt_seed + 0x9E3779B97F4A7C15ull * (*calls)++, 0.0, &o));
+            return DeviceTensor(o, x.zd, x.xd, x.yd, x.batch);
+        };
+    }
+    ~CrtEnsemble() {
+        net_.reencrypt_dev = nullptr;
+        crcnn_crt_free(Runtime::get().ctx(), crt_);
+        crcnn_comm_destroy(Runtime::get().ctx(), comm_);
+    }
+    CrtEnsemble(const CrtEnsemble &) = delete;
+    CrtEnsemble &operator=(const CrtEnsemble &) = delete;
+
+    // Network::decrypt_images_dev under T (collective, crcnn_crt_decrypt_values): the same floats on every rank.
+    std::vector<floatCube> decrypt_images_dev(const DeviceTensor &x, int zd, int xd, int yd) {
+        crcnn_keys *keys = net_.require_keys();
+        const long per = (long)zd * xd * yd;
+        if (per <= 0 || x.count() % per) throw std::invalid_argument("tensor is not a whole number of images of that shape");
+        std::vector<float> v((size_t)x.count());
+        Runtime::get().check(crcnn_crt_decrypt_values(Runtime::get().ctx(), crt_, keys, x.t, v.data()));
+        return Network::images_of(v, zd, xd, yd);
+    }
+    // Network::predict of the ensemble: this rank's instance encrypts the images (encrypt_images_dev) and runs forward_batch_dev,
+    // re-encrypting collectively before layer_before_reenc; the scores are decrypted collectively.  Every rank calls it with the
+    // same images and gets the same floats.
+    std::vector<floatCube> predict(const std::vector<floatCube> &images, std::uint64_t seed) {
+        refuse_budget_policy();
+        DeviceTensor y = net_.forward_batch_dev(net_.encrypt_images_dev(images, seed));
+        return decrypt_images_dev(y, y.zd, y.xd, y.yd);
+    }
+
+private:
+    static constexpr const char *budget_policy_refused =
+        "crcnn_b200::CrtEnsemble: the budget-driven re-encryption (reencrypt_below_budget >= 0) would let each rank decide alone whether "
+        "to enter the collective re-encryption";
+    void refuse_budget_policy() const { if (net_.reencrypt_below_budget >= 0) throw std::logic_error(budget_policy_refused); }
+    Network &net_;
+    crcnn_comm *comm_ = nullptr;
+    crcnn_crt *crt_ = nullptr;
 };
 
 }  // namespace crcnn_b200

@@ -17,6 +17,7 @@ using namespace crcnn_b200;
 namespace {
 std::string g_err;
 std::unique_ptr<Network> g_net;
+std::unique_ptr<CrtEnsemble> g_crt;   // crcnn_host_crt_begin: this rank's place in a CRT ensemble over g_net
 std::unique_ptr<BatchServer> g_srv;
 std::unique_ptr<DeviceTensor> g_x0;   // resident input of crcnn_host_resident_*
 int g_zd = 0, g_xd = 0, g_yd = 0, g_outputs = 0, g_batch = 0;
@@ -37,7 +38,7 @@ const char *crcnn_host_last_error() { return g_err.c_str(); }
 
 // setParameters (CrCNN/src/globals.cpp:25-56) as far as evaluation goes
 int crcnn_host_init(int n, int K, const uint64_t *q, uint64_t t, int device) {
-    return guarded([&] { g_x0.reset(); g_srv.reset(); g_net.reset(); Runtime::get().init(n, std::vector<uint64_t>(q, q + K), t, device); });
+    return guarded([&] { g_x0.reset(); g_srv.reset(); g_crt.reset(); g_net.reset(); Runtime::get().init(n, std::vector<uint64_t>(q, q + K), t, device); });
 }
 int crcnn_host_set_evk(const uint64_t *words, const int *sizes, int dbc) {
     return guarded([&] { Runtime::get().setEvaluationKeys(words, sizes, dbc); });
@@ -48,7 +49,7 @@ void *crcnn_host_ctx() { try { return Runtime::get().ctx(); } catch (...) { retu
 // made from nccl_id (crcnn_comm_unique_id on rank 0, handed to every rank by the launcher).
 int crcnn_host_build(const char *h5_path, const char *topology, int world, int rank, const void *nccl_id, int skip_reencryption) {
     return guarded([&] {
-        g_x0.reset(); g_srv.reset(); g_net.reset();
+        g_x0.reset(); g_srv.reset(); g_crt.reset(); g_net.reset();
         CnnBuilder builder(h5_path);
         if (world > 1 || nccl_id) g_net.reset(new ShardedNetwork(world, rank, nccl_id));
         else g_net.reset(new Network());
@@ -253,6 +254,41 @@ int crcnn_host_serve_times(double *out, int cap) {
     return n;
 }
 
-void crcnn_host_shutdown() { g_x0.reset(); g_srv.reset(); g_net.reset(); Runtime::get().reset(); }
+// CrtEnsemble over the built network (after crcnn_host_build with world 1 and crcnn_host_use_keys): this rank holds the instance under
+// moduli[rank] (the plain modulus of crcnn_host_init); collective, every rank of the M calls it with the same list and nccl_id.
+// reencrypt_seed keys the noise of the collective re-encryption before layer 6.
+int crcnn_host_crt_begin(const uint64_t *moduli, int M, int rank, const void *nccl_id, uint64_t reencrypt_seed) {
+    return guarded([&] {
+        if (!g_net) throw std::invalid_argument("no network built");
+        if (!moduli || M < 1 || !nccl_id) throw std::invalid_argument("bad ensemble arguments");
+        g_crt.reset();
+        g_crt.reset(new CrtEnsemble(*g_net, std::vector<uint64_t>(moduli, moduli + M), M, rank, nccl_id, reencrypt_seed));
+    });
+}
+// CrtEnsemble::predict, images and scores as in crcnn_host_predict_values; the same scores on every rank.
+int crcnn_host_crt_predict_values(const float *images, int batch, uint64_t seed, float *scores) {
+    return guarded([&] {
+        if (!g_crt) throw std::invalid_argument("crcnn_host_crt_begin has not been called");
+        if (!images || !scores || batch <= 0) throw std::invalid_argument("bad predict arguments");
+        std::vector<floatCube> in((size_t)batch, floatCube(g_zd, std::vector<std::vector<float>>(g_xd, std::vector<float>(g_yd))));
+        const float *p = images;
+        for (auto &img : in)
+            for (auto &plane : img)
+                for (auto &row : plane)
+                    for (auto &f : row) f = *p++;
+        const std::vector<floatCube> out = g_crt->predict(in, seed);
+        size_t i = 0;
+        for (auto &img : out)
+            for (auto &plane : img)
+                for (auto &row : plane)
+                    for (float f : row) {
+                        if (i == (size_t)batch * g_outputs) throw std::logic_error("network output is not [batch][outputs] values");
+                        scores[i++] = f;
+                    }
+        if (i != (size_t)batch * g_outputs) throw std::logic_error("network output is not [batch][outputs] values");
+    });
+}
+
+void crcnn_host_shutdown() { g_x0.reset(); g_srv.reset(); g_crt.reset(); g_net.reset(); Runtime::get().reset(); }
 
 }  // extern "C"

@@ -7,6 +7,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <map>
+#include <numeric>
 #include <unordered_map>
 #include <string>
 #include <vector>
@@ -1984,6 +1985,7 @@ struct NcclApi {
     int (*GroupEnd)() = nullptr;
     int (*Send)(const void *, size_t, int, int, void *, cudaStream_t) = nullptr;
     int (*Recv)(void *, size_t, int, int, void *, cudaStream_t) = nullptr;
+    int (*AllGather)(const void *, void *, size_t, int, void *, cudaStream_t) = nullptr;
     const char *(*GetErrorString)(int) = nullptr;
     std::string why;
 };
@@ -2005,6 +2007,7 @@ NcclApi &nccl() {
         a.GroupEnd = (decltype(a.GroupEnd))sym("ncclGroupEnd");
         a.Send = (decltype(a.Send))sym("ncclSend");
         a.Recv = (decltype(a.Recv))sym("ncclRecv");
+        a.AllGather = (decltype(a.AllGather))sym("ncclAllGather");
         a.GetErrorString = (decltype(a.GetErrorString))sym("ncclGetErrorString");
         return a;
     }();
@@ -2091,6 +2094,15 @@ int crcnn_comm_all_gather(crcnn_ctx *ctx, crcnn_comm *c, crcnn_tensor *local, in
     *out = full;
     return CRCNN_OK;
 }
+
+namespace {
+// recv[world][words] = every rank's send[words], rank r's block at recv + r words; raw device words, one NCCL all-gather on the
+// context's stream (send may be recv's own block: NCCL's in-place form)
+int comm_all_gather_words(crcnn_ctx *ctx, crcnn_comm *c, const uint64_t *send, size_t words, uint64_t *recv) {
+    NCCLCHECK(nccl().AllGather(send, recv, words, kNcclUint64, c->comm, ctx->stream));
+    return CRCNN_OK;
+}
+}  // namespace
 
 // ---------------------------------------------------------------------------------------- re-encryption (SURVEY 8(f) N4)
 int crcnn_keys_upload(crcnn_ctx *ctx, const uint64_t *secret_key_ntt, const uint64_t *public_key_ntt, crcnn_keys **out) {
@@ -2374,6 +2386,208 @@ int crcnn_decrypt_values(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, float *
         if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(er));
     }
     dev_free(ctx, scratch); dev_free(ctx, plain); dev_free(ctx, vals);
+    return rc;
+}
+
+// ---------------------------------------------------------------------------------------- CRT plaintext-modulus ensembles
+struct crcnn_crt {
+    crcnn_comm *comm = nullptr;          // not owned
+    std::vector<uint64_t> moduli;
+    CrtConsts c;
+};
+
+namespace {
+// What every list of moduli must satisfy: 1 to CRT_MAX_MODULI of them, each >= 2, pairwise coprime, and a product below every
+// coefficient prime of ctx -- the condition params.cpp puts on a single plain modulus, so a context under T exists to check an
+// ensemble against, and the decoder's signed 64-bit arithmetic holds under T.
+int crt_check_moduli(crcnn_ctx *ctx, const uint64_t *moduli, int M) {
+    REQUIRE(moduli && M >= 1 && M <= CRT_MAX_MODULI, "an ensemble takes 1 to 16 plain moduli");
+    unsigned __int128 T = 1;
+    for (int i = 0; i < M; i++) {
+        REQUIRE(moduli[i] >= 2, "every plain modulus of an ensemble must be at least 2");
+        for (int j = 0; j < i; j++) REQUIRE(std::gcd(moduli[i], moduli[j]) == 1, "the plain moduli of an ensemble must be pairwise coprime");
+        if (!(T >> 64)) T *= moduli[i];
+    }
+    for (int j = 0; j < ctx->K; j++)
+        REQUIRE(T < ctx->hp.d.tab[j].mod.q, "the product of the plain moduli must be below every coefficient prime");
+    return CRCNN_OK;
+}
+
+// slots[count][96] of ciphertexts [first, first+count) of t: decrypt_range restricted to the coefficients the decoder reads
+int decrypt_slots_range(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, long first, long count, uint64_t *scratch, uint64_t *slots) {
+    ProfScope ps(ctx, KC_REENC, lp_bytes(ctx, (double)count * 2 * ctx->K) + (double)count * REENC_SLOTS * 8, lp_bfly(ctx, (double)count * 2 * ctx->K));
+    const uint64_t *c0 = nullptr;
+    int rc = dec_dot_range(ctx, k, t, first, count, scratch, &c0);
+    if (rc) return rc;
+    CU(launch_dec_scale_slots(k->c, c0, scratch, slots, count, ctx->stream));
+    return CRCNN_OK;
+}
+
+// *gathered = every instance's slots of its tensor t, [world][count][96]: this rank decrypts its block in decrypt_step chunks, then ONE
+// all-gather -- the chunking is each rank's own affair, only the block size (the tensor's count) has to agree
+int crt_gather_slots(crcnn_ctx *ctx, crcnn_crt *crt, crcnn_keys *k, crcnn_tensor *t, uint64_t **gathered) {
+    const long count = t->count, step = decrypt_step(ctx, count);
+    const size_t block = (size_t)count * REENC_SLOTS;
+    uint64_t *scratch = nullptr, *g = nullptr;
+    int rc = dev_alloc(ctx, (size_t)step * ctx->K * ctx->n * 8, (void **)&scratch);
+    if (!rc) rc = dev_alloc(ctx, (size_t)crt->comm->world * block * 8, (void **)&g);
+    uint64_t *mine = rc ? nullptr : g + (size_t)crt->comm->rank * block;
+    for (long c0 = 0; c0 < count && !rc; c0 += step)
+        rc = decrypt_slots_range(ctx, k, t, c0, std::min<long>(step, count - c0), scratch, mine + c0 * REENC_SLOTS);
+    if (!rc) rc = comm_all_gather_words(ctx, crt->comm, mine, block, g);
+    dev_free(ctx, scratch);
+    if (rc) { dev_free(ctx, g); return rc; }
+    *gathered = g;
+    return CRCNN_OK;
+}
+
+int crt_call_check(crcnn_ctx *ctx, crcnn_crt *crt, crcnn_keys *k, crcnn_tensor *t) {
+    REQUIRE(crt && k && t, "null argument");
+    REQUIRE(t->size == 2, "decrypt is implemented for size-2 ciphertexts");
+    REQUIRE(t->count > 0, "empty tensor");
+    REQUIRE(crt->c.t_own == ctx->hp.d.t, "the ensemble was made for a context under another plain modulus");
+    return CRCNN_OK;
+}
+}  // namespace
+
+int crcnn_crt_create(crcnn_ctx *ctx, crcnn_comm *comm, const uint64_t *moduli, int M, crcnn_crt **out) {
+    if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
+    REQUIRE(comm && moduli && out && M >= 1 && M <= CRT_MAX_MODULI, "bad ensemble arguments");
+    // Every check of this rank's arguments runs before the first NCCL call.  A rank that refuses its list still enters the one
+    // fixed-size all-gather, carrying its verdict: a list that fails on some ranks only must not leave the others waiting there.
+    int rc = M == comm->world ? CRCNN_OK : fail(ctx, CRCNN_ERR_INVALID_ARGUMENT, "an ensemble has one plain modulus per rank");
+    if (!rc) rc = crt_check_moduli(ctx, moduli, M);
+    if (!rc && ctx->hp.d.t != moduli[comm->rank]) rc = fail(ctx, CRCNN_ERR_INVALID_ARGUMENT, "the context's plain modulus is not moduli[rank]");
+    const std::string why = ctx->err;
+    constexpr int W = CRT_MAX_MODULI + 2;     // verdict, M, the moduli padded with zeros
+    std::vector<uint64_t> rec(W, 0), all((size_t)comm->world * W);
+    rec[0] = rc == CRCNN_OK; rec[1] = (uint64_t)M;
+    std::copy(moduli, moduli + M, rec.begin() + 2);
+    CU(cudaSetDevice(ctx->device));
+    uint64_t *d = nullptr;
+    int grc = dev_alloc(ctx, all.size() * 8, (void **)&d);
+    if (!grc) {
+        cudaError_t e = cudaMemcpyAsync(d + (size_t)comm->rank * W, rec.data(), W * 8, cudaMemcpyHostToDevice, ctx->stream);
+        if (e != cudaSuccess) grc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
+    }
+    if (!grc) grc = comm_all_gather_words(ctx, comm, d + (size_t)comm->rank * W, W, d);
+    if (!grc) {
+        cudaError_t e = cudaMemcpyAsync(all.data(), d, all.size() * 8, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+        if (e != cudaSuccess) grc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
+    }
+    dev_free(ctx, d);
+    if (rc) return fail(ctx, rc, why);
+    if (grc) return grc;
+    for (int r = 0; r < comm->world; r++) {
+        REQUIRE(all[(size_t)r * W] == 1, "rank " + std::to_string(r) + " refused the ensemble's plain moduli");
+        REQUIRE(std::equal(rec.begin() + 1, rec.end(), all.begin() + (size_t)r * W + 1), "the ranks passed different lists of plain moduli");
+    }
+    auto *c = new crcnn_crt;
+    c->comm = comm;
+    c->moduli.assign(moduli, moduli + M);
+    c->c = make_crt_consts(moduli, M, comm->rank);
+    *out = c;
+    return CRCNN_OK;
+}
+
+int crcnn_crt_free(crcnn_ctx *ctx, crcnn_crt *crt) {
+    if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
+    delete crt;
+    return CRCNN_OK;
+}
+
+int crcnn_crt_decrypt_values(crcnn_ctx *ctx, crcnn_crt *crt, crcnn_keys *k, crcnn_tensor *t, float *host_values) {
+    if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
+    int rc = crt_call_check(ctx, crt, k, t);
+    if (rc) return rc;
+    REQUIRE(host_values, "null argument");
+    CU(cudaSetDevice(ctx->device));
+    uint64_t *g = nullptr;
+    float *vals = nullptr;
+    rc = crt_gather_slots(ctx, crt, k, t, &g);
+    if (!rc) rc = dev_alloc(ctx, (size_t)t->count * 4, (void **)&vals);
+    if (!rc) {
+        cudaError_t er;
+        {
+            ProfScope ps(ctx, KC_REENC, (double)crt->c.M * t->count * REENC_SLOTS * 8 + (double)t->count * 4, 0);
+            er = launch_crt_decode_values(crt->c, g, vals, t->count, ctx->stream);
+        }
+        if (er == cudaSuccess) er = cudaMemcpyAsync(host_values, vals, (size_t)t->count * 4, cudaMemcpyDeviceToHost, ctx->stream);
+        if (er == cudaSuccess) er = cudaStreamSynchronize(ctx->stream);
+        if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(er));
+    }
+    dev_free(ctx, g); dev_free(ctx, vals);
+    return rc;
+}
+
+int crcnn_crt_reencrypt(crcnn_ctx *ctx, crcnn_crt *crt, crcnn_keys *k, crcnn_tensor *in, uint64_t seed, double noise_standard_deviation,
+                        crcnn_tensor **out) {
+    if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
+    int rc = crt_call_check(ctx, crt, k, in);
+    if (rc) return rc;
+    REQUIRE(out, "null argument");
+    CU(cudaSetDevice(ctx->device));
+    const size_t n = ctx->n, pw = poly_words(ctx);
+    const long count = in->count, step = encrypt_step(ctx, count);
+    crcnn_tensor *o = nullptr;
+    uint64_t *g = nullptr, *U = nullptr, *slots = nullptr;
+    int8_t *e = nullptr;
+    rc = crt_gather_slots(ctx, crt, k, in, &g);
+    if (!rc) rc = new_tensor(ctx, count, 2, 0, &o);
+    if (!rc) rc = dev_alloc(ctx, (size_t)step * ctx->K * n * 8, (void **)&U);
+    if (!rc) rc = dev_alloc(ctx, (size_t)step * REENC_SLOTS * 8, (void **)&slots);
+    if (!rc) rc = dev_alloc(ctx, (size_t)step * 2 * n, (void **)&e);
+    // ciphertext counters of rank r start at r 2^48: instances sharing a seed (and perhaps a key set) never share u
+    const long first = (long)((uint64_t)crt->comm->rank << 48);
+    for (long c0 = 0; c0 < count && !rc; c0 += step) {
+        const long cnt = std::min<long>(step, count - c0);
+        cudaError_t er;
+        {
+            ProfScope ps(ctx, KC_REENC, lp_bytes(ctx, (double)cnt * 2 * ctx->K), lp_bfly(ctx, (double)cnt * 3 * ctx->K));
+            er = launch_crt_reencode(crt->c, g, count, c0, slots, cnt, ctx->stream);
+            if (er == cudaSuccess)
+                er = encrypt_range(ctx, k, slots, seed, first + c0, noise_standard_deviation, nullptr, nullptr, U, e, o->d + c0 * 2 * pw, cnt);
+        }
+        if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, std::string("re-encryption: ") + cudaGetErrorString(er));
+    }
+    dev_free(ctx, g); dev_free(ctx, U); dev_free(ctx, slots); dev_free(ctx, e);
+    if (rc) { if (o) crcnn_tensor_free(ctx, o); return rc; }
+    *out = o;
+    return CRCNN_OK;
+}
+
+int crcnn_crt_decode_values(crcnn_ctx *ctx, int M, const uint64_t *moduli, const uint64_t *const *host_plain, long count, float *host_values) {
+    if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
+    int rc = crt_check_moduli(ctx, moduli, M);
+    if (rc) return rc;
+    REQUIRE(host_plain && host_values && count > 0, "bad decode arguments");
+    const size_t n = ctx->n;
+    std::vector<uint64_t> slots((size_t)M * count * REENC_SLOTS);
+    for (int m = 0; m < M; m++) {
+        REQUIRE(host_plain[m], "null plaintext array");
+        for (long r = 0; r < count; r++) {
+            const uint64_t *p = host_plain[m] + (size_t)r * (n + 1);
+            uint64_t *s = slots.data() + ((size_t)m * count + r) * REENC_SLOTS;
+            for (int j = 0; j < REENC_SLOTS; j++) {
+                s[j] = p[j < 64 ? j : n - REENC_SLOTS + j];
+                REQUIRE(s[j] < moduli[m], "a plaintext coefficient is not below its plain modulus");
+            }
+        }
+    }
+    CU(cudaSetDevice(ctx->device));
+    uint64_t *d = nullptr;
+    float *vals = nullptr;
+    rc = dev_alloc(ctx, slots.size() * 8, (void **)&d);
+    if (!rc) rc = dev_alloc(ctx, (size_t)count * 4, (void **)&vals);
+    if (!rc) {
+        cudaError_t er = cudaMemcpyAsync(d, slots.data(), slots.size() * 8, cudaMemcpyHostToDevice, ctx->stream);
+        if (er == cudaSuccess) er = launch_crt_decode_values(make_crt_consts(moduli, M, 0), d, vals, count, ctx->stream);
+        if (er == cudaSuccess) er = cudaMemcpyAsync(host_values, vals, (size_t)count * 4, cudaMemcpyDeviceToHost, ctx->stream);
+        if (er == cudaSuccess) er = cudaStreamSynchronize(ctx->stream);
+        if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(er));
+    }
+    dev_free(ctx, d); dev_free(ctx, vals);
     return rc;
 }
 

@@ -33,6 +33,21 @@ ReencConsts make_reenc_consts(const DeviceParams &d) {
     return c;
 }
 
+CrtConsts make_crt_consts(const uint64_t *moduli, int M, int own) {
+    CrtConsts c{};
+    c.M = M;
+    uint64_t p = 1;
+    for (int k = 0; k < M; k++) {
+        c.tm[k] = make_mod(moduli[k]);
+        c.prefix[k] = p;
+        c.inv[k] = k ? inv_mod(p % moduli[k], moduli[k]) : 0;
+        p *= moduli[k];
+    }
+    c.T = p; c.half = (p + 1) >> 1;
+    c.t_own = moduli[own];
+    return c;
+}
+
 // w[NB_WORDS] *= v
 static void words_mul(uint64_t *w, uint64_t v) {
     u128h carry = 0;
@@ -83,15 +98,10 @@ dec_dot_kernel(const __grid_constant__ ReencConsts c, const uint64_t *__restrict
     }
 }
 
-// One thread per coefficient: the K residues of c0 + c1 s -> the plaintext coefficient (decryptor.cpp:172-234)
-__global__ void __launch_bounds__(128)
-dec_scale_kernel(const __grid_constant__ ReencConsts c, const uint64_t *__restrict__ ct, const uint64_t *__restrict__ tmp,
-                 uint64_t *__restrict__ plain, long total) {
-    const long w = (long)blockIdx.x * 128 + threadIdx.x;
-    if (w >= total) return;
+// The K residues of c0 + c1 s at coefficient k of ciphertext cti -> the plaintext coefficient (decryptor.cpp:172-234)
+__device__ __forceinline__ uint64_t dec_scale_coeff(const ReencConsts &c, const uint64_t *__restrict__ ct, const uint64_t *__restrict__ tmp,
+                                                    long cti, int k) {
     const int n = c.n, K = c.K;
-    const int k = (int)(w % n);
-    const long cti = w / n;
     Acc7 at = acc7_zero(), ag = acc7_zero();
     for (int i = 0; i < K; i++) {
         uint64_t d = __ldg(tmp + (cti * K + i) * (long)n + k);
@@ -105,7 +115,26 @@ dec_scale_kernel(const __grid_constant__ ReencConsts c, const uint64_t *__restri
     uint64_t r;
     if (a_g > (c.gamma >> 1)) r = addmod(a_t, reduce64(c.gamma - a_g, c.tm), c.t);          // :207-217
     else r = submod(a_t, reduce64(a_g, c.tm), c.t);                                         // :219-224
-    plain[w] = mulmod(r, c.inv_gamma_t, c.tm);                                              // :233-234
+    return mulmod(r, c.inv_gamma_t, c.tm);                                                  // :233-234
+}
+
+// One thread per coefficient: plain[count][n]
+__global__ void __launch_bounds__(128)
+dec_scale_kernel(const __grid_constant__ ReencConsts c, const uint64_t *__restrict__ ct, const uint64_t *__restrict__ tmp,
+                 uint64_t *__restrict__ plain, long total) {
+    const long w = (long)blockIdx.x * 128 + threadIdx.x;
+    if (w >= total) return;
+    plain[w] = dec_scale_coeff(c, ct, tmp, w / c.n, (int)(w % c.n));
+}
+
+// One thread per slot: slots[count][96], slot j < 64 is coefficient j, slot j >= 64 coefficient n - 96 + j
+__global__ void __launch_bounds__(128)
+dec_scale_slots_kernel(const __grid_constant__ ReencConsts c, const uint64_t *__restrict__ ct, const uint64_t *__restrict__ tmp,
+                       uint64_t *__restrict__ slots, long total) {
+    const long w = (long)blockIdx.x * 128 + threadIdx.x;
+    if (w >= total) return;
+    const int j = (int)(w % REENC_SLOTS);
+    slots[w] = dec_scale_coeff(c, ct, tmp, w / REENC_SLOTS, j < 64 ? j : c.n - REENC_SLOTS + j);
 }
 
 // x -= y when x >= y (NB_WORDS words each); returns whether it subtracted
@@ -193,29 +222,34 @@ noise_bits_kernel(const __grid_constant__ BudgetConsts c, const uint64_t *__rest
 // ---------------------------------------------------------------------------------------------- decode -> float -> encode
 // IEEE double arithmetic with explicit round-to-nearest intrinsics: no fused multiply-add may change a digit.
 
-// BalancedFractionalEncoder::decode / BalancedEncoder::decode_int64 (SEAL/seal/encoder.cpp) of the plaintext p[n]
-__device__ __forceinline__ double decode_fractional(const ReencConsts &c, const uint64_t *p) {
-    const int n = c.n;
-    const uint64_t t = c.t, neg = c.half;          // coeff_neg_threshold_ = (t + 1) >> 1
+// BalancedFractionalEncoder::decode / BalancedEncoder::decode_int64 (SEAL/seal/encoder.cpp) under plain modulus t with
+// coeff_neg_threshold_ half = (t + 1) >> 1; coef(j) is slot j of the plaintext: coefficient j for j < 64, coefficient n - 96 + j above.
+// The single-modulus path reads a decrypted plaintext, the CRT ensembles compose each coefficient from the instances' residues.
+template <class Coef>
+__device__ __forceinline__ double decode_fractional(uint64_t t, uint64_t half, const Coef &coef) {
     long long ip = 0;
     for (int i = 63; i >= 0; i--) {
-        const uint64_t cf = p[i];
-        const long long v = cf >= neg ? -(long long)(t - cf) : (long long)cf;
+        const uint64_t cf = coef(i);
+        const long long v = cf >= half ? -(long long)(t - cf) : (long long)cf;
         ip = (long long)((unsigned long long)ip * 3ull) + v;
     }
     double frac = 0;
     for (int i = 0; i < 32; i++) {
-        const uint64_t cf = p[n - 32 + i];
-        const long long v = cf >= neg ? -(long long)(t - cf) : (long long)cf;
+        const uint64_t cf = coef(64 + i);
+        const long long v = cf >= half ? -(long long)(t - cf) : (long long)cf;
         frac = __ddiv_rn(__dadd_rn(frac, (double)v), 3.0);
     }
     return __dadd_rn((double)ip, -frac);
 }
 
+__device__ __forceinline__ double decode_plain(const ReencConsts &c, const uint64_t *p) {
+    const int tail = c.n - REENC_SLOTS;
+    return decode_fractional(c.t, c.half, [p, tail](int j) { return p[j < 64 ? j : tail + j]; });
+}
+
 // BalancedFractionalEncoder::encode of value (the restatement of params.cpp: encode_fractional_sparse, checked against the oracle):
 // s[96] = coefficients 0..63 and n-32..n-1
-__device__ __forceinline__ void encode_fractional(const ReencConsts &c, double value, uint64_t *s) {
-    const uint64_t t = c.t;
+__device__ __forceinline__ void encode_fractional(uint64_t t, double value, uint64_t *s) {
     for (int i = 0; i < REENC_SLOTS; i++) s[i] = 0;
     const long long ipart = (long long)round(value);
     {
@@ -246,9 +280,9 @@ reencode_kernel(const __grid_constant__ ReencConsts c, const uint64_t *__restric
                 float *__restrict__ values, long count) {
     const long cti = (long)blockIdx.x * 128 + threadIdx.x;
     if (cti >= count) return;
-    const float f = (float)decode_fractional(c, plain + cti * (long)c.n);     // floatCube (CrCNN/src/globals.h:16): the value passes through a float
+    const float f = (float)decode_plain(c, plain + cti * (long)c.n);          // floatCube (CrCNN/src/globals.h:16): the value passes through a float
     if (values) values[cti] = f;
-    encode_fractional(c, (double)f, slots + cti * REENC_SLOTS);
+    encode_fractional(c.t, (double)f, slots + cti * REENC_SLOTS);
 }
 
 // encryptImage's encoding: fraencoder->encode(image[z][x][y]), the float promoted to double (CrCNN/src/globals.cpp:207-226)
@@ -256,7 +290,7 @@ __global__ void __launch_bounds__(128)
 encode_values_kernel(const __grid_constant__ ReencConsts c, const float *__restrict__ values, uint64_t *__restrict__ slots, long count) {
     const long cti = (long)blockIdx.x * 128 + threadIdx.x;
     if (cti >= count) return;
-    encode_fractional(c, (double)values[cti], slots + cti * REENC_SLOTS);
+    encode_fractional(c.t, (double)values[cti], slots + cti * REENC_SLOTS);
 }
 
 // decryptImage's decoding: (float) fraencoder->decode(plain) (CrCNN/src/globals.cpp:127-142)
@@ -264,7 +298,42 @@ __global__ void __launch_bounds__(128)
 decode_values_kernel(const __grid_constant__ ReencConsts c, const uint64_t *__restrict__ plain, float *__restrict__ values, long count) {
     const long cti = (long)blockIdx.x * 128 + threadIdx.x;
     if (cti >= count) return;
-    values[cti] = (float)decode_fractional(c, plain + cti * (long)c.n);
+    values[cti] = (float)decode_plain(c, plain + cti * (long)c.n);
+}
+
+// ---------------------------------------------------------------------------------------------- CRT ensembles
+// Garner's recombination of slot j of ciphertext cti from slots[M][total][96]
+__device__ __forceinline__ uint64_t crt_compose(const CrtConsts &c, const uint64_t *__restrict__ slots, long total, long cti, int j) {
+    const long stride = total * REENC_SLOTS, at = cti * REENC_SLOTS + j;
+    uint64_t x = __ldg(slots + at);
+    for (int k = 1; k < c.M; k++) {
+        const Mod &m = c.tm[k];
+        const uint64_t v = mulmod(submod(__ldg(slots + k * stride + at), reduce64(x, m), m.q), c.inv[k], m);
+        x += v * c.prefix[k];                 // x < t_1 ... t_k <= T
+    }
+    return x;
+}
+
+__device__ __forceinline__ double crt_decode(const CrtConsts &c, const uint64_t *slots, long total, long cti) {
+    return decode_fractional(c.T, c.half, [&](int j) { return crt_compose(c, slots, total, cti, j); });
+}
+
+// decryptImage's decoding under T: (float) FractionalEncoder::decode of the composed plaintext
+__global__ void __launch_bounds__(128)
+crt_decode_values_kernel(const __grid_constant__ CrtConsts c, const uint64_t *__restrict__ slots, float *__restrict__ values, long count) {
+    const long cti = (long)blockIdx.x * 128 + threadIdx.x;
+    if (cti >= count) return;
+    values[cti] = (float)crt_decode(c, slots, count, cti);
+}
+
+// reencode_kernel's step for an ensemble: decode under T, through a float (floatCube), encode under this instance's t
+__global__ void __launch_bounds__(128)
+crt_reencode_kernel(const __grid_constant__ CrtConsts c, const uint64_t *__restrict__ slots, long total, long first,
+                    uint64_t *__restrict__ out, long count) {
+    const long r = (long)blockIdx.x * 128 + threadIdx.x;
+    if (r >= count) return;
+    const float f = (float)crt_decode(c, slots, total, first + r);
+    encode_fractional(c.t_own, (double)f, out + r * REENC_SLOTS);
 }
 
 // ---------------------------------------------------------------------------------------------- encrypt
@@ -371,6 +440,12 @@ cudaError_t launch_dec_scale(const ReencConsts &c, const uint64_t *ct, const uin
     dec_scale_kernel<<<blocks(total, 128), 128, 0, s>>>(c, ct, tmp, plain, total);
     return cudaGetLastError();
 }
+cudaError_t launch_dec_scale_slots(const ReencConsts &c, const uint64_t *ct, const uint64_t *tmp, uint64_t *slots, long count, cudaStream_t s) {
+    const long total = count * REENC_SLOTS;
+    if (total <= 0) return cudaSuccess;
+    dec_scale_slots_kernel<<<blocks(total, 128), 128, 0, s>>>(c, ct, tmp, slots, total);
+    return cudaGetLastError();
+}
 cudaError_t launch_noise_bits(const BudgetConsts &c, const uint64_t *ct, const uint64_t *tmp, int *bits, long count, cudaStream_t s) {
     const long total = count * (long)c.n;
     if (total <= 0) return cudaSuccess;
@@ -391,6 +466,16 @@ cudaError_t launch_encode_values(const ReencConsts &c, const float *values, uint
 cudaError_t launch_decode_values(const ReencConsts &c, const uint64_t *plain, float *values, long count, cudaStream_t s) {
     if (count <= 0) return cudaSuccess;
     decode_values_kernel<<<blocks(count, 128), 128, 0, s>>>(c, plain, values, count);
+    return cudaGetLastError();
+}
+cudaError_t launch_crt_decode_values(const CrtConsts &c, const uint64_t *slots, float *values, long count, cudaStream_t s) {
+    if (count <= 0) return cudaSuccess;
+    crt_decode_values_kernel<<<blocks(count, 128), 128, 0, s>>>(c, slots, values, count);
+    return cudaGetLastError();
+}
+cudaError_t launch_crt_reencode(const CrtConsts &c, const uint64_t *slots, long total, long first, uint64_t *out, long count, cudaStream_t s) {
+    if (count <= 0) return cudaSuccess;
+    crt_reencode_kernel<<<blocks(count, 128), 128, 0, s>>>(c, slots, total, first, out, count);
     return cudaGetLastError();
 }
 cudaError_t launch_enc_sample(const ReencConsts &c, uint64_t seed, long first_ct, double sigma, double max_dev, const int8_t *given,

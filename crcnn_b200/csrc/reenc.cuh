@@ -60,6 +60,9 @@ cudaError_t launch_reencode(const ReencConsts &c, const uint64_t *plain, uint64_
 cudaError_t launch_encode_values(const ReencConsts &c, const float *values, uint64_t *slots, long count, cudaStream_t s);
 // values[count] = (float) FractionalEncoder::decode(plain[i]), plain[count][n] as launch_dec_scale leaves it
 cudaError_t launch_decode_values(const ReencConsts &c, const uint64_t *plain, float *values, long count, cudaStream_t s);
+// Decryptor::decrypt restricted to the coefficients the fractional decoder reads: slots[count][96] = coefficients 0..63 and
+// n-32..n-1 of launch_dec_scale's plaintexts (tmp and ct as for launch_dec_scale)
+cudaError_t launch_dec_scale_slots(const ReencConsts &c, const uint64_t *ct, const uint64_t *tmp, uint64_t *slots, long count, cudaStream_t s);
 // u (as residues, U[count][K][n]) and e[count][2][n] (int8): sampled from (seed, ciphertext index, coefficient) or copied from `given`
 // ([count][3][n] int8: u, e0, e1)
 cudaError_t launch_enc_sample(const ReencConsts &c, uint64_t seed, long first_ct, double sigma, double max_dev, const int8_t *given,
@@ -68,5 +71,27 @@ cudaError_t launch_enc_sample(const ReencConsts &c, uint64_t seed, long first_ct
 cudaError_t launch_enc_mul(const ReencConsts &c, const uint64_t *U, const uint64_t *pk, uint64_t *out, long count, cudaStream_t s);
 // out (coefficient form after the inverse transform) += e_p (+ Delta * m on polynomial 0)
 cudaError_t launch_enc_finish(const ReencConsts &c, const uint64_t *slots, const int8_t *e, uint64_t *out, long count, cudaStream_t s);
+
+// CRT plaintext-modulus ensembles: M instances under pairwise coprime t_1 .. t_M stand for one under T = t_1 ... t_M.  A coefficient
+// is rebuilt modulo T from its M residues by Garner's mixed-radix recombination, x = r_1 + v_2 t_1 + v_3 t_1 t_2 + ..., with
+// v_k = (r_k - x_{k-1}) (t_1 ... t_{k-1})^-1 mod t_k; T is below every coefficient prime (< 2^61), so every partial sum fits a word.
+constexpr int CRT_MAX_MODULI = 16;
+struct CrtConsts {
+    int M;
+    uint64_t T, half;                     // the product and BalancedEncoder's negative threshold (T + 1) >> 1 under it
+    Mod tm[CRT_MAX_MODULI];               // t_k
+    uint64_t prefix[CRT_MAX_MODULI];      // t_1 ... t_{k-1} (prefix[0] = 1)
+    uint64_t inv[CRT_MAX_MODULI];         // (t_1 ... t_{k-1})^-1 mod t_k (inv[0] unused)
+    uint64_t t_own;                       // this instance's modulus, the one re-encoded plaintexts are written under
+};
+
+// moduli[M] pairwise coprime with a product below 2^62 (the caller checks); own: index of this instance's modulus
+CrtConsts make_crt_consts(const uint64_t *moduli, int M, int own);
+// values[count] = (float) BalancedFractionalEncoder::decode under T of the coefficients composed from slots[M][count][96]
+// (instance k's block of launch_dec_scale_slots output at slots + k count 96)
+cudaError_t launch_crt_decode_values(const CrtConsts &c, const uint64_t *slots, float *values, long count, cudaStream_t s);
+// ciphertexts [first, first + count) of slots[M][total][96]: compose, decode under T, round to float, encode under t_own into
+// out[count][96] (launch_reencode's layout, ready for launch_enc_finish)
+cudaError_t launch_crt_reencode(const CrtConsts &c, const uint64_t *slots, long total, long first, uint64_t *out, long count, cudaStream_t s);
 
 }  // namespace crcnn

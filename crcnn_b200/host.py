@@ -48,6 +48,8 @@ def load():
     h.crcnn_host_budget_log.argtypes = [C.POINTER(_I)] * 3 + [_I]
     h.crcnn_host_budget_log.restype = _I
     h.crcnn_host_predict_values.argtypes = [C.POINTER(C.c_float), _I, C.c_uint64, C.POINTER(C.c_float), C.POINTER(_I)]
+    h.crcnn_host_crt_begin.argtypes = [_vp, _I, _I, _vp, C.c_uint64]
+    h.crcnn_host_crt_predict_values.argtypes = [C.POINTER(C.c_float), _I, C.c_uint64, C.POINTER(C.c_float)]
     _h = h
     return h
 
@@ -206,6 +208,24 @@ class HostNetwork:
         if rc == CRCNN_ERR_OUT_OF_BUDGET:
             raise OutOfBudget(self.h.crcnn_host_last_error().decode(), failed.value)
         self._chk(rc)
+        return out
+
+    def crt_begin(self, moduli, rank, nccl_id, reencrypt_seed):
+        """CrtEnsemble over this network (built with world 1, keys installed with use_keys): this process holds the instance under
+        moduli[rank], the network's own plain modulus.  Collective: every rank calls it with the same moduli and nccl_id."""
+        m = np.ascontiguousarray([int(v) for v in moduli], dtype=np.uint64)
+        idbuf = (C.c_char * 128).from_buffer_copy(nccl_id)
+        self._chk(self.h.crcnn_host_crt_begin(m.ctypes.data, len(m), int(rank), C.cast(idbuf, _vp), C.c_uint64(reencrypt_seed)))
+
+    def crt_predict_values(self, images, batch=1, seed=0):
+        """CrtEnsemble::predict (collective): predict_values of the ensemble, the scores decoded under the product of the moduli
+        -> float32 [batch][outputs], the same on every rank."""
+        x = np.ascontiguousarray(images, dtype=np.float32).ravel()
+        if x.size != batch * self.zd * self.xd * self.yd:
+            raise ValueError("images must hold batch * %d values" % (self.zd * self.xd * self.yd))
+        out = np.zeros((batch, self.outputs), dtype=np.float32)
+        fp = C.POINTER(C.c_float)
+        self._chk(self.h.crcnn_host_crt_predict_values(x.ctypes.data_as(fp), batch, C.c_uint64(seed), out.ctypes.data_as(fp)))
         return out
 
     def budget_log(self):

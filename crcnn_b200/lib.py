@@ -103,6 +103,11 @@ SYMBOLS = [
     ("crcnn_reencrypt", _I, [_vp, _vp, _vp, C.c_uint64, C.c_double, _vp, _vpp, _vp, _vp]),
     ("crcnn_encrypt_values", _I, [_vp, _vp, _f32p, C.c_long, C.c_uint64, C.c_double, _vp, _vpp]),
     ("crcnn_decrypt_values", _I, [_vp, _vp, _vp, _f32p]),
+    ("crcnn_crt_create", _I, [_vp, _vp, _u64p, _I, _vpp]),
+    ("crcnn_crt_free", _I, [_vp, _vp]),
+    ("crcnn_crt_decrypt_values", _I, [_vp, _vp, _vp, _vp, _f32p]),
+    ("crcnn_crt_reencrypt", _I, [_vp, _vp, _vp, _vp, C.c_uint64, C.c_double, _vpp]),
+    ("crcnn_crt_decode_values", _I, [_vp, _I, _u64p, C.POINTER(_u64p), _L, _f32p]),
     ("crcnn_probe_pipe", _I, [_vp, _I, _I, _I, _I, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
 ]
 
@@ -375,6 +380,34 @@ class Engine:
         """(float) FractionalEncoder::decode(Decryptor::decrypt(ct)) of every ciphertext of t -> float32[count]."""
         out = np.zeros(self.count(t), dtype=np.float32)
         self._chk(self.lib.crcnn_decrypt_values(self.h, keys.ptr if keys is not None else None, t.ptr, out.ctypes.data_as(_f32p)))
+        return out
+
+    # ---- CRT plaintext-modulus ensembles (include/crcnn_b200.h)
+    def crt_create(self, comm_ptr, moduli):
+        """Collective: this context's place in the ensemble of `moduli` over the NCCL communicator comm_ptr (crcnn_comm_create)."""
+        m = np.ascontiguousarray([int(v) for v in moduli], dtype=np.uint64)
+        return self._new(self.lib.crcnn_crt_create, "crt", C.c_void_p(comm_ptr), m.ctypes.data_as(_u64p), len(m))
+
+    def crt_decrypt_values(self, crt, keys, t):
+        """Collective: (float) FractionalEncoder::decode under the product modulus of the instances' plaintexts -> float32[count]."""
+        out = np.zeros(self.count(t), dtype=np.float32)
+        self._chk(self.lib.crcnn_crt_decrypt_values(self.h, crt.ptr, keys.ptr, t.ptr, out.ctypes.data_as(_f32p)))
+        return out
+
+    def crt_reencrypt(self, crt, keys, t, seed=0, sigma=0.0):
+        """Collective: decrypt, recombine and decode under the product modulus, float, encode under this context's t, encrypt."""
+        return self._new(self.lib.crcnn_crt_reencrypt, "tensor", crt.ptr, keys.ptr, t.ptr, C.c_uint64(seed), C.c_double(sigma))
+
+    def crt_decode_values(self, moduli, plains):
+        """(float) FractionalEncoder::decode under prod(moduli) of the plaintexts recombined from plains[m] ([count][n+1] words of
+        the instance under moduli[m], as decrypt() returns them) -> float32[count]."""
+        m = np.ascontiguousarray([int(v) for v in moduli], dtype=np.uint64)
+        arrs = [np.ascontiguousarray(p, dtype=np.uint64).reshape(-1, self.stride) for p in plains]
+        count = arrs[0].shape[0] if arrs else 0
+        assert len(arrs) == len(m) and all(a.shape[0] == count for a in arrs)
+        ptrs = (_u64p * len(arrs))(*[a.ctypes.data_as(_u64p) for a in arrs])
+        out = np.zeros(count, dtype=np.float32)
+        self._chk(self.lib.crcnn_crt_decode_values(self.h, len(m), m.ctypes.data_as(_u64p), ptrs, count, out.ctypes.data_as(_f32p)))
         return out
 
     # ---- layers

@@ -36,6 +36,7 @@ typedef struct crcnn_plain crcnn_plain;   /* device pack of plaintexts (weights,
 typedef struct crcnn_evk crcnn_evk;       /* device copy of evaluation (relinearisation) keys */
 typedef struct crcnn_keys crcnn_keys;     /* device copy of the key holder's secret and public key (opt-in: GPU re-encryption) */
 typedef struct crcnn_comm crcnn_comm;     /* NCCL communicator of a group of contexts, one per GPU (output-neuron sharding) */
+typedef struct crcnn_crt crcnn_crt;       /* CRT plaintext-modulus ensemble: this rank's place in it (plain moduli, recombination constants) */
 
 typedef enum {
     CRCNN_OK = 0,
@@ -330,6 +331,35 @@ int crcnn_encrypt_values(crcnn_ctx *ctx, crcnn_keys *keys, const float *host_val
 /* decryptImage's inner loop: host_values[i] = (float) FractionalEncoder::decode(Decryptor::decrypt(ciphertext i of t)), size-2
  * ciphertexts in either domain; only the count floats leave the device. */
 int crcnn_decrypt_values(crcnn_ctx *ctx, crcnn_keys *keys, crcnn_tensor *t, float *host_values);
+
+/* ---- CRT plaintext-modulus ensembles (opt-in, the same keys) ----------------------------------------------
+ * A plain modulus T is split into pairwise coprime t_1 .. t_M (M <= 16); instance i is an ordinary context under t_i, one per GPU
+ * and process, running the whole network; the instances' plaintexts are recombined modulo T by CRT (Garner's mixed radix) on the
+ * device, so decryption and the re-encryption before layer 6 see exactly what one context under T would see.  FV keys depend on
+ * n and q only: the instances may share one key set or have one each.  The scores equal a single-modulus run under T bit for bit
+ * as long as every instance keeps a noise budget.  T must be below every coefficient prime, the condition of a context under T. */
+/* Replaces: setParameters' single plain modulus (CrCNN/src/globals.cpp:25-56) for the ensemble.  Collective: every rank of comm
+ * calls it with its context (plain modulus moduli[rank]) and the same list.  Every check of the arguments (M == world, t_i >= 2,
+ * pairwise coprime, product below every coefficient prime, the context's t == moduli[rank]) runs before the first NCCL call; then
+ * one fixed-size all-gather carries each rank's list and verdict, so every rank returns CRCNN_ERR_INVALID_ARGUMENT when any rank
+ * refused its list or the lists differ -- no rank is left waiting.  comm must outlive the ensemble. */
+int crcnn_crt_create(crcnn_ctx *ctx, crcnn_comm *comm, const uint64_t *moduli, int M, crcnn_crt **out);
+int crcnn_crt_free(crcnn_ctx *ctx, crcnn_crt *crt);
+/* Replaces: decryptImage (CrCNN/src/globals.cpp:127-142) under T.  Collective: every rank passes its instance's tensor (same
+ * count on every rank); Decryptor::decrypt of the coefficients the fractional decoder reads, one all-gather of them, then
+ * host_values[i] = (float) FractionalEncoder::decode under T of the recombined plaintext -- the same floats on every rank. */
+int crcnn_crt_decrypt_values(crcnn_ctx *ctx, crcnn_crt *crt, crcnn_keys *keys, crcnn_tensor *t, float *host_values);
+/* Replaces: the noise reset inside Network::forward (CrCNN/src/network.cpp:30-33) under T.  Collective, like
+ * crcnn_crt_decrypt_values; the decoded float of every ciphertext is encoded under this rank's t_i and encrypted as
+ * crcnn_reencrypt does.  Noise from the generator keyed by seed, with rank r's ciphertext counters offset by r 2^48: ranks that
+ * share a seed never share u. */
+int crcnn_crt_reencrypt(crcnn_ctx *ctx, crcnn_crt *crt, crcnn_keys *keys, crcnn_tensor *in, uint64_t seed,
+                        double noise_standard_deviation, crcnn_tensor **out);
+/* Replaces: the key holder's recombination on the host.  Not collective: host_plain[m] holds count plaintexts of instance m as
+ * crcnn_decrypt returns them (n+1 words each, values below moduli[m]); host_values[i] = (float) FractionalEncoder::decode under
+ * T of plaintext i recombined from the M instances.  The moduli are checked as crcnn_crt_create checks them against ctx. */
+int crcnn_crt_decode_values(crcnn_ctx *ctx, int M, const uint64_t *moduli, const uint64_t *const *host_plain, long count,
+                            float *host_values);
 
 /* ---- measurement ------------------------------------------------------------------------------
  * Kernel classes are timed with CUDA events on the context's stream while profiling is on. */
