@@ -7,8 +7,9 @@
 //     the host members are filled on demand (materializeHostParameters) when a caller asks for them or saves the net;
 //   * buildNetwork(file_name) builds the reference's ACTIVE block (PlainModelTiny, cnnBuilder.cpp:157-169);
 //     buildNetwork(topology, file_name) also offers the two blocks the reference keeps commented out (Approx, WoPad,
-//     cnnBuilder.cpp:115-155) and "PlainModel" = the weights file PlainModel.h5 run on a 32x32 zero-bordered input
-//     (SURVEY.md 8(a): that file was trained with padding 2 and has no builder block in the reference).
+//     cnnBuilder.cpp:115-155), "PlainModelPadded" = the weights file PlainModel.h5 as it was trained, conv1 with padding 2 on a
+//     28x28 input, and "PlainModel" = the same weights run on a 32x32 input that carries the zero border itself
+//     (SURVEY.md 8(a): that file has no builder block in the reference, whose layers have no padding).
 // The simulator builders (buildSimulatedNetwork, ChooserPoly) are out of scope: noise estimation, not the forward path.
 #pragma once
 #include <cmath>
@@ -39,6 +40,13 @@ public:
         if (infile != NULL) return new ConvolutionalLayer(name, xd, yd, zd, xs, ys, xf, yf, nf, th_count, infile);
         std::vector<float> weights = getPretrained(name + ".weight"), biases = getPretrained(name + ".bias");
         return new ConvolutionalLayer(name, xd, yd, zd, xs, ys, xf, yf, nf, th_count, weights, biases);
+    }
+    // the same with zero padding (xp, yp) (ConvolutionalLayer's padded constructors)
+    ConvolutionalLayer *buildConvolutionalLayer(std::string name, int xd, int yd, int zd, int xs, int ys, int xf, int yf, int nf, int xp, int yp,
+                                                int th_count, std::istream *infile) {
+        if (infile != NULL) return new ConvolutionalLayer(name, xd, yd, zd, xs, ys, xf, yf, nf, xp, yp, th_count, infile);
+        std::vector<float> weights = getPretrained(name + ".weight"), biases = getPretrained(name + ".bias");
+        return new ConvolutionalLayer(name, xd, yd, zd, xs, ys, xf, yf, nf, xp, yp, th_count, weights, biases);
     }
     // cnnBuilder.cpp:54-77
     FullyConnectedLayer *buildFullyConnectedLayer(std::string name, int in_dim, int out_dim, int th_count, std::istream *infile) {
@@ -86,12 +94,13 @@ public:
                 add(buildAvgPoolingLayer("pool2", 8, 8, 64, 2, 2, 2, 2));
                 add(buildFullyConnectedLayer("classifier.fc3", 4 * 4 * 64, 512, th_tiny2, infile));
                 add(buildFullyConnectedLayer("classifier.fc4", 512, 10, th_tiny2, infile));
-            } else if (topology == "Approx" || topology == "WoPad" || topology == "PlainModel") {
-                // cnnBuilder.cpp:115-134 (avg-pool) / 136-155 (sum-pool); PlainModel: 32x32 zero-bordered input, fc3 1250 -> 500
+            } else if (topology == "Approx" || topology == "WoPad" || topology == "PlainModel" || topology == "PlainModelPadded") {
+                // cnnBuilder.cpp:115-134 (avg-pool) / 136-155 (sum-pool); PlainModel: 32x32 zero-bordered input, PlainModelPadded: 28x28 input
+                // and conv1 with padding 2 (as PlainModel.h5 was trained); both 14 -> 13 -> 6 -> 5, fc3 1250 -> 500
                 const bool avg = topology != "WoPad";
-                const int in = topology == "PlainModel" ? 32 : 28;
-                const int c1 = (in - 5) / 2 + 1, p1 = c1 - 1, c2 = (p1 - 3) / 2 + 1, p2 = c2 - 1;
-                add(buildConvolutionalLayer("pool1_features.conv1", in, in, 1, 2, 2, 5, 5, 20, th_count, infile));
+                const int in = topology == "PlainModel" ? 32 : 28, pad = topology == "PlainModelPadded" ? 2 : 0;
+                const int c1 = (in + 2 * pad - 5) / 2 + 1, p1 = c1 - 1, c2 = (p1 - 3) / 2 + 1, p2 = c2 - 1;
+                add(buildConvolutionalLayer("pool1_features.conv1", in, in, 1, 2, 2, 5, 5, 20, pad, pad, th_count, infile));
                 if (avg) add(buildAvgPoolingLayer("pool1", c1, c1, 20, 1, 1, 2, 2)); else add(buildPoolingLayer("pool1", c1, c1, 20, 1, 1, 2, 2));
                 add(buildBatchNormLayer("pool1_features.norm1", 20, infile));
                 add(buildConvolutionalLayer("pool2_features.conv2", p1, p1, 20, 2, 2, 3, 3, 50, th_count2, infile));

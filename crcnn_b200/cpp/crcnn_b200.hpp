@@ -363,6 +363,7 @@ class BatchNormLayer;
 class ConvolutionalLayer : public Layer {
 public:
     int xd, yd, zd, xs, ys, xf, yf, nf, th_count;  // th_count is accepted and ignored (the GPU schedules the work)
+    int xp, yp;   // zero padding: xp columns and yp rows of all-zero ciphertexts on each side of the input (0 in the reference's layers)
     int xo, yo, zo;
     plaintext4D filters;  // nf,zd,xf,yf -- never modified by forward (the reference NTT-transforms them in place)
     std::vector<Plaintext> biases;
@@ -370,21 +371,34 @@ public:
 
     ConvolutionalLayer(std::string name, int xd, int yd, int zd, int xs, int ys, int xf, int yf, int nf, int th_count,
                        plaintext4D &filters, std::vector<Plaintext> &biases)
-        : Layer(name), xd(xd), yd(yd), zd(zd), xs(xs), ys(ys), xf(xf), yf(yf), nf(nf), th_count(th_count),
-          xo((xd - xf) / xs + 1), yo((yd - yf) / ys + 1), zo(nf), filters(filters), biases(biases), filters_already_ntt(false) {}
+        : ConvolutionalLayer(name, xd, yd, zd, xs, ys, xf, yf, nf, 0, 0, th_count, filters, biases) {}
     ConvolutionalLayer(std::string name, int xd, int yd, int zd, int xs, int ys, int xf, int yf, int nf, int th_count,
                        std::istream *infile)
-        : Layer(name), xd(xd), yd(yd), zd(zd), xs(xs), ys(ys), xf(xf), yf(yf), nf(nf), th_count(th_count),
-          xo((xd - xf) / xs + 1), yo((yd - yf) / ys + 1), zo(nf), filters_already_ntt(false) {
-        loadPlaintextParameters(infile);
-    }
-
+        : ConvolutionalLayer(name, xd, yd, zd, xs, ys, xf, yf, nf, 0, 0, th_count, infile) {}
     // Trained floats in the reference's order [nf][zd][xf][yf] (cnnBuilder.cpp:36-47), encoded on the device; the host
     // members `filters` / `biases` stay empty until materializeHostParameters() (getKernel, getBias and save call it).
     ConvolutionalLayer(std::string name, int xd, int yd, int zd, int xs, int ys, int xf, int yf, int nf, int th_count,
                        const std::vector<float> &weights, const std::vector<float> &bias_values)
-        : Layer(name), xd(xd), yd(yd), zd(zd), xs(xs), ys(ys), xf(xf), yf(yf), nf(nf), th_count(th_count),
-          xo((xd - xf) / xs + 1), yo((yd - yf) / ys + 1), zo(nf), filters_already_ntt(false) {
+        : ConvolutionalLayer(name, xd, yd, zd, xs, ys, xf, yf, nf, 0, 0, th_count, weights, bias_values) {}
+
+    // The same three forms with zero padding (xp, yp), 0 <= xp < xf and 0 <= yp < yf: the layer computes what the reference's
+    // forward computes on the input with a border of all-zero ciphertexts (crcnn_conv_forward_padded), and its output is
+    // (xd + 2 xp - xf) / xs + 1 by (yd + 2 yp - yf) / ys + 1.  Padding is geometry: the parameter stream format is unchanged.
+    ConvolutionalLayer(std::string name, int xd, int yd, int zd, int xs, int ys, int xf, int yf, int nf, int xp, int yp, int th_count,
+                       plaintext4D &filters, std::vector<Plaintext> &biases)
+        : Layer(name), xd(xd), yd(yd), zd(zd), xs(xs), ys(ys), xf(xf), yf(yf), nf(nf), th_count(th_count), xp(checked_pad(xp, xf)),
+          yp(checked_pad(yp, yf)), xo((xd + 2 * xp - xf) / xs + 1), yo((yd + 2 * yp - yf) / ys + 1), zo(nf), filters(filters), biases(biases),
+          filters_already_ntt(false) {}
+    ConvolutionalLayer(std::string name, int xd, int yd, int zd, int xs, int ys, int xf, int yf, int nf, int xp, int yp, int th_count,
+                       std::istream *infile)
+        : Layer(name), xd(xd), yd(yd), zd(zd), xs(xs), ys(ys), xf(xf), yf(yf), nf(nf), th_count(th_count), xp(checked_pad(xp, xf)),
+          yp(checked_pad(yp, yf)), xo((xd + 2 * xp - xf) / xs + 1), yo((yd + 2 * yp - yf) / ys + 1), zo(nf), filters_already_ntt(false) {
+        loadPlaintextParameters(infile);
+    }
+    ConvolutionalLayer(std::string name, int xd, int yd, int zd, int xs, int ys, int xf, int yf, int nf, int xp, int yp, int th_count,
+                       const std::vector<float> &weights, const std::vector<float> &bias_values)
+        : Layer(name), xd(xd), yd(yd), zd(zd), xs(xs), ys(ys), xf(xf), yf(yf), nf(nf), th_count(th_count), xp(checked_pad(xp, xf)),
+          yp(checked_pad(yp, yf)), xo((xd + 2 * xp - xf) / xs + 1), yo((yd + 2 * yp - yf) / ys + 1), zo(nf), filters_already_ntt(false) {
         if ((long)weights.size() != (long)nf * zd * xf * yf || (int)bias_values.size() != nf) throw std::invalid_argument("kernel shape does not match the layer");
         w_.encode(weights); b_.encode(bias_values);
     }
@@ -405,7 +419,7 @@ public:
         Runtime &rt = Runtime::get();
         ensure_packs();
         crcnn_tensor *o = nullptr;
-        rt.check(crcnn_conv_forward(rt.ctx(), in.t, w_.p, b_.p, in.batch, xd, yd, zd, xs, ys, xf, yf, nf, &o));
+        rt.check(crcnn_conv_forward_padded(rt.ctx(), in.t, w_.p, b_.p, in.batch, xd, yd, zd, xs, ys, xf, yf, nf, xp, yp, 0, nf, &o));
         return DeviceTensor(o, zo, xo, yo, in.batch);
     }
     // Output channels [k0, k0+kc) only: this GPU's share of the reference's filter split (convolutionalLayer.cpp:177-187)
@@ -413,7 +427,7 @@ public:
         Runtime &rt = Runtime::get();
         ensure_packs();
         crcnn_tensor *o = nullptr;
-        rt.check(crcnn_conv_forward_shard(rt.ctx(), in.t, w_.p, b_.p, in.batch, xd, yd, zd, xs, ys, xf, yf, nf, k0, kc, &o));
+        rt.check(crcnn_conv_forward_padded(rt.ctx(), in.t, w_.p, b_.p, in.batch, xd, yd, zd, xs, ys, xf, yf, nf, xp, yp, k0, kc, &o));
         return DeviceTensor(o, kc, xo, yo, in.batch);
     }
     crcnn_plain *weight_pack() { ensure_packs(); return w_.p; }
@@ -445,11 +459,15 @@ public:
         w_.clear(); b_.clear();
     }
     void printLayerStructure() override {
-        std::fprintf(stderr, "Convolutional %s : input (%d,%d,%d); kernel(%d,%d,%d,%d); stride(%d,%d); output(%d,%d,%d)\n",
-                     name.c_str(), zd, xd, yd, nf, zd, xf, yf, xs, ys, zo, xo, yo);
+        std::fprintf(stderr, "Convolutional %s : input (%d,%d,%d); kernel(%d,%d,%d,%d); stride(%d,%d); padding(%d,%d); output(%d,%d,%d)\n",
+                     name.c_str(), zd, xd, yd, nf, zd, xf, yf, xs, ys, xp, yp, zo, xo, yo);
     }
 
 private:
+    static int checked_pad(int pad, int filter) {
+        if (pad < 0 || pad >= filter) throw std::invalid_argument("convolution padding must be in [0, filter - 1]");
+        return pad;
+    }
     void ensure_packs() {
         if (w_.p) return;
         std::vector<const Plaintext *> ws, bs;
@@ -719,8 +737,9 @@ inline DeviceTensor BatchNormLayer::forward_after_conv_avgpool(DeviceTensor in, 
     if (conv.nf != num_channels || pool.xd != conv.xo || pool.yd != conv.yo)
         throw std::invalid_argument("convolution / pooling / batch-norm shapes do not chain");
     crcnn_tensor *o = nullptr;
-    rt.check(crcnn_conv_pool_bn_forward(rt.ctx(), in.t, conv.weight_pack(), conv.bias_pack(), in.batch, conv.xd, conv.yd, conv.zd, conv.xs, conv.ys,
-                                        conv.xf, conv.yf, conv.nf, pool.xs, pool.ys, pool.xf, pool.yf, pool.scale_or_null(), m_.p, v_.p, &o));
+    rt.check(crcnn_conv_pool_bn_forward_padded(rt.ctx(), in.t, conv.weight_pack(), conv.bias_pack(), in.batch, conv.xd, conv.yd, conv.zd, conv.xs,
+                                               conv.ys, conv.xf, conv.yf, conv.nf, pool.xs, pool.ys, pool.xf, pool.yf, pool.scale_or_null(), m_.p,
+                                               v_.p, conv.xp, conv.yp, 0, conv.nf, &o));
     return DeviceTensor(o, conv.nf, pool.xo, pool.yo, in.batch);
 }
 
@@ -742,9 +761,9 @@ inline bool BatchNormLayer::forward_after_conv_avgpool_shard(const DeviceTensor 
     if (conv.nf != num_channels || pool.xd != conv.xo || pool.yd != conv.yo)
         throw std::invalid_argument("convolution / pooling / batch-norm shapes do not chain");
     crcnn_tensor *o = nullptr;
-    const int rc = crcnn_conv_pool_bn_forward_shard(rt.ctx(), in.t, conv.weight_pack(), conv.bias_pack(), in.batch, conv.xd, conv.yd, conv.zd, conv.xs,
-                                                    conv.ys, conv.xf, conv.yf, conv.nf, pool.xs, pool.ys, pool.xf, pool.yf, pool.scale_or_null(), m_.p,
-                                                    v_.p, k0, kc, &o);
+    const int rc = crcnn_conv_pool_bn_forward_padded(rt.ctx(), in.t, conv.weight_pack(), conv.bias_pack(), in.batch, conv.xd, conv.yd, conv.zd, conv.xs,
+                                                     conv.ys, conv.xf, conv.yf, conv.nf, pool.xs, pool.ys, pool.xf, pool.yf, pool.scale_or_null(), m_.p,
+                                                     v_.p, conv.xp, conv.yp, k0, kc, &o);
     if (rc == CRCNN_ERR_UNSUPPORTED) return false;
     rt.check(rc);
     *out = DeviceTensor(o, kc, pool.xo, pool.yo, in.batch);
@@ -1033,9 +1052,9 @@ public:
                 IdentityBn &id = identity_bn(conv->nf);
                 Runtime &rt = Runtime::get();
                 crcnn_tensor *o = nullptr;
-                rt.check(crcnn_conv_pool_bn_forward(rt.ctx(), x.t, conv->weight_pack(), conv->bias_pack(), x.batch, conv->xd, conv->yd, conv->zd,
-                                                    conv->xs, conv->ys, conv->xf, conv->yf, conv->nf, pool->xs, pool->ys, pool->xf, pool->yf,
-                                                    pool->scale_or_null(), id.mean.p, id.invstd.p, &o));
+                rt.check(crcnn_conv_pool_bn_forward_padded(rt.ctx(), x.t, conv->weight_pack(), conv->bias_pack(), x.batch, conv->xd, conv->yd,
+                                                           conv->zd, conv->xs, conv->ys, conv->xf, conv->yf, conv->nf, pool->xs, pool->ys, pool->xf,
+                                                           pool->yf, pool->scale_or_null(), id.mean.p, id.invstd.p, conv->xp, conv->yp, 0, conv->nf, &o));
                 x = DeviceTensor(o, conv->nf, pool->xo, pool->yo, x.batch);
                 break;
             }

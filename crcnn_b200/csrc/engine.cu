@@ -1074,24 +1074,29 @@ int crcnn_evk_free(crcnn_ctx *ctx, crcnn_evk *k) {
 }
 
 // ---------------------------------------------------------------------------- layers
-int crcnn_conv_forward_shard(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_plain *b, int batch, int xd, int yd,
-                             int zd, int xs, int ys, int xf, int yf, int nf, int k0, int kc, crcnn_tensor **out) {
+// Zero padding (xp, yp): the convolution of the input with a border of xp columns and yp rows of all-zero ciphertexts on each side.
+// No bordered copy is made: the index table holds -1 where a window reaches into the border, and the gather kernels read -1 as the
+// zero ciphertext (its products add nothing), so the result is the canonical residues of the bordered input's convolution.
+int crcnn_conv_forward_padded(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_plain *b, int batch, int xd, int yd, int zd,
+                              int xs, int ys, int xf, int yf, int nf, int xp, int yp, int k0, int kc, crcnn_tensor **out) {
     if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
     REQUIRE(in && w && b && out, "null argument");
-    REQUIRE(batch > 0 && xd > 0 && yd > 0 && zd > 0 && xs > 0 && ys > 0 && xf > 0 && yf > 0 && nf > 0 && xf <= xd && yf <= yd,
+    REQUIRE(xp >= 0 && yp >= 0 && xp < xf && yp < yf, "padding must be in [0, filter - 1]");
+    const int xe = xd + 2 * xp, ye = yd + 2 * yp;       // the padded extent
+    REQUIRE(batch > 0 && xd > 0 && yd > 0 && zd > 0 && xs > 0 && ys > 0 && xf > 0 && yf > 0 && nf > 0 && xf <= xe && yf <= ye,
             "bad convolution geometry");
     REQUIRE(k0 >= 0 && kc >= 0 && k0 + kc <= nf, "bad output-channel shard");
     REQUIRE(in->size == 2 && in->count == (long)batch * zd * xd * yd, "input tensor does not match the layer geometry");
     const int R = zd * xf * yf;
     REQUIRE(w->count == (long)nf * R && b->count == nf, "kernel/bias count does not match the layer geometry");  // convolutionalLayer.cpp:57-59
     CU(cudaSetDevice(ctx->device));
-    const int xo = (xd - xf) / xs + 1, yo = (yd - yf) / ys + 1;  // convolutionalLayer.cpp:24
+    const int xo = (xe - xf) / xs + 1, yo = (ye - yf) / ys + 1;  // convolutionalLayer.cpp:24
     int xl, yl;
-    boundaries(xd, yd, xs, ys, xf, yf, &xl, &yl);
+    boundaries(xe, ye, xs, ys, xf, yf, &xl, &yl);
     if ((xl + xs - 1) / xs != xo || (yl + ys - 1) / ys != yo)
         return fail(ctx, CRCNN_ERR_UNSUPPORTED, "stride larger than the filter leaves outputs the reference never computes");
     const int P = xo * yo, Npos = batch * P, nin = zd * xd * yd;
-    std::vector<int> key = {1, batch, xd, yd, zd, xs, ys, xf, yf};
+    std::vector<int> key = {1, batch, xd, yd, zd, xs, ys, xf, yf, xp, yp};
     const int *d_index = nullptr;
     if (ctx->index_cache.find(key) == ctx->index_cache.end()) {
         std::vector<int> table((size_t)Npos * R);
@@ -1102,7 +1107,10 @@ int crcnn_conv_forward_shard(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, c
                     int r = 0;
                     for (int z = 0; z < zd; z++)
                         for (int kx = 0; kx < xf; kx++)
-                            for (int ky = 0; ky < yf; ky++) row[r++] = bi * nin + (z * xd + i * xs + kx) * yd + j * ys + ky;
+                            for (int ky = 0; ky < yf; ky++) {
+                                const int u = i * xs + kx - xp, v = j * ys + ky - yp;
+                                row[r++] = (u >= 0 && u < xd && v >= 0 && v < yd) ? bi * nin + (z * xd + u) * yd + v : -1;
+                            }
                 }
         int rc = get_index_table(ctx, key, table, &d_index);
         if (rc) return rc;
@@ -1118,9 +1126,14 @@ int crcnn_conv_forward_shard(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, c
     return CRCNN_OK;
 }
 
+int crcnn_conv_forward_shard(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_plain *b, int batch, int xd, int yd,
+                             int zd, int xs, int ys, int xf, int yf, int nf, int k0, int kc, crcnn_tensor **out) {
+    return crcnn_conv_forward_padded(ctx, in, w, b, batch, xd, yd, zd, xs, ys, xf, yf, nf, 0, 0, k0, kc, out);
+}
+
 int crcnn_conv_forward(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_plain *b, int batch, int xd, int yd, int zd,
                        int xs, int ys, int xf, int yf, int nf, crcnn_tensor **out) {
-    return crcnn_conv_forward_shard(ctx, in, w, b, batch, xd, yd, zd, xs, ys, xf, yf, nf, 0, nf, out);
+    return crcnn_conv_forward_padded(ctx, in, w, b, batch, xd, yd, zd, xs, ys, xf, yf, nf, 0, 0, 0, nf, out);
 }
 
 int crcnn_fc_forward_shard(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_plain *b, int batch, int in_dim,
@@ -1461,15 +1474,17 @@ int crcnn_pool_bn_forward(crcnn_ctx *ctx, crcnn_tensor *in, int batch, int xd, i
 //     W'[k,r] = W[k,r] (.) C_k,      B'_k = |window| * B_k (.) C_k - D_k        (NTT domain, computed once per network).
 // One weighted sum with (pooled positions / convolution positions) of the columns replaces three layers and two full-size
 // intermediates; the residues are the canonical ones of the same ring elements, hence the reference's bytes.
-int crcnn_conv_pool_bn_forward_shard(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_plain *b, int batch, int xd, int yd, int zd,
-                                     int xs, int ys, int xf, int yf, int nf, int pxs, int pys, int pxf, int pyf, crcnn_plain *scale,
-                                     crcnn_plain *mean, crcnn_plain *invstd, int k0, int kc, crcnn_tensor **out) {
+int crcnn_conv_pool_bn_forward_padded(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_plain *b, int batch, int xd, int yd, int zd,
+                                      int xs, int ys, int xf, int yf, int nf, int pxs, int pys, int pxf, int pyf, crcnn_plain *scale,
+                                      crcnn_plain *mean, crcnn_plain *invstd, int xp, int yp, int k0, int kc, crcnn_tensor **out) {
     if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
     REQUIRE(k0 >= 0 && kc >= 0 && k0 + kc <= nf, "bad output-channel shard");
     REQUIRE(in && w && b && mean && invstd && out, "null argument");      // scale == NULL: PoolingLayer (window sum without a factor)
-    REQUIRE(batch > 0 && xd > 0 && yd > 0 && zd > 0 && xs > 0 && ys > 0 && xf > 0 && yf > 0 && nf > 0 && xf <= xd && yf <= yd,
+    REQUIRE(xp >= 0 && yp >= 0 && xp < xf && yp < yf, "padding must be in [0, filter - 1]");
+    const int xe = xd + 2 * xp, ye = yd + 2 * yp;                           // the convolution's padded extent
+    REQUIRE(batch > 0 && xd > 0 && yd > 0 && zd > 0 && xs > 0 && ys > 0 && xf > 0 && yf > 0 && nf > 0 && xf <= xe && yf <= ye,
             "bad convolution geometry");
-    const int cxo = (xd - xf) / xs + 1, cyo = (yd - yf) / ys + 1;          // convolution output (convolutionalLayer.cpp:24)
+    const int cxo = (xe - xf) / xs + 1, cyo = (ye - yf) / ys + 1;          // convolution output (convolutionalLayer.cpp:24)
     REQUIRE(pxs > 0 && pys > 0 && pxf > 0 && pyf > 0 && pxf <= cxo && pyf <= cyo, "bad pooling geometry");
     const int pxo = (cxo - pxf) / pxs + 1, pyo = (cyo - pyf) / pys + 1;    // pooled output (poolingLayer.cpp:18)
     const int Rp = pxf * pyf, R = zd * xf * yf;
@@ -1486,7 +1501,7 @@ int crcnn_conv_pool_bn_forward_shard(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_pla
         if (k0 != 0 || kc != nf)    // a channel shard of the layer-by-layer path is the caller's: conv shard, then pool and batch-norm on its channels
             return fail(ctx, CRCNN_ERR_UNSUPPORTED, "channel shards of conv + pool + batch-norm need the pooled-grid path");
         crcnn_tensor *mid = nullptr;
-        int rc = crcnn_conv_forward(ctx, in, w, b, batch, xd, yd, zd, xs, ys, xf, yf, nf, &mid);
+        int rc = crcnn_conv_forward_padded(ctx, in, w, b, batch, xd, yd, zd, xs, ys, xf, yf, nf, xp, yp, 0, nf, &mid);
         if (rc) return rc;
         rc = crcnn_pool_bn_forward(ctx, mid, batch, cxo, cyo, nf, pxs, pys, pxf, pyf, scale, mean, invstd, out);
         crcnn_tensor_free(ctx, mid);
@@ -1517,10 +1532,12 @@ int crcnn_conv_pool_bn_forward_shard(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_pla
         CU(launch_fold_affine(ctx->dP, w->folded_b->ntt_add, (long)nf, (long)pw, 1, invstd->fused_C, invstd->fused_D, ctx->stream));
         memcpy(w->folded_key, key, sizeof(key));
     }
-    // S: dilated window sums of the input, (zd, sxd, syd) per image, in the input's domain
-    const int sxd = xd - (pxf - 1) * xs, syd = yd - (pyf - 1) * ys;
+    // S: dilated window sums of the input, (zd, sxd, syd) per image, in the input's domain.  With padding S spans the padded extent and
+    // its table holds -1 for border positions; the convolution over S then needs no padding, and its bias |window| * B stays as it is
+    // because the convolution output carries the bias at every position, border included.
+    const int sxd = xe - (pxf - 1) * xs, syd = ye - (pyf - 1) * ys;
     const int Nsum = batch * zd * sxd * syd;
-    std::vector<int> skey = {4, batch, xd, yd, zd, xs, ys, pxf, pyf};
+    std::vector<int> skey = {4, batch, xd, yd, zd, xs, ys, pxf, pyf, xp, yp};
     const int *d_index = nullptr;
     if (ctx->index_cache.find(skey) == ctx->index_cache.end()) {
         std::vector<int> table((size_t)Nsum * Rp);
@@ -1529,7 +1546,10 @@ int crcnn_conv_pool_bn_forward_shard(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_pla
             for (int u = 0; u < sxd; u++)
                 for (int v = 0; v < syd; v++)
                     for (int a = 0; a < pxf; a++)
-                        for (int c = 0; c < pyf; c++) table[o++] = (bz * xd + u + a * xs) * yd + v + c * ys;
+                        for (int c = 0; c < pyf; c++) {
+                            const int x = u + a * xs - xp, y = v + c * ys - yp;
+                            table[o++] = (x >= 0 && x < xd && y >= 0 && y < yd) ? (bz * xd + x) * yd + y : -1;
+                        }
         rc = get_index_table(ctx, skey, table, &d_index);
         if (rc) return rc;
     } else {
@@ -1554,10 +1574,18 @@ int crcnn_conv_pool_bn_forward_shard(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_pla
     return CRCNN_OK;
 }
 
+int crcnn_conv_pool_bn_forward_shard(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_plain *b, int batch, int xd, int yd, int zd,
+                                     int xs, int ys, int xf, int yf, int nf, int pxs, int pys, int pxf, int pyf, crcnn_plain *scale,
+                                     crcnn_plain *mean, crcnn_plain *invstd, int k0, int kc, crcnn_tensor **out) {
+    return crcnn_conv_pool_bn_forward_padded(ctx, in, w, b, batch, xd, yd, zd, xs, ys, xf, yf, nf, pxs, pys, pxf, pyf, scale, mean, invstd, 0, 0,
+                                             k0, kc, out);
+}
+
 int crcnn_conv_pool_bn_forward(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_plain *b, int batch, int xd, int yd, int zd,
                                int xs, int ys, int xf, int yf, int nf, int pxs, int pys, int pxf, int pyf, crcnn_plain *scale,
                                crcnn_plain *mean, crcnn_plain *invstd, crcnn_tensor **out) {
-    return crcnn_conv_pool_bn_forward_shard(ctx, in, w, b, batch, xd, yd, zd, xs, ys, xf, yf, nf, pxs, pys, pxf, pyf, scale, mean, invstd, 0, nf, out);
+    return crcnn_conv_pool_bn_forward_padded(ctx, in, w, b, batch, xd, yd, zd, xs, ys, xf, yf, nf, pxs, pys, pxf, pyf, scale, mean, invstd, 0, 0,
+                                             0, nf, out);
 }
 
 int crcnn_bn_forward(crcnn_ctx *ctx, crcnn_tensor *in, int batch, int zd, int xd, int yd, crcnn_plain *mean,

@@ -334,9 +334,11 @@ mac_kernel(const DeviceParams *__restrict__ P, MacArgs a) {
             for (int m = 0; m < TM; m++) { W[m] = __ldg(reinterpret_cast<const uint64_t *>(wptr[m])); wptr[m] += w_step; }
 #pragma unroll
             for (int t = 0; t < TN; t++) {
-                const unsigned long long off = (unsigned long long)(unsigned)s_idx[t * R + r] * ct_step;
-                X[t][0] = __ldg(reinterpret_cast<const uint64_t *>(x0 + off));
-                X[t][1] = __ldg(reinterpret_cast<const uint64_t *>(x1 + off));
+                // index -1: the all-zero ciphertext of a padded convolution's border, whose products are zero
+                const int ix = s_idx[t * R + r];
+                const unsigned long long off = (unsigned long long)(unsigned)max(ix, 0) * ct_step;
+                X[t][0] = ix >= 0 ? __ldg(reinterpret_cast<const uint64_t *>(x0 + off)) : 0;
+                X[t][1] = ix >= 0 ? __ldg(reinterpret_cast<const uint64_t *>(x1 + off)) : 0;
             }
 #pragma unroll
             for (int m = 0; m < TM; m++)
@@ -426,7 +428,9 @@ pool_kernel(const DeviceParams *__restrict__ P, const uint64_t *__restrict__ in,
 #pragma unroll
         for (int k = 0; k < EW_PER; k++) res[k] = make_ulonglong2(0, 0);
         for (int r = 0; r < R; r++) {
-            const uint64_t *src = in + (long)__ldg(in_index + o * R + r) * ctw + word0;
+            const int ix = __ldg(in_index + o * R + r);
+            if (ix < 0) continue;       // the all-zero ciphertext of a padded border: adds nothing
+            const uint64_t *src = in + (long)ix * ctw + word0;
 #pragma unroll
             for (int k = 0; k < EW_PER; k++)
                 if (k < per) {
@@ -441,7 +445,8 @@ pool_kernel(const DeviceParams *__restrict__ P, const uint64_t *__restrict__ in,
             if (k >= per) continue;
             U128 s0{0, 0}, s1{0, 0};
             for (int r = 0; r < R; r++) {
-                const ulonglong2 v = __ldg(reinterpret_cast<const ulonglong2 *>(in + (long)__ldg(in_index + o * R + r) * ctw + word0 + 512 * k));
+                const int ix = __ldg(in_index + o * R + r);
+                const ulonglong2 v = ix >= 0 ? __ldg(reinterpret_cast<const ulonglong2 *>(in + (long)ix * ctw + word0 + 512 * k)) : make_ulonglong2(0, 0);
                 add128_64(s0, v.x);
                 add128_64(s1, v.y);
             }

@@ -268,8 +268,8 @@ tc_split_kernel(const DeviceParams *__restrict__ P, TcMacArgs a) {
     for (int rr = warp; rr < 128; rr += 8) {
         const int r = r0 + rr;
         uint64_t v = 0;
-        if (r < a.R) {
-            const long ctx = __ldg(a.in_index + (long)p * a.R + r);
+        const long ctx = r < a.R ? __ldg(a.in_index + (long)p * a.R + r) : -1;
+        if (ctx >= 0) {             // index -1: a padded border's zero ciphertext, zero wrap coefficients included
             const uint64_t *src = a.x + ((ctx * 2 + poly) * K + j) * (long)n;
             if (!wrap) v = __ldg(src + ct * 32 + lane);
             else { v = __ldg(src + lane); v = v ? q - v : 0; }

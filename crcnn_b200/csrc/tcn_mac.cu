@@ -699,7 +699,7 @@ __global__ void tcn_preshift_kernel(const uint64_t *__restrict__ src, uint64_t *
 __global__ void __launch_bounds__(256)
 tcn_split_kernel(TcnSplitArgs a) {
     __shared__ uint64_t tile[32][133];    // [slot][(e & 3) * 33 + (e >> 2)], e = byte within the 128; row stride 133 = 5 mod 16: conflict free both ways
-    __shared__ long src_off[128];         // word offset of source row e (-1: padding)
+    __shared__ long src_off[128];         // word offset of source row e (-1: tile padding or a zero ciphertext)
     const int n = a.n, K = a.K;
     const int rows_per = a.Kpad < 128 ? 128 / a.Kpad : 1;   // columns per CTA
     const int col0 = blockIdx.x * rows_per;
@@ -716,7 +716,7 @@ tcn_split_kernel(TcnSplitArgs a) {
         if (r < a.R && col < a.ncols) {
             const int group = col / a.item_polys, poly = col - group * a.item_polys;
             const long item = a.index ? (long)__ldg(a.index + (long)group * a.R + r) : (long)group * a.R + r;
-            off = ((item * a.item_polys + poly) * K + j) * (long)n + c0;
+            if (item >= 0) off = ((item * a.item_polys + poly) * K + j) * (long)n + c0;   // index -1: a padded border's zero ciphertext
         }
         src_off[e] = off;
     }

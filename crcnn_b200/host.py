@@ -13,7 +13,8 @@ from .h5write import write_h5
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 HOST_LIB_PATH = os.path.join(_HERE, "libcrcnn_b200_host.so")
-TOPOLOGY_OF = {"PlainModel": "PlainModel", "ApproxPlainModel": "Approx", "PlainModelWoPad": "WoPad", "PlainModelTiny": "Tiny"}
+TOPOLOGY_OF = {"PlainModel": "PlainModel", "ApproxPlainModel": "Approx", "PlainModelWoPad": "WoPad", "PlainModelTiny": "Tiny",
+               "PlainModelPadded": "PlainModelPadded"}
 MODEL_OF = {v: k for k, v in TOPOLOGY_OF.items()}
 _vp, _I, _dp = C.c_void_p, C.c_int, C.POINTER(C.c_double)
 
@@ -105,7 +106,7 @@ class HostNetwork:
         self._chk(self.h.crcnn_host_shape(*[C.byref(x) for x in v]))
         self.zd, self.xd, self.yd, self.outputs, self.num_layers = [x.value for x in v]
         # the largest activation per image (input or any layer's output): what forward() on any layer range may hand back
-        topo = nets.TOPOLOGIES[MODEL_OF.get(model, model)]
+        topo = nets.topology(MODEL_OF.get(model, model))
         self.max_cts = max([self.zd * self.xd * self.yd] + [nets.layer_io_counts(layer)[1] for layer in topo["layers"]])
         name = C.create_string_buffer(128)
         self.layer_names = []

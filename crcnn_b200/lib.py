@@ -60,6 +60,7 @@ SYMBOLS = [
     ("crcnn_evk_free", _I, [_vp, _vp]),
     ("crcnn_conv_forward", _I, [_vp, _vp, _vp, _vp] + [_I] * 9 + [_vpp]),
     ("crcnn_conv_forward_shard", _I, [_vp, _vp, _vp, _vp] + [_I] * 11 + [_vpp]),
+    ("crcnn_conv_forward_padded", _I, [_vp, _vp, _vp, _vp] + [_I] * 13 + [_vpp]),
     ("crcnn_fc_forward", _I, [_vp, _vp, _vp, _vp, _I, _I, _I, _vpp]),
     ("crcnn_fc_forward_shard", _I, [_vp, _vp, _vp, _vp, _I, _I, _I, _I, _I, _vpp]),
     ("crcnn_pool_forward", _I, [_vp, _vp] + [_I] * 8 + [_vp, _vpp]),
@@ -69,6 +70,7 @@ SYMBOLS = [
     ("crcnn_fc_fc_forward", _I, [_vp, _vp, _vp, _vp, _vp, _vp, _I, _I, _I, _I, _vpp]),
     ("crcnn_conv_pool_bn_forward", _I, [_vp, _vp, _vp, _vp] + [_I] * 13 + [_vp, _vp, _vp, _vpp]),
     ("crcnn_conv_pool_bn_forward_shard", _I, [_vp, _vp, _vp, _vp] + [_I] * 13 + [_vp, _vp, _vp, _I, _I, _vpp]),
+    ("crcnn_conv_pool_bn_forward_padded", _I, [_vp, _vp, _vp, _vp] + [_I] * 13 + [_vp, _vp, _vp, _I, _I, _I, _I, _vpp]),
     ("crcnn_square_forward", _I, [_vp, _vp, _vp, _vpp]),
     ("crcnn_transform_to_ntt", _I, [_vp, _vp]),
     ("crcnn_transform_from_ntt", _I, [_vp, _vp]),
@@ -411,7 +413,12 @@ class Engine:
         return out
 
     # ---- layers
-    def conv(self, x, w, b, batch, xd, yd, zd, xs, ys, xf, yf, nf, shard=None):
+    def conv(self, x, w, b, batch, xd, yd, zd, xs, ys, xf, yf, nf, xp=0, yp=0, shard=None):
+        """Convolution (crcnn_conv_forward[_shard]); padding (xp, yp) of all-zero ciphertexts runs crcnn_conv_forward_padded."""
+        if xp or yp:
+            k0, kc = shard if shard is not None else (0, nf)
+            return self._new(self.lib.crcnn_conv_forward_padded, "tensor", x.ptr, w.ptr, b.ptr, batch, xd, yd, zd, xs, ys, xf, yf, nf,
+                             xp, yp, k0, kc)
         if shard is None:
             return self._new(self.lib.crcnn_conv_forward, "tensor", x.ptr, w.ptr, b.ptr, batch, xd, yd, zd, xs, ys, xf, yf, nf)
         return self._new(self.lib.crcnn_conv_forward_shard, "tensor", x.ptr, w.ptr, b.ptr, batch, xd, yd, zd, xs, ys,
@@ -430,8 +437,13 @@ class Engine:
     def bn(self, x, batch, zd, xd, yd, mean, invstd):
         return self._new(self.lib.crcnn_bn_forward, "tensor", x.ptr, batch, zd, xd, yd, mean.ptr, invstd.ptr)
 
-    def conv_pool_bn(self, x, w, b, batch, xd, yd, zd, xs, ys, xf, yf, nf, pxs, pys, pxf, pyf, scale, mean, invstd, shard=None):
-        """Convolution + average pooling + batch-norm on the pooled grid (crcnn_conv_pool_bn_forward[_shard])."""
+    def conv_pool_bn(self, x, w, b, batch, xd, yd, zd, xs, ys, xf, yf, nf, pxs, pys, pxf, pyf, scale, mean, invstd, shard=None, xp=0, yp=0):
+        """Convolution + average pooling + batch-norm on the pooled grid (crcnn_conv_pool_bn_forward[_shard]; with a padded convolution
+        crcnn_conv_pool_bn_forward_padded)."""
+        if xp or yp:
+            k0, kc = shard if shard is not None else (0, nf)
+            return self._new(self.lib.crcnn_conv_pool_bn_forward_padded, "tensor", x.ptr, w.ptr, b.ptr, batch, xd, yd, zd, xs, ys, xf, yf, nf,
+                             pxs, pys, pxf, pyf, scale.ptr if scale is not None else None, mean.ptr, invstd.ptr, xp, yp, k0, kc)
         if shard is not None:
             return self._new(self.lib.crcnn_conv_pool_bn_forward_shard, "tensor", x.ptr, w.ptr, b.ptr, batch, xd, yd, zd, xs, ys, xf, yf, nf,
                              pxs, pys, pxf, pyf, scale.ptr if scale is not None else None, mean.ptr, invstd.ptr, shard[0], shard[1])

@@ -3,6 +3,8 @@
 Topologies mirror CnnBuilder::buildNetwork (CrCNN/src/cnnBuilder.cpp:108-179: Approx, WoPad and
 Tiny blocks); `PlainModel` is the weights file PlainModel.h5 run through the unchanged layer API on
 a 32x32 zero-bordered input (SURVEY.md section 8(a), table of topologies, and Appendix B3).
+PADDED_TOPOLOGIES holds the networks whose convolutions have zero padding: `PlainModelPadded` is
+PlainModel.h5 as it was trained, conv1 with padding 2 on the 28x28 image.
 
 Network.forward mirrors Network::forward (CrCNN/src/network.cpp:22-47) without the hard-coded
 re-encryption before layer 6: re-encryption needs the SECRET key and therefore belongs to the
@@ -70,16 +72,38 @@ TOPOLOGIES = {
         ("fc", "classifier.fc4", 500, 10)]),
 }
 
+# Networks with zero-padded convolutions: conv tuples carry two more fields, the padding (xp, yp) (ConvolutionalLayer's padded
+# constructors).  Kept apart from TOPOLOGIES, whose conv tuples have the reference's ten fields.  "weights": the .npz they read.
+PADDED_TOPOLOGIES = {
+    # PlainModel.h5 as trained: conv1 5x5 / 2 with padding 2 on 28x28, then the same eight layers as "PlainModel"
+    "PlainModelPadded": dict(input=(1, 28, 28), weights="PlainModel", layers=[
+        ("conv", "pool1_features.conv1", 28, 28, 1, 2, 2, 5, 5, 20, 2, 2)] + TOPOLOGIES["PlainModel"]["layers"][1:]),
+}
+
+
+def topology(model):
+    """The topology dict of `model`, from TOPOLOGIES or PADDED_TOPOLOGIES."""
+    return TOPOLOGIES[model] if model in TOPOLOGIES else PADDED_TOPOLOGIES[model]
+
 
 def load_weights(model):
-    return dict(np.load(os.path.join(WEIGHTS_DIR, model + ".npz")))
+    name = PADDED_TOPOLOGIES[model]["weights"] if model in PADDED_TOPOLOGIES else model
+    return dict(np.load(os.path.join(WEIGHTS_DIR, name + ".npz")))
+
+
+def conv_out(layer):
+    """(xo, yo) of a conv tuple, with its padding (0 for the reference's ten-field tuples)."""
+    _, _, xd, yd, zd, xs, ys, xf, yf, nf = layer[:10]
+    xp, yp = layer[10:12] if len(layer) > 10 else (0, 0)
+    return (xd + 2 * xp - xf) // xs + 1, (yd + 2 * yp - yf) // ys + 1
 
 
 def layer_terms(layer):
     """Weighted-sum terms (ciphertext x plaintext products) per image of one layer."""
     if layer[0] == "conv":
-        _, _, xd, yd, zd, xs, ys, xf, yf, nf = layer
-        return nf * ((xd - xf) // xs + 1) * ((yd - yf) // ys + 1) * zd * xf * yf
+        _, _, xd, yd, zd, xs, ys, xf, yf, nf = layer[:10]
+        xo, yo = conv_out(layer)
+        return nf * xo * yo * zd * xf * yf
     if layer[0] == "fc":
         return layer[2] * layer[3]
     return 0
@@ -89,8 +113,9 @@ def layer_io_counts(layer):
     """(input ciphertexts, output ciphertexts) per image."""
     k = layer[0]
     if k == "conv":
-        _, _, xd, yd, zd, xs, ys, xf, yf, nf = layer
-        return zd * xd * yd, nf * ((xd - xf) // xs + 1) * ((yd - yf) // ys + 1)
+        _, _, xd, yd, zd, xs, ys, xf, yf, nf = layer[:10]
+        xo, yo = conv_out(layer)
+        return zd * xd * yd, nf * xo * yo
     if k in ("pool", "avgpool"):
         _, _, xd, yd, zd, xs, ys, xf, yf = layer
         return zd * xd * yd, zd * ((xd - xf) // xs + 1) * ((yd - yf) // ys + 1)
@@ -109,7 +134,7 @@ class Network:
         """limit: optional dict {layer_name: max_outputs} to build a cropped network (used only by the
         bounded CPU-baseline sample; the GPU path always runs the full layers)."""
         self.eng, self.model = eng, model
-        topo = TOPOLOGIES[model]
+        topo = topology(model)
         self.input_shape = topo["input"]
         self.layers = list(topo["layers"])
         w = weights if weights is not None else load_weights(model)

@@ -179,6 +179,15 @@ int crcnn_conv_forward(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *weights, c
 int crcnn_conv_forward_shard(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *weights, crcnn_plain *biases, int batch,
                              int xd, int yd, int zd, int xs, int ys, int xf, int yf, int nf, int k0, int kc,
                              crcnn_tensor **out);
+/* As above with zero padding: the convolution of the input with a border of xp columns and yp rows of all-zero ciphertexts on
+ * each side (PyTorch Conv2d(padding=(xp, yp)) over a plaintext-zero border; PlainModel.h5's conv1 was trained with padding 2).
+ * Output (xd + 2xp - xf)/xs + 1 by (yd + 2yp - yf)/ys + 1; computeBoundaries applies to the padded extent.  The bytes are those of
+ * crcnn_conv_forward on the bordered input, without a bordered copy ever being made.  0 <= xp <= xf - 1 and 0 <= yp <= yf - 1 (every
+ * window holds a real input), otherwise CRCNN_ERR_INVALID_ARGUMENT.  Output channels [k0, k0+kc); k0 = 0, kc = nf is the whole
+ * layer.  crcnn_conv_forward[_shard] are this call with xp = yp = 0. */
+int crcnn_conv_forward_padded(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *weights, crcnn_plain *biases, int batch,
+                              int xd, int yd, int zd, int xs, int ys, int xf, int yf, int nf, int xp, int yp,
+                              int k0, int kc, crcnn_tensor **out);
 /* Replaces FullyConnectedLayer::forward (CrCNN/src/fullyConnectedLayer.cpp:113-168); the input is
  * the row-major flattening reshapeInput produces (:38-56).  weights [out_dim][in_dim]. */
 int crcnn_fc_forward(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *weights, crcnn_plain *biases, int batch,
@@ -220,6 +229,13 @@ int crcnn_conv_pool_bn_forward(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w,
 int crcnn_conv_pool_bn_forward_shard(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_plain *b, int batch, int xd, int yd, int zd,
                                      int xs, int ys, int xf, int yf, int nf, int pxs, int pys, int pxf, int pyf, crcnn_plain *scale,
                                      crcnn_plain *mean, crcnn_plain *invstd, int k0, int kc, crcnn_tensor **out);
+/* crcnn_conv_pool_bn_forward_shard with a zero-padded convolution (padding (xp, yp) as in crcnn_conv_forward_padded): the same bytes
+ * as crcnn_conv_forward_padded, then the pooling and batch-norm.  On the pooled grid the window sums span the padded extent and read
+ * border positions as the zero ciphertext; the fallback is crcnn_conv_forward_padded + crcnn_pool_bn_forward.  The other two entries
+ * are this call with xp = yp = 0. */
+int crcnn_conv_pool_bn_forward_padded(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_plain *b, int batch, int xd, int yd, int zd,
+                                      int xs, int ys, int xf, int yf, int nf, int pxs, int pys, int pxf, int pyf, crcnn_plain *scale,
+                                      crcnn_plain *mean, crcnn_plain *invstd, int xp, int yp, int k0, int kc, crcnn_tensor **out);
 /* Two FullyConnectedLayer::forward calls in a row with no layer between them (fc3 -> fc4, the tail of every reference topology:
  * CrCNN/src/cnnBuilder.cpp:121-122, 132-133, 153-154; fullyConnectedLayer.cpp:96-166), producing the second layer's output
  * ciphertexts -- the same bytes as the two calls.  fc2(fc1(x)) = (W2 W1) x + (W2 Delta b1 + Delta b2) over Z_q[x]/(x^n+1): the composed
