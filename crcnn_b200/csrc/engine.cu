@@ -7,6 +7,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <numeric>
 #include <unordered_map>
 #include <string>
@@ -158,6 +159,9 @@ int fail(crcnn_ctx *ctx, int code, const std::string &msg) {
 #define REQUIRE(cond, msg) \
     do { if (!(cond)) return fail(ctx, CRCNN_ERR_INVALID_ARGUMENT, msg); } while (0)
 
+#define TRY(call) \
+    do { int rc__ = (call); if (rc__) return rc__; } while (0)
+
 struct ProfScope {
     crcnn_ctx *c; int cls; cudaEvent_t a = nullptr, b = nullptr;
     ProfScope(crcnn_ctx *ctx, int k, double bytes = 0, double ops = 0) : c(ctx), cls(k) {
@@ -174,6 +178,13 @@ struct ProfScope {
         cudaEventRecord(b, c->stream);
         c->pending.push_back({cls, a, b});
     }
+};
+
+// Build-time work is not part of any step's profile: no timing events while the guard lives, prof_on as it was on every exit.
+struct ProfPause {
+    crcnn_ctx *c; bool was;
+    explicit ProfPause(crcnn_ctx *ctx) : c(ctx), was(ctx->prof_on) { c->prof_on = false; }
+    ~ProfPause() { c->prof_on = was; }
 };
 
 void prof_collect(crcnn_ctx *c) {
@@ -241,6 +252,33 @@ void dev_free(crcnn_ctx *ctx, void *p) {
     cudaFreeAsync(p, ctx->stream);
 }
 
+// What a call takes from the context -- a device block, a tensor, a pack, a key object -- held for the length of a scope: whichever
+// return leaves it gives the object back through Free (on the context's stream, after everything enqueued so far), unless release()
+// has handed it to the caller.
+template <class T, int (*Free)(crcnn_ctx *, T *)>
+class Owned {
+  public:
+    explicit Owned(crcnn_ctx *ctx, T *p = nullptr) : ctx_(ctx), p_(p) {}
+    Owned(const Owned &) = delete;
+    Owned &operator=(const Owned &) = delete;
+    ~Owned() { reset(); }
+    operator T *() const { return p_; }
+    T *operator->() const { return p_; }
+    T **out() { reset(); return &p_; }
+    T *release() { T *p = p_; p_ = nullptr; return p; }
+    void reset() { if (p_) Free(ctx_, p_); p_ = nullptr; }
+
+  private:
+    crcnn_ctx *ctx_;
+    T *p_;
+};
+template <class T> int dev_release(crcnn_ctx *ctx, T *p) { dev_free(ctx, p); return CRCNN_OK; }
+template <class T> using DevBuf = Owned<T, dev_release<T>>;
+using TensorOwner = Owned<crcnn_tensor, crcnn_tensor_free>;
+using PlainOwner = Owned<crcnn_plain, crcnn_plain_free>;
+
+template <class T> int dev_alloc(crcnn_ctx *ctx, size_t bytes, DevBuf<T> &buf) { return dev_alloc(ctx, bytes, (void **)buf.out()); }
+
 int new_tensor(crcnn_ctx *ctx, long count, int size, int ntt, crcnn_tensor **out) {
     auto *t = new crcnn_tensor{count, size, ntt, nullptr};
     int rc = dev_alloc(ctx, (size_t)count * size * poly_words(ctx) * 8, (void **)&t->d);
@@ -277,45 +315,46 @@ int ensure_form(crcnn_ctx *ctx, crcnn_plain *p, PlainForm f) {
     uint64_t **slot = f == PF_NTT_MUL ? &p->ntt_mul : (f == PF_NTT_ADD ? &p->ntt_add : &p->coef_add);
     if (*slot) return CRCNN_OK;
     if (p->dense_only) return fail(ctx, CRCNN_ERR_UNSUPPORTED, "this derived plaintext pack has no such form");
-    int rc = dev_alloc(ctx, (size_t)p->count * poly_words(ctx) * 8, (void **)slot);
-    if (rc) return rc;
-    rc = expand_range(ctx, p, 0, p->count, f, *slot);
-    if (!rc && f != PF_NTT_MUL && p->add_mult != 1)
-        CU(launch_scale_small(ctx->dP, *slot, (long)((size_t)p->count * poly_words(ctx)), p->add_mult, ctx->stream));
-    return rc;
+    DevBuf<uint64_t> d(ctx);
+    TRY(dev_alloc(ctx, (size_t)p->count * poly_words(ctx) * 8, d));
+    TRY(expand_range(ctx, p, 0, p->count, f, d));
+    if (f != PF_NTT_MUL && p->add_mult != 1)
+        CU(launch_scale_small(ctx->dP, d, (long)((size_t)p->count * poly_words(ctx)), p->add_mult, ctx->stream));
+    *slot = d.release();
+    return CRCNN_OK;
 }
 
 int make_plain(crcnn_ctx *ctx, std::vector<uint32_t> &&off, std::vector<uint32_t> &&idx, std::vector<uint64_t> &&val,
                crcnn_plain **out) {
-    auto *p = new crcnn_plain();
+    PlainOwner p(ctx, new crcnn_plain());
     p->count = (long)off.size() - 1;
     p->off = std::move(off); p->idx = std::move(idx); p->val = std::move(val);
     p->sparse_shape = true;
     for (uint32_t ix : p->idx)
         if (ix >= 64 && ix < (uint32_t)(ctx->n - 32)) { p->sparse_shape = false; break; }
-    int rc = dev_alloc(ctx, p->off.size() * 4, (void **)&p->d_off);
-    if (!rc) rc = dev_alloc(ctx, std::max<size_t>(p->idx.size(), 1) * 4, (void **)&p->d_idx);
-    if (!rc) rc = dev_alloc(ctx, std::max<size_t>(p->val.size(), 1) * 8, (void **)&p->d_val);
-    if (rc) { delete p; return rc; }
+    TRY(dev_alloc(ctx, p->off.size() * 4, (void **)&p->d_off));
+    TRY(dev_alloc(ctx, std::max<size_t>(p->idx.size(), 1) * 4, (void **)&p->d_idx));
+    TRY(dev_alloc(ctx, std::max<size_t>(p->val.size(), 1) * 8, (void **)&p->d_val));
     CU(cudaMemcpyAsync(p->d_off, p->off.data(), p->off.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
     if (!p->idx.empty()) {
         CU(cudaMemcpyAsync(p->d_idx, p->idx.data(), p->idx.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
         CU(cudaMemcpyAsync(p->d_val, p->val.data(), p->val.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
     }
     CU(cudaStreamSynchronize(ctx->stream));  // host vectors are pageable; make the staging explicit
-    *out = p;
+    *out = p.release();
     return CRCNN_OK;
 }
 
 // Shoup companions of the multiplicative NTT form (element-wise layers multiply by a per-channel constant:
 // one mulhi + two mullo instead of a 128-bit Barrett reduction per residue).
 int ensure_shoup(crcnn_ctx *ctx, crcnn_plain *p) {
-    int rc = ensure_form(ctx, p, PF_NTT_MUL);
-    if (rc || p->ntt_mul_sh) return rc;
+    TRY(ensure_form(ctx, p, PF_NTT_MUL));
+    if (p->ntt_mul_sh) return CRCNN_OK;
     const size_t words = (size_t)p->count * poly_words(ctx);
-    rc = dev_alloc(ctx, words * 8, (void **)&p->ntt_mul_sh);
-    if (rc) return rc;
-    CU(launch_shoup_companion(ctx->dP, p->ntt_mul, (long)words, p->ntt_mul_sh, ctx->stream));
+    DevBuf<uint64_t> sh(ctx);
+    TRY(dev_alloc(ctx, words * 8, sh));
+    CU(launch_shoup_companion(ctx->dP, p->ntt_mul, (long)words, sh, ctx->stream));
+    p->ntt_mul_sh = sh.release();
     return CRCNN_OK;
 }
 
@@ -323,36 +362,68 @@ int ensure_shoup(crcnn_ctx *ctx, crcnn_plain *p) {
 // C[z] = scale (.) invstd[z] (with Shoup companions), D[z] = mean[z] (.) invstd[z];  x -> x (.) C[z] - D[z] (D on polynomial 0 only).
 int ensure_pool_bn_consts(crcnn_ctx *ctx, crcnn_plain *scale, crcnn_plain *mean, crcnn_plain *invstd) {
     // scale == nullptr: sum pooling (PoolingLayer, the WoPad topology) -- C[z] = invstd[z]
-    int rc = scale ? ensure_form(ctx, scale, PF_NTT_MUL) : CRCNN_OK;
-    if (!rc) rc = ensure_form(ctx, mean, PF_NTT_ADD);
-    if (!rc) rc = ensure_form(ctx, invstd, PF_NTT_MUL);
-    if (rc) return rc;
+    if (scale) TRY(ensure_form(ctx, scale, PF_NTT_MUL));
+    TRY(ensure_form(ctx, mean, PF_NTT_ADD));
+    TRY(ensure_form(ctx, invstd, PF_NTT_MUL));
     const long scale_id = scale ? scale->serial : -1;
     if (invstd->fused_C && invstd->fused_scale == scale_id && invstd->fused_mean == mean->serial) return CRCNN_OK;
     const size_t words = (size_t)invstd->count * poly_words(ctx);
+    DevBuf<uint64_t> C(ctx), Csh(ctx), D(ctx);
+    TRY(dev_alloc(ctx, words * 8, C));
+    TRY(dev_alloc(ctx, words * 8, Csh));
+    TRY(dev_alloc(ctx, words * 8, D));
+    CU(launch_pool_bn_consts(ctx->dP, scale ? scale->ntt_mul : nullptr, invstd->ntt_mul, mean->ntt_add, (long)words, C, D, ctx->stream));
+    CU(launch_shoup_companion(ctx->dP, C, (long)words, Csh, ctx->stream));
     dev_free(ctx, invstd->fused_C); dev_free(ctx, invstd->fused_Csh); dev_free(ctx, invstd->fused_D);
-    invstd->fused_C = invstd->fused_Csh = invstd->fused_D = nullptr;
-    rc = dev_alloc(ctx, words * 8, (void **)&invstd->fused_C);
-    if (!rc) rc = dev_alloc(ctx, words * 8, (void **)&invstd->fused_Csh);
-    if (!rc) rc = dev_alloc(ctx, words * 8, (void **)&invstd->fused_D);
-    if (rc) return rc;
-    CU(launch_pool_bn_consts(ctx->dP, scale ? scale->ntt_mul : nullptr, invstd->ntt_mul, mean->ntt_add, (long)words, invstd->fused_C, invstd->fused_D, ctx->stream));
-    CU(launch_shoup_companion(ctx->dP, invstd->fused_C, (long)words, invstd->fused_Csh, ctx->stream));
+    invstd->fused_C = C.release(); invstd->fused_Csh = Csh.release(); invstd->fused_D = D.release();
     invstd->fused_scale = scale_id; invstd->fused_mean = mean->serial;
     return CRCNN_OK;
 }
 
-// Device copy of an index table, cached by content key.
-int get_index_table(crcnn_ctx *ctx, const std::vector<int> &key, const std::vector<int> &table, const int **out) {
+// A composed layer's constants folded from weight pack w, kept in w->folded_w / folded_b for the packs and shape in `key`:
+// build(&folded_w, &folded_b) makes them when the key differs; a failed build leaves the pack as it was.
+template <class Build>
+int ensure_folded(crcnn_ctx *ctx, crcnn_plain *w, const long (&key)[9], Build build) {
+    if (w->folded_w && memcmp(key, w->folded_key, sizeof(key)) == 0) return CRCNN_OK;
+    PlainOwner fw(ctx), fb(ctx);
+    TRY(build(fw.out(), fb.out()));
+    crcnn_plain_free(ctx, w->folded_w);
+    crcnn_plain_free(ctx, w->folded_b);
+    w->folded_w = fw.release(); w->folded_b = fb.release();
+    memcpy(w->folded_key, key, sizeof(key));
+    return CRCNN_OK;
+}
+
+// Index tables of the gather kernels; the kind is the first word of every key, so tables of different kinds never share one.
+enum TableKind { TAB_CONV = 1, TAB_FC, TAB_POOL, TAB_WINDOW_SUM, TAB_COMPOSE, TAB_ADD_MANY };
+
+struct CudaFree { void operator()(int *p) const { cudaFree(p); } };
+
+// The device copy of the table of `kind` under `dims`: built by fill() (-> std::vector<int>) on the first request, kept until the
+// context is destroyed.
+template <class Fill>
+int index_table(crcnn_ctx *ctx, TableKind kind, std::initializer_list<int> dims, Fill fill, const int **out) {
+    std::vector<int> key{(int)kind};
+    key.insert(key.end(), dims);
     auto it = ctx->index_cache.find(key);
     if (it != ctx->index_cache.end()) { *out = it->second; return CRCNN_OK; }
-    int *d = nullptr;
-    CU(cudaMalloc((void **)&d, std::max<size_t>(table.size(), 1) * sizeof(int)));
-    CU(cudaMemcpyAsync(d, table.data(), table.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+    const std::vector<int> table = fill();
+    int *raw = nullptr;
+    CU(cudaMalloc((void **)&raw, std::max<size_t>(table.size(), 1) * sizeof(int)));
+    std::unique_ptr<int, CudaFree> d(raw);
+    CU(cudaMemcpyAsync(d.get(), table.data(), table.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
-    ctx->index_cache[key] = d;
-    *out = d;
+    *out = ctx->index_cache[key] = d.release();
     return CRCNN_OK;
+}
+
+// A fully connected layer's gather: image b reads the in_dim ciphertexts from b * in_dim on.
+int fc_index_table(crcnn_ctx *ctx, int batch, int in_dim, const int **out) {
+    return index_table(ctx, TAB_FC, {batch, in_dim}, [&] {
+        std::vector<int> table((size_t)batch * in_dim);
+        std::iota(table.begin(), table.end(), 0);
+        return table;
+    }, out);
 }
 
 // The coefficient-domain multiply (tapmul_kernel) applies to this pack: FractionalEncoder digits only, primes below 2^56.
@@ -383,6 +454,32 @@ void boundaries(int xd, int yd, int xs, int ys, int xf, int yf, int *xl, int *yl
     *yl = (yf > ys) ? yd - yf + 1 : yd - ys + 1;
 }
 
+// Windows of xf x yf at strides (xs, ys) over the batch * zd images of xd x yd in `in` (poolingLayer.cpp:18): the output extent and
+// the device table of every output's R = xf * yf inputs.
+struct PoolWindows { int xo, yo, R, Nout; const int *d_index; };
+
+int pool_windows(crcnn_ctx *ctx, const crcnn_tensor *in, int batch, int xd, int yd, int zd, int xs, int ys, int xf, int yf, PoolWindows *g) {
+    REQUIRE(batch > 0 && xd > 0 && yd > 0 && zd > 0 && xs > 0 && ys > 0 && xf > 0 && yf > 0 && xf <= xd && yf <= yd, "bad pooling geometry");
+    REQUIRE(in->size == 2 && in->count == (long)batch * zd * xd * yd, "input tensor does not match the layer geometry");
+    CU(cudaSetDevice(ctx->device));
+    const int xo = (xd - xf) / xs + 1, yo = (yd - yf) / ys + 1;
+    int xl, yl;
+    boundaries(xd, yd, xs, ys, xf, yf, &xl, &yl);
+    if ((xl + xs - 1) / xs != xo || (yl + ys - 1) / ys != yo)
+        return fail(ctx, CRCNN_ERR_UNSUPPORTED, "stride larger than the window leaves outputs the reference never computes");
+    *g = {xo, yo, xf * yf, batch * zd * xo * yo, nullptr};
+    return index_table(ctx, TAB_POOL, {batch, xd, yd, zd, xs, ys, xf, yf}, [&] {
+        std::vector<int> table((size_t)g->Nout * g->R);
+        size_t o = 0;
+        for (int bz = 0; bz < batch * zd; bz++)
+            for (int i = 0; i < xo; i++)
+                for (int j = 0; j < yo; j++)
+                    for (int kx = 0; kx < xf; kx++)
+                        for (int ky = 0; ky < yf; ky++) table[o++] = (bz * xd + i * xs + kx) * yd + j * ys + ky;
+        return table;
+    }, &g->d_index);
+}
+
 // Weighted-sum driver shared by conv and fc: M output channels [m_first, m_first+M) of Mall.
 // Ternary tap matrix of a weight pack for fan-in R (tc_mac.cuh): built once, on the host, from the sparse form.
 int ensure_tc_form(crcnn_ctx *ctx, crcnn_plain *w, int R) {
@@ -407,11 +504,12 @@ int ensure_tc_form(crcnn_ctx *ctx, crcnn_plain *w, int R) {
             A[((size_t)m * TC_TAPS + tap - 1) * Kpad + r] = w->val[e] == 1 ? (int8_t)-1 : (int8_t)1;
         }
     }
-    if (w->tc_A) { dev_free(ctx, w->tc_A); w->tc_A = nullptr; }
-    int rc = dev_alloc(ctx, A.size(), (void **)&w->tc_A);
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(w->tc_A, A.data(), A.size(), cudaMemcpyHostToDevice, ctx->stream));
+    DevBuf<int8_t> dA(ctx);
+    TRY(dev_alloc(ctx, A.size(), dA));
+    CU(cudaMemcpyAsync(dA, A.data(), A.size(), cudaMemcpyHostToDevice, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
+    dev_free(ctx, w->tc_A);
+    w->tc_A = dA.release();
     w->tc_state = 1; w->tc_R = R; w->tc_Kpad = Kpad;
     return CRCNN_OK;
 }
@@ -419,9 +517,8 @@ int ensure_tc_form(crcnn_ctx *ctx, crcnn_plain *w, int R) {
 // Weighted sum on the tensor cores: coefficient-domain inputs and outputs, no transform anywhere.
 int run_weighted_sum_tc(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_plain *b, const int *d_index, int R,
                         int Npos, int Pimg, int m_first, int M, crcnn_tensor *out) {
-    int rc = ensure_domain(ctx, in, 0);
-    if (!rc) rc = ensure_form(ctx, b, PF_COEF_ADD);
-    if (rc) return rc;
+    TRY(ensure_domain(ctx, in, 0));
+    TRY(ensure_form(ctx, b, PF_COEF_ADD));
     const size_t pw = poly_words(ctx);
     TcMacArgs a{};
     a.A = w->tc_A + (size_t)m_first * TC_TAPS * w->tc_Kpad;
@@ -433,11 +530,10 @@ int run_weighted_sum_tc(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_
     const size_t per_pos = tc_b_bytes(a);
     long chunk = (long)std::max<size_t>(1, ctx->tc_scratch_bytes / per_pos);
     chunk = std::min<long>(std::min<long>(chunk, Npos), 65535 / (2 * ctx->K));
-    uint8_t *scratch = nullptr;
-    rc = dev_alloc(ctx, (size_t)chunk * per_pos, (void **)&scratch);
-    if (rc) return rc;
+    DevBuf<uint8_t> scratch(ctx);
+    TRY(dev_alloc(ctx, (size_t)chunk * per_pos, scratch));
     a.B = scratch;
-    for (long p0 = 0; p0 < Npos && !rc; p0 += chunk) {
+    for (long p0 = 0; p0 < Npos; p0 += chunk) {
         a.npos = (int)std::min<long>(chunk, Npos - p0);
         a.p0 = (int)p0;
         a.in_index = d_index + p0 * R;
@@ -451,11 +547,10 @@ int run_weighted_sum_tc(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_
                          (double)a.npos * 2 * ctx->K * ctx->n * a.planes * (double)M * TC_TAPS * R);
             e = launch_tc_mac(ctx->dP, a, ctx->sm_count, ctx->stream);
         }
-        if (e != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, std::string("tensor-core weighted sum: ") + cudaGetErrorString(e));
+        if (e != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, std::string("tensor-core weighted sum: ") + cudaGetErrorString(e));
     }
-    dev_free(ctx, scratch);
-    if (!rc) out->ntt = 0;
-    return rc;
+    out->ntt = 0;
+    return CRCNN_OK;
 }
 
 // Byte planes of the whole pack's NTT-form weights, staged once (tcn_mac.cuh); the dense NTT form is released afterwards.
@@ -463,20 +558,15 @@ int run_weighted_sum_tc(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_
 // pre-shifted one serves the 13-class kernels through its first block.
 int ensure_tcn_weights(crcnn_ctx *ctx, crcnn_plain *w, int R, bool preshift) {
     if (w->tcn_W && w->tcn_R == R) return CRCNN_OK;
-    int rc = ensure_form(ctx, w, PF_NTT_MUL);
-    if (rc) return rc;
-    if (w->tcn_W) { dev_free(ctx, w->tcn_W); w->tcn_W = nullptr; }
+    TRY(ensure_form(ctx, w, PF_NTT_MUL));
     const int Mall = (int)(w->count / R), Kpad = tcn_kpad(R);
     const size_t block = tcn_w_bytes(7, Mall, Kpad, ctx->K, ctx->n);
     const int blocks = preshift ? 7 : 1;
-    rc = dev_alloc(ctx, block * blocks, (void **)&w->tcn_W);
-    if (rc) return rc;
+    DevBuf<uint8_t> planes(ctx);
+    TRY(dev_alloc(ctx, block * blocks, planes));
     const long words = (long)w->count * (long)poly_words(ctx);
-    uint64_t *shifted = nullptr;
-    if (preshift) {
-        rc = dev_alloc(ctx, (size_t)words * 8, (void **)&shifted);
-        if (rc) { dev_free(ctx, w->tcn_W); w->tcn_W = nullptr; return rc; }
-    }
+    DevBuf<uint64_t> shifted(ctx);
+    if (preshift) TRY(dev_alloc(ctx, (size_t)words * 8, shifted));
     uint64_t q[MAXK];
     for (int j = 0; j < ctx->K; j++) q[j] = ctx->hp.d.tab[j].mod.q;
     TcnSplitArgs s{};
@@ -485,11 +575,12 @@ int ensure_tcn_weights(crcnn_ctx *ctx, crcnn_plain *w, int R, bool preshift) {
     for (int b = 0; b < blocks; b++) {
         if (b) CU(launch_tcn_preshift(q, w->ntt_mul, shifted, words, b, ctx->n, ctx->K, ctx->stream));
         s.src = b ? shifted : w->ntt_mul;
-        s.dst = w->tcn_W + block * b;
+        s.dst = planes + block * b;
         ProfScope ps(ctx, KC_TCN_SPLIT, lp_bytes(ctx, (double)w->count * ctx->K) + (double)block, 0);
         CU(launch_tcn_split(s, ctx->stream));
     }
-    if (shifted) dev_free(ctx, shifted);
+    dev_free(ctx, w->tcn_W);
+    w->tcn_W = planes.release();
     dev_free(ctx, w->ntt_mul); w->ntt_mul = nullptr;
     if (w->ntt_mul_sh) { dev_free(ctx, w->ntt_mul_sh); w->ntt_mul_sh = nullptr; }
     w->tcn_R = R;
@@ -505,17 +596,15 @@ int run_weighted_sum_tcn(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn
     // fan-in <= 32: pre-shifted weights (7x the planes) and the seven-class kernel, when they fit the weight cache
     const bool want_pre = tcn_preshift_shape(R, ncols, M, variant) &&
                           7 * tcn_w_bytes(7, (int)(w->count / R), Kpad, ctx->K, ctx->n) <= ctx->weight_cache_bytes;
-    int rc = ensure_domain(ctx, in, 1);
-    if (!rc) rc = ensure_form(ctx, b, PF_NTT_ADD);
-    if (!rc) rc = ensure_tcn_weights(ctx, w, R, want_pre);
-    if (rc) return rc;
+    TRY(ensure_domain(ctx, in, 1));
+    TRY(ensure_form(ctx, b, PF_NTT_ADD));
+    TRY(ensure_tcn_weights(ctx, w, R, want_pre));
     const size_t pw = poly_words(ctx);
     const size_t per_slot = tcn_x_bytes_per_slot(7, ncols, Kpad);
     long chunk = (long)(ctx->tc_scratch_bytes / per_slot) / 32 * 32;
     chunk = std::max<long>(32, std::min<long>(chunk, total));
-    uint8_t *scratch = nullptr;
-    rc = dev_alloc(ctx, (size_t)chunk * per_slot, (void **)&scratch);
-    if (rc) return rc;
+    DevBuf<uint8_t> scratch(ctx);
+    TRY(dev_alloc(ctx, (size_t)chunk * per_slot, scratch));
     TcnSplitArgs s{};
     s.src = in->d; s.index = d_index; s.dst = scratch; s.item_polys = 2;
     s.R = R; s.Kpad = Kpad; s.planes = 7; s.ncols = ncols; s.n = ctx->n; s.K = ctx->K;
@@ -528,7 +617,7 @@ int run_weighted_sum_tcn(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn
     a.preshift = want_pre && w->tcn_pre;
     a.use_fold = ctx->tcn_fold;
     for (int j = 0; j < ctx->K; j++) a.fold[j] = tcn_fold_make(ctx->hp.d.tab[j].mod.q);
-    for (long s0 = 0; s0 < total && !rc; s0 += chunk) {
+    for (long s0 = 0; s0 < total; s0 += chunk) {
         const int ns = (int)std::min<long>(chunk, total - s0);
         s.slot0 = a.slot0 = (int)s0; s.nslots = a.nslots = ns;
         const double xbytes = (double)ns * per_slot;
@@ -539,30 +628,35 @@ int run_weighted_sum_tcn(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn
             ProfScope ps(ctx, KC_TCN_MAC, xbytes + (double)ns * 7 * M * Kpad * (a.preshift ? 7 : 1) + (double)ncols * M * ns * 8.0, (double)ns * ncols * M * R * 49.0);
             e = launch_tcn_mac(ctx->dP, a, ctx->sm_count, ctx->stream);
         }
-        if (e != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, std::string("limb-split tensor-core weighted sum: ") + cudaGetErrorString(e));
+        if (e != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, std::string("limb-split tensor-core weighted sum: ") + cudaGetErrorString(e));
     }
-    dev_free(ctx, scratch);
-    if (!rc) out->ntt = 1;
-    return rc;
+    out->ntt = 1;
+    return CRCNN_OK;
 }
 
+// The NTT-domain limb-split GEMM can run a weighted sum of fan-in R whose byte planes of `rows` output rows fit the weight cache
+// (rows = 0: planes already staged).
+bool limb_split_fits(const crcnn_ctx *ctx, int R, int rows) {
+    return ctx->tcn_mode && tcn_planes_for(ctx->hp.d) == 7 && R <= TCN_MAX_R && tc_mac_available() == cudaSuccess &&
+           tcn_w_bytes(7, rows, tcn_kpad(R), ctx->K, ctx->n) <= ctx->weight_cache_bytes;
+}
+
+// ntt_only: the inputs are NTT-form plaintexts posing as ciphertexts (compose_fc), so the coefficient-domain ternary GEMM is not
+// considered.
 int run_weighted_sum(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_plain *b, const int *d_index, int R,
-                     int Npos, int Pimg, int Mall, int m_first, int M, crcnn_tensor *out) {
+                     int Npos, int Pimg, int Mall, int m_first, int M, crcnn_tensor *out, bool ntt_only) {
     // the kernel (and with it the domain of the output) is chosen from the LAYER's output count Mall, not the shard's M: every rank of a
     // neuron-sharded layer then produces its rows in the same domain, whatever the split (63 rows on 2 ranks: 32 + 31)
-    if (ctx->tc_mode && R >= ctx->tc_min_fanin && (ctx->tc_mode == 2 || Mall >= ctx->tc_min_outputs) && w->sparse_shape && tc_mac_available() == cudaSuccess) {
-        int rc = ensure_tc_form(ctx, w, R);
-        if (rc) return rc;
+    if (!ntt_only && ctx->tc_mode && R >= ctx->tc_min_fanin && (ctx->tc_mode == 2 || Mall >= ctx->tc_min_outputs) && w->sparse_shape &&
+        tc_mac_available() == cudaSuccess) {
+        TRY(ensure_tc_form(ctx, w, R));
         if (w->tc_state == 1) return run_weighted_sum_tc(ctx, in, w, b, d_index, R, Npos, Pimg, m_first, M, out);
     }
     // any weights, NTT domain: the limb-split GEMM, as long as the staged weight planes fit the weight cache
-    if (ctx->tcn_mode && tcn_planes_for(ctx->hp.d) == 7 && R <= TCN_MAX_R && w->count % R == 0 && tc_mac_available() == cudaSuccess &&
-        (w->tcn_W || tcn_w_bytes(7, (int)(w->count / R), tcn_kpad(R), ctx->K, ctx->n) <= ctx->weight_cache_bytes))
+    if (w->count % R == 0 && limb_split_fits(ctx, R, w->tcn_W ? 0 : (int)(w->count / R)))
         return run_weighted_sum_tcn(ctx, in, w, b, d_index, R, Npos, Pimg, m_first, M, out);
-    int rc = ensure_domain(ctx, in, 1);
-    if (rc) return rc;
-    rc = ensure_form(ctx, b, PF_NTT_ADD);
-    if (rc) return rc;
+    TRY(ensure_domain(ctx, in, 1));
+    TRY(ensure_form(ctx, b, PF_NTT_ADD));
     MacArgs a{};
     a.x = in->d; a.in_index = d_index; a.out = out->d;
     a.R = R; a.Npos = Npos; a.Pimg = Pimg; a.Mtotal = M; a.K = ctx->K; a.n = ctx->n;
@@ -570,8 +664,7 @@ int run_weighted_sum(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_pla
     const size_t pw = poly_words(ctx);
     const size_t all_bytes = (size_t)w->count * pw * 8;
     if (w->ntt_mul || all_bytes <= ctx->weight_cache_bytes) {
-        rc = ensure_form(ctx, w, PF_NTT_MUL);  // first forward pays the transform, like the reference's lazy transform_kernel_to_ntt
-        if (rc) return rc;
+        TRY(ensure_form(ctx, w, PF_NTT_MUL));  // first forward pays the transform, like the reference's lazy transform_kernel_to_ntt
         a.w = w->ntt_mul + (size_t)m_first * R * pw;
         a.bias = b->ntt_add + (size_t)m_first * pw;
         a.M = M; a.m0 = 0;
@@ -583,22 +676,19 @@ int run_weighted_sum(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_pla
     // weights do not fit: expand `rows` output rows at a time into a scratch buffer
     long rows = (long)std::max<size_t>(1, ctx->weight_cache_bytes / ((size_t)R * pw * 8));
     rows = std::min<long>(rows, M);
-    uint64_t *scratch = nullptr;
-    rc = dev_alloc(ctx, (size_t)rows * R * pw * 8, (void **)&scratch);
-    if (rc) return rc;
+    DevBuf<uint64_t> scratch(ctx);
+    TRY(dev_alloc(ctx, (size_t)rows * R * pw * 8, scratch));
     for (long m0 = 0; m0 < M; m0 += rows) {
         long cur = std::min<long>(rows, M - m0);
-        rc = expand_range(ctx, w, (long)(m_first + m0) * R, cur * R, PF_NTT_MUL, scratch);
-        if (rc) break;
+        TRY(expand_range(ctx, w, (long)(m_first + m0) * R, cur * R, PF_NTT_MUL, scratch));
         a.w = scratch; a.bias = b->ntt_add + (size_t)(m_first + m0) * pw;
         a.M = (int)cur; a.m0 = (int)m0;
         ProfScope ps(ctx, KC_MAC, lp_bytes(ctx, ((double)in->count + (double)cur * Npos) * 2 * ctx->K + (double)cur * R * ctx->K),
                      (double)cur * Npos * R * 2 * ctx->K * ctx->n);
         cudaError_t e = launch_mac(ctx->dP, a, ctx->stream);
-        if (e != cudaSuccess) { rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e)); break; }
+        if (e != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
     }
-    dev_free(ctx, scratch);
-    return rc;
+    return CRCNN_OK;
 }
 
 // Host (SEAL layout, limb stride n+1) -> device (stride n): one contiguous H2D copy into a staging buffer, then a
@@ -805,16 +895,11 @@ int crcnn_tensor_upload_ex(crcnn_ctx *ctx, const uint64_t *host, long count, int
     if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
     REQUIRE(host && out && count >= 0 && size >= 2 && size <= 3, "bad tensor upload arguments");
     CU(cudaSetDevice(ctx->device));
-    crcnn_tensor *t = nullptr;
-    int rc = new_tensor(ctx, count, size, ntt_form ? 1 : 0, &t);
-    if (rc) return rc;
-    const size_t n = ctx->n, rows = (size_t)count * size * ctx->K;
-    if (rows) {
-        int rc2 = upload_rows(ctx, host, rows, t->d, ctx->stream);
-        if (rc2) { crcnn_tensor_free(ctx, t); return rc2; }
-    }
-    (void)n;
-    *out = t;
+    TensorOwner t(ctx);
+    TRY(new_tensor(ctx, count, size, ntt_form ? 1 : 0, t.out()));
+    const size_t rows = (size_t)count * size * ctx->K;
+    if (rows) TRY(upload_rows(ctx, host, rows, t->d, ctx->stream));
+    *out = t.release();
     return CRCNN_OK;
 }
 int crcnn_tensor_upload_on(crcnn_ctx *ctx, const uint64_t *host, long count, int size, int ntt_form, void *copy_stream,
@@ -875,18 +960,15 @@ int crcnn_tensor_download_ex(crcnn_ctx *ctx, crcnn_tensor *t, int want_ntt, uint
     CU(cudaSetDevice(ctx->device));
     const size_t n = ctx->n, rows = (size_t)t->count * t->size * ctx->K;
     const uint64_t *src = t->d;
-    uint64_t *tmp = nullptr;
+    DevBuf<uint64_t> tmp(ctx);
     if ((t->ntt != 0) != (want_ntt != 0)) {  // convert a copy; the tensor itself keeps its domain
-        int rc = dev_alloc(ctx, rows * n * 8, (void **)&tmp);
-        if (rc) return rc;
+        TRY(dev_alloc(ctx, rows * n * 8, tmp));
         CU(cudaMemcpyAsync(tmp, t->d, rows * n * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-        rc = ntt_inplace(ctx, tmp, (long)rows, 0, ctx->K, want_ntt == 0);
-        if (rc) return rc;
+        TRY(ntt_inplace(ctx, tmp, (long)rows, 0, ctx->K, want_ntt == 0));
         src = tmp;
     }
     if (rows) CU(cudaMemcpy2DAsync(host, (n + 1) * 8, src, n * 8, n * 8, rows, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
-    dev_free(ctx, tmp);
     for (size_t r = 0; r < rows; r++) host[r * (n + 1) + n] = 0;  // SEAL's pad word
     prof_collect(ctx);
     return CRCNN_OK;
@@ -906,12 +988,11 @@ int crcnn_tensor_ct_size(const crcnn_tensor *t) { return t ? t->size : -1; }
 int crcnn_tensor_slice(crcnn_ctx *ctx, crcnn_tensor *t, long first, long count, crcnn_tensor **out) {
     if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
     REQUIRE(t && out && first >= 0 && count >= 0 && first + count <= t->count, "slice out of range");
-    crcnn_tensor *s = nullptr;
-    int rc = new_tensor(ctx, count, t->size, t->ntt, &s);
-    if (rc) return rc;
+    TensorOwner s(ctx);
+    TRY(new_tensor(ctx, count, t->size, t->ntt, s.out()));
     size_t ctw = (size_t)t->size * poly_words(ctx);
     if (count) CU(cudaMemcpyAsync(s->d, t->d + first * ctw, count * ctw * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-    *out = s;
+    *out = s.release();
     return CRCNN_OK;
 }
 
@@ -1003,15 +1084,12 @@ int crcnn_plain_get_ntt(crcnn_ctx *ctx, crcnn_plain *p, long index, uint64_t *ou
     if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
     REQUIRE(p && out_words && index >= 0 && index < p->count, "plaintext index out of range");
     REQUIRE(!p->dense_only, "derived plaintext pack: no host form");
-    uint64_t *tmp = nullptr;
-    int rc = dev_alloc(ctx, poly_words(ctx) * 8, (void **)&tmp);
-    if (rc) return rc;
-    rc = expand_range(ctx, p, index, 1, PF_NTT_MUL, tmp);
-    if (rc) return rc;
+    DevBuf<uint64_t> tmp(ctx);
+    TRY(dev_alloc(ctx, poly_words(ctx) * 8, tmp));
+    TRY(expand_range(ctx, p, index, 1, PF_NTT_MUL, tmp));
     const size_t n = ctx->n;
     CU(cudaMemcpy2DAsync(out_words, (n + 1) * 8, tmp, n * 8, n * 8, ctx->K, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
-    dev_free(ctx, tmp);
     for (int j = 0; j < ctx->K; j++) out_words[j * (n + 1) + n] = 0;
     return CRCNN_OK;
 }
@@ -1034,19 +1112,18 @@ int crcnn_evk_upload(crcnn_ctx *ctx, const uint64_t *host, int dbc, const int *s
     if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
     REQUIRE(host && sizes && out && dbc >= 1 && dbc <= 60, "bad evaluation key arguments");
     CU(cudaSetDevice(ctx->device));
-    auto *k = new crcnn_evk();
+    Owned<crcnn_evk, crcnn_evk_free> k(ctx, new crcnn_evk());
     k->dbc = dbc;
     long polys = 0;
     const size_t pw = poly_words(ctx);
     for (int i = 0; i < MAXK; i++) { k->key_off[i] = 0; k->digits[i] = 0; }
     for (int i = 0; i < ctx->K; i++) {
-        if (sizes[i] < 2 || (sizes[i] & 1)) { delete k; return fail(ctx, CRCNN_ERR_INVALID_ARGUMENT, "evaluation key sizes must be even and >= 2"); }
+        REQUIRE(sizes[i] >= 2 && !(sizes[i] & 1), "evaluation key sizes must be even and >= 2");
         k->key_off[i] = polys * (long)pw;
         k->digits[i] = sizes[i] / 2;
         polys += sizes[i];
     }
-    int rc = dev_alloc(ctx, (size_t)polys * pw * 8, (void **)&k->d);
-    if (rc) { delete k; return rc; }
+    TRY(dev_alloc(ctx, (size_t)polys * pw * 8, (void **)&k->d));
     const size_t n = ctx->n, rows = (size_t)polys * ctx->K;
     CU(cudaMemcpy2DAsync(k->d, n * 8, host, (n + 1) * 8, n * 8, rows, cudaMemcpyHostToDevice, ctx->stream));
     CU(launch_canonicalize(ctx->dP, k->d, (long)(rows * n), ctx->stream));
@@ -1055,11 +1132,11 @@ int crcnn_evk_upload(crcnn_ctx *ctx, const uint64_t *host, int dbc, const int *s
         for (int i = 0; i < ctx->K; i++) q[i] = ctx->hp.d.tab[i].mod.q;
         if (relin32_applicable(ctx->n, ctx->K, q, k->digits, dbc, k->r32.c)) {
             cudaError_t e = relin32_build(ctx->dP, ctx->logn, ctx->K, q, k->d, k->key_off, polys, k->r32, ctx->stream);
-            if (e != cudaSuccess) { relin32_free(k->r32); dev_free(ctx, k->d); delete k; return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e)); }
+            if (e != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
             k->has_r32 = true;
         }
     }
-    *out = k;
+    *out = k.release();
     return CRCNN_OK;
 }
 int crcnn_evk_free(crcnn_ctx *ctx, crcnn_evk *k) {
@@ -1096,9 +1173,8 @@ int crcnn_conv_forward_padded(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, 
     if ((xl + xs - 1) / xs != xo || (yl + ys - 1) / ys != yo)
         return fail(ctx, CRCNN_ERR_UNSUPPORTED, "stride larger than the filter leaves outputs the reference never computes");
     const int P = xo * yo, Npos = batch * P, nin = zd * xd * yd;
-    std::vector<int> key = {1, batch, xd, yd, zd, xs, ys, xf, yf, xp, yp};
     const int *d_index = nullptr;
-    if (ctx->index_cache.find(key) == ctx->index_cache.end()) {
+    TRY(index_table(ctx, TAB_CONV, {batch, xd, yd, zd, xs, ys, xf, yf, xp, yp}, [&] {
         std::vector<int> table((size_t)Npos * R);
         for (int bi = 0; bi < batch; bi++)
             for (int i = 0; i < xo; i++)
@@ -1112,17 +1188,12 @@ int crcnn_conv_forward_padded(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, 
                                 row[r++] = (u >= 0 && u < xd && v >= 0 && v < yd) ? bi * nin + (z * xd + u) * yd + v : -1;
                             }
                 }
-        int rc = get_index_table(ctx, key, table, &d_index);
-        if (rc) return rc;
-    } else {
-        d_index = ctx->index_cache[key];
-    }
-    crcnn_tensor *o = nullptr;
-    int rc = new_tensor(ctx, (long)batch * kc * P, 2, 1, &o);
-    if (rc) return rc;
-    rc = run_weighted_sum(ctx, in, w, b, d_index, R, Npos, P, nf, k0, kc, o);
-    if (rc) { crcnn_tensor_free(ctx, o); return rc; }
-    *out = o;
+        return table;
+    }, &d_index));
+    TensorOwner o(ctx);
+    TRY(new_tensor(ctx, (long)batch * kc * P, 2, 1, o.out()));
+    TRY(run_weighted_sum(ctx, in, w, b, d_index, R, Npos, P, nf, k0, kc, o, false));
+    *out = o.release();
     return CRCNN_OK;
 }
 
@@ -1145,22 +1216,12 @@ int crcnn_fc_forward_shard(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crc
     REQUIRE(in->size == 2 && in->count == (long)batch * in_dim, "input tensor does not match the layer geometry");
     REQUIRE(w->count == (long)out_dim * in_dim && b->count == out_dim, "weight/bias count does not match the layer geometry");
     CU(cudaSetDevice(ctx->device));
-    std::vector<int> key = {2, batch, in_dim};
     const int *d_index = nullptr;
-    if (ctx->index_cache.find(key) == ctx->index_cache.end()) {
-        std::vector<int> table((size_t)batch * in_dim);
-        for (size_t i = 0; i < table.size(); i++) table[i] = (int)i;
-        int rc = get_index_table(ctx, key, table, &d_index);
-        if (rc) return rc;
-    } else {
-        d_index = ctx->index_cache[key];
-    }
-    crcnn_tensor *o = nullptr;
-    int rc = new_tensor(ctx, (long)batch * oc, 2, 1, &o);
-    if (rc) return rc;
-    rc = run_weighted_sum(ctx, in, w, b, d_index, in_dim, batch, 1, out_dim, o0, oc, o);
-    if (rc) { crcnn_tensor_free(ctx, o); return rc; }
-    *out = o;
+    TRY(fc_index_table(ctx, batch, in_dim, &d_index));
+    TensorOwner o(ctx);
+    TRY(new_tensor(ctx, (long)batch * oc, 2, 1, o.out()));
+    TRY(run_weighted_sum(ctx, in, w, b, d_index, in_dim, batch, 1, out_dim, o0, oc, o, false));
+    *out = o.release();
     return CRCNN_OK;
 }
 
@@ -1179,87 +1240,61 @@ int crcnn_fc_forward(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w, crcnn_pla
 // With C / D (per input channel, `per_channel` inputs each; ensure_pool_bn_consts) the layer in front of fc1 -- x = P (.) C_c - D_c, the pooling
 // scale and batch-norm applied to window sums P -- goes into the composed constants as well: W[k,r] (.)= C_c(r), B_k -= sum_r W[k,r] (.) D_c(r).
 static int compose_fc(crcnn_ctx *ctx, crcnn_plain *w1, crcnn_plain *b1, crcnn_plain *w2, crcnn_plain *b2, int in_dim, int mid_dim, int out_dim,
-                      const uint64_t *C = nullptr, const uint64_t *D = nullptr, int per_channel = 1) {
+                      crcnn_plain **folded_w, crcnn_plain **folded_b, const uint64_t *C = nullptr, const uint64_t *D = nullptr,
+                      int per_channel = 1) {
     const size_t pw = poly_words(ctx);
-    const int saved_tc = ctx->tc_mode;
-    const bool saved_prof = ctx->prof_on;
-    ctx->tc_mode = 0;           // NTT-domain kernels only: the "ciphertexts" below are NTT-form plaintexts
-    ctx->prof_on = false;       // build-time work is not part of any step's profile
-    crcnn_plain *zero = nullptr, *W = nullptr, *B = nullptr;
-    crcnn_tensor *T = nullptr, *O = nullptr;
-    uint64_t *dense = nullptr;
-    int rc = CRCNN_OK;
-    auto done = [&](int code) {
-        if (T) crcnn_tensor_free(ctx, T);
-        if (O) crcnn_tensor_free(ctx, O);
-        if (zero) crcnn_plain_free(ctx, zero);
-        dev_free(ctx, dense);
-        if (code) { if (W) crcnn_plain_free(ctx, W); if (B) crcnn_plain_free(ctx, B); }
-        ctx->tc_mode = saved_tc; ctx->prof_on = saved_prof;
-        return code;
-    };
-    rc = make_plain(ctx, std::vector<uint32_t>((size_t)out_dim + 1, 0), {}, {}, &zero);
-    if (rc) return done(rc);
-    rc = dev_alloc(ctx, (size_t)out_dim * in_dim * pw * 8, (void **)&dense);
-    if (rc) return done(rc);
+    ProfPause quiet(ctx);       // build-time work is not part of any step's profile
+    PlainOwner zero(ctx);
+    TRY(make_plain(ctx, std::vector<uint32_t>((size_t)out_dim + 1, 0), {}, {}, zero.out()));
+    DevBuf<uint64_t> dense(ctx);
+    TRY(dev_alloc(ctx, (size_t)out_dim * in_dim * pw * 8, dense));
     // column pairs per pass: the staged columns of W1 (mid_dim pseudo-ciphertexts per pair) stay below ~8 GB
     const int pairs_all = (in_dim + 1) / 2;
     int Bc = (int)std::max<size_t>(1, std::min<size_t>((size_t)pairs_all, (8ull << 30) / ((size_t)mid_dim * 2 * pw * 8)));
     if (const char *e = getenv("CRCNN_FC_COMPOSE_PAIRS")) Bc = std::max(1, std::min(Bc, atoi(e)));   // tests: several passes on small layers
-    std::vector<int> table((size_t)Bc * mid_dim);
-    for (int bi = 0; bi < Bc; bi++)
-        for (int o = 0; o < mid_dim; o++) table[(size_t)bi * mid_dim + o] = o * Bc + bi;
     const int *d_index = nullptr;
-    rc = get_index_table(ctx, {5, Bc, mid_dim}, table, &d_index);
-    if (rc) return done(rc);
-    rc = new_tensor(ctx, (long)mid_dim * Bc, 2, 1, &T);
-    if (!rc) rc = new_tensor(ctx, (long)Bc * out_dim, 2, 1, &O);
-    if (rc) return done(rc);
+    TRY(index_table(ctx, TAB_COMPOSE, {Bc, mid_dim}, [&] {
+        std::vector<int> table((size_t)Bc * mid_dim);
+        for (int bi = 0; bi < Bc; bi++)
+            for (int o = 0; o < mid_dim; o++) table[(size_t)bi * mid_dim + o] = o * Bc + bi;
+        return table;
+    }, &d_index));
+    TensorOwner T(ctx), O(ctx);
+    TRY(new_tensor(ctx, (long)mid_dim * Bc, 2, 1, T.out()));
+    TRY(new_tensor(ctx, (long)Bc * out_dim, 2, 1, O.out()));
     CU(cudaMemsetAsync(T->d, 0, (size_t)T->count * 2 * pw * 8, ctx->stream));
-    for (int r0 = 0; r0 < in_dim && !rc; r0 += 2 * Bc) {
+    // NTT-domain kernels only (ntt_only): the "ciphertexts" below are NTT-form plaintexts
+    for (int r0 = 0; r0 < in_dim; r0 += 2 * Bc) {
         const int cols = std::min(2 * Bc, in_dim - r0);
-        for (int o = 0; o < mid_dim && !rc; o++)
-            rc = expand_range(ctx, w1, (long)o * in_dim + r0, cols, PF_NTT_MUL, T->d + (size_t)o * Bc * 2 * pw);
-        if (rc) break;
-        rc = run_weighted_sum(ctx, T, w2, zero, d_index, mid_dim, Bc, 1, out_dim, 0, out_dim, O);
-        if (rc) break;
+        for (int o = 0; o < mid_dim; o++)
+            TRY(expand_range(ctx, w1, (long)o * in_dim + r0, cols, PF_NTT_MUL, T->d + (size_t)o * Bc * 2 * pw));
+        TRY(run_weighted_sum(ctx, T, w2, zero, d_index, mid_dim, Bc, 1, out_dim, 0, out_dim, O, true));
         // O[b][k] = (W[k][r0+2b], W[k][r0+2b+1])  ->  dense[k][r]
         for (int bi = 0; 2 * bi < cols; bi++) {
             const int polys = std::min(2, cols - 2 * bi);
-            cudaError_t e = cudaMemcpy2DAsync(dense + ((size_t)r0 + 2 * bi) * pw, (size_t)in_dim * pw * 8, O->d + (size_t)bi * out_dim * 2 * pw,
-                                              2 * pw * 8, (size_t)polys * pw * 8, out_dim, cudaMemcpyDeviceToDevice, ctx->stream);
-            if (e != cudaSuccess) { rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e)); break; }
+            CU(cudaMemcpy2DAsync(dense + ((size_t)r0 + 2 * bi) * pw, (size_t)in_dim * pw * 8, O->d + (size_t)bi * out_dim * 2 * pw,
+                                 2 * pw * 8, (size_t)polys * pw * 8, out_dim, cudaMemcpyDeviceToDevice, ctx->stream));
         }
     }
-    if (rc) return done(rc);
-    W = new crcnn_plain();
+    PlainOwner W(ctx, new crcnn_plain());
     W->count = (long)out_dim * in_dim; W->dense_only = true; W->sparse_shape = false; W->tc_state = -1; W->tap_state = -1;
-    W->ntt_mul = dense; dense = nullptr;
+    W->ntt_mul = dense.release();
     // bias: fc2 applied to the Delta-scaled b1 (polynomial 0 of one pseudo-ciphertext per middle neuron), plus Delta b2
-    rc = ensure_form(ctx, b1, PF_NTT_ADD);
-    if (rc) return done(rc);
-    crcnn_tensor_free(ctx, T); T = nullptr;
-    crcnn_tensor_free(ctx, O); O = nullptr;
-    rc = new_tensor(ctx, mid_dim, 2, 1, &T);
-    if (!rc) rc = new_tensor(ctx, out_dim, 2, 1, &O);
-    if (rc) return done(rc);
+    TRY(ensure_form(ctx, b1, PF_NTT_ADD));
+    TRY(new_tensor(ctx, mid_dim, 2, 1, T.out()));
+    TRY(new_tensor(ctx, out_dim, 2, 1, O.out()));
     CU(cudaMemsetAsync(T->d, 0, (size_t)mid_dim * 2 * pw * 8, ctx->stream));
     CU(cudaMemcpy2DAsync(T->d, 2 * pw * 8, b1->ntt_add, pw * 8, pw * 8, mid_dim, cudaMemcpyDeviceToDevice, ctx->stream));
-    std::vector<int> ident(mid_dim);
-    for (int o = 0; o < mid_dim; o++) ident[o] = o;
-    rc = get_index_table(ctx, {2, 1, mid_dim}, ident, &d_index);
-    if (!rc) rc = run_weighted_sum(ctx, T, w2, b2, d_index, mid_dim, 1, 1, out_dim, 0, out_dim, O);
-    if (rc) return done(rc);
-    B = new crcnn_plain();
+    TRY(fc_index_table(ctx, 1, mid_dim, &d_index));
+    TRY(run_weighted_sum(ctx, T, w2, b2, d_index, mid_dim, 1, 1, out_dim, 0, out_dim, O, true));
+    PlainOwner B(ctx, new crcnn_plain());
     B->count = out_dim; B->dense_only = true; B->sparse_shape = false; B->tc_state = -1; B->tap_state = -1;
-    rc = dev_alloc(ctx, (size_t)out_dim * pw * 8, (void **)&B->ntt_add);
-    if (rc) return done(rc);
+    TRY(dev_alloc(ctx, (size_t)out_dim * pw * 8, (void **)&B->ntt_add));
     CU(cudaMemcpy2DAsync(B->ntt_add, pw * 8, O->d, 2 * pw * 8, pw * 8, out_dim, cudaMemcpyDeviceToDevice, ctx->stream));
     if (C) CU(launch_fold_fc_input_affine(ctx->dP, W->ntt_mul, out_dim, in_dim, (long)pw, per_channel, C, D, B->ntt_add, ctx->stream));
-    rc = ensure_tcn_weights(ctx, W, in_dim, false);   // byte planes of the composed weights; releases the dense form
-    if (rc) return done(rc);
-    w1->folded_w = W; w1->folded_b = B;
-    return done(CRCNN_OK);
+    TRY(ensure_tcn_weights(ctx, W, in_dim, false));   // byte planes of the composed weights; releases the dense form
+    *folded_w = W.release(); *folded_b = B.release();
+    return CRCNN_OK;
 }
 
 int crcnn_fc_fc_forward(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w1, crcnn_plain *b1, crcnn_plain *w2, crcnn_plain *b2, int batch,
@@ -1273,25 +1308,16 @@ int crcnn_fc_fc_forward(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_plain *w1, crcnn
     CU(cudaSetDevice(ctx->device));
     // worth it when the composed layer is the smaller one, and possible when its byte planes fit the weight cache
     const bool composed = (double)out_dim * in_dim < (double)mid_dim * (in_dim + out_dim) && !w1->dense_only && !w2->dense_only &&
-                          ctx->tcn_mode && tcn_planes_for(ctx->hp.d) == 7 && in_dim <= TCN_MAX_R && mid_dim <= TCN_MAX_R &&
-                          tc_mac_available() == cudaSuccess && tcn_w_bytes(7, out_dim, tcn_kpad(in_dim), ctx->K, ctx->n) <= ctx->weight_cache_bytes &&
-                          !getenv("CRCNN_NO_FC_COMPOSE");
+                          mid_dim <= TCN_MAX_R && limb_split_fits(ctx, in_dim, out_dim) && !getenv("CRCNN_NO_FC_COMPOSE");
     if (!composed) {
-        crcnn_tensor *mid = nullptr;
-        int rc = crcnn_fc_forward(ctx, in, w1, b1, batch, in_dim, mid_dim, &mid);
-        if (rc) return rc;
-        rc = crcnn_fc_forward(ctx, mid, w2, b2, batch, mid_dim, out_dim, out);
-        crcnn_tensor_free(ctx, mid);
-        return rc;
+        TensorOwner mid(ctx);
+        TRY(crcnn_fc_forward(ctx, in, w1, b1, batch, in_dim, mid_dim, mid.out()));
+        return crcnn_fc_forward(ctx, mid, w2, b2, batch, mid_dim, out_dim, out);
     }
     const long key[9] = {b1->serial, w2->serial, b2->serial, (long)mid_dim, (long)out_dim, 0, 0, 0, 0};
-    if (!w1->folded_w || memcmp(key, w1->folded_key, sizeof(key)) != 0) {
-        if (w1->folded_w) { crcnn_plain_free(ctx, w1->folded_w); w1->folded_w = nullptr; }
-        if (w1->folded_b) { crcnn_plain_free(ctx, w1->folded_b); w1->folded_b = nullptr; }
-        int rc = compose_fc(ctx, w1, b1, w2, b2, in_dim, mid_dim, out_dim);
-        if (rc) return rc;
-        memcpy(w1->folded_key, key, sizeof(key));
-    }
+    TRY(ensure_folded(ctx, w1, key, [&](crcnn_plain **fw, crcnn_plain **fb) {
+        return compose_fc(ctx, w1, b1, w2, b2, in_dim, mid_dim, out_dim, fw, fb);
+    }));
     return crcnn_fc_forward(ctx, in, w1->folded_w, w1->folded_b, batch, in_dim, out_dim, out);
 }
 
@@ -1314,96 +1340,57 @@ int crcnn_pool_bn_fc_fc_forward(crcnn_ctx *ctx, crcnn_tensor *in, int batch, int
     CU(cudaSetDevice(ctx->device));
     const bool composed = pxs <= pxf && pys <= pyf && sum_fits_64(ctx, Rp) &&
                           (double)out_dim * in_dim < (double)mid_dim * (in_dim + out_dim) && !w1->dense_only && !w2->dense_only &&
-                          ctx->tcn_mode && tcn_planes_for(ctx->hp.d) == 7 && in_dim <= TCN_MAX_R && mid_dim <= TCN_MAX_R &&
-                          tc_mac_available() == cudaSuccess && tcn_w_bytes(7, out_dim, tcn_kpad(in_dim), ctx->K, ctx->n) <= ctx->weight_cache_bytes &&
-                          !getenv("CRCNN_NO_FC_COMPOSE");
+                          mid_dim <= TCN_MAX_R && limb_split_fits(ctx, in_dim, out_dim) && !getenv("CRCNN_NO_FC_COMPOSE");
     if (!composed) {
-        crcnn_tensor *mid = nullptr;
-        int rc = crcnn_pool_bn_forward(ctx, in, batch, xd, yd, zd, pxs, pys, pxf, pyf, scale, mean, invstd, &mid);
-        if (rc) return rc;
-        rc = crcnn_fc_fc_forward(ctx, mid, w1, b1, w2, b2, batch, in_dim, mid_dim, out_dim, out);
-        crcnn_tensor_free(ctx, mid);
-        return rc;
+        TensorOwner mid(ctx);
+        TRY(crcnn_pool_bn_forward(ctx, in, batch, xd, yd, zd, pxs, pys, pxf, pyf, scale, mean, invstd, mid.out()));
+        return crcnn_fc_fc_forward(ctx, mid, w1, b1, w2, b2, batch, in_dim, mid_dim, out_dim, out);
     }
-    int rc = ensure_pool_bn_consts(ctx, scale, mean, invstd);
-    if (rc) return rc;
+    TRY(ensure_pool_bn_consts(ctx, scale, mean, invstd));
     const long key[9] = {b1->serial, w2->serial, b2->serial, (long)mid_dim, (long)out_dim, scale ? scale->serial : -1, mean->serial, invstd->serial, (long)(pxo * pyo)};
-    if (!w1->folded_w || memcmp(key, w1->folded_key, sizeof(key)) != 0) {
-        if (w1->folded_w) { crcnn_plain_free(ctx, w1->folded_w); w1->folded_w = nullptr; }
-        if (w1->folded_b) { crcnn_plain_free(ctx, w1->folded_b); w1->folded_b = nullptr; }
-        rc = compose_fc(ctx, w1, b1, w2, b2, in_dim, mid_dim, out_dim, invstd->fused_C, invstd->fused_D, pxo * pyo);
-        if (rc) return rc;
-        memcpy(w1->folded_key, key, sizeof(key));
-    }
+    TRY(ensure_folded(ctx, w1, key, [&](crcnn_plain **fw, crcnn_plain **fb) {
+        return compose_fc(ctx, w1, b1, w2, b2, in_dim, mid_dim, out_dim, fw, fb, invstd->fused_C, invstd->fused_D, pxo * pyo);
+    }));
     // window sums (no scale), in the input's domain: the pooling layer's own index table
-    crcnn_tensor *sums = nullptr;
-    rc = crcnn_pool_forward(ctx, in, batch, xd, yd, zd, pxs, pys, pxf, pyf, nullptr, &sums);
-    if (rc) return rc;
-    rc = crcnn_fc_forward(ctx, sums, w1->folded_w, w1->folded_b, batch, in_dim, out_dim, out);
-    crcnn_tensor_free(ctx, sums);
-    return rc;
+    TensorOwner sums(ctx);
+    TRY(crcnn_pool_forward(ctx, in, batch, xd, yd, zd, pxs, pys, pxf, pyf, nullptr, sums.out()));
+    return crcnn_fc_forward(ctx, sums, w1->folded_w, w1->folded_b, batch, in_dim, out_dim, out);
 }
 
 int crcnn_pool_forward(crcnn_ctx *ctx, crcnn_tensor *in, int batch, int xd, int yd, int zd, int xs, int ys, int xf, int yf,
                        crcnn_plain *scale, crcnn_tensor **out) {
     if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
     REQUIRE(in && out, "null argument");
-    REQUIRE(batch > 0 && xd > 0 && yd > 0 && zd > 0 && xs > 0 && ys > 0 && xf > 0 && yf > 0 && xf <= xd && yf <= yd, "bad pooling geometry");
-    REQUIRE(in->size == 2 && in->count == (long)batch * zd * xd * yd, "input tensor does not match the layer geometry");
     REQUIRE(!scale || scale->count >= 1, "empty scale pack");
-    CU(cudaSetDevice(ctx->device));
-    const int xo = (xd - xf) / xs + 1, yo = (yd - yf) / ys + 1;  // poolingLayer.cpp:18
-    int xl, yl;
-    boundaries(xd, yd, xs, ys, xf, yf, &xl, &yl);
-    if ((xl + xs - 1) / xs != xo || (yl + ys - 1) / ys != yo)
-        return fail(ctx, CRCNN_ERR_UNSUPPORTED, "stride larger than the window leaves outputs the reference never computes");
-    const int R = xf * yf, Nout = batch * zd * xo * yo;
-    std::vector<int> key = {3, batch, xd, yd, zd, xs, ys, xf, yf};
-    const int *d_index = nullptr;
-    if (ctx->index_cache.find(key) == ctx->index_cache.end()) {
-        std::vector<int> table((size_t)Nout * R);
-        size_t o = 0;
-        for (int bz = 0; bz < batch * zd; bz++)
-            for (int i = 0; i < xo; i++)
-                for (int j = 0; j < yo; j++)
-                    for (int kx = 0; kx < xf; kx++)
-                        for (int ky = 0; ky < yf; ky++) table[o++] = (bz * xd + i * xs + kx) * yd + j * ys + ky;
-        int rc = get_index_table(ctx, key, table, &d_index);
-        if (rc) return rc;
-    } else {
-        d_index = ctx->index_cache[key];
-    }
-    int rc = CRCNN_OK;
+    PoolWindows g;
+    TRY(pool_windows(ctx, in, batch, xd, yd, zd, xs, ys, xf, yf, &g));
+    const int R = g.R, Nout = g.Nout;
+    TensorOwner o(ctx);
     if (scale && !in->ntt && ctx->tap_mode && tap_eligible(ctx, scale) && sum_fits_64(ctx, R)) {
         // coefficient-form input (after the square activation): stay there, no transform in either direction
-        crcnn_tensor *o = nullptr;
-        rc = new_tensor(ctx, Nout, 2, 0, &o);
-        if (rc) return rc;
+        TRY(new_tensor(ctx, Nout, 2, 0, o.out()));
         TapMulArgs a{};
-        a.in = in->d; a.in_index = d_index; a.R = R; a.sub = nullptr;
+        a.in = in->d; a.in_index = g.d_index; a.R = R; a.sub = nullptr;
         a.t_off = scale->d_off; a.t_idx = scale->d_idx; a.t_val = scale->d_val; a.per_channel = 1; a.channels = 1;
         a.out = o->d; a.nout = Nout;
         ProfScope ps(ctx, KC_POOL, lp_bytes(ctx, ((double)in->count + Nout) * 2 * ctx->K), (double)Nout * R * 2 * ctx->K * ctx->n);
         cudaError_t e = launch_tapmul(ctx->dP, ctx->n, ctx->K, a, ctx->stream);
-        if (e != cudaSuccess) { crcnn_tensor_free(ctx, o); return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e)); }
-        *out = o;
+        if (e != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
+        *out = o.release();
         return CRCNN_OK;
     }
     if (scale) {
-        rc = ensure_domain(ctx, in, 1);
-        if (!rc) rc = ensure_shoup(ctx, scale);
-        if (rc) return rc;
+        TRY(ensure_domain(ctx, in, 1));
+        TRY(ensure_shoup(ctx, scale));
     }
-    crcnn_tensor *o = nullptr;
-    rc = new_tensor(ctx, Nout, 2, in->ntt, &o);
-    if (rc) return rc;
+    TRY(new_tensor(ctx, Nout, 2, in->ntt, o.out()));
     {
         ProfScope ps(ctx, KC_POOL, lp_bytes(ctx, ((double)in->count + Nout) * 2 * ctx->K), (double)Nout * R * 2 * ctx->K * ctx->n);
-        cudaError_t e = launch_pool(ctx->dP, ctx->n, ctx->K, in->d, d_index, Nout, R, scale ? scale->ntt_mul : nullptr,
+        cudaError_t e = launch_pool(ctx->dP, ctx->n, ctx->K, in->d, g.d_index, Nout, R, scale ? scale->ntt_mul : nullptr,
                                     scale ? scale->ntt_mul_sh : nullptr, sum_fits_64(ctx, R), o->d, ctx->stream);
-        if (e != cudaSuccess) { crcnn_tensor_free(ctx, o); return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e)); }
+        if (e != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
     }
-    *out = o;
+    *out = o.release();
     return CRCNN_OK;
 }
 
@@ -1416,52 +1403,23 @@ int crcnn_pool_bn_forward(crcnn_ctx *ctx, crcnn_tensor *in, int batch, int xd, i
     if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
     REQUIRE(in && mean && invstd && out, "null argument");      // scale == NULL: PoolingLayer (window sum without a factor)
     REQUIRE((!scale || scale->count >= 1) && mean->count == zd && invstd->count == zd, "mean/var count does not match the channel count");
-    const int xo = (xd - xf) / xs + 1, yo = (yd - yf) / ys + 1;
-    const int R = xf * yf;
-    if (!in->ntt || !sum_fits_64(ctx, R)) {      // not the fused kernel's case: the two layers one after the other
-        crcnn_tensor *mid = nullptr;
-        int rc = crcnn_pool_forward(ctx, in, batch, xd, yd, zd, xs, ys, xf, yf, scale, &mid);
-        if (rc) return rc;
-        rc = crcnn_bn_forward(ctx, mid, batch, zd, xo, yo, mean, invstd, out);
-        crcnn_tensor_free(ctx, mid);
-        return rc;
+    if (!in->ntt || !sum_fits_64(ctx, xf * yf)) {      // not the fused kernel's case: the two layers one after the other
+        TensorOwner mid(ctx);
+        TRY(crcnn_pool_forward(ctx, in, batch, xd, yd, zd, xs, ys, xf, yf, scale, mid.out()));
+        return crcnn_bn_forward(ctx, mid, batch, zd, (xd - xf) / xs + 1, (yd - yf) / ys + 1, mean, invstd, out);
     }
-    // geometry checks and the window index table are those of the pooling layer: run it on an empty batch? no -- build the table here
-    REQUIRE(batch > 0 && xd > 0 && yd > 0 && zd > 0 && xs > 0 && ys > 0 && xf > 0 && yf > 0 && xf <= xd && yf <= yd, "bad pooling geometry");
-    REQUIRE(in->size == 2 && in->count == (long)batch * zd * xd * yd, "input tensor does not match the layer geometry");
-    CU(cudaSetDevice(ctx->device));
-    int xl, yl;
-    boundaries(xd, yd, xs, ys, xf, yf, &xl, &yl);
-    if ((xl + xs - 1) / xs != xo || (yl + ys - 1) / ys != yo)
-        return fail(ctx, CRCNN_ERR_UNSUPPORTED, "stride larger than the window leaves outputs the reference never computes");
-    const int Nout = batch * zd * xo * yo;
-    std::vector<int> key = {3, batch, xd, yd, zd, xs, ys, xf, yf};
-    const int *d_index = nullptr;
-    if (ctx->index_cache.find(key) == ctx->index_cache.end()) {
-        std::vector<int> table((size_t)Nout * R);
-        size_t o = 0;
-        for (int bz = 0; bz < batch * zd; bz++)
-            for (int i = 0; i < xo; i++)
-                for (int j = 0; j < yo; j++)
-                    for (int kx = 0; kx < xf; kx++)
-                        for (int ky = 0; ky < yf; ky++) table[o++] = (bz * xd + i * xs + kx) * yd + j * ys + ky;
-        int rc = get_index_table(ctx, key, table, &d_index);
-        if (rc) return rc;
-    } else {
-        d_index = ctx->index_cache[key];
-    }
-    int rc = ensure_pool_bn_consts(ctx, scale, mean, invstd);
-    if (rc) return rc;
-    crcnn_tensor *o = nullptr;
-    rc = new_tensor(ctx, Nout, 2, 1, &o);
-    if (rc) return rc;
+    PoolWindows g;
+    TRY(pool_windows(ctx, in, batch, xd, yd, zd, xs, ys, xf, yf, &g));
+    TRY(ensure_pool_bn_consts(ctx, scale, mean, invstd));
+    TensorOwner o(ctx);
+    TRY(new_tensor(ctx, g.Nout, 2, 1, o.out()));
     {
-        ProfScope ps(ctx, KC_POOL, lp_bytes(ctx, ((double)in->count + Nout) * 2 * ctx->K), (double)Nout * (R + 1) * 2 * ctx->K * ctx->n);
-        cudaError_t e = launch_pool(ctx->dP, ctx->n, ctx->K, in->d, d_index, Nout, R, invstd->fused_C, invstd->fused_Csh, true, o->d, ctx->stream,
-                                    xo * yo, zd, invstd->fused_D);
-        if (e != cudaSuccess) { crcnn_tensor_free(ctx, o); return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e)); }
+        ProfScope ps(ctx, KC_POOL, lp_bytes(ctx, ((double)in->count + g.Nout) * 2 * ctx->K), (double)g.Nout * (g.R + 1) * 2 * ctx->K * ctx->n);
+        cudaError_t e = launch_pool(ctx->dP, ctx->n, ctx->K, in->d, g.d_index, g.Nout, g.R, invstd->fused_C, invstd->fused_Csh, true, o->d,
+                                    ctx->stream, g.xo * g.yo, zd, invstd->fused_D);
+        if (e != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
     }
-    *out = o;
+    *out = o.release();
     return CRCNN_OK;
 }
 
@@ -1495,51 +1453,39 @@ int crcnn_conv_pool_bn_forward_padded(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_pl
     // the pooled grid needs: strides that leave no output the reference skips (computeBoundaries), window sums below 2^64, and the
     // limb-split weighted sum (any NTT-form weights) with the folded weight planes resident
     const bool pooled_grid = pxs <= pxf && pys <= pyf && xs <= xf && ys <= yf && pxs * xs <= xf && pys * ys <= yf && Rp <= 64 && sum_fits_64(ctx, Rp) &&
-                             ctx->tcn_mode && tcn_planes_for(ctx->hp.d) == 7 && R <= TCN_MAX_R && tc_mac_available() == cudaSuccess &&
-                             tcn_w_bytes(7, nf, tcn_kpad(R), ctx->K, ctx->n) <= ctx->weight_cache_bytes && !getenv("CRCNN_NO_POOLED_CONV");
+                             limb_split_fits(ctx, R, nf) && !getenv("CRCNN_NO_POOLED_CONV");
     if (!pooled_grid) {   // the three layers one after the other (the last two in one pass when the activations are in NTT form)
         if (k0 != 0 || kc != nf)    // a channel shard of the layer-by-layer path is the caller's: conv shard, then pool and batch-norm on its channels
             return fail(ctx, CRCNN_ERR_UNSUPPORTED, "channel shards of conv + pool + batch-norm need the pooled-grid path");
-        crcnn_tensor *mid = nullptr;
-        int rc = crcnn_conv_forward_padded(ctx, in, w, b, batch, xd, yd, zd, xs, ys, xf, yf, nf, xp, yp, 0, nf, &mid);
-        if (rc) return rc;
-        rc = crcnn_pool_bn_forward(ctx, mid, batch, cxo, cyo, nf, pxs, pys, pxf, pyf, scale, mean, invstd, out);
-        crcnn_tensor_free(ctx, mid);
-        return rc;
+        TensorOwner mid(ctx);
+        TRY(crcnn_conv_forward_padded(ctx, in, w, b, batch, xd, yd, zd, xs, ys, xf, yf, nf, xp, yp, 0, nf, mid.out()));
+        return crcnn_pool_bn_forward(ctx, mid, batch, cxo, cyo, nf, pxs, pys, pxf, pyf, scale, mean, invstd, out);
     }
-    int rc = ensure_pool_bn_consts(ctx, scale, mean, invstd);
-    if (rc) return rc;
+    TRY(ensure_pool_bn_consts(ctx, scale, mean, invstd));
     const long key[9] = {b->serial, scale ? scale->serial : -1, mean->serial, invstd->serial, (long)Rp, 0, 0, 0, 0};
-    if (!w->folded_w || memcmp(key, w->folded_key, sizeof(key)) != 0) {
-        if (w->folded_w) { crcnn_plain_free(ctx, w->folded_w); w->folded_w = nullptr; }
-        if (w->folded_b) { crcnn_plain_free(ctx, w->folded_b); w->folded_b = nullptr; }
+    TRY(ensure_folded(ctx, w, key, [&](crcnn_plain **fw, crcnn_plain **fb) -> int {
         const size_t pw = poly_words(ctx);
-        // W' : the NTT form of W, row m*R + r times C[m]; staged as byte planes right away (the dense form is released by the staging)
-        rc = make_plain(ctx, std::vector<uint32_t>(w->off), std::vector<uint32_t>(w->idx), std::vector<uint64_t>(w->val), &w->folded_w);
-        if (rc) return rc;
-        w->folded_w->sparse_shape = false;   // never the ternary-tap path: these weights are general residues
-        w->folded_w->tc_state = -1; w->folded_w->tap_state = -1;
-        rc = ensure_form(ctx, w->folded_w, PF_NTT_MUL);
-        if (rc) return rc;
-        CU(launch_fold_affine(ctx->dP, w->folded_w->ntt_mul, (long)nf * R, (long)pw, R, invstd->fused_C, nullptr, ctx->stream));
+        // W' : the NTT form of W, row m*R + r times C[m]
+        TRY(make_plain(ctx, std::vector<uint32_t>(w->off), std::vector<uint32_t>(w->idx), std::vector<uint64_t>(w->val), fw));
+        (*fw)->sparse_shape = false;   // never the ternary-tap path: these weights are general residues
+        (*fw)->tc_state = -1; (*fw)->tap_state = -1;
+        TRY(ensure_form(ctx, *fw, PF_NTT_MUL));
+        CU(launch_fold_affine(ctx->dP, (*fw)->ntt_mul, (long)nf * R, (long)pw, R, invstd->fused_C, nullptr, ctx->stream));
         // staged as byte planes by the first weighted sum below, which knows the shape (pre-shifted or not); it releases the dense form
         // B' : |window| * (Delta-scaled bias) in NTT form, times C[m], minus D[m]
-        rc = make_plain(ctx, std::vector<uint32_t>(b->off), std::vector<uint32_t>(b->idx), std::vector<uint64_t>(b->val), &w->folded_b);
-        if (rc) return rc;
-        w->folded_b->add_mult = Rp;
-        rc = ensure_form(ctx, w->folded_b, PF_NTT_ADD);
-        if (rc) return rc;
-        CU(launch_fold_affine(ctx->dP, w->folded_b->ntt_add, (long)nf, (long)pw, 1, invstd->fused_C, invstd->fused_D, ctx->stream));
-        memcpy(w->folded_key, key, sizeof(key));
-    }
+        TRY(make_plain(ctx, std::vector<uint32_t>(b->off), std::vector<uint32_t>(b->idx), std::vector<uint64_t>(b->val), fb));
+        (*fb)->add_mult = Rp;
+        TRY(ensure_form(ctx, *fb, PF_NTT_ADD));
+        CU(launch_fold_affine(ctx->dP, (*fb)->ntt_add, (long)nf, (long)pw, 1, invstd->fused_C, invstd->fused_D, ctx->stream));
+        return CRCNN_OK;
+    }));
     // S: dilated window sums of the input, (zd, sxd, syd) per image, in the input's domain.  With padding S spans the padded extent and
     // its table holds -1 for border positions; the convolution over S then needs no padding, and its bias |window| * B stays as it is
     // because the convolution output carries the bias at every position, border included.
     const int sxd = xe - (pxf - 1) * xs, syd = ye - (pyf - 1) * ys;
     const int Nsum = batch * zd * sxd * syd;
-    std::vector<int> skey = {4, batch, xd, yd, zd, xs, ys, pxf, pyf, xp, yp};
     const int *d_index = nullptr;
-    if (ctx->index_cache.find(skey) == ctx->index_cache.end()) {
+    TRY(index_table(ctx, TAB_WINDOW_SUM, {batch, xd, yd, zd, xs, ys, pxf, pyf, xp, yp}, [&] {
         std::vector<int> table((size_t)Nsum * Rp);
         size_t o = 0;
         for (int bz = 0; bz < batch * zd; bz++)
@@ -1550,27 +1496,19 @@ int crcnn_conv_pool_bn_forward_padded(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_pl
                             const int x = u + a * xs - xp, y = v + c * ys - yp;
                             table[o++] = (x >= 0 && x < xd && y >= 0 && y < yd) ? (bz * xd + x) * yd + y : -1;
                         }
-        rc = get_index_table(ctx, skey, table, &d_index);
-        if (rc) return rc;
-    } else {
-        d_index = ctx->index_cache[skey];
-    }
-    crcnn_tensor *sums = nullptr, *pooled = nullptr;
-    rc = new_tensor(ctx, Nsum, 2, in->ntt, &sums);
-    if (rc) return rc;
+        return table;
+    }, &d_index));
+    TensorOwner sums(ctx), pooled(ctx);
+    TRY(new_tensor(ctx, Nsum, 2, in->ntt, sums.out()));
     {
         ProfScope ps(ctx, KC_POOL, lp_bytes(ctx, ((double)in->count + Nsum) * 2 * ctx->K), (double)Nsum * Rp * 2 * ctx->K * ctx->n);
         cudaError_t e = launch_pool(ctx->dP, ctx->n, ctx->K, in->d, d_index, Nsum, Rp, nullptr, nullptr, true, sums->d, ctx->stream);
-        if (e != cudaSuccess) { crcnn_tensor_free(ctx, sums); return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e)); }
+        if (e != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
     }
-    rc = crcnn_conv_forward_shard(ctx, sums, w->folded_w, w->folded_b, batch, sxd, syd, zd, pxs * xs, pys * ys, xf, yf, nf, k0, kc, &pooled);
-    crcnn_tensor_free(ctx, sums);
-    if (rc) return rc;
-    if (pooled->count != (long)batch * kc * pxo * pyo || !pooled->ntt) {
-        crcnn_tensor_free(ctx, pooled);
+    TRY(crcnn_conv_forward_shard(ctx, sums, w->folded_w, w->folded_b, batch, sxd, syd, zd, pxs * xs, pys * ys, xf, yf, nf, k0, kc, pooled.out()));
+    if (pooled->count != (long)batch * kc * pxo * pyo || !pooled->ntt)
         return fail(ctx, CRCNN_ERR_UNSUPPORTED, "pooled-grid convolution produced an unexpected shape");
-    }
-    *out = pooled;
+    *out = pooled.release();
     return CRCNN_OK;
 }
 
@@ -1596,35 +1534,30 @@ int crcnn_bn_forward(crcnn_ctx *ctx, crcnn_tensor *in, int batch, int zd, int xd
     REQUIRE(in->size == 2 && in->count == (long)batch * zd * xd * yd, "input tensor does not match the layer geometry");
     REQUIRE(mean->count == zd && invstd->count == zd, "mean/var count does not match the channel count");
     CU(cudaSetDevice(ctx->device));
+    TensorOwner o(ctx);
     if (!in->ntt && ctx->tap_mode && tap_eligible(ctx, invstd)) {
-        int rc = ensure_form(ctx, mean, PF_COEF_ADD);
-        if (rc) return rc;
-        crcnn_tensor *o = nullptr;
-        rc = new_tensor(ctx, in->count, 2, 0, &o);
-        if (rc) return rc;
+        TRY(ensure_form(ctx, mean, PF_COEF_ADD));
+        TRY(new_tensor(ctx, in->count, 2, 0, o.out()));
         TapMulArgs a{};
         a.in = in->d; a.in_index = nullptr; a.R = 1; a.sub = mean->coef_add;
         a.t_off = invstd->d_off; a.t_idx = invstd->d_idx; a.t_val = invstd->d_val; a.per_channel = xd * yd; a.channels = zd;
         a.out = o->d; a.nout = in->count;
         ProfScope ps(ctx, KC_BN, lp_bytes(ctx, (double)in->count * 4 * ctx->K), (double)in->count * 2 * ctx->K * ctx->n);
         cudaError_t e = launch_tapmul(ctx->dP, ctx->n, ctx->K, a, ctx->stream);
-        if (e != cudaSuccess) { crcnn_tensor_free(ctx, o); return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e)); }
-        *out = o;
+        if (e != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
+        *out = o.release();
         return CRCNN_OK;
     }
-    int rc = ensure_domain(ctx, in, 1);
-    if (!rc) rc = ensure_form(ctx, mean, PF_NTT_ADD);
-    if (!rc) rc = ensure_shoup(ctx, invstd);
-    if (rc) return rc;
-    crcnn_tensor *o = nullptr;
-    rc = new_tensor(ctx, in->count, 2, 1, &o);
-    if (rc) return rc;
+    TRY(ensure_domain(ctx, in, 1));
+    TRY(ensure_form(ctx, mean, PF_NTT_ADD));
+    TRY(ensure_shoup(ctx, invstd));
+    TRY(new_tensor(ctx, in->count, 2, 1, o.out()));
     {
         ProfScope ps(ctx, KC_BN, lp_bytes(ctx, (double)in->count * 4 * ctx->K), (double)in->count * 2 * ctx->K * ctx->n);
         cudaError_t e = launch_bn(ctx->dP, ctx->n, ctx->K, in->d, in->count, xd * yd, zd, mean->ntt_add, invstd->ntt_mul, invstd->ntt_mul_sh, o->d, ctx->stream);
-        if (e != cudaSuccess) { crcnn_tensor_free(ctx, o); return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e)); }
+        if (e != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
     }
-    *out = o;
+    *out = o.release();
     return CRCNN_OK;
 }
 
@@ -1639,19 +1572,17 @@ int crcnn_square(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_tensor **out3) {
     // The tensor stage leaves n^-1 to the floor's constants (and reduces on the fold where it applies); so does the INTT copy
     // to the lift's -- not a coefficient-form input, whose q limbs the lift copies into ext unscaled
     const bool fold = behz_fold_ok(ctx->hp.d);
-    crcnn_tensor *o = nullptr;
-    int rc = new_tensor(ctx, in->count, 3, 0, &o);
-    if (rc) return rc;
+    TensorOwner o(ctx);
+    TRY(new_tensor(ctx, in->count, 3, 0, o.out()));
     const int KS = ctx->K + ctx->S;
     const size_t n = ctx->n, pw = poly_words(ctx);
     // bound the scratch: chunks of at most `step` ciphertexts
     const long step = std::max<long>(1, std::min<long>(in->count, (long)((2ull << 30) / (5 * (size_t)KS * n * 8))));
-    uint64_t *ext = nullptr, *prod = nullptr, *coef = nullptr;
-    rc = dev_alloc(ctx, (size_t)step * 2 * KS * n * 8, (void **)&ext);
-    if (!rc) rc = dev_alloc(ctx, (size_t)step * 3 * KS * n * 8, (void **)&prod);
-    if (!rc && have_ntt) rc = dev_alloc(ctx, (size_t)step * 2 * pw * 8, (void **)&coef);
-    if (rc) { crcnn_tensor_free(ctx, o); return rc; }
-    for (long c0 = 0; c0 < in->count && !rc; c0 += step) {
+    DevBuf<uint64_t> ext(ctx), prod(ctx), coef(ctx);
+    TRY(dev_alloc(ctx, (size_t)step * 2 * KS * n * 8, ext));
+    TRY(dev_alloc(ctx, (size_t)step * 3 * KS * n * 8, prod));
+    if (have_ntt) TRY(dev_alloc(ctx, (size_t)step * 2 * pw * 8, coef));
+    for (long c0 = 0; c0 < in->count; c0 += step) {
         const long cur = std::min<long>(step, in->count - c0);
         const uint64_t *src = in->d + c0 * 2 * pw;
         cudaError_t e = cudaSuccess;
@@ -1677,12 +1608,9 @@ int crcnn_square(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_tensor **out3) {
         }
         if (e == cudaSuccess) { ProfScope ps(ctx, KC_BEHZ_FLOOR, lp_bytes(ctx, (double)cur * 3 * (KS + ctx->K)),
                                                      (double)cur * 3 * n * (ctx->S * (ctx->K + 1) + ctx->S + ctx->K * ctx->S)); e = launch_behz_floor(ctx->hp.d, ctx->n, prod, cur, o->d + c0 * 3 * pw, ctx->stream); }
-        if (e != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
+        if (e != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
     }
-    dev_free(ctx, coef);
-    dev_free(ctx, ext); dev_free(ctx, prod);
-    if (rc) { crcnn_tensor_free(ctx, o); return rc; }
-    *out3 = o;
+    *out3 = o.release();
     return CRCNN_OK;
 }
 
@@ -1698,31 +1626,26 @@ int crcnn_relinearize(crcnn_ctx *ctx, crcnn_tensor *in3, crcnn_evk *evk, crcnn_t
     }
     REQUIRE(total_digits <= 63, "too many key digits for 128-bit lazy accumulation");  // evaluator.cpp:972-976
     CU(cudaSetDevice(ctx->device));
-    int rc = ensure_domain(ctx, in3, 0);
-    if (rc) return rc;
-    crcnn_tensor *o = nullptr;
-    rc = new_tensor(ctx, in3->count, 2, 0, &o);
-    if (rc) return rc;
+    TRY(ensure_domain(ctx, in3, 0));
+    TensorOwner o(ctx);
+    TRY(new_tensor(ctx, in3->count, 2, 0, o.out()));
     const size_t pw = poly_words(ctx);
     if (evk->has_r32 && ctx->relin_mode == 1) {
         // word-size auxiliary-prime path: D*S3 forward + 2K*S3 inverse 32-bit transforms per ciphertext
         const Relin32Consts &c = evk->r32.c;
         const size_t per_ct = relin32_scratch_bytes(ctx->n, ctx->K, c);
         const long step = std::max<long>(1, std::min<long>(std::min<long>(in3->count, 200000), (long)((2ull << 30) / per_ct)));
-        void *scratch = nullptr;
-        rc = dev_alloc(ctx, (size_t)step * per_ct, &scratch);
-        if (rc) { crcnn_tensor_free(ctx, o); return rc; }
-        for (long c0 = 0; c0 < in3->count && !rc; c0 += step) {
+        DevBuf<uint8_t> scratch(ctx);
+        TRY(dev_alloc(ctx, (size_t)step * per_ct, scratch));
+        for (long c0 = 0; c0 < in3->count; c0 += step) {
             const long cnt = std::min<long>(step, in3->count - c0);
             // work: bytes = in (3 polys) + out (2 polys) per ciphertext; operations = 32-bit butterflies
             ProfScope ps(ctx, KC_RELIN32, lp_bytes(ctx, (double)cnt * 5 * ctx->K),
                          lp_bfly(ctx, (double)cnt * (c.D + 2 * ctx->K) * c.S3));
             cudaError_t e = relin32_run(ctx->dP, ctx->logn, ctx->K, evk->r32, in3->d + c0 * 3 * pw, o->d + c0 * 2 * pw, cnt, scratch, ctx->stream);
-            if (e != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
+            if (e != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
         }
-        dev_free(ctx, scratch);
-        if (rc) { crcnn_tensor_free(ctx, o); return rc; }
-        *out2 = o;
+        *out2 = o.release();
         return CRCNN_OK;
     }
     RelinArgs a{};
@@ -1732,13 +1655,12 @@ int crcnn_relinearize(crcnn_ctx *ctx, crcnn_tensor *in3, crcnn_evk *evk, crcnn_t
     // chunked so it stays near 2 GB
     const size_t per_ct = (size_t)(1 + total_digits + 2) * pw * 8;
     const long step = std::max<long>(1, std::min<long>(in3->count, (long)((2ull << 30) / per_ct)));
-    uint64_t *scratch = nullptr;
-    rc = dev_alloc(ctx, (size_t)step * per_ct, (void **)&scratch);
-    if (rc) { crcnn_tensor_free(ctx, o); return rc; }
+    DevBuf<uint64_t> scratch(ctx);
+    TRY(dev_alloc(ctx, (size_t)step * per_ct, scratch));
     a.dsc = scratch;
     a.dig = scratch + (size_t)step * pw;
     a.acc = a.dig + (size_t)step * total_digits * pw;
-    for (long c0 = 0; c0 < in3->count && !rc; c0 += step) {
+    for (long c0 = 0; c0 < in3->count; c0 += step) {
         a.count = std::min<long>(step, in3->count - c0);
         a.in3 = in3->d + c0 * 3 * pw;
         a.out = o->d + c0 * 2 * pw;
@@ -1750,22 +1672,17 @@ int crcnn_relinearize(crcnn_ctx *ctx, crcnn_tensor *in3, crcnn_evk *evk, crcnn_t
             e = launch_ntt_grouped(ctx->dP, ctx->logn, a.out, a.count * 2 * ctx->K, 0, ctx->K, true, ctx->K, 0, ctx->stream, a.acc, a.in3,
                                    2 * ctx->K, 3 * ctx->K);
         }
-        if (e != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
+        if (e != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
     }
-    dev_free(ctx, scratch);
-    if (rc) { crcnn_tensor_free(ctx, o); return rc; }
-    *out2 = o;
+    *out2 = o.release();
     return CRCNN_OK;
 }
 
 int crcnn_square_forward(crcnn_ctx *ctx, crcnn_tensor *in, crcnn_evk *evk, crcnn_tensor **out) {
     if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
-    crcnn_tensor *t3 = nullptr;
-    int rc = crcnn_square(ctx, in, &t3);
-    if (rc) return rc;
-    rc = crcnn_relinearize(ctx, t3, evk, out);
-    crcnn_tensor_free(ctx, t3);
-    return rc;
+    TensorOwner t3(ctx);
+    TRY(crcnn_square(ctx, in, t3.out()));
+    return crcnn_relinearize(ctx, t3, evk, out);
 }
 
 // ---------------------------------------------------------------------------- evaluator-level ops
@@ -1788,17 +1705,15 @@ int crcnn_plain_op(crcnn_ctx *ctx, crcnn_tensor *t, crcnn_plain *p, long index, 
     if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
     REQUIRE(t && p && index >= 0 && index < p->count && op >= 0 && op <= 2, "bad plain_op arguments");
     CU(cudaSetDevice(ctx->device));
-    int rc;
     const uint64_t *pl, *pl_sh = nullptr;
     if (op == 0) {
-        rc = ensure_domain(ctx, t, 1);
-        if (!rc) rc = ensure_shoup(ctx, p);
-        if (rc) return rc;
+        TRY(ensure_domain(ctx, t, 1));
+        TRY(ensure_shoup(ctx, p));
         pl = p->ntt_mul + index * poly_words(ctx);
         pl_sh = p->ntt_mul_sh + index * poly_words(ctx);
     } else {
-        rc = ensure_form(ctx, p, t->ntt ? PF_NTT_ADD : PF_COEF_ADD);
-        if (rc) return rc;
+        TRY(ensure_form(ctx, p, t->ntt ? PF_NTT_ADD : PF_COEF_ADD));
+
         pl = (t->ntt ? p->ntt_add : p->coef_add) + index * poly_words(ctx);
     }
     ProfScope ps(ctx, KC_PLAIN_OP, lp_bytes(ctx, (double)t->count * (op == 0 ? t->size : 1) * 2 * ctx->K), (double)t->count * (op == 0 ? t->size : 1) * ctx->K * ctx->n);
@@ -1814,24 +1729,20 @@ int crcnn_add_many(crcnn_ctx *ctx, crcnn_tensor *t, crcnn_tensor **out) {
     CU(cudaSetDevice(ctx->device));
     // sum of ciphertexts [first, first + count) of `src` in groups of `g` -> `nout` ciphertexts at dst (identity index table, cached)
     auto pass = [&](const uint64_t *src, long first, int nout, int g, uint64_t *dst) -> int {
-        std::vector<int> key = {4, (int)first, nout, g};
         const int *d_index = nullptr;
-        auto it = ctx->index_cache.find(key);
-        if (it == ctx->index_cache.end()) {
+        TRY(index_table(ctx, TAB_ADD_MANY, {(int)first, nout, g}, [&] {
             std::vector<int> table((size_t)nout * g);
-            for (size_t i = 0; i < table.size(); i++) table[i] = (int)(first + (long)i);
-            int rc = get_index_table(ctx, key, table, &d_index);
-            if (rc) return rc;
-        } else d_index = it->second;
+            std::iota(table.begin(), table.end(), (int)first);
+            return table;
+        }, &d_index));
         ProfScope ps(ctx, KC_POOL, lp_bytes(ctx, ((double)nout * g + nout) * 2 * ctx->K), (double)nout * g * 2 * ctx->K * ctx->n);
         CU(launch_pool(ctx->dP, ctx->n, ctx->K, src, d_index, nout, g, nullptr, nullptr, sum_fits_64(ctx, g), dst, ctx->stream));
         return CRCNN_OK;
     };
-    crcnn_tensor *o = nullptr;
-    int rc = new_tensor(ctx, 1, 2, t->ntt, &o);
-    if (rc) return rc;
+    TensorOwner o(ctx);
+    TRY(new_tensor(ctx, 1, 2, t->ntt, o.out()));
     if (t->count <= 128) {
-        rc = pass(t->d, 0, 1, (int)t->count, o->d);
+        TRY(pass(t->d, 0, 1, (int)t->count, o->d));
     } else {
         // ONE output ciphertext keeps 2K CTAs busy: reduce in two levels -- groups of ~sqrt(count) summed in parallel (every input read
         // once, in full coalesced rows), then the canonical partial sums.  Modular addition is associative: same residues as the
@@ -1839,15 +1750,13 @@ int crcnn_add_many(crcnn_ctx *ctx, crcnn_tensor *t, crcnn_tensor **out) {
         int g = 1;
         while ((long)g * g < t->count) g++;
         const long full = t->count / g, tail = t->count % g, groups = full + (tail ? 1 : 0);
-        crcnn_tensor *part = nullptr;
-        rc = new_tensor(ctx, groups, 2, t->ntt, &part);
-        if (!rc) rc = pass(t->d, 0, (int)full, g, part->d);
-        if (!rc && tail) rc = pass(t->d, full * g, 1, (int)tail, part->d + full * 2 * poly_words(ctx));
-        if (!rc) rc = pass(part->d, 0, 1, (int)groups, o->d);
-        crcnn_tensor_free(ctx, part);
+        TensorOwner part(ctx);
+        TRY(new_tensor(ctx, groups, 2, t->ntt, part.out()));
+        TRY(pass(t->d, 0, (int)full, g, part->d));
+        if (tail) TRY(pass(t->d, full * g, 1, (int)tail, part->d + full * 2 * poly_words(ctx)));
+        TRY(pass(part->d, 0, 1, (int)groups, o->d));
     }
-    if (rc) { crcnn_tensor_free(ctx, o); return rc; }
-    *out = o;
+    *out = o.release();
     return CRCNN_OK;
 }
 
@@ -1886,9 +1795,8 @@ int crcnn_probe_pipe(crcnn_ctx *ctx, int which, int blocks, int threads, int ite
     if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
     REQUIRE(which >= 0 && which <= 4 && blocks > 0 && threads > 0 && threads <= 1024 && iters > 0 && ms, "bad probe arguments");
     CU(cudaSetDevice(ctx->device));
-    uint64_t *sink = nullptr;
-    int rc = dev_alloc(ctx, 8, (void **)&sink);
-    if (rc) return rc;
+    DevBuf<uint64_t> sink(ctx);
+    TRY(dev_alloc(ctx, 8, sink));
     cudaEvent_t a, b;
     CU(cudaEventCreate(&a));
     CU(cudaEventCreate(&b));
@@ -1905,7 +1813,6 @@ int crcnn_probe_pipe(crcnn_ctx *ctx, int which, int blocks, int threads, int ite
     *ms = t;
     if (ops) *ops = work;
     cudaEventDestroy(a); cudaEventDestroy(b);
-    dev_free(ctx, sink);
     return CRCNN_OK;
 }
 int crcnn_probe_imad(crcnn_ctx *ctx, int blocks, int threads, int iters, double *ms) {
@@ -1979,18 +1886,15 @@ int crcnn_tensor_download_async(crcnn_ctx *ctx, crcnn_tensor *t, uint64_t *host)
     if (!ctx) return CRCNN_ERR_INVALID_ARGUMENT;
     REQUIRE(t && host, "null argument");
     CU(cudaSetDevice(ctx->device));
-    int rc = ensure_domain(ctx, t, 0);
-    if (rc) return rc;
+    TRY(ensure_domain(ctx, t, 0));
     const size_t n = ctx->n, rows = (size_t)t->count * t->size * ctx->K;
     if (!rows) return CRCNN_OK;
     // re-pad on the device (pad word = 0), then ONE contiguous copy: a strided cudaMemcpy2D reaches a tenth of the link rate
-    uint64_t *padded = nullptr;
-    rc = dev_alloc(ctx, rows * (n + 1) * 8, (void **)&padded);
-    if (rc) return rc;
+    DevBuf<uint64_t> padded(ctx);
+    TRY(dev_alloc(ctx, rows * (n + 1) * 8, padded));
     CU(cudaMemsetAsync(padded, 0, rows * (n + 1) * 8, ctx->stream));
     CU(cudaMemcpy2DAsync(padded, (n + 1) * 8, t->d, n * 8, n * 8, rows, cudaMemcpyDeviceToDevice, ctx->stream));
     CU(cudaMemcpyAsync(host, padded, rows * (n + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    dev_free(ctx, padded);
     return CRCNN_OK;
 }
 
@@ -2095,11 +1999,9 @@ int crcnn_comm_all_gather(crcnn_ctx *ctx, crcnn_comm *c, crcnn_tensor *local, in
     // the gathered tensor carries ONE domain flag: with want_ntt_form >= 0 every rank first brings its block into that domain; with -1 the
     // blocks are exchanged as they are (all ranks of a sharded layer produce the same domain: the kernel is chosen from the layer's
     // total output count, run_weighted_sum, and pooling / batch-norm / square map a domain to a domain)
-    int rc = want_ntt_form >= 0 ? ensure_domain(ctx, local, want_ntt_form ? 1 : 0) : CRCNN_OK;
-    if (rc) return rc;
-    crcnn_tensor *full = nullptr;
-    rc = new_tensor(ctx, (long)batch * total, local->size, local->ntt, &full);
-    if (rc) return rc;
+    if (want_ntt_form >= 0) TRY(ensure_domain(ctx, local, want_ntt_form ? 1 : 0));
+    TensorOwner full(ctx);
+    TRY(new_tensor(ctx, (long)batch * total, local->size, local->ntt, full.out()));
     const size_t ctw = (size_t)local->size * poly_words(ctx);
     // image b of the gathered tensor = [rank 0's ciphertexts of b | rank 1's | ...]
     if (c->world > 1) NCCLCHECK(nccl().GroupStart());
@@ -2119,7 +2021,7 @@ int crcnn_comm_all_gather(crcnn_ctx *ctx, crcnn_comm *c, crcnn_tensor *local, in
     }
     if (c->world > 1) NCCLCHECK(nccl().GroupEnd());
     (void)before;
-    *out = full;
+    *out = full.release();
     return CRCNN_OK;
 }
 
@@ -2138,17 +2040,16 @@ int crcnn_keys_upload(crcnn_ctx *ctx, const uint64_t *secret_key_ntt, const uint
     REQUIRE(secret_key_ntt && public_key_ntt && out, "null argument");
     REQUIRE(ctx->hp.d.t >= 2 && REENC_GAMMA % ctx->hp.d.t != 0, "plain modulus not usable with the decryptor's gamma");
     CU(cudaSetDevice(ctx->device));
-    auto *k = new crcnn_keys;
+    Owned<crcnn_keys, crcnn_keys_free> k(ctx, new crcnn_keys);
     k->c = make_reenc_consts(ctx->hp.d);
     k->b = make_budget_consts(ctx->hp.d);
     const size_t pw = poly_words(ctx);
-    int rc = dev_alloc(ctx, pw * 8, (void **)&k->sk);
-    if (!rc) rc = dev_alloc(ctx, 2 * pw * 8, (void **)&k->pk);
-    if (!rc) rc = upload_rows(ctx, secret_key_ntt, (size_t)ctx->K, k->sk, ctx->stream);
-    if (!rc) rc = upload_rows(ctx, public_key_ntt, (size_t)2 * ctx->K, k->pk, ctx->stream);
-    if (!rc) { cudaError_t e = cudaStreamSynchronize(ctx->stream); if (e != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e)); }
-    if (rc) { dev_free(ctx, k->sk); dev_free(ctx, k->pk); delete k; return rc; }
-    *out = k;
+    TRY(dev_alloc(ctx, pw * 8, (void **)&k->sk));
+    TRY(dev_alloc(ctx, 2 * pw * 8, (void **)&k->pk));
+    TRY(upload_rows(ctx, secret_key_ntt, (size_t)ctx->K, k->sk, ctx->stream));
+    TRY(upload_rows(ctx, public_key_ntt, (size_t)2 * ctx->K, k->pk, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    *out = k.release();
     return CRCNN_OK;
 }
 int crcnn_keys_free(crcnn_ctx *ctx, crcnn_keys *k) {
@@ -2236,21 +2137,17 @@ int crcnn_decrypt(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, uint64_t *host
     CU(cudaSetDevice(ctx->device));
     const size_t n = ctx->n;
     const long step = decrypt_step(ctx, t->count);
-    uint64_t *scratch = nullptr, *plain = nullptr;
-    int rc = dev_alloc(ctx, (size_t)step * ctx->K * n * 8, (void **)&scratch);
-    if (!rc) rc = dev_alloc(ctx, (size_t)step * n * 8, (void **)&plain);
-    for (long c0 = 0; c0 < t->count && !rc; c0 += step) {
+    DevBuf<uint64_t> scratch(ctx), plain(ctx);
+    TRY(dev_alloc(ctx, (size_t)step * ctx->K * n * 8, scratch));
+    TRY(dev_alloc(ctx, (size_t)step * n * 8, plain));
+    for (long c0 = 0; c0 < t->count; c0 += step) {
         const long cnt = std::min<long>(step, t->count - c0);
-        rc = decrypt_range(ctx, k, t, c0, cnt, scratch, plain);
-        if (!rc) {
-            cudaError_t e = cudaMemcpy2DAsync(host_plain + c0 * (n + 1), (n + 1) * 8, plain, n * 8, n * 8, cnt, cudaMemcpyDeviceToHost, ctx->stream);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-            if (e != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
-            for (long r = 0; r < cnt; r++) host_plain[(c0 + r) * (n + 1) + n] = 0;
-        }
+        TRY(decrypt_range(ctx, k, t, c0, cnt, scratch, plain));
+        CU(cudaMemcpy2DAsync(host_plain + c0 * (n + 1), (n + 1) * 8, plain, n * 8, n * 8, cnt, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));
+        for (long r = 0; r < cnt; r++) host_plain[(c0 + r) * (n + 1) + n] = 0;
     }
-    dev_free(ctx, scratch); dev_free(ctx, plain);
-    return rc;
+    return CRCNN_OK;
 }
 
 int crcnn_noise_budget(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, int *host_budgets, int *min_budget) {
@@ -2261,22 +2158,16 @@ int crcnn_noise_budget(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, int *host
     CU(cudaSetDevice(ctx->device));
     const size_t n = ctx->n;
     const long step = decrypt_step(ctx, t->count);
-    uint64_t *scratch = nullptr;
-    int *bits = nullptr;
-    int rc = dev_alloc(ctx, (size_t)step * ctx->K * n * 8, (void **)&scratch);
-    if (!rc) rc = dev_alloc(ctx, (size_t)t->count * sizeof(int), (void **)&bits);
-    if (!rc) { cudaError_t e = cudaMemsetAsync(bits, 0, (size_t)t->count * sizeof(int), ctx->stream); if (e != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e)); }
-    for (long c0 = 0; c0 < t->count && !rc; c0 += step)
-        rc = noise_bits_range(ctx, k, t, c0, std::min<long>(step, t->count - c0), scratch, bits + c0);
-    std::vector<int> hb;
-    if (!rc) {
-        hb.resize((size_t)t->count);
-        cudaError_t e = cudaMemcpyAsync(hb.data(), bits, hb.size() * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-        if (e != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
-    }
-    dev_free(ctx, scratch); dev_free(ctx, bits);
-    if (rc) return rc;
+    DevBuf<uint64_t> scratch(ctx);
+    DevBuf<int> bits(ctx);
+    TRY(dev_alloc(ctx, (size_t)step * ctx->K * n * 8, scratch));
+    TRY(dev_alloc(ctx, (size_t)t->count * sizeof(int), bits));
+    CU(cudaMemsetAsync(bits, 0, (size_t)t->count * sizeof(int), ctx->stream));
+    for (long c0 = 0; c0 < t->count; c0 += step)
+        TRY(noise_bits_range(ctx, k, t, c0, std::min<long>(step, t->count - c0), scratch, bits + c0));
+    std::vector<int> hb((size_t)t->count);
+    CU(cudaMemcpyAsync(hb.data(), bits, hb.size() * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
     int mn = k->b.q_bits;
     for (long i = 0; i < t->count; i++) {
         const int b = std::max(0, k->b.q_bits - hb[(size_t)i] - 1);     // the -1 accounts for scaling the invariant noise by 2
@@ -2295,53 +2186,47 @@ int crcnn_reencrypt(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *in, uint64_t se
     CU(cudaSetDevice(ctx->device));
     const size_t n = ctx->n, pw = poly_words(ctx);
     const int K = ctx->K;
-    crcnn_tensor *o = nullptr;
-    int rc = new_tensor(ctx, in->count, 2, 0, &o);
-    if (rc) return rc;
+    TensorOwner o(ctx);
+    TRY(new_tensor(ctx, in->count, 2, 0, o.out()));
     const long step = encrypt_step(ctx, in->count);
-    uint64_t *scratch = nullptr, *plain = nullptr, *slots = nullptr;
-    int8_t *e = nullptr, *given = nullptr;
-    float *vals = nullptr;
-    rc = dev_alloc(ctx, (size_t)step * K * n * 8, (void **)&scratch);
-    if (!rc) rc = dev_alloc(ctx, (size_t)step * n * 8, (void **)&plain);
-    if (!rc) rc = dev_alloc(ctx, (size_t)step * REENC_SLOTS * 8, (void **)&slots);
-    if (!rc) rc = dev_alloc(ctx, (size_t)step * 2 * n, (void **)&e);
-    if (!rc && host_noise) rc = dev_alloc(ctx, (size_t)step * 3 * n, (void **)&given);
-    if (!rc && host_values) rc = dev_alloc(ctx, (size_t)step * 4, (void **)&vals);
-    for (long c0 = 0; c0 < in->count && !rc; c0 += step) {
+    DevBuf<uint64_t> scratch(ctx), plain(ctx), slots(ctx);
+    DevBuf<int8_t> e(ctx), given(ctx);
+    DevBuf<float> vals(ctx);
+    TRY(dev_alloc(ctx, (size_t)step * K * n * 8, scratch));
+    TRY(dev_alloc(ctx, (size_t)step * n * 8, plain));
+    TRY(dev_alloc(ctx, (size_t)step * REENC_SLOTS * 8, slots));
+    TRY(dev_alloc(ctx, (size_t)step * 2 * n, e));
+    if (host_noise) TRY(dev_alloc(ctx, (size_t)step * 3 * n, given));
+    if (host_values) TRY(dev_alloc(ctx, (size_t)step * 4, vals));
+    for (long c0 = 0; c0 < in->count; c0 += step) {
         const long cnt = std::min<long>(step, in->count - c0);
-        rc = decrypt_range(ctx, k, in, c0, cnt, scratch, plain);
-        if (rc) break;
-        uint64_t *dst = o->d + c0 * 2 * pw;
-        cudaError_t er = cudaSuccess;
+        TRY(decrypt_range(ctx, k, in, c0, cnt, scratch, plain));
         {
             ProfScope ps(ctx, KC_REENC, lp_bytes(ctx, (double)cnt * 2 * K), lp_bfly(ctx, (double)cnt * 3 * K));
-            er = launch_reencode(k->c, plain, slots, vals, cnt, ctx->stream);
+            cudaError_t er = launch_reencode(k->c, plain, slots, vals, cnt, ctx->stream);
             if (er == cudaSuccess)
                 er = encrypt_range(ctx, k, slots, seed, c0, noise_standard_deviation, host_noise ? host_noise + c0 * 3 * n : nullptr, given, scratch, e,
-                                   dst, cnt);
+                                   o->d + c0 * 2 * pw, cnt);
+            if (er != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, std::string("re-encryption: ") + cudaGetErrorString(er));
         }
-        if (er == cudaSuccess && host_reencoded) {     // the re-encoded plaintexts, n+1 words each (parity checks)
+        if (host_reencoded) {     // the re-encoded plaintexts, n+1 words each (parity checks)
             std::vector<uint64_t> hs((size_t)cnt * REENC_SLOTS);
-            er = cudaMemcpyAsync(hs.data(), slots, hs.size() * 8, cudaMemcpyDeviceToHost, ctx->stream);
-            if (er == cudaSuccess) er = cudaStreamSynchronize(ctx->stream);
-            for (long r = 0; r < cnt && er == cudaSuccess; r++) {
+            CU(cudaMemcpyAsync(hs.data(), slots, hs.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
+            CU(cudaStreamSynchronize(ctx->stream));
+            for (long r = 0; r < cnt; r++) {
                 uint64_t *p = host_reencoded + (c0 + r) * (n + 1);
                 memset(p, 0, (n + 1) * 8);
                 memcpy(p, hs.data() + r * REENC_SLOTS, 64 * 8);
                 memcpy(p + n - 32, hs.data() + r * REENC_SLOTS + 64, 32 * 8);
             }
         }
-        if (er == cudaSuccess && host_values) {
-            er = cudaMemcpyAsync(host_values + c0, vals, (size_t)cnt * 4, cudaMemcpyDeviceToHost, ctx->stream);
-            if (er == cudaSuccess) er = cudaStreamSynchronize(ctx->stream);
+        if (host_values) {
+            CU(cudaMemcpyAsync(host_values + c0, vals, (size_t)cnt * 4, cudaMemcpyDeviceToHost, ctx->stream));
+            CU(cudaStreamSynchronize(ctx->stream));
         }
-        if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, std::string("re-encryption: ") + cudaGetErrorString(er));
     }
-    if (host_noise && !rc) { cudaError_t er = cudaStreamSynchronize(ctx->stream); if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(er)); }
-    dev_free(ctx, scratch); dev_free(ctx, plain); dev_free(ctx, slots); dev_free(ctx, e); dev_free(ctx, given); dev_free(ctx, vals);
-    if (rc) { crcnn_tensor_free(ctx, o); return rc; }
-    *out = o;
+    if (host_noise) CU(cudaStreamSynchronize(ctx->stream));
+    *out = o.release();
     return CRCNN_OK;
 }
 
@@ -2353,36 +2238,30 @@ int crcnn_encrypt_values(crcnn_ctx *ctx, crcnn_keys *k, const float *host_values
     CU(cudaSetDevice(ctx->device));
     const size_t n = ctx->n, pw = poly_words(ctx);
     const int K = ctx->K;
-    crcnn_tensor *o = nullptr;
-    int rc = new_tensor(ctx, count, 2, 0, &o);
-    if (rc) return rc;
+    TensorOwner o(ctx);
+    TRY(new_tensor(ctx, count, 2, 0, o.out()));
     const long step = encrypt_step(ctx, count);
-    uint64_t *U = nullptr, *slots = nullptr;
-    int8_t *e = nullptr, *given = nullptr;
-    float *vals = nullptr;
-    rc = dev_alloc(ctx, (size_t)step * K * n * 8, (void **)&U);
-    if (!rc) rc = dev_alloc(ctx, (size_t)step * REENC_SLOTS * 8, (void **)&slots);
-    if (!rc) rc = dev_alloc(ctx, (size_t)step * 2 * n, (void **)&e);
-    if (!rc && host_noise) rc = dev_alloc(ctx, (size_t)step * 3 * n, (void **)&given);
-    if (!rc) rc = dev_alloc(ctx, (size_t)count * 4, (void **)&vals);
-    if (!rc) { cudaError_t er = cudaMemcpyAsync(vals, host_values, (size_t)count * 4, cudaMemcpyHostToDevice, ctx->stream); if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(er)); }
-    for (long c0 = 0; c0 < count && !rc; c0 += step) {
+    DevBuf<uint64_t> U(ctx), slots(ctx);
+    DevBuf<int8_t> e(ctx), given(ctx);
+    DevBuf<float> vals(ctx);
+    TRY(dev_alloc(ctx, (size_t)step * K * n * 8, U));
+    TRY(dev_alloc(ctx, (size_t)step * REENC_SLOTS * 8, slots));
+    TRY(dev_alloc(ctx, (size_t)step * 2 * n, e));
+    if (host_noise) TRY(dev_alloc(ctx, (size_t)step * 3 * n, given));
+    TRY(dev_alloc(ctx, (size_t)count * 4, vals));
+    CU(cudaMemcpyAsync(vals, host_values, (size_t)count * 4, cudaMemcpyHostToDevice, ctx->stream));
+    for (long c0 = 0; c0 < count; c0 += step) {
         const long cnt = std::min<long>(step, count - c0);
-        cudaError_t er;
-        {
-            ProfScope ps(ctx, KC_REENC, lp_bytes(ctx, (double)cnt * 2 * K), lp_bfly(ctx, (double)cnt * 3 * K));
-            er = launch_encode_values(k->c, vals + c0, slots, cnt, ctx->stream);
-            if (er == cudaSuccess)
-                er = encrypt_range(ctx, k, slots, seed, c0, noise_standard_deviation, host_noise ? host_noise + c0 * 3 * n : nullptr, given, U, e,
-                                   o->d + c0 * 2 * pw, cnt);
-        }
-        if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, std::string("encryption: ") + cudaGetErrorString(er));
+        ProfScope ps(ctx, KC_REENC, lp_bytes(ctx, (double)cnt * 2 * K), lp_bfly(ctx, (double)cnt * 3 * K));
+        cudaError_t er = launch_encode_values(k->c, vals + c0, slots, cnt, ctx->stream);
+        if (er == cudaSuccess)
+            er = encrypt_range(ctx, k, slots, seed, c0, noise_standard_deviation, host_noise ? host_noise + c0 * 3 * n : nullptr, given, U, e,
+                               o->d + c0 * 2 * pw, cnt);
+        if (er != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, std::string("encryption: ") + cudaGetErrorString(er));
     }
     // the host buffers must stay untouched until their copies have run
-    if (!rc) { cudaError_t er = cudaStreamSynchronize(ctx->stream); if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(er)); }
-    dev_free(ctx, U); dev_free(ctx, slots); dev_free(ctx, e); dev_free(ctx, given); dev_free(ctx, vals);
-    if (rc) { crcnn_tensor_free(ctx, o); return rc; }
-    *out = o;
+    CU(cudaStreamSynchronize(ctx->stream));
+    *out = o.release();
     return CRCNN_OK;
 }
 
@@ -2394,27 +2273,21 @@ int crcnn_decrypt_values(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, float *
     CU(cudaSetDevice(ctx->device));
     const size_t n = ctx->n;
     const long step = decrypt_step(ctx, t->count);
-    uint64_t *scratch = nullptr, *plain = nullptr;
-    float *vals = nullptr;
-    int rc = dev_alloc(ctx, (size_t)step * ctx->K * n * 8, (void **)&scratch);
-    if (!rc) rc = dev_alloc(ctx, (size_t)step * n * 8, (void **)&plain);
-    if (!rc) rc = dev_alloc(ctx, (size_t)t->count * 4, (void **)&vals);
-    for (long c0 = 0; c0 < t->count && !rc; c0 += step) {
+    DevBuf<uint64_t> scratch(ctx), plain(ctx);
+    DevBuf<float> vals(ctx);
+    TRY(dev_alloc(ctx, (size_t)step * ctx->K * n * 8, scratch));
+    TRY(dev_alloc(ctx, (size_t)step * n * 8, plain));
+    TRY(dev_alloc(ctx, (size_t)t->count * 4, vals));
+    for (long c0 = 0; c0 < t->count; c0 += step) {
         const long cnt = std::min<long>(step, t->count - c0);
-        rc = decrypt_range(ctx, k, t, c0, cnt, scratch, plain);
-        if (!rc) {
-            ProfScope ps(ctx, KC_REENC, (double)cnt * n * 8 + (double)cnt * 4, 0);
-            cudaError_t er = launch_decode_values(k->c, plain, vals + c0, cnt, ctx->stream);
-            if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(er));
-        }
+        TRY(decrypt_range(ctx, k, t, c0, cnt, scratch, plain));
+        ProfScope ps(ctx, KC_REENC, (double)cnt * n * 8 + (double)cnt * 4, 0);
+        cudaError_t er = launch_decode_values(k->c, plain, vals + c0, cnt, ctx->stream);
+        if (er != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(er));
     }
-    if (!rc) {
-        cudaError_t er = cudaMemcpyAsync(host_values, vals, (size_t)t->count * 4, cudaMemcpyDeviceToHost, ctx->stream);
-        if (er == cudaSuccess) er = cudaStreamSynchronize(ctx->stream);
-        if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(er));
-    }
-    dev_free(ctx, scratch); dev_free(ctx, plain); dev_free(ctx, vals);
-    return rc;
+    CU(cudaMemcpyAsync(host_values, vals, (size_t)t->count * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    return CRCNN_OK;
 }
 
 // ---------------------------------------------------------------------------------------- CRT plaintext-modulus ensembles
@@ -2451,22 +2324,18 @@ int decrypt_slots_range(crcnn_ctx *ctx, crcnn_keys *k, crcnn_tensor *t, long fir
     return CRCNN_OK;
 }
 
-// *gathered = every instance's slots of its tensor t, [world][count][96]: this rank decrypts its block in decrypt_step chunks, then ONE
+// gathered = every instance's slots of its tensor t, [world][count][96]: this rank decrypts its block in decrypt_step chunks, then ONE
 // all-gather -- the chunking is each rank's own affair, only the block size (the tensor's count) has to agree
-int crt_gather_slots(crcnn_ctx *ctx, crcnn_crt *crt, crcnn_keys *k, crcnn_tensor *t, uint64_t **gathered) {
+int crt_gather_slots(crcnn_ctx *ctx, crcnn_crt *crt, crcnn_keys *k, crcnn_tensor *t, DevBuf<uint64_t> &gathered) {
     const long count = t->count, step = decrypt_step(ctx, count);
     const size_t block = (size_t)count * REENC_SLOTS;
-    uint64_t *scratch = nullptr, *g = nullptr;
-    int rc = dev_alloc(ctx, (size_t)step * ctx->K * ctx->n * 8, (void **)&scratch);
-    if (!rc) rc = dev_alloc(ctx, (size_t)crt->comm->world * block * 8, (void **)&g);
-    uint64_t *mine = rc ? nullptr : g + (size_t)crt->comm->rank * block;
-    for (long c0 = 0; c0 < count && !rc; c0 += step)
-        rc = decrypt_slots_range(ctx, k, t, c0, std::min<long>(step, count - c0), scratch, mine + c0 * REENC_SLOTS);
-    if (!rc) rc = comm_all_gather_words(ctx, crt->comm, mine, block, g);
-    dev_free(ctx, scratch);
-    if (rc) { dev_free(ctx, g); return rc; }
-    *gathered = g;
-    return CRCNN_OK;
+    DevBuf<uint64_t> scratch(ctx);
+    TRY(dev_alloc(ctx, (size_t)step * ctx->K * ctx->n * 8, scratch));
+    TRY(dev_alloc(ctx, (size_t)crt->comm->world * block * 8, gathered));
+    uint64_t *mine = gathered + (size_t)crt->comm->rank * block;
+    for (long c0 = 0; c0 < count; c0 += step)
+        TRY(decrypt_slots_range(ctx, k, t, c0, std::min<long>(step, count - c0), scratch, mine + c0 * REENC_SLOTS));
+    return comm_all_gather_words(ctx, crt->comm, mine, block, gathered);
 }
 
 int crt_call_check(crcnn_ctx *ctx, crcnn_crt *crt, crcnn_keys *k, crcnn_tensor *t) {
@@ -2492,19 +2361,15 @@ int crcnn_crt_create(crcnn_ctx *ctx, crcnn_comm *comm, const uint64_t *moduli, i
     rec[0] = rc == CRCNN_OK; rec[1] = (uint64_t)M;
     std::copy(moduli, moduli + M, rec.begin() + 2);
     CU(cudaSetDevice(ctx->device));
-    uint64_t *d = nullptr;
-    int grc = dev_alloc(ctx, all.size() * 8, (void **)&d);
-    if (!grc) {
-        cudaError_t e = cudaMemcpyAsync(d + (size_t)comm->rank * W, rec.data(), W * 8, cudaMemcpyHostToDevice, ctx->stream);
-        if (e != cudaSuccess) grc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
-    }
-    if (!grc) grc = comm_all_gather_words(ctx, comm, d + (size_t)comm->rank * W, W, d);
-    if (!grc) {
-        cudaError_t e = cudaMemcpyAsync(all.data(), d, all.size() * 8, cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-        if (e != cudaSuccess) grc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(e));
-    }
-    dev_free(ctx, d);
+    const int grc = [&]() -> int {
+        DevBuf<uint64_t> d(ctx);
+        TRY(dev_alloc(ctx, all.size() * 8, d));
+        CU(cudaMemcpyAsync(d + (size_t)comm->rank * W, rec.data(), W * 8, cudaMemcpyHostToDevice, ctx->stream));
+        TRY(comm_all_gather_words(ctx, comm, d + (size_t)comm->rank * W, W, d));
+        CU(cudaMemcpyAsync(all.data(), d, all.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));
+        return CRCNN_OK;
+    }();
     if (rc) return fail(ctx, rc, why);
     if (grc) return grc;
     for (int r = 0; r < comm->world; r++) {
@@ -2531,22 +2396,17 @@ int crcnn_crt_decrypt_values(crcnn_ctx *ctx, crcnn_crt *crt, crcnn_keys *k, crcn
     if (rc) return rc;
     REQUIRE(host_values, "null argument");
     CU(cudaSetDevice(ctx->device));
-    uint64_t *g = nullptr;
-    float *vals = nullptr;
-    rc = crt_gather_slots(ctx, crt, k, t, &g);
-    if (!rc) rc = dev_alloc(ctx, (size_t)t->count * 4, (void **)&vals);
-    if (!rc) {
-        cudaError_t er;
-        {
-            ProfScope ps(ctx, KC_REENC, (double)crt->c.M * t->count * REENC_SLOTS * 8 + (double)t->count * 4, 0);
-            er = launch_crt_decode_values(crt->c, g, vals, t->count, ctx->stream);
-        }
-        if (er == cudaSuccess) er = cudaMemcpyAsync(host_values, vals, (size_t)t->count * 4, cudaMemcpyDeviceToHost, ctx->stream);
-        if (er == cudaSuccess) er = cudaStreamSynchronize(ctx->stream);
-        if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(er));
+    DevBuf<uint64_t> g(ctx);
+    DevBuf<float> vals(ctx);
+    TRY(crt_gather_slots(ctx, crt, k, t, g));
+    TRY(dev_alloc(ctx, (size_t)t->count * 4, vals));
+    {
+        ProfScope ps(ctx, KC_REENC, (double)crt->c.M * t->count * REENC_SLOTS * 8 + (double)t->count * 4, 0);
+        CU(launch_crt_decode_values(crt->c, g, vals, t->count, ctx->stream));
     }
-    dev_free(ctx, g); dev_free(ctx, vals);
-    return rc;
+    CU(cudaMemcpyAsync(host_values, vals, (size_t)t->count * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    return CRCNN_OK;
 }
 
 int crcnn_crt_reencrypt(crcnn_ctx *ctx, crcnn_crt *crt, crcnn_keys *k, crcnn_tensor *in, uint64_t seed, double noise_standard_deviation,
@@ -2558,30 +2418,25 @@ int crcnn_crt_reencrypt(crcnn_ctx *ctx, crcnn_crt *crt, crcnn_keys *k, crcnn_ten
     CU(cudaSetDevice(ctx->device));
     const size_t n = ctx->n, pw = poly_words(ctx);
     const long count = in->count, step = encrypt_step(ctx, count);
-    crcnn_tensor *o = nullptr;
-    uint64_t *g = nullptr, *U = nullptr, *slots = nullptr;
-    int8_t *e = nullptr;
-    rc = crt_gather_slots(ctx, crt, k, in, &g);
-    if (!rc) rc = new_tensor(ctx, count, 2, 0, &o);
-    if (!rc) rc = dev_alloc(ctx, (size_t)step * ctx->K * n * 8, (void **)&U);
-    if (!rc) rc = dev_alloc(ctx, (size_t)step * REENC_SLOTS * 8, (void **)&slots);
-    if (!rc) rc = dev_alloc(ctx, (size_t)step * 2 * n, (void **)&e);
+    DevBuf<uint64_t> g(ctx), U(ctx), slots(ctx);
+    DevBuf<int8_t> e(ctx);
+    TensorOwner o(ctx);
+    TRY(crt_gather_slots(ctx, crt, k, in, g));
+    TRY(new_tensor(ctx, count, 2, 0, o.out()));
+    TRY(dev_alloc(ctx, (size_t)step * ctx->K * n * 8, U));
+    TRY(dev_alloc(ctx, (size_t)step * REENC_SLOTS * 8, slots));
+    TRY(dev_alloc(ctx, (size_t)step * 2 * n, e));
     // ciphertext counters of rank r start at r 2^48: instances sharing a seed (and perhaps a key set) never share u
     const long first = (long)((uint64_t)crt->comm->rank << 48);
-    for (long c0 = 0; c0 < count && !rc; c0 += step) {
+    for (long c0 = 0; c0 < count; c0 += step) {
         const long cnt = std::min<long>(step, count - c0);
-        cudaError_t er;
-        {
-            ProfScope ps(ctx, KC_REENC, lp_bytes(ctx, (double)cnt * 2 * ctx->K), lp_bfly(ctx, (double)cnt * 3 * ctx->K));
-            er = launch_crt_reencode(crt->c, g, count, c0, slots, cnt, ctx->stream);
-            if (er == cudaSuccess)
-                er = encrypt_range(ctx, k, slots, seed, first + c0, noise_standard_deviation, nullptr, nullptr, U, e, o->d + c0 * 2 * pw, cnt);
-        }
-        if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, std::string("re-encryption: ") + cudaGetErrorString(er));
+        ProfScope ps(ctx, KC_REENC, lp_bytes(ctx, (double)cnt * 2 * ctx->K), lp_bfly(ctx, (double)cnt * 3 * ctx->K));
+        cudaError_t er = launch_crt_reencode(crt->c, g, count, c0, slots, cnt, ctx->stream);
+        if (er == cudaSuccess)
+            er = encrypt_range(ctx, k, slots, seed, first + c0, noise_standard_deviation, nullptr, nullptr, U, e, o->d + c0 * 2 * pw, cnt);
+        if (er != cudaSuccess) return fail(ctx, CRCNN_ERR_CUDA, std::string("re-encryption: ") + cudaGetErrorString(er));
     }
-    dev_free(ctx, g); dev_free(ctx, U); dev_free(ctx, slots); dev_free(ctx, e);
-    if (rc) { if (o) crcnn_tensor_free(ctx, o); return rc; }
-    *out = o;
+    *out = o.release();
     return CRCNN_OK;
 }
 
@@ -2604,19 +2459,15 @@ int crcnn_crt_decode_values(crcnn_ctx *ctx, int M, const uint64_t *moduli, const
         }
     }
     CU(cudaSetDevice(ctx->device));
-    uint64_t *d = nullptr;
-    float *vals = nullptr;
-    rc = dev_alloc(ctx, slots.size() * 8, (void **)&d);
-    if (!rc) rc = dev_alloc(ctx, (size_t)count * 4, (void **)&vals);
-    if (!rc) {
-        cudaError_t er = cudaMemcpyAsync(d, slots.data(), slots.size() * 8, cudaMemcpyHostToDevice, ctx->stream);
-        if (er == cudaSuccess) er = launch_crt_decode_values(make_crt_consts(moduli, M, 0), d, vals, count, ctx->stream);
-        if (er == cudaSuccess) er = cudaMemcpyAsync(host_values, vals, (size_t)count * 4, cudaMemcpyDeviceToHost, ctx->stream);
-        if (er == cudaSuccess) er = cudaStreamSynchronize(ctx->stream);
-        if (er != cudaSuccess) rc = fail(ctx, CRCNN_ERR_CUDA, cudaGetErrorString(er));
-    }
-    dev_free(ctx, d); dev_free(ctx, vals);
-    return rc;
+    DevBuf<uint64_t> d(ctx);
+    DevBuf<float> vals(ctx);
+    TRY(dev_alloc(ctx, slots.size() * 8, d));
+    TRY(dev_alloc(ctx, (size_t)count * 4, vals));
+    CU(cudaMemcpyAsync(d, slots.data(), slots.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CU(launch_crt_decode_values(make_crt_consts(moduli, M, 0), d, vals, count, ctx->stream));
+    CU(cudaMemcpyAsync(host_values, vals, (size_t)count * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    return CRCNN_OK;
 }
 
 }  // extern "C"
